@@ -3,7 +3,8 @@
 
   python bench.py [--gpus N] [--steps K] [--warmup W]            # our arm (CUDA, one process per GPU)
   python bench.py --impl reference [--steps K] [--warmup W]       # reference arm: CPU env classes on all host cores
-  torchrun --nproc-per-node N ... bench.py --gpus N ...           # N > 1 (the driver launches this)
+  torchrun --nproc-per-node N ... bench.py --gpus N ...           # N > 1
+  python bench.py --steps K --warmup W --dump-outputs DIR         # also write what the last timed step computed
 
 Workload (BASELINE.json configs[1], the configuration the metric is quoted on): one synthetic
 thor-cached scene, 1,500 positions x 4 rotations = 6,000 states, 84x84 RGB + depth + goal frame,
@@ -13,13 +14,21 @@ random actions, TimeLimit 900, no curriculum by default (start states uniform ov
 initial hardness 0.01 - `--hardness 0.01` - the envs cluster around the goals and most reads hit L2).
 One "step" = one vectorised step of all envs.  Rank 0 prints ONE JSON line.
 
-Timed region: R back-to-back blocks of exactly K steps, each block bracketed by a pair of CUDA events on the
-launching stream, the whole group bracketed by barrier + synchronize.  `ms_per_step` / `value` are the MEDIAN
-block (each block's time is first maximised over the ranks); min / max are reported next to it.  R grows until
-the region lasts >= ~0.2 s, so `--steps 20` is as stable as `--steps 20000`.  NO collective, host
-synchronisation or allocation sits between two event records (`timed_blocks`, checked by
+Timed region: exactly K steps (`--steps K`) bracketed by a pair of CUDA events on the launching stream, preceded by
+the `--mix` and the W warm-up steps (`--warmup W`), which are enqueued without waiting for them so that the region
+opens with the device busy and the host ahead of it; barrier + synchronize before those and after the region.
+`ms_per_step` / `value` are the region's time over K (maximised over the ranks).  NO collective, host
+synchronisation or allocation sits between the two event records (`timed_blocks`, checked by
 tests/test_bench_contract.py); the one NCCL call near this path - the episode-statistics all-reduce - is timed
-on its own and reported as `collective_ms`.
+on its own and reported as `collective_ms`.  Every input of the timed steps is seeded and the number of steps before
+the region is fixed by the arguments, so the same command line steps the same envs through the same states on every
+run.
+
+`--dump-outputs DIR` writes what the last timed step computed, as seen by its caller, to DIR/<name>.npy (float32,
+or float64 where float32 would not hold the values exactly; at most 64 MB in all): every observation leaf
+(`obs_<leaf>`), `last_action_reward`, `reward`, `done`.  Where the observation batch is larger than that, the same
+fixed, seeded sample of env rows is written for every leaf.  `--workload c5` writes the rollout builder's results
+instead.  With more than one rank, rank 0 writes its own shard.
 """
 import argparse
 import importlib
@@ -46,6 +55,7 @@ WORKLOAD = "C2 synthetic thor-cached scene: 1,500 positions x 4 rotations, 84x84
 METRIC = "env-steps/s (obs gather+step+reset)"
 MIN_REGION_S = 0.2          # the timed region is repeated until it lasts at least this long
 MAX_BLOCKS = 4000
+DUMP_BYTES = 60_000_000     # --dump-outputs: array data of all files together (headers add a few hundred bytes)
 
 
 def make_scene(vn, planes=("rgb", "depth")):
@@ -219,10 +229,15 @@ class Harness:
         self.dist.all_reduce(t, op=self.dist.ReduceOp.MAX)
         return [float(v) for v in t.tolist()]
 
-    def blocks(self, run_block, n_blocks):
-        """ms of each block (max over ranks)."""
-        make_event = lambda: self.torch.cuda.Event(enable_timing=True)
+    def blocks(self, run_block, n_blocks, lead=None):
+        """ms of each block (max over ranks).  `lead()` enqueues un-timed work between the opening barrier and the
+        first event, so that the device is still busy with it when the region opens.  The events are created before
+        the barrier: nothing but `lead` runs on the host between the two."""
+        pool = [self.torch.cuda.Event(enable_timing=True) for _ in range(2 * n_blocks)][::-1]
+        make_event = pool.pop
         self.barrier()
+        if lead is not None:
+            lead()
         events = timed_blocks(make_event, run_block, n_blocks)
         self.barrier()
         return self.max_over_ranks([a.elapsed_time(b) for a, b in events])
@@ -257,6 +272,53 @@ def e2e_loop(step, n_steps, sync):
     dt = time.perf_counter() - t0
     # <<< timed region
     return dt
+
+
+# ------------------------------------------------------------------------------------------ --dump-outputs
+def obs_leaves(env):
+    """(name, tensor) of every observation leaf a step of `env` hands back, in layout order, then last_action_reward."""
+    lv = env.leaves
+    names = list(lv) if isinstance(lv, dict) else (list(lv) if isinstance(lv, tuple) else [lv])
+    obs = env._obs()
+    inner, lar = obs if env.unreal_wrapper else (obs, None)
+    tensors = [inner[k] for k in names] if isinstance(lv, dict) else (list(inner) if isinstance(lv, tuple) else [inner])
+    out = [("obs_" + n, t) for n, t in zip(names, tensors)]
+    return out + ([("last_action_reward", lar)] if lar is not None else [])
+
+
+def dump_outputs(out_dir, arrays, sampled, budget=DUMP_BYTES, seed=0):
+    """Writes every (name, tensor) of `arrays` to out_dir/<name>.npy: floating point as float32 (float64 stays
+    float64), integers and booleans as float32, or float64 where float32 would not hold them exactly.  When all of it
+    would exceed `budget` bytes, the arrays named in `sampled` (same first dimension) keep the same fixed, seeded
+    sample of rows (ascending); the others are always written whole."""
+    import torch
+    host = []
+    for name, t in arrays:
+        if t.dtype in (torch.bool, torch.uint8, torch.int8, torch.int16):
+            t = t.to(torch.float32)
+        elif not t.is_floating_point():
+            x = t.to(torch.float64)
+            t = x.to(torch.float32) if torch.equal(x.to(torch.float32).to(torch.float64), x) else x
+        elif t.dtype != torch.float64:
+            t = t.to(torch.float32)
+        host.append((name, t))
+    rowed = [name in sampled for name, _ in host]
+    batch = {t.shape[0] for (_, t), r in zip(host, rowed) if r}
+    assert len(batch) <= 1, "sampled arrays must share their first dimension"
+    batch = batch.pop() if batch else 0
+    fixed = sum(t.numel() * t.element_size() for (_, t), r in zip(host, rowed) if not r)
+    per_row = sum(t[0].numel() * t.element_size() for (_, t), r in zip(host, rowed) if r)
+    rows = batch if per_row == 0 else min(batch, max(1, (budget - fixed) // per_row))
+    if fixed + rows * per_row > budget:
+        raise ValueError("--dump-outputs: %d bytes of whole arrays alone exceed %d" % (fixed, budget))
+    idx = None
+    if rows < batch:
+        idx = np.sort(np.random.RandomState(seed).choice(batch, rows, replace=False))
+    os.makedirs(out_dir, exist_ok=True)
+    for (name, t), r in zip(host, rowed):
+        if r and idx is not None:
+            t = t.index_select(0, torch.from_numpy(idx).to(t.device))
+        np.save(os.path.join(out_dir, name + ".npy"), t.cpu().numpy())
 
 
 # ------------------------------------------------------------------------------------------ CPU arm
@@ -549,34 +611,44 @@ def run_cuda(args):
         # launch-bound batches (C1): replay CUDA graphs of `graph_len` steps instead of 2 launches per step
         graph_len = min(64, n_rows)
         graph = env.capture_steps(actions[:graph_len])
-        K = ((K + graph_len - 1) // graph_len) * graph_len      # whole graphs
 
     def device_loop(k0, k):
+        """Enqueues exactly k steps: action rows k0 .. k0 + k - 1, or with --cuda-graph k // graph_len replays (rows
+        0 .. graph_len - 1 each) followed by k % graph_len eager steps on rows 0, 1, ..."""
         if graph_len:
-            for _ in range((k + graph_len - 1) // graph_len):
+            for _ in range(k // graph_len):
                 graph.replay()
+            for i in range(k % graph_len):
+                env.step_enqueue(actions[i], actions_ready=not args.serial)
             return
         for i in range(k0, k0 + k):
             # the action stream is pre-computed and resident: VN_STEP_ACTIONS_READY lets the scalar part of
             # step i + 1 run while the gather of step i is still copying
             env.step_enqueue(actions[i % n_rows], actions_ready=not args.serial)
 
-    device_loop(0, args.mix)      # un-timed: lets the state distribution settle (random-walk mixing)
-    device_loop(0, W)
     # the only collective anywhere near this path - the episode-statistics all-reduce - is exercised once here so that
     # its first-use cost (NCCL channel setup) cannot leak into anything timed later
     stats_vec = env.stats.to(torch.float64)
     if world_size > 1:
         dist.all_reduce(stats_vec)
-    est_ms = min(H.blocks(lambda r: device_loop(0, K), 2))
-    n_blocks = H.n_blocks_for(est_ms)
-    env.stats.zero_()
+    mark = {}
+
+    def warm_up():
+        device_loop(0, args.mix)      # un-timed: lets the state distribution settle (random-walk mixing)
+        # the statistics count the warm-up and the timed steps: nothing but steps may sit between the two, or the
+        # first timed step could not overlap the last warm-up gather
+        env.stats.zero_()
+        device_loop(0, W)
+        mark["launches0"] = env.kernel_launches
+
     sampler.start()
-    launches0 = env.kernel_launches
-    block_ms = H.blocks(lambda r: device_loop(W + r * K, K), n_blocks)
+    ms = H.blocks(lambda r: device_loop(W, K), 1, lead=warm_up)[0]
     clocks = sampler.stop()
-    launches = (launches_per_step * K * n_blocks) if graph_len else env.kernel_launches - launches0
-    ms = float(np.median(block_ms))
+    launches = (launches_per_step * K) if graph_len else env.kernel_launches - mark["launches0"]
+    if args.dump_outputs and rank == 0:
+        leaves = obs_leaves(env)
+        dump_outputs(args.dump_outputs, leaves + [("reward", env.reward), ("done", env.done)],
+                     sampled=[n for n, _ in leaves if n.startswith("obs_")])
     stats = env.episode_stats(reduce=True)
     value = n_total * K / (ms * 1e-3)
     p_reset = stats["resets"] / max(1.0, stats["steps"])
@@ -666,8 +738,8 @@ def run_cuda(args):
                 "traffic_source": prof.get("source") if prof else None,
                 "kernel": kname,
                 "kernel_ms": situ_ms, "algorithmic_bytes_per_launch": alg_bytes, "peak_source": peak_src,
-                "how": "in situ: CUDA events around blocks of K timed steps / K launches, median block (the scalar part "
-                       "of a step overlaps the previous gather, so this is the gather's launch-to-launch period)",
+                "how": "in situ: CUDA events around the K timed steps / K launches (the scalar part of a step overlaps "
+                       "the previous gather, so this is the gather's launch-to-launch period)",
                 "rows_skipped_rate": p_skip, "isolated": iso,
                 "same_size_copy_ms": copy_ms, "same_size_copy_gbs": 2 * nb / (copy_ms * 1e-3) / 1e9,
                 # the DRAM rate of the gather next to what a plain copy of this size reaches on this GPU (a 36 us
@@ -678,14 +750,12 @@ def run_cuda(args):
     run_stats = {"p_reset": p_reset, "collision_rate": coll, "rows_skipped_rate": p_skip,
                  "launches_per_step": launches_per_step, "states": world.n_states, "store_bytes": env.dw.nbytes(),
                  "batch_bytes_per_step": N * F_OBS, "gather": args.gather, "mix_steps": args.mix,
-                 "cuda_graph_steps": graph_len, "blocks": n_blocks, "timed_steps_total": K * n_blocks,
-                 "timed_region_ms": float(sum(block_ms)), "ms_per_step_min": min(block_ms) / K,
-                 "ms_per_step_max": max(block_ms) / K, "collective_ms": collective_ms}
+                 "cuda_graph_steps": graph_len, "blocks": 1, "timed_steps_total": K,
+                 "timed_region_ms": ms, "collective_ms": collective_ms}
 
     if args.quick:
         if rank == 0:
-            emit({"value": value, "ms_per_step": ms / K, "min": min(block_ms) / K, "max": max(block_ms) / K,
-                  "blocks": n_blocks, "frac": roofline["frac"], "iso": iso and iso["kernel_ms"],
+            emit({"value": value, "ms_per_step": ms / K, "frac": roofline["frac"], "iso": iso and iso["kernel_ms"],
                   "iso_frac": iso and iso["frac"], "p_reset": p_reset, "p_skip": p_skip,
                   "launches_per_step": launches_per_step})
         if world_size > 1:
@@ -889,8 +959,8 @@ def run_rollout(args):
     for _ in range(T):
         a = torch.randint(0, 4, (N,), device=dev, generator=gen, dtype=torch.int32)
         buf.step(env, a)
-    v_last = torch.randn(N, device=dev)
-    q_last = torch.rand(N, 400, device=dev)
+    v_last = torch.randn(N, device=dev, generator=gen)           # seeded like the actions: same inputs on every run
+    q_last = torch.rand(N, 400, device=dev, generator=gen)
 
     def builder(with_aux):
         ret = buf.returns(v_last, 0.99)
@@ -899,6 +969,8 @@ def run_rollout(args):
         aux = buf.auxiliary_targets(4, (20, 20)) if with_aux else None
         return ret, pcr, lab, aux
 
+    last = {}
+
     def timed(fn, k):
         for _ in range(W):
             fn()
@@ -906,12 +978,18 @@ def run_rollout(args):
         torch.cuda.synchronize(dev)
         e0.record()
         for _ in range(k):
-            fn()
+            last["out"] = fn()
         e1.record()
         torch.cuda.synchronize(dev)
         return e0.elapsed_time(e1) / k
 
     ms_core = timed(lambda: builder(False), K)
+    if args.dump_outputs:
+        ret, pcr, (labels, zero, nonzero, counts), _ = last["out"]
+        nz, nnz = (int(c) for c in counts.tolist())         # the position lists are valid up to their counts
+        dump_outputs(args.dump_outputs, [("returns", ret), ("pixel_control_returns", pcr), ("rp_labels", labels),
+                                         ("rp_zero_positions", zero[:nz]), ("rp_nonzero_positions", nonzero[:nnz])],
+                     sampled=["pixel_control_returns"])
     ms_all = timed(lambda: builder(True), max(2, K // 4))
     ms_pc = timed(lambda: buf.pixel_control(4, (20, 20)), K)
     ms_ret = timed(lambda: buf.returns(v_last, 0.99), K)
@@ -976,7 +1054,13 @@ def main():
     ap.add_argument("--hardness", default="none", help="curriculum hardness (set_complexity); 'none' = uniform starts")
     ap.add_argument("--mix", type=int, default=1000, help="un-timed steps before warm-up")
     ap.add_argument("--envs-per-gpu", type=int, default=None, help="development: override the envs per GPU")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step computed to DIR/<name>.npy (float32 / float64, <= 64 MB)")
     args = ap.parse_args()
+    if args.steps is not None and args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the CUDA path's outputs; the reference arm has none")
     if args.impl == "reference":
         run_reference(args)
     elif args.workload == "c5":

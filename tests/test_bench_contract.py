@@ -148,3 +148,32 @@ def test_timed_blocks_under_gloo_world_size_2(tmp_path):
     for r, p in enumerate(procs):
         out, err = p.communicate(timeout=180)
         assert p.returncode == 0 and "OK %d" % r in out, err[-3000:]
+
+
+def test_dump_outputs_types_budget_and_fixed_row_sample(tmp_path):
+    """--dump-outputs' writer: float32 / float64 files only, integers kept exact, and arrays too large for the budget
+    reduced to the same seeded rows in every array named as sampled (the others written whole)."""
+    import numpy as np
+    import torch
+    import bench
+    g = torch.Generator().manual_seed(0)
+    obs = torch.randint(0, 256, (64, 5, 5, 3), dtype=torch.uint8, generator=g)
+    arrays = [("obs", obs), ("v64", torch.rand(64, dtype=torch.float64, generator=g)),
+              ("reward", torch.rand(64, generator=g)), ("done", torch.rand(64, generator=g) < 0.5),
+              ("big", torch.arange(64) + (1 << 30)), ("lists", torch.arange(10, dtype=torch.int32))]
+    sampled = ["obs", "v64"]
+    bench.dump_outputs(str(tmp_path / "all"), arrays, sampled)
+    a = {k: np.load(tmp_path / "all" / (k + ".npy")) for k, _ in arrays}
+    assert a["obs"].dtype == np.float32 and np.array_equal(a["obs"], obs.numpy().astype(np.float32))
+    assert a["reward"].dtype == np.float32 and a["done"].dtype == np.float32 and a["v64"].dtype == np.float64
+    assert a["big"].dtype == np.float64 and np.array_equal(a["big"], np.arange(64) + (1 << 30))    # > 2^24: float64
+    assert a["lists"].dtype == np.float32 and np.array_equal(a["lists"], np.arange(10))
+    budget = 20 * (75 * 4 + 8) + 64 * (4 + 4 + 8) + 10 * 4
+    for d in ("s0", "s1"):
+        bench.dump_outputs(str(tmp_path / d), arrays, sampled, budget=budget)
+    s = {k: np.load(tmp_path / "s0" / (k + ".npy")) for k, _ in arrays}
+    assert all(np.array_equal(s[k], np.load(tmp_path / "s1" / (k + ".npy"))) for k in s)
+    rows = np.flatnonzero((a["obs"][:, None] == s["obs"][None]).all(axis=(2, 3, 4)).any(axis=1))
+    assert len(rows) == s["obs"].shape[0] == 20 and np.array_equal(s["v64"], a["v64"][rows])
+    assert all(np.array_equal(s[k], a[k]) for k in ("reward", "done", "big", "lists"))
+    assert sum(v.nbytes for v in s.values()) <= budget
