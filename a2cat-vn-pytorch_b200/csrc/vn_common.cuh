@@ -15,8 +15,43 @@
 namespace vn {
 
 void set_error(const char *fmt, ...);
-int32_t check_launch(const char *what);
+// Counts a kernel launch whose enqueue returned `e`; VN_ECUDA with `what` in vn_last_error when it failed.
+int32_t launch_result(const char *what, cudaError_t e);
+// The same for a launch written as kernel<<<...>>>, which reports through cudaGetLastError.
+inline int32_t check_launch(const char *what) { return launch_result(what, cudaGetLastError()); }
 int sm_count();  // multiprocessors of the current device (cached per device)
+// Raises the kernel's dynamic shared-memory limit on the current device to `bytes` unless an earlier call did; a size
+// is remembered only once the attribute was set.  VN_ECUDA with a message when it cannot be set.
+int32_t ensure_smem(const void *kernel, int bytes);
+template <typename... KArgs>
+int32_t ensure_smem(void (*kernel)(KArgs...), int bytes) {
+    return ensure_smem(reinterpret_cast<const void *>(kernel), bytes);
+}
+// CTAs of `smem` bytes of dynamic shared memory that fit on one SM (220 KB usable, ~1 KB reserved per CTA), 1 .. cap.
+inline int ctas_per_sm(int smem, int cap = 32) {
+    const int fit = (220 * 1024) / (smem + 1024);
+    return fit < 1 ? 1 : (fit < cap ? fit : cap);
+}
+
+// Launches kernel(args...) on `stream` and counts it.  programmatic: the kernel may be scheduled while its predecessor
+// in the stream is still running (programmatic dependent launch); it synchronises itself with griddepcontrol.wait.
+template <typename... KArgs, typename... Args>
+int32_t launch(void (*kernel)(KArgs...), const char *name, dim3 grid, dim3 block, size_t smem, cudaStream_t stream,
+               bool programmatic, Args... args) {
+    cudaLaunchConfig_t cfg = {};
+    cfg.gridDim = grid;
+    cfg.blockDim = block;
+    cfg.dynamicSmemBytes = smem;
+    cfg.stream = stream;
+    cudaLaunchAttribute attr[1];
+    attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
+    attr[0].val.programmaticStreamSerializationAllowed = 1;
+    cfg.attrs = attr;
+    cfg.numAttrs = programmatic ? 1 : 0;
+    cudaError_t e = cudaLaunchKernelEx(&cfg, kernel, static_cast<KArgs>(args)...);
+    const cudaError_t last = cudaGetLastError();  // also clears what a failed launch left behind
+    return launch_result(name, e != cudaSuccess ? e : last);
+}
 // All float leaves of one step in one launch (vn_rollout.cu); in_step = enqueued by vn_env_reset / vn_env_step* right
 // after the kernels that wrote `desc` (programmatic launch, releases its stream successor early).
 int32_t launch_float_leaves(const vn_store_t *store, const vn_float_leaf_t *leaves, int32_t n_leaves, const int32_t *desc,

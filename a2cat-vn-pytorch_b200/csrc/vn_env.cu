@@ -1,29 +1,24 @@
 // Vectorised env step / reset and the frame gather (sm_100a).
 //
-// Two launches per vectorised step, in stream order:
+// A vectorised step is, in stream order, programmatically chained:
 //   K1 vn_step_kernel   one thread per env: adjacency lookup, collision + goal test, reward, TimeLimit,
 //                       done, auto-reset (Philox4x32-10 or injected stream), RewardCollector accumulators,
 //                       last_action_reward, warp-aggregated episode statistics.  ~40 B per env.
-//   K2 vn_gather_*      one CTA per env: copies the env's observation planes (and, only if the env just
-//                       reset, its goal planes) from the HBM store into the contiguous policy batch.
-//                       >99.9 % of the bytes; HBM-bound; two variants (LDG.128 registers / bulk async copy).
+//   K2 vn_gather_*      copies each env's observation planes (and, only if the env just reset, its goal planes)
+//                       from the HBM store into the contiguous policy batch.  >99.9 % of the bytes; HBM-bound; two
+//                       variants: LDG.128 through registers (one CTA per env) and bulk async copies (persistent
+//                       one-warp CTAs that take (env, slice) units, see vn_gather_bulk_kernel).
+// or ONE launch that does both: vn_step_fused_kernel (a CTA per env, batches of one wave) and vn_step_gather_kernel
+// (a persistent grid, mid-size batches); choose_mode decides.
 #include <atomic>
 #include <chrono>
-#include <cstdlib>
 #include <cstring>
+#include <map>
+#include <mutex>
 #include <string>
+#include <utility>
 
 #include "vn_common.cuh"
-
-#ifndef VN_BULK_GROUPS_DEFAULT
-#define VN_BULK_GROUPS_DEFAULT 1  // chunks (own mbarrier each) per record slice in the bulk copies, see bulk_copy_slice
-#endif
-#ifndef VN_BULK_TAIL_DEFAULT
-#define VN_BULK_TAIL_DEFAULT 1  // slices per record for the last wave's worth of envs of a bulk gather (1 = whole records)
-#endif
-#ifndef VN_PERSISTENT_DEFAULT
-#define VN_PERSISTENT_DEFAULT 1  // VN_GATHER_AUTO beyond one wave: 0 never, 1 mid-size device-resident batches, 2 always
-#endif
 
 namespace vn {
 
@@ -40,13 +35,12 @@ void set_error(const char *fmt, ...) {
     g_error = buf;
 }
 
-int32_t check_launch(const char *what) {
-    g_launches.fetch_add(1, std::memory_order_relaxed);
-    cudaError_t e = cudaGetLastError();
+int32_t launch_result(const char *what, cudaError_t e) {
     if (e != cudaSuccess) {
         set_error("%s: %s", what, cudaGetErrorString(e));
         return VN_ECUDA;
     }
+    g_launches.fetch_add(1, std::memory_order_relaxed);
     return VN_OK;
 }
 
@@ -67,8 +61,6 @@ struct StepParams {
 
 constexpr int kStepThreads = 128;  // envs per block of the scalar half (= envs per host_seq word)
 
-__device__ __forceinline__ uint32_t warp_sum(uint32_t v) { return __reduce_add_sync(0xffffffffu, v); }
-
 // Programmatic dependent launch: every kernel of the step path lets its successor be scheduled early
 // (launch latency overlaps this kernel's execution) and waits for its predecessor's memory to be visible
 // before touching any env data.  Both are no-ops when the launch was not programmatic.
@@ -81,7 +73,37 @@ __device__ __forceinline__ void pdl_wait_then_release() {
 struct EnvStats {
     uint32_t episodes = 0, len = 0, succ = 0, coll = 0, steps = 0, trunc = 0, resets = 0, skipped = 0;
     float ret = 0.f;
+
+    __device__ __forceinline__ EnvStats &operator+=(const EnvStats &o) {
+        episodes += o.episodes;
+        len += o.len;
+        succ += o.succ;
+        coll += o.coll;
+        steps += o.steps;
+        trunc += o.trunc;
+        resets += o.resets;
+        skipped += o.skipped;
+        ret += o.ret;
+        return *this;
+    }
 };
+
+// Sum over the (full) warp; every lane receives it.
+__device__ __forceinline__ EnvStats warp_reduce(const EnvStats &s) {
+    EnvStats w;
+    w.episodes = __reduce_add_sync(0xffffffffu, s.episodes);
+    w.len = __reduce_add_sync(0xffffffffu, s.len);
+    w.succ = __reduce_add_sync(0xffffffffu, s.succ);
+    w.coll = __reduce_add_sync(0xffffffffu, s.coll);
+    w.steps = __reduce_add_sync(0xffffffffu, s.steps);
+    w.trunc = __reduce_add_sync(0xffffffffu, s.trunc);
+    w.resets = __reduce_add_sync(0xffffffffu, s.resets);
+    w.skipped = __reduce_add_sync(0xffffffffu, s.skipped);
+    w.ret = s.ret;
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) w.ret += __shfl_xor_sync(0xffffffffu, w.ret, o);
+    return w;
+}
 
 // One env, one step (or reset): everything the reference does between receiving the action and calling
 // observe().  Returns the store record whose frames must be in the batch (rec; -1 = the batch row already
@@ -298,18 +320,7 @@ __global__ void __launch_bounds__(kStepThreads) vn_step_kernel(const StepParams 
 
     if (p.out.stats) {
         // warp-aggregated statistics: one atomic per counter per warp
-        EnvStats w;
-        w.episodes = warp_sum(st.episodes);
-        w.len = warp_sum(st.len);
-        w.succ = warp_sum(st.succ);
-        w.coll = warp_sum(st.coll);
-        w.steps = warp_sum(st.steps);
-        w.trunc = warp_sum(st.trunc);
-        w.resets = warp_sum(st.resets);
-        w.skipped = warp_sum(st.skipped);
-        w.ret = st.ret;
-#pragma unroll
-        for (int o = 16; o > 0; o >>= 1) w.ret += __shfl_xor_sync(0xffffffffu, w.ret, o);
+        const EnvStats w = warp_reduce(st);
         if ((threadIdx.x & 31) == 0) add_stats(p.out.stats, w);
     }
     if (p.out.host_seq) signal_host(p.out);
@@ -335,7 +346,7 @@ struct GatherParams {
     // memory - often env.state / obs_state / goal themselves - that a following step kernel REWRITES, so the successor
     // must not start before this grid has completed.
     int32_t early_release;
-    // development: per-CTA timeline (vn_debug_gather_trace): [grid][8] globaltimer stamps, NULL = off
+    // development: per-CTA timeline (vn_debug_gather_trace): [grid][16] words, see vn_gather_bulk_kernel; NULL = off
     unsigned long long *trace;
 };
 
@@ -414,60 +425,29 @@ __global__ void __launch_bounds__(kThreads) vn_gather_ldg_kernel(const GatherPar
 // Work unit = (env, slice): each plane is cut into `split` slices of whole 16-byte units, so that
 // split > 1 gives more, smaller CTAs per SM.  Units are handed out by an atomic ticket counter
 // (persistent CTAs, dynamic scheduling): no CTA idles while another still has a queue of records.
-// The ticket counter is CALLER-OWNED scratch (vn_step_out_t.sched: [0] next ticket, [1] CTAs finished), zero
-// before the first launch and re-armed by the last CTA of every launch, so gathers of different env batches
-// on different streams never share a counter.  Without scratch the units are dealt statically.
-
-struct BulkHints {
-    int mode;  // bit 0: loads evict_last, bit 1: stores evict_first
-    uint64_t load_policy, store_policy;
-    int groups = 1;  // chunks per record slice, each with its own mbarrier (1 .. kCopyGroups)
-    int whole_record = 0;  // bit 0 / 1: the observation / goal plane set is contiguous in the record and shared memory was
-                           // sized for its SPAN: one load per record (see bulk_copy_slice)
+// The ticket counter is CALLER-OWNED scratch (vn_step_out_t.sched[parity & 1]), zero before the first launch and
+// zeroed again by the scalar half of the step that next uses it, so gathers of different env batches on different
+// streams never share a counter.  Without scratch the units are dealt statically.
+//
+// L2 policies of the copies: the store is re-read across envs and steps, a batch row is written once and read by a
+// later kernel, so loads are evict_last and stores evict_first (measured +2.5 % C2, +4 % at hardness 0.01,
+// profiles/r1b_l2_hint_sweep.txt).
+struct L2Policies {
+    uint64_t load, store;
 };
 
-struct NoPrefetch {
-    __device__ __forceinline__ void operator()() const {}
-};
-
-// `while_loading()` runs after the global->shared copies of the slice have been issued and before the wait for them: the
-// place to fetch whatever the NEXT unit needs (ticket, descriptor) so that its latency hides behind this transfer.
-// One record slice through shared memory in kCopyGroups chunks, each with its own mbarrier: all loads are issued at once,
-// and the stores of chunk g go out as soon as chunk g has landed - while chunks g+1.. are still loading.  With ONE barrier
-// for the whole record (round 1) a CTA alternated between a pure load phase and a pure store phase: the first 6.5 us of
-// every launch were reads only, and every unit paid load latency + store drain back to back.
-constexpr int kCopyGroups = 4;
-
-// Calls op(group, plane, first 16-byte unit in the plane, units, shared-memory offset in units) for every piece of the
-// slice; pieces are cut at plane ends and at group boundaries (gsize units of shared memory per group).
-template <typename Op>
-__device__ __forceinline__ void for_each_piece(const vn_store_t &st, uint8_t *const *dst, int slice, int split, int gsize,
-                                               int groups, Op op) {
-    int off = 0;
-    for (int pl = 0; pl < st.n_planes; ++pl)
-        if (dst[pl]) {
-            const int n16 = st.plane_bytes[pl] >> 4, per = (n16 + split - 1) / split;
-            const int lo = min(slice * per, n16), hi = min(lo + per, n16);
-            int pos = lo;
-            while (pos < hi) {
-                const int g = min(off / gsize, groups - 1);
-                const int room = g == groups - 1 ? hi - pos : (g + 1) * gsize - off;
-                const int cnt = min(hi - pos, room);
-                op(g, pl, pos, cnt, off);
-                pos += cnt;
-                off += cnt;
-            }
-        }
-}
-
-template <typename F = NoPrefetch>
-__device__ __forceinline__ void bulk_copy_slice(const vn_store_t &st, const uint8_t *src, uint8_t *const *dst,
-                                                int env, int slice, int split, uint8_t *smem, uint64_t *bar,
-                                                uint32_t &parity, const BulkHints &hints, F while_loading = F(),
-                                                bool whole = false) {
+// One record slice through shared memory: all its loads complete on one mbarrier, then its stores go out.
+// `while_loading()` runs after the loads have been issued and before the wait for them: the place to fetch whatever the
+// NEXT unit needs (ticket, descriptor) so that its latency hides behind this transfer.  whole: the plane set is
+// contiguous in the record and shared memory was sized for its SPAN (plane_set_bytes), so one load brings the record.
+template <typename F>
+__device__ __forceinline__ void bulk_copy_slice(const vn_store_t &st, const uint8_t *src, uint8_t *const *dst, int env,
+                                                int slice, int split, uint8_t *smem, uint64_t *bar, uint32_t &parity,
+                                                const L2Policies &pol, F while_loading, bool whole) {
     // the previous shared->global reads of this buffer must have drained before it is refilled
     bulk_wait_read<0>();
     int total = 0;
+#pragma unroll 1
     for (int pl = 0; pl < st.n_planes; ++pl)
         if (dst[pl]) {
             const int n16 = st.plane_bytes[pl] >> 4, per = (n16 + split - 1) / split;
@@ -488,94 +468,77 @@ __device__ __forceinline__ void bulk_copy_slice(const vn_store_t &st, const uint
         const uint32_t base = (uint32_t)st.plane_off[first];
         const uint32_t span = (uint32_t)st.plane_off[last] + (uint32_t)st.plane_bytes[last] - base;
         mbar_expect_tx(bar, span);
-        if (hints.mode & 1)
-            bulk_g2s_hint(smem, src + base, span, bar, hints.load_policy);
-        else
-            bulk_g2s(smem, src + base, span, bar);
+        bulk_g2s_hint(smem, src + base, span, bar, pol.load);
         while_loading();
         mbar_wait(bar, parity & 1u);
         parity ^= 1u;
         for (int pl = first; pl <= last; ++pl)
-            if (dst[pl]) {
-                uint8_t *to = dst[pl] + (size_t)env * st.plane_bytes[pl];
-                const uint8_t *from = smem + ((uint32_t)st.plane_off[pl] - base);
-                if (hints.mode & 2)
-                    bulk_s2g_hint(to, from, (uint32_t)st.plane_bytes[pl], hints.store_policy);
-                else
-                    bulk_s2g(to, from, (uint32_t)st.plane_bytes[pl]);
-            }
+            if (dst[pl])
+                bulk_s2g_hint(dst[pl] + (size_t)env * st.plane_bytes[pl], smem + ((uint32_t)st.plane_off[pl] - base),
+                              (uint32_t)st.plane_bytes[pl], pol.store);
         bulk_commit();
         return;
     }
-    const int groups = hints.groups;
-    const int gsize = (total + groups - 1) / groups;
-    for (int g = 0; g < groups; ++g) {
-        const int units = min(total, g == groups - 1 ? total : (g + 1) * gsize) - min(total, g * gsize);
-        if (units > 0) mbar_expect_tx(bar + g, (uint32_t)units << 4);
-    }
-    for_each_piece(st, dst, slice, split, gsize, groups, [&](int g, int pl, int pos, int cnt, int off) {
-        const uint8_t *from = src + st.plane_off[pl] + ((size_t)pos << 4);
-        if (hints.mode & 1)
-            bulk_g2s_hint(smem + ((size_t)off << 4), from, (uint32_t)cnt << 4, bar + g, hints.load_policy);
-        else
-            bulk_g2s(smem + ((size_t)off << 4), from, (uint32_t)cnt << 4, bar + g);
-    });
-    while_loading();
+    // the slices of the planes, packed back to back in shared memory
+    mbar_expect_tx(bar, (uint32_t)total << 4);
+    int off = 0;
 #pragma unroll 1
-    for (int g = 0; g < groups; ++g) {
-        if (min(total, g * gsize) >= total) break;   // no bytes in this group (tiny slices)
-        mbar_wait(bar + g, (parity >> g) & 1u);
-        parity ^= 1u << g;
-        for_each_piece(st, dst, slice, split, gsize, groups, [&](int pg, int pl, int pos, int cnt, int off) {
-            if (pg != g) return;
-            uint8_t *to = dst[pl] + (size_t)env * st.plane_bytes[pl] + ((size_t)pos << 4);
-            if (hints.mode & 2)
-                bulk_s2g_hint(to, smem + ((size_t)off << 4), (uint32_t)cnt << 4, hints.store_policy);
-            else
-                bulk_s2g(to, smem + ((size_t)off << 4), (uint32_t)cnt << 4);
-        });
-    }
+    for (int pl = 0; pl < st.n_planes; ++pl)
+        if (dst[pl]) {
+            const int n16 = st.plane_bytes[pl] >> 4, per = (n16 + split - 1) / split;
+            const int lo = min(slice * per, n16), hi = min(lo + per, n16);
+            if (hi > lo)
+                bulk_g2s_hint(smem + ((size_t)off << 4), src + st.plane_off[pl] + ((size_t)lo << 4),
+                              (uint32_t)(hi - lo) << 4, bar, pol.load);
+            off += hi - lo;
+        }
+    while_loading();
+    mbar_wait(bar, parity & 1u);
+    parity ^= 1u;
+    off = 0;
+#pragma unroll 1
+    for (int pl = 0; pl < st.n_planes; ++pl)
+        if (dst[pl]) {
+            const int n16 = st.plane_bytes[pl] >> 4, per = (n16 + split - 1) / split;
+            const int lo = min(slice * per, n16), hi = min(lo + per, n16);
+            if (hi > lo)
+                bulk_s2g_hint(dst[pl] + (size_t)env * st.plane_bytes[pl] + ((size_t)lo << 4), smem + ((size_t)off << 4),
+                              (uint32_t)(hi - lo) << 4, pol.store);
+            off += hi - lo;
+        }
     bulk_commit();
 }
 
-// Work units: envs [0, n_whole) are one unit each (the whole record); every env from n_whole on is cut into `split`
-// slices, one unit per slice.  n_whole = 0: every record sliced (small batches, records larger than shared memory
-// allows); n_whole = n: no slicing; in between: only the LAST units of a launch are small ("guided" scheduling - the
-// spread of the last units' durations is what a launch pays at its end).
-__global__ void __launch_bounds__(32) vn_gather_bulk_kernel(const GatherParams p, int split, int n_whole,
-                                                            unsigned int *sched, int hint_mode) {
+// whole: bit 0 / 1 = the observation / goal plane set is loaded as one span (bulk_copy_slice), only with split == 1.
+// Trace record of a CTA (16 words): [0] resident, [1] predecessor complete, [2] first unit issued, [3] last unit
+// issued, [4] shared memory drained, [5] units, [6] SM id, [8 + k] unit k issued (bit 63: nothing copied), k < 8.
+__global__ void __launch_bounds__(32) vn_gather_bulk_kernel(const GatherParams p, int split, unsigned int *sched,
+                                                            int whole) {
     extern __shared__ __align__(128) uint8_t smem[];
-    __shared__ uint64_t bar[kCopyGroups];
+    __shared__ uint64_t bar;
     if (threadIdx.x != 0) return;
     unsigned long long *tr = p.trace ? p.trace + (size_t)blockIdx.x * 16 : nullptr;
     if (tr) {
-        tr[0] = globaltimer_ns();   // CTA resident
+        tr[0] = globaltimer_ns();
         unsigned int smid;
         asm volatile("mov.u32 %0, %smid;" : "=r"(smid));
         tr[6] = smid;
     }
-#pragma unroll
-    for (int g = 0; g < kCopyGroups; ++g) mbar_init(bar + g, 1);
+    mbar_init(&bar, 1);
     asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
     // the prologue above overlapped the scalar kernel; its results are needed from here on
     asm volatile("griddepcontrol.wait;" ::: "memory");
     if (p.early_release) asm volatile("griddepcontrol.launch_dependents;" ::: "memory");
-    if (tr) tr[1] = globaltimer_ns();   // predecessor complete
+    if (tr) tr[1] = globaltimer_ns();
     int n_units = 0;
     uint32_t parity = 0;
-    BulkHints hints;
-    // bits: 1 loads evict_last, 2 stores evict_first, 4 loads evict_first, 8 stores evict_last
-    hints.load_policy = (hint_mode & 1) ? l2_policy_evict_last() : (hint_mode & 4) ? l2_policy_evict_first() : 0;
-    hints.store_policy = (hint_mode & 2) ? l2_policy_evict_first() : (hint_mode & 8) ? l2_policy_evict_last() : 0;
-    hints.mode = ((hint_mode & 5) ? 1 : 0) | ((hint_mode & 10) ? 2 : 0);
-    hints.groups = max(1, min(kCopyGroups, (hint_mode >> 8) & 7));
-    hints.whole_record = (hint_mode >> 16) & 3;
-    const int units = n_whole + (p.n - n_whole) * split;
+    const L2Policies pol{l2_policy_evict_last(), l2_policy_evict_first()};
+    const int units = p.n * split;
     const bool dynamic = sched != nullptr;
     // (record, goal record) of a unit; -1 = nothing to copy (row unchanged / no reset / past the end)
     auto unit_desc = [&](int u) -> int2 {
         if (u >= units) return make_int2(-1, -1);
-        const int env = u < n_whole ? u : n_whole + (u - n_whole) / split;
+        const int env = split == 1 ? u : u / split;
         if (p.desc) return p.desc[env];
         int2 d = make_int2(p.obs_state[env], -1);
         if (p.goal && (!p.did_reset || p.did_reset[env])) d.y = p.goal[env];
@@ -587,10 +550,8 @@ __global__ void __launch_bounds__(32) vn_gather_bulk_kernel(const GatherParams p
     int u = (int)blockIdx.x;
     int2 d = unit_desc(u);
     while (u < units) {
-        const bool whole_unit = u < n_whole;
-        const int env = whole_unit ? u : n_whole + (u - n_whole) / split;
-        const int slice = whole_unit ? 0 : (u - n_whole) % split;
-        const int sp = whole_unit ? 1 : split;
+        const int env = split == 1 ? u : u / split;
+        const int slice = split == 1 ? 0 : u - env * split;
         int u_next = 0;
         int2 d_next = make_int2(-1, -1);
         bool have_next = false;
@@ -602,19 +563,19 @@ __global__ void __launch_bounds__(32) vn_gather_bulk_kernel(const GatherParams p
         };
         if (d.x >= 0) {  // < 0: the row already holds this record (VN_STEP_SKIP_UNCHANGED)
             const uint8_t *src = p.store.base + (size_t)d.x * p.store.state_pitch;
-            bulk_copy_slice(p.store, src, p.obs, env, slice, sp, smem, bar, parity, hints, fetch_next,
-                            (hints.whole_record & 1) != 0);
+            bulk_copy_slice(p.store, src, p.obs, env, slice, split, smem, &bar, parity, pol, fetch_next,
+                            (whole & 1) != 0);
         }
         if (d.y >= 0) {
             const uint8_t *gsrc = p.store.base + (size_t)d.y * p.store.state_pitch;
-            bulk_copy_slice(p.store, gsrc, p.goal_obs, env, slice, sp, smem, bar, parity, hints, fetch_next,
-                            (hints.whole_record & 2) != 0);
+            bulk_copy_slice(p.store, gsrc, p.goal_obs, env, slice, split, smem, &bar, parity, pol, fetch_next,
+                            (whole & 2) != 0);
         }
         fetch_next();
         if (tr) {
-            if (n_units == 0) tr[2] = globaltimer_ns();   // first unit issued (its stores are in flight)
-            tr[3] = globaltimer_ns();                      // last unit issued
-            if (n_units < 8) tr[8 + n_units] = tr[3] | ((unsigned long long)(d.x < 0 && d.y < 0) << 63);  // bit 63: nothing copied
+            if (n_units == 0) tr[2] = globaltimer_ns();
+            tr[3] = globaltimer_ns();
+            if (n_units < 8) tr[8 + n_units] = tr[3] | ((unsigned long long)(d.x < 0 && d.y < 0) << 63);
             ++n_units;
         }
         u = u_next;
@@ -622,7 +583,7 @@ __global__ void __launch_bounds__(32) vn_gather_bulk_kernel(const GatherParams p
     }
     bulk_wait_read<0>();
     if (tr) {
-        tr[4] = globaltimer_ns();   // shared memory drained
+        tr[4] = globaltimer_ns();
         tr[5] = (unsigned long long)n_units;
     }
     // no epilogue: the ticket counter of this launch (sched[parity]) is zeroed by the scalar half of the step that
@@ -636,6 +597,9 @@ __global__ void __launch_bounds__(32) vn_gather_bulk_kernel(const GatherParams p
 // env, then lane 0 of warp w moves slice w of every plane - the observation record and, after a reset, the goal
 // record, both in flight at once - with bulk async copies through a record-shaped region of shared memory.
 constexpr int kFusedWarps = 4;
+// VN_GATHER_AUTO runs a batch fused up to this many envs per SM (fewer when shared memory holds fewer records): beyond,
+// the step is no longer bound by launch latency and the two-kernel path (pipelined, bandwidth-tuned) wins
+constexpr int kFusedPerSm = 4;
 
 template <bool kReset>
 __global__ void __launch_bounds__(kFusedWarps * 32) vn_step_fused_kernel(const StepParams sp, const GatherParams gp) {
@@ -717,14 +681,14 @@ __global__ void __launch_bounds__(kFusedWarps * 32) vn_step_fused_kernel(const S
 // No CTA ever waits for another one (ownership is static), nothing goes through a second launch, and there is no
 // descriptor hand-off between kernels: the scalar kernel, the PDL hand-off and the ticket counter of the two-kernel
 // path are gone.  Records that need slicing (split > 1) stay on the two-kernel path.
+// whole: as for vn_gather_bulk_kernel.
 template <bool kReset>
-__global__ void __launch_bounds__(32) vn_step_gather_kernel(const StepParams sp, const GatherParams gp, int hint_mode) {
+__global__ void __launch_bounds__(32) vn_step_gather_kernel(const StepParams sp, const GatherParams gp, int whole) {
     extern __shared__ __align__(128) uint8_t smem[];
-    __shared__ uint64_t bar[kCopyGroups];
+    __shared__ uint64_t bar;
     const int lane = threadIdx.x;
     if (lane == 0) {
-#pragma unroll
-        for (int g = 0; g < kCopyGroups; ++g) mbar_init(bar + g, 1);
+        mbar_init(&bar, 1);
         asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
     }
     // everything above overlapped the previous kernel of the stream; its env state is needed from here on
@@ -742,30 +706,11 @@ __global__ void __launch_bounds__(32) vn_step_gather_kernel(const StepParams sp,
             int rec, grec;
             step_env<kReset>(sp, e, st, rec, grec);
             desc[e] = make_int2(rec, grec);
-            acc.episodes += st.episodes;
-            acc.len += st.len;
-            acc.succ += st.succ;
-            acc.coll += st.coll;
-            acc.steps += st.steps;
-            acc.trunc += st.trunc;
-            acc.resets += st.resets;
-            acc.skipped += st.skipped;
-            acc.ret += st.ret;
+            acc += st;
         }
     }
     if (sp.out.stats) {
-        EnvStats w;
-        w.episodes = warp_sum(acc.episodes);
-        w.len = warp_sum(acc.len);
-        w.succ = warp_sum(acc.succ);
-        w.coll = warp_sum(acc.coll);
-        w.steps = warp_sum(acc.steps);
-        w.trunc = warp_sum(acc.trunc);
-        w.resets = warp_sum(acc.resets);
-        w.skipped = warp_sum(acc.skipped);
-        w.ret = acc.ret;
-#pragma unroll
-        for (int o = 16; o > 0; o >>= 1) w.ret += __shfl_xor_sync(0xffffffffu, w.ret, o);
+        const EnvStats w = warp_reduce(acc);
         if (lane == 0) add_stats(sp.out.stats, w);
     }
     __syncwarp();   // the lanes' descriptor / host-pack writes are ordered before what lanes 0 and 1 do next
@@ -784,12 +729,7 @@ __global__ void __launch_bounds__(32) vn_step_gather_kernel(const StepParams sp,
 
     // ---- phase B: copy the records of the same envs
     uint32_t parity = 0;
-    BulkHints hints;
-    hints.load_policy = (hint_mode & 1) ? l2_policy_evict_last() : (hint_mode & 4) ? l2_policy_evict_first() : 0;
-    hints.store_policy = (hint_mode & 2) ? l2_policy_evict_first() : (hint_mode & 8) ? l2_policy_evict_last() : 0;
-    hints.mode = ((hint_mode & 5) ? 1 : 0) | ((hint_mode & 10) ? 2 : 0);
-    hints.groups = max(1, min(kCopyGroups, (hint_mode >> 8) & 7));
-    hints.whole_record = (hint_mode >> 16) & 3;
+    const L2Policies pol{l2_policy_evict_last(), l2_policy_evict_first()};
     int2 d = desc[b];
     for (int e = b; e < n; e += G) {
         int2 d_next = make_int2(-1, -1);
@@ -799,11 +739,11 @@ __global__ void __launch_bounds__(32) vn_step_gather_kernel(const StepParams sp,
             have_next = true;
         };
         if (d.x >= 0)  // < 0: the row already holds this record (VN_STEP_SKIP_UNCHANGED)
-            bulk_copy_slice(gp.store, gp.store.base + (size_t)d.x * gp.store.state_pitch, gp.obs, e, 0, 1, smem, bar,
-                            parity, hints, fetch_next, (hints.whole_record & 1) != 0);
+            bulk_copy_slice(gp.store, gp.store.base + (size_t)d.x * gp.store.state_pitch, gp.obs, e, 0, 1, smem, &bar,
+                            parity, pol, fetch_next, (whole & 1) != 0);
         if (d.y >= 0 && gp.goal)
-            bulk_copy_slice(gp.store, gp.store.base + (size_t)d.y * gp.store.state_pitch, gp.goal_obs, e, 0, 1, smem, bar,
-                            parity, hints, fetch_next, (hints.whole_record & 2) != 0);
+            bulk_copy_slice(gp.store, gp.store.base + (size_t)d.y * gp.store.state_pitch, gp.goal_obs, e, 0, 1, smem,
+                            &bar, parity, pol, fetch_next, (whole & 2) != 0);
         fetch_next();
         d = d_next;
     }
@@ -857,25 +797,6 @@ static int32_t validate_store(const vn_store_t *s) {
     return VN_OK;
 }
 
-// Launch with programmatic stream serialisation allowed (PDL): the kernel may be scheduled while its
-// predecessor in the stream is still running; it synchronises itself with griddepcontrol.wait.
-template <typename... KArgs, typename... Args>
-static cudaError_t launch_pdl(void (*kernel)(KArgs...), dim3 grid, dim3 block, size_t smem, cudaStream_t stream,
-                              Args... args) {
-    cudaLaunchConfig_t cfg = {};
-    cfg.gridDim = grid;
-    cfg.blockDim = block;
-    cfg.dynamicSmemBytes = smem;
-    cfg.stream = stream;
-    cudaLaunchAttribute attr[1];
-    attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-    attr[0].val.programmaticStreamSerializationAllowed = 1;
-    static const bool pdl = !(getenv("VN_NO_PDL") && atoi(getenv("VN_NO_PDL")));
-    cfg.attrs = attr;
-    cfg.numAttrs = pdl ? 1 : 0;
-    return cudaLaunchKernelEx(&cfg, kernel, static_cast<KArgs>(args)...);
-}
-
 constexpr int kMaxDevices = 64;
 static int current_device() {
     int dev = 0;
@@ -892,6 +813,33 @@ int sm_count() {
     return cached[dev];
 }
 
+int32_t ensure_smem(const void *kernel, int bytes) {
+    static std::mutex mu;
+    static std::map<std::pair<const void *, int>, int> configured;  // (kernel, device) -> bytes
+    const int dev = current_device();
+    std::lock_guard<std::mutex> lock(mu);
+    int &have = configured[{kernel, dev}];
+    if (bytes <= have) return VN_OK;
+    const cudaError_t e = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, bytes);
+    if (e != cudaSuccess) {
+        cudaGetLastError();
+        set_error("%d bytes of dynamic shared memory: %s", bytes, cudaGetErrorString(e));
+        return VN_ECUDA;
+    }
+    have = bytes;
+    return VN_OK;
+}
+
+static int32_t check_rows_aligned(const GatherParams &gp) {
+    for (int pl = 0; pl < gp.store.n_planes; ++pl) {
+        VN_REQUIRE(!gp.obs[pl] || (reinterpret_cast<uintptr_t>(gp.obs[pl]) & 15) == 0,
+                   "gather: obs[%d] must be 16-byte aligned", pl);
+        VN_REQUIRE(!gp.goal_obs[pl] || (reinterpret_cast<uintptr_t>(gp.goal_obs[pl]) & 15) == 0,
+                   "gather: goal_obs[%d] must be 16-byte aligned", pl);
+    }
+    return VN_OK;
+}
+
 // Shared memory a CTA needs for one whole record of a plane set, and whether that set is CONTIGUOUS in the record
 // (nothing but alignment padding between its planes): then *span covers it with one load.
 static int plane_set_bytes(const vn_store_t &st, uint8_t *const *dst, bool use, int *span, bool *contiguous) {
@@ -903,94 +851,62 @@ static int plane_set_bytes(const vn_store_t &st, uint8_t *const *dst, bool use, 
             last = pl;
         }
     *span = first < 0 ? 0 : st.plane_off[last] + st.plane_bytes[last] - st.plane_off[first];
-    static const bool off = getenv("VN_NO_WHOLE_RECORD") && atoi(getenv("VN_NO_WHOLE_RECORD"));
-    *contiguous = !off && first >= 0 && last > first && *span - sum <= 128 * (last - first);
+    *contiguous = first >= 0 && last > first && *span - sum <= 128 * (last - first);
     return sum;
 }
 
+// The gather half of a two-kernel step, and the gather-only entry points (vn_env_gather, vn_gather_plane): there is
+// no scalar half here, so the one-launch modes mean VN_GATHER_BULK.
 static int32_t launch_gather(const GatherParams &gp, int32_t variant, cudaStream_t stream) {
     if (gp.n == 0) return VN_OK;
-    for (int pl = 0; pl < gp.store.n_planes; ++pl) {
-        VN_REQUIRE(!gp.obs[pl] || (reinterpret_cast<uintptr_t>(gp.obs[pl]) & 15) == 0,
-                   "gather: obs[%d] must be 16-byte aligned", pl);
-        VN_REQUIRE(!gp.goal_obs[pl] || (reinterpret_cast<uintptr_t>(gp.goal_obs[pl]) & 15) == 0,
-                   "gather: goal_obs[%d] must be 16-byte aligned", pl);
-    }
-    if (variant == VN_GATHER_FUSED || variant == VN_GATHER_PERSISTENT)
-        variant = VN_GATHER_BULK;  // no scalar half here: the one-launch modes do not apply
+    int32_t rc = check_rows_aligned(gp);
+    if (rc) return rc;
     // measured on B200 (profiles/): the bulk-copy variant reaches 94 % of the copy peak, LDG.128 86 %
-    if (variant == VN_GATHER_AUTO) variant = VN_GATHER_BULK;
+    if (variant == VN_GATHER_AUTO || variant == VN_GATHER_FUSED || variant == VN_GATHER_PERSISTENT)
+        variant = VN_GATHER_BULK;
     if (variant == VN_GATHER_LDG) {
         constexpr int kThreads = 256;
-        launch_pdl(vn_gather_ldg_kernel<kThreads, 4>, dim3(gp.n), dim3(kThreads), 0, stream, gp);
-        return check_launch("vn_gather_ldg_kernel");
+        return launch(vn_gather_ldg_kernel<kThreads, 4>, "vn_gather_ldg_kernel", dim3(gp.n), dim3(kThreads), 0, stream,
+                      true, gp);
     }
-    if (variant == VN_GATHER_BULK) {
-        // tunables (development overrides through the environment; defaults chosen from profiles/)
-        static const int env_split = getenv("VN_BULK_SPLIT") ? atoi(getenv("VN_BULK_SPLIT")) : 0;
-        static const int env_per_sm = getenv("VN_BULK_PER_SM") ? atoi(getenv("VN_BULK_PER_SM")) : 0;
-        static const int env_dynamic = getenv("VN_BULK_DYNAMIC") ? atoi(getenv("VN_BULK_DYNAMIC")) : 1;
-        // L2 policy hints: loads evict_last + stores evict_first measured +2.5 % (C2) / +4 % (hardness 0.01)
-        static const int env_groups = getenv("VN_BULK_GROUPS") ? atoi(getenv("VN_BULK_GROUPS")) : VN_BULK_GROUPS_DEFAULT;
-        static const int env_hints =
-            (getenv("VN_BULK_L2_HINTS") ? atoi(getenv("VN_BULK_L2_HINTS")) : 3) | (max(1, min(7, env_groups)) << 8);
-        // small batches (C1: 16 envs) cannot fill 148 SMs with one record per CTA: cut each record into
-        // slices until there are ~2 units per SM (latency-bound regime; one slice >= 2 KB)
-        int split = env_split > 0 ? env_split : 1;
-        if (env_split <= 0 && gp.n < 2 * sm_count()) split = min(16, (2 * sm_count() + gp.n - 1) / gp.n);
-        if (env_split <= 0) {
-            // large records (the reference's native 174 x 174 frames: 212 KB for rgb + depth + segmentation) are
-            // cut into slices of at most 52 KB so that at least 4 CTAs stay resident per SM (84 x 84 rgb + depth +
-            // segmentation = 49.6 KB stays whole: one load per record instead of two slices of three)
-            int per_env = 0, per_goal = 0;
-            for (int pl = 0; pl < gp.store.n_planes; ++pl) {
-                if (gp.obs[pl]) per_env += gp.store.plane_bytes[pl];
-                if (gp.goal && gp.goal_obs[pl]) per_goal += gp.store.plane_bytes[pl];
-            }
-            split = max(split, (max(per_env, per_goal) + 52 * 1024 - 1) / (52 * 1024));
-        }
-        int smem_obs = 0, smem_goal = 0;
-        for (int pl = 0; pl < gp.store.n_planes; ++pl) {
-            const int n16 = gp.store.plane_bytes[pl] >> 4, per = (n16 + split - 1) / split;
-            if (gp.obs[pl]) smem_obs += per << 4;
-            if (gp.goal && gp.goal_obs[pl]) smem_goal += per << 4;
-        }
-        int smem = max(smem_obs, smem_goal), whole = 0;
-        int n_whole = split == 1 ? gp.n : 0, k_split = split;
-        if (split == 1) {
-            int span_o, span_g;
-            bool co, cg;
-            plane_set_bytes(gp.store, gp.obs, true, &span_o, &co);
-            plane_set_bytes(gp.store, gp.goal_obs, gp.goal != nullptr, &span_g, &cg);
-            if (co) smem = max(smem, span_o);
-            if (cg) smem = max(smem, span_g);
-            whole = (co ? 1 : 0) | (cg ? 2 : 0);
-        }
-        VN_REQUIRE(smem <= 200 * 1024, "gather(bulk): %d bytes of planes per env exceed shared memory", smem);
-        static int configured[kMaxDevices] = {0};  // the attribute is per device
-        const int dev = current_device();
-        if (smem > configured[dev]) {
-            cudaFuncSetAttribute(vn_gather_bulk_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
-            configured[dev] = smem;
-        }
-        int per_sm = max(1, min(32, (220 * 1024) / (smem + 1024)));
-        if (env_per_sm > 0) per_sm = min(per_sm, env_per_sm);
-        int grid = (int)min((int64_t)gp.n * split, (int64_t)sm_count() * per_sm);
-        static const int env_grid = getenv("VN_BULK_GRID") ? atoi(getenv("VN_BULK_GRID")) : 0;   // development
-        if (env_grid > 0) grid = min(grid, env_grid);
-        // guided scheduling: the last wave's worth of envs in `tail` slices each (development knob, default off = 1)
-        static const int env_tail = getenv("VN_BULK_TAIL_SPLIT") ? atoi(getenv("VN_BULK_TAIL_SPLIT")) : VN_BULK_TAIL_DEFAULT;
-        static const int env_tail_waves16 = getenv("VN_BULK_TAIL_WAVES16") ? atoi(getenv("VN_BULK_TAIL_WAVES16")) : 16;
-        if (split == 1 && env_tail > 1 && gp.n > 2 * grid) {
-            n_whole = gp.n - min(gp.n, grid * env_tail_waves16 / 16);
-            k_split = min(env_tail, 8);
-        }
-        launch_pdl(vn_gather_bulk_kernel, dim3(grid), dim3(32), (size_t)smem, stream, gp, k_split, n_whole,
-                   (env_dynamic && gp.sched) ? gp.sched + (gp.parity & 1) : nullptr, env_hints | (whole << 16));
-        return check_launch("vn_gather_bulk_kernel");
+    if (variant != VN_GATHER_BULK) {
+        set_error("gather: unknown variant %d", variant);
+        return VN_EINVAL;
     }
-    set_error("gather: unknown variant %d", variant);
-    return VN_EINVAL;
+    // small batches (C1: 16 envs) cannot fill 148 SMs with one record per CTA: cut each record into
+    // slices until there are ~2 units per SM (latency-bound regime; one slice >= 2 KB)
+    int split = gp.n < 2 * sm_count() ? min(16, (2 * sm_count() + gp.n - 1) / gp.n) : 1;
+    // large records (the reference's native 174 x 174 frames: 212 KB for rgb + depth + segmentation) are
+    // cut into slices of at most 52 KB so that at least 4 CTAs stay resident per SM (84 x 84 rgb + depth +
+    // segmentation = 49.6 KB stays whole: one load per record instead of two slices of three)
+    int per_env = 0, per_goal = 0;
+    for (int pl = 0; pl < gp.store.n_planes; ++pl) {
+        if (gp.obs[pl]) per_env += gp.store.plane_bytes[pl];
+        if (gp.goal && gp.goal_obs[pl]) per_goal += gp.store.plane_bytes[pl];
+    }
+    split = max(split, (max(per_env, per_goal) + 52 * 1024 - 1) / (52 * 1024));
+    int smem_obs = 0, smem_goal = 0;
+    for (int pl = 0; pl < gp.store.n_planes; ++pl) {
+        const int n16 = gp.store.plane_bytes[pl] >> 4, per = (n16 + split - 1) / split;
+        if (gp.obs[pl]) smem_obs += per << 4;
+        if (gp.goal && gp.goal_obs[pl]) smem_goal += per << 4;
+    }
+    int smem = max(smem_obs, smem_goal), whole = 0;
+    if (split == 1) {
+        int span_o, span_g;
+        bool co, cg;
+        plane_set_bytes(gp.store, gp.obs, true, &span_o, &co);
+        plane_set_bytes(gp.store, gp.goal_obs, gp.goal != nullptr, &span_g, &cg);
+        if (co) smem = max(smem, span_o);
+        if (cg) smem = max(smem, span_g);
+        whole = (co ? 1 : 0) | (cg ? 2 : 0);
+    }
+    VN_REQUIRE(smem <= 200 * 1024, "gather(bulk): %d bytes of planes per env exceed shared memory", smem);
+    rc = ensure_smem(vn_gather_bulk_kernel, smem);
+    if (rc) return rc;
+    const int grid = (int)min((int64_t)gp.n * split, (int64_t)sm_count() * ctas_per_sm(smem));
+    return launch(vn_gather_bulk_kernel, "vn_gather_bulk_kernel", dim3(grid), dim3(32), (size_t)smem, stream, true, gp,
+                  split, gp.sched ? gp.sched + (gp.parity & 1) : nullptr, whole);
 }
 
 static int32_t make_step_params(StepParams &sp, const vn_tables_t *tab, const vn_envs_t *envs, const vn_rules_t *rules,
@@ -1031,14 +947,9 @@ static int32_t run_scalar(const vn_tables_t *tab, const vn_envs_t *envs, const v
     StepParams sp;
     int32_t rc = make_step_params(sp, tab, envs, rules, inj, actions, mask, out, reset, actions_copy);
     if (rc) return rc;
-    const int threads = kStepThreads;
-    const int blocks = (envs->n_envs + threads - 1) / threads;
-    cudaStream_t st = static_cast<cudaStream_t>(stream);
-    if (reset)
-        launch_pdl(vn_step_kernel<true>, dim3(blocks), dim3(threads), 0, st, sp);
-    else
-        launch_pdl(vn_step_kernel<false>, dim3(blocks), dim3(threads), 0, st, sp);
-    return check_launch("vn_step_kernel");
+    const int blocks = (envs->n_envs + kStepThreads - 1) / kStepThreads;
+    return launch(reset ? vn_step_kernel<true> : vn_step_kernel<false>, "vn_step_kernel", dim3(blocks),
+                  dim3(kStepThreads), 0, static_cast<cudaStream_t>(stream), true, sp);
 }
 
 // *any = whether there is anything to gather at all
@@ -1081,8 +992,6 @@ static int32_t run_gather(const vn_store_t *store, const vn_envs_t *envs, const 
     int32_t rc = make_gather_params(gp, store, envs, out, &any);
     if (rc) return rc;
     if (!any) return VN_OK;
-    if (variant == VN_GATHER_FUSED || variant == VN_GATHER_PERSISTENT)
-        variant = VN_GATHER_BULK;  // the halves were requested separately
     return launch_gather(gp, variant, static_cast<cudaStream_t>(stream));
 }
 
@@ -1105,28 +1014,13 @@ static int32_t run_fused(const vn_store_t *store, const vn_tables_t *tab, const 
     GatherParams gp;
     bool any = false;
     rc = make_gather_params(gp, store, envs, out, &any);
+    if (!rc) rc = check_rows_aligned(gp);
     if (rc) return rc;
-    for (int pl = 0; pl < gp.store.n_planes; ++pl) {
-        VN_REQUIRE(!gp.obs[pl] || (reinterpret_cast<uintptr_t>(gp.obs[pl]) & 15) == 0,
-                   "gather: obs[%d] must be 16-byte aligned", pl);
-        VN_REQUIRE(!gp.goal_obs[pl] || (reinterpret_cast<uintptr_t>(gp.goal_obs[pl]) & 15) == 0,
-                   "gather: goal_obs[%d] must be 16-byte aligned", pl);
-    }
-    static int configured[kMaxDevices][2] = {{0, 0}};  // the attribute is per device and per instantiation
-    const int dev = current_device();
-    if (smem > configured[dev][reset]) {
-        if (reset)
-            cudaFuncSetAttribute(vn_step_fused_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
-        else
-            cudaFuncSetAttribute(vn_step_fused_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
-        configured[dev][reset] = smem;
-    }
-    cudaStream_t st = static_cast<cudaStream_t>(stream);
-    if (reset)
-        launch_pdl(vn_step_fused_kernel<true>, dim3(envs->n_envs), dim3(kFusedWarps * 32), (size_t)smem, st, sp, gp);
-    else
-        launch_pdl(vn_step_fused_kernel<false>, dim3(envs->n_envs), dim3(kFusedWarps * 32), (size_t)smem, st, sp, gp);
-    return check_launch("vn_step_fused_kernel");
+    const auto kernel = reset ? vn_step_fused_kernel<true> : vn_step_fused_kernel<false>;
+    rc = ensure_smem(kernel, smem);
+    if (rc) return rc;
+    return launch(kernel, "vn_step_fused_kernel", dim3(envs->n_envs), dim3(kFusedWarps * 32), (size_t)smem,
+                  static_cast<cudaStream_t>(stream), true, sp, gp);
 }
 
 // Shared memory of one CTA of the persistent single launch (largest of the observation / goal plane sets), or 0 when
@@ -1155,37 +1049,16 @@ static int32_t run_persistent(const vn_store_t *store, const vn_tables_t *tab, c
     GatherParams gp;
     bool any = false;
     rc = make_gather_params(gp, store, envs, out, &any);
+    if (!rc) rc = check_rows_aligned(gp);
     if (rc) return rc;
-    for (int pl = 0; pl < gp.store.n_planes; ++pl) {
-        VN_REQUIRE(!gp.obs[pl] || (reinterpret_cast<uintptr_t>(gp.obs[pl]) & 15) == 0,
-                   "gather: obs[%d] must be 16-byte aligned", pl);
-        VN_REQUIRE(!gp.goal_obs[pl] || (reinterpret_cast<uintptr_t>(gp.goal_obs[pl]) & 15) == 0,
-                   "gather: goal_obs[%d] must be 16-byte aligned", pl);
-    }
-    static int configured[kMaxDevices][2] = {{0, 0}};
-    const int dev = current_device();
-    if (smem > configured[dev][reset]) {
-        if (reset)
-            cudaFuncSetAttribute(vn_step_gather_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
-        else
-            cudaFuncSetAttribute(vn_step_gather_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
-        configured[dev][reset] = smem;
-    }
+    const auto kernel = reset ? vn_step_gather_kernel<true> : vn_step_gather_kernel<false>;
+    rc = ensure_smem(kernel, smem);
+    if (rc) return rc;
     int whole = 0;
     persistent_smem_bytes(store, out, &whole);
-    static const int env_per_sm = getenv("VN_BULK_PER_SM") ? atoi(getenv("VN_BULK_PER_SM")) : 0;
-    static const int env_groups = getenv("VN_BULK_GROUPS") ? atoi(getenv("VN_BULK_GROUPS")) : VN_BULK_GROUPS_DEFAULT;
-    static const int env_hints =
-        (getenv("VN_BULK_L2_HINTS") ? atoi(getenv("VN_BULK_L2_HINTS")) : 3) | (max(1, min(7, env_groups)) << 8);
-    int per_sm = max(1, min(32, (220 * 1024) / (smem + 1024)));
-    if (env_per_sm > 0) per_sm = min(per_sm, env_per_sm);
-    const int grid = (int)min((int64_t)envs->n_envs, (int64_t)sm_count() * per_sm);
-    cudaStream_t st = static_cast<cudaStream_t>(stream);
-    if (reset)
-        launch_pdl(vn_step_gather_kernel<true>, dim3(grid), dim3(32), (size_t)smem, st, sp, gp, env_hints | (whole << 16));
-    else
-        launch_pdl(vn_step_gather_kernel<false>, dim3(grid), dim3(32), (size_t)smem, st, sp, gp, env_hints | (whole << 16));
-    return check_launch("vn_step_gather_kernel");
+    const int grid = (int)min((int64_t)envs->n_envs, (int64_t)sm_count() * ctas_per_sm(smem));
+    return launch(kernel, "vn_step_gather_kernel", dim3(grid), dim3(32), (size_t)smem, static_cast<cudaStream_t>(stream),
+                  true, sp, gp, whole);
 }
 
 enum StepMode { kModeError = -1, kModeSplit = 0, kModeFused = 1, kModePersistent = 2 };
@@ -1199,8 +1072,6 @@ static StepMode choose_mode(const vn_store_t *store, const vn_envs_t *envs, cons
 // -1: error already set; 0: two launches; > 0: fused, shared memory bytes
 static int32_t choose_fused(const vn_store_t *store, const vn_envs_t *envs, const vn_step_out_t *out, int32_t variant) {
     if (variant != VN_GATHER_FUSED && variant != VN_GATHER_AUTO) return 0;
-    static const bool off = getenv("VN_NO_FUSED") && atoi(getenv("VN_NO_FUSED"));
-    if (off && variant == VN_GATHER_AUTO) return 0;
     if (!out) return 0;  // reported by the parameter checks
     const int32_t smem = fused_smem_bytes(store, out);
     if (smem < 0) {
@@ -1209,13 +1080,8 @@ static int32_t choose_fused(const vn_store_t *store, const vn_envs_t *envs, cons
                   (long long)store->state_pitch);
         return -1;
     }
-    if (variant == VN_GATHER_AUTO) {
-        // one wave of CTAs: as many envs as fit at once (shared memory bound), at most 4 per SM - beyond that the
-        // step is no longer bound by launch latency and the two-kernel path (pipelined, bandwidth-tuned) wins
-        static const int env_waves = getenv("VN_FUSED_PER_SM") ? atoi(getenv("VN_FUSED_PER_SM")) : 4;
-        const int per_sm = max(1, min(env_waves, (220 * 1024) / (smem + 1024)));
-        if (envs->n_envs > sm_count() * per_sm) return 0;
-    }
+    // one wave of CTAs: as many envs as fit at once, at most kFusedPerSm per SM
+    if (variant == VN_GATHER_AUTO && envs->n_envs > sm_count() * ctas_per_sm(smem, kFusedPerSm)) return 0;
     return smem;
 }
 
@@ -1259,15 +1125,11 @@ static StepMode choose_mode(const vn_store_t *store, const vn_envs_t *envs, cons
         // A HOST caller (out->host_pack) always takes two kernels: the stepping phase of a persistent grid cannot become
         // resident before the previous launch's CTAs release their shared memory, so the host would get its rewards a
         // whole gather late, and lanes that own strided envs read / write the mapped host buffers 4 bytes at a time.
-        // VN_PERSISTENT=0 / 2 (development): never / whenever the batch qualifies.
-        static const int env_persistent = getenv("VN_PERSISTENT") ? atoi(getenv("VN_PERSISTENT")) : VN_PERSISTENT_DEFAULT;
-        const int32_t ps = env_persistent ? persistent_smem_bytes(store, out) : 0;
+        const int32_t ps = persistent_smem_bytes(store, out);
         if (ps > 0) {
-            const int per_sm = max(1, min(32, (220 * 1024) / (ps + 1024)));
-            const int64_t wave = (int64_t)sm_count() * per_sm, n = envs->n_envs;
+            const int64_t wave = (int64_t)sm_count() * ctas_per_sm(ps), n = envs->n_envs;
             const bool pipelined = (out->flags & VN_STEP_ACTIONS_READY) != 0;
-            const bool mid_size = !out->host_pack && (pipelined ? 4 * n <= 3 * wave : n <= 4 * wave);
-            if (env_persistent >= 2 || mid_size) {
+            if (!out->host_pack && (pipelined ? 4 * n <= 3 * wave : n <= 4 * wave)) {
                 *smem = ps;
                 return kModePersistent;
             }
@@ -1365,8 +1227,8 @@ int32_t vn_fill_store(const vn_store_t *store, int32_t record0, int32_t n_record
     const int64_t total = (store->state_pitch >> 3) * n_records;
     const int blocks = (int)((total + 255) / 256 < (int64_t)vn::sm_count() * 32 ? (total + 255) / 256
                                                                                  : (int64_t)vn::sm_count() * 32);
-    vn::vn_fill_kernel<<<blocks, 256, 0, static_cast<cudaStream_t>(stream)>>>(fp);
-    return vn::check_launch("vn_fill_kernel");
+    return vn::launch(vn::vn_fill_kernel, "vn_fill_kernel", dim3(blocks), dim3(256), 0, static_cast<cudaStream_t>(stream),
+                      false, fp);
 }
 
 int32_t vn_env_reset(const vn_store_t *store, const vn_tables_t *tables, const vn_envs_t *envs,

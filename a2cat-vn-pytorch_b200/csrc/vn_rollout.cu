@@ -3,19 +3,6 @@
 // and the fused gather -> float32 CHW conversion for the policy input.
 #include "vn_common.cuh"
 
-// cudaFuncAttributeMaxDynamicSharedMemorySize is a per-device attribute: remember the largest request per device
-#define VN_ENSURE_SMEM(kernel, bytes)                                                              \
-    do {                                                                                           \
-        static int configured_[64] = {0};                                                          \
-        int dev_ = 0;                                                                              \
-        cudaGetDevice(&dev_);                                                                      \
-        dev_ = (dev_ >= 0 && dev_ < 64) ? dev_ : 0;                                                \
-        if ((bytes) > configured_[dev_]) {                                                         \
-            cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (bytes));    \
-            configured_[dev_] = (bytes);                                                           \
-        }                                                                                          \
-    } while (0)
-
 namespace vn {
 
 // Programmatic dependent launch inside a builder CHAIN (several kernels enqueued by one C call): every kernel waits for
@@ -25,22 +12,6 @@ namespace vn {
 __device__ __forceinline__ void chain_wait(int release_successor) {
     asm volatile("griddepcontrol.wait;" ::: "memory");
     if (release_successor) asm volatile("griddepcontrol.launch_dependents;" ::: "memory");
-}
-
-template <typename... KArgs, typename... Args>
-static cudaError_t launch_chain(void (*kernel)(KArgs...), dim3 grid, dim3 block, size_t smem, cudaStream_t stream,
-                                Args... args) {
-    cudaLaunchConfig_t cfg = {};
-    cfg.gridDim = grid;
-    cfg.blockDim = block;
-    cfg.dynamicSmemBytes = smem;
-    cfg.stream = stream;
-    cudaLaunchAttribute attr[1];
-    attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-    attr[0].val.programmaticStreamSerializationAllowed = 1;
-    cfg.attrs = attr;
-    cfg.numAttrs = 1;
-    return cudaLaunchKernelEx(&cfg, kernel, static_cast<KArgs>(args)...);
 }
 
 // =====================================================================================================
@@ -813,12 +784,12 @@ static int32_t pool_geom(int h, int w, int c, int cell, int out_h, int out_w, Po
 static int32_t launch_pc_list(const vn_store_t *store, int plane, const int32_t *states, int t, int64_t sn, int64_t st,
                               const PoolGeom &g, const int32_t *pos, const int32_t *count, int max_count, int compact,
                               float *out, int smem, int per_sm, cudaStream_t stream, bool chained) {
-    VN_ENSURE_SMEM(vn_pixel_control_list_kernel, smem);
+    int32_t rc = ensure_smem(vn_pixel_control_list_kernel, smem);
+    if (rc) return rc;
     const int want = sm_count() * (per_sm < 4 ? per_sm : 4);
     const int grid = max_count < want ? max_count : want;
-    launch_chain(vn_pixel_control_list_kernel, dim3(grid), dim3(512), (size_t)smem, stream, *store, plane, states, t, sn,
-                 st, g, pos, count, max_count, compact, out, chained ? 1 : 0);
-    return check_launch("vn_pixel_control_list_kernel");
+    return launch(vn_pixel_control_list_kernel, "vn_pixel_control_list_kernel", dim3(grid), dim3(512), (size_t)smem,
+                  stream, true, *store, plane, states, t, sn, st, g, pos, count, max_count, compact, out, chained ? 1 : 0);
 }
 
 }  // namespace vn
@@ -931,27 +902,25 @@ int32_t vn_pixel_control_returns_from_states(const vn_store_t *store, int32_t pl
     // time-major `rows` costs the back-up kernel: there every step's row index is a dependent load in front of the table
     // load, and batch-major keeps an env's T indices in one or two cache lines - 42 vs 58 us at 4,096 x 20)
     const int64_t rsn = t, rst = 1;
-    vn::launch_chain(vn::vn_transition_rows_kernel, dim3((unsigned)((total + 255) / 256)), dim3(256), 0, st, adj, states, n,
-                     t, state_stride_n, state_stride_t, rsn, rst, rows, miss_pos, miss_count, 1);
-    rc = vn::check_launch("vn_transition_rows_kernel");
+    rc = vn::launch(vn::vn_transition_rows_kernel, "vn_transition_rows_kernel", dim3((unsigned)((total + 255) / 256)),
+                    dim3(256), 0, st, true, adj, states, n, t, state_stride_n, state_stride_t, rsn, rst, rows, miss_pos,
+                    miss_count, 1);
     if (rc) return rc;
     // (2) the misses computed directly from their two frames into the compact side buffer
     const int fb = (h * w * c + 15) & ~15;
     const int smem = 2 * fb;
     VN_REQUIRE(smem <= 220 * 1024, "pixel_control_returns: frame too large for shared memory");
-    const int per_sm = (220 * 1024) / (smem + 1024) < 1 ? 1 : (220 * 1024) / (smem + 1024);
     rc = vn::launch_pc_list(store, plane, states, t, state_stride_n, state_stride_t, g, miss_pos, miss_count, max_miss, 1,
-                            miss_rows, smem, per_sm, st, true);
+                            miss_rows, smem, vn::ctas_per_sm(smem), st, true);
     if (rc) return rc;
     // (3) rewards gathered on the fly + discounted back-up
     const int d4 = cells >> 2;
     const int64_t threads = (int64_t)n * d4;
-    vn::launch_chain(vn::vn_pc_returns_kernel, dim3((unsigned)((threads + 255) / 256)), dim3(256), 0, st,
-                     reinterpret_cast<const float4 *>(pc_table), rows, rsn, rst,
-                     reinterpret_cast<const float4 *>(miss_rows), done, done_stride_n, done_stride_t,
-                     reinterpret_cast<const float4 *>(bootstrap), gamma, n, t, d4,
-                     reinterpret_cast<float4 *>(out_returns), reinterpret_cast<float4 *>(out_reward), miss_count);
-    return vn::check_launch("vn_pc_returns_kernel");
+    return vn::launch(vn::vn_pc_returns_kernel, "vn_pc_returns_kernel", dim3((unsigned)((threads + 255) / 256)), dim3(256),
+                      0, st, true, reinterpret_cast<const float4 *>(pc_table), rows, rsn, rst,
+                      reinterpret_cast<const float4 *>(miss_rows), done, done_stride_n, done_stride_t,
+                      reinterpret_cast<const float4 *>(bootstrap), gamma, n, t, d4,
+                      reinterpret_cast<float4 *>(out_returns), reinterpret_cast<float4 *>(out_reward), miss_count);
 }
 
 int32_t vn_pixel_control(const vn_store_t *store, int32_t plane, const int32_t *states, int32_t n, int32_t t,
@@ -968,7 +937,8 @@ int32_t vn_pixel_control(const vn_store_t *store, int32_t plane, const int32_t *
     const int fb = (h * w * c + 15) & ~15;
     const int smem = 2 * fb;
     VN_REQUIRE(smem <= 220 * 1024, "pixel_control: frame too large for shared memory");
-    VN_ENSURE_SMEM(vn::vn_pixel_control_kernel<kChunk>, smem);
+    rc = vn::ensure_smem(vn::vn_pixel_control_kernel<kChunk>, smem);
+    if (rc) return rc;
     const int64_t blocks = (int64_t)n * ((t + kChunk - 1) / kChunk);
     VN_REQUIRE(blocks < (1ll << 31), "pixel_control: too many blocks");
     vn::vn_pixel_control_kernel<kChunk><<<(unsigned)blocks, 256, smem, static_cast<cudaStream_t>(stream)>>>(
@@ -1021,10 +991,8 @@ int32_t vn_pixel_control_list(const vn_store_t *store, int32_t plane, const int3
     const int fb = (h * w * c + 15) & ~15;
     const int smem = 2 * fb;
     VN_REQUIRE(smem <= 220 * 1024, "pixel_control_list: frame too large for shared memory");
-    VN_ENSURE_SMEM(vn::vn_pixel_control_list_kernel, smem);
-    const int per_sm = (220 * 1024) / (smem + 1024) < 8 ? ((220 * 1024) / (smem + 1024) < 1 ? 1 : (220 * 1024) / (smem + 1024)) : 8;
     return vn::launch_pc_list(store, plane, states, t, state_stride_n, state_stride_t, g, pos, count, max_count, compact, out,
-                              smem, per_sm, static_cast<cudaStream_t>(stream), false);
+                              smem, vn::ctas_per_sm(smem, 8), static_cast<cudaStream_t>(stream), false);
 }
 
 int32_t vn_replay_sample(const vn_replay_t *ring, int32_t length, int32_t mode, uint64_t seed, uint32_t call,
@@ -1079,7 +1047,8 @@ int32_t vn_aux_target(const vn_store_t *store, int32_t plane, const int32_t *idx
     if (m == 0) return VN_OK;
     const int smem = (h * w * c + 15) & ~15;
     VN_REQUIRE(smem <= 220 * 1024, "aux_target: frame too large for shared memory");
-    VN_ENSURE_SMEM(vn::vn_aux_target_kernel, smem);
+    rc = vn::ensure_smem(vn::vn_aux_target_kernel, smem);
+    if (rc) return rc;
     const int grid = m < vn::sm_count() * 8 ? m : vn::sm_count() * 8;
     vn::vn_aux_target_kernel<<<grid, 256, smem, static_cast<cudaStream_t>(stream)>>>(*store, plane, idx, m, g, out);
     return vn::check_launch("vn_aux_target_kernel");
@@ -1113,7 +1082,8 @@ int32_t vn_gather_plane_f32_chw_rows(const vn_store_t *store, int32_t plane, con
     }
     const int smem = (h * w * c + 15) & ~15;
     VN_REQUIRE(smem <= 220 * 1024, "gather_plane_f32_chw: frame too large for shared memory");
-    VN_ENSURE_SMEM(vn::vn_gather_f32_chw_kernel, smem);
+    rc = vn::ensure_smem(vn::vn_gather_f32_chw_kernel, smem);
+    if (rc) return rc;
     const int grid = n < vn::sm_count() * 8 ? n : vn::sm_count() * 8;
     vn::vn_gather_f32_chw_kernel<<<grid, 256, smem, static_cast<cudaStream_t>(stream)>>>(*store, plane, idx, idx_stride,
                                                                                         n, h, w, c, out);
@@ -1164,25 +1134,12 @@ int32_t launch_float_leaves(const vn_store_t *store, const vn_float_leaf_t *leav
     const int2 *d2 = reinterpret_cast<const int2 *>(desc);
     const int64_t pitch = store->state_pitch;
     const int hw = h * w, early = in_step ? 1 : 0;
+    void (*const kernels[])(FloatLeaves, int64_t, const int2 *, int, int, int) = {
+        vn_gather_leaves_f32_kernel<1, 4>, vn_gather_leaves_f32_kernel<2, 2>, vn_gather_leaves_f32_kernel<3, 2>,
+        vn_gather_leaves_f32_kernel<4, 1>, vn_gather_leaves_f32_kernel<5, 1>, vn_gather_leaves_f32_kernel<6, 1>};
     // programmatic launch only as part of a step: there the predecessor is the step's own scalar / gather kernel
-    cudaLaunchConfig_t cfg = {};
-    cfg.gridDim = dim3(grid);
-    cfg.blockDim = dim3(256);
-    cfg.stream = static_cast<cudaStream_t>(stream);
-    cudaLaunchAttribute attr[1];
-    attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-    attr[0].val.programmaticStreamSerializationAllowed = 1;
-    cfg.attrs = attr;
-    cfg.numAttrs = in_step ? 1 : 0;
-    switch (n_leaves) {
-        case 1: cudaLaunchKernelEx(&cfg, vn_gather_leaves_f32_kernel<1, 4>, L, pitch, d2, n, hw, early); break;
-        case 2: cudaLaunchKernelEx(&cfg, vn_gather_leaves_f32_kernel<2, 2>, L, pitch, d2, n, hw, early); break;
-        case 3: cudaLaunchKernelEx(&cfg, vn_gather_leaves_f32_kernel<3, 2>, L, pitch, d2, n, hw, early); break;
-        case 4: cudaLaunchKernelEx(&cfg, vn_gather_leaves_f32_kernel<4, 1>, L, pitch, d2, n, hw, early); break;
-        case 5: cudaLaunchKernelEx(&cfg, vn_gather_leaves_f32_kernel<5, 1>, L, pitch, d2, n, hw, early); break;
-        default: cudaLaunchKernelEx(&cfg, vn_gather_leaves_f32_kernel<6, 1>, L, pitch, d2, n, hw, early); break;
-    }
-    return check_launch("vn_gather_leaves_f32_kernel");
+    return launch(kernels[n_leaves - 1], "vn_gather_leaves_f32_kernel", dim3(grid), dim3(256), 0,
+                  static_cast<cudaStream_t>(stream), in_step, L, pitch, d2, n, hw, early);
 }
 
 }  // namespace vn
@@ -1202,21 +1159,17 @@ int32_t vn_rp_labels(const float *reward, int32_t n, int32_t t, int64_t stride_n
     if (n == 0) return VN_OK;
     cudaStream_t st = static_cast<cudaStream_t>(stream);
     const int blocks = (n + vn::kRpBlock - 1) / vn::kRpBlock;
-    vn::launch_chain(vn::vn_rp_count_kernel, dim3(blocks), dim3(vn::kRpBlock), 0, st, reward, n, t, stride_n, stride_t,
-                     labels, scratch);
-    vn::check_launch("vn_rp_count_kernel");
-    if (blocks <= 256) {
-        // few blocks (an A2C rollout: 80 blocks at 4,096 envs x 20 steps): no separate scan launch
-        vn::launch_chain(vn::vn_rp_scatter_kernel, dim3(blocks), dim3(vn::kRpBlock), 0, st, reward, n, t, stride_n,
-                         stride_t, scratch, 0, counts, zero_idx, nonzero_idx);
-        return vn::check_launch("vn_rp_scatter_kernel");
-    }
-    vn::launch_chain(vn::vn_rp_scan_kernel, dim3(1), dim3(1024), 0, st, scratch, blocks, n, counts);
-    vn::check_launch("vn_rp_scan_kernel");
-    if (zero_idx || nonzero_idx)
-        vn::launch_chain(vn::vn_rp_scatter_kernel, dim3(blocks), dim3(vn::kRpBlock), 0, st, reward, n, t, stride_n,
-                         stride_t, scratch, 1, (int32_t *)nullptr, zero_idx, nonzero_idx);
-    return vn::check_launch("vn_rp_labels");
+    int32_t rc = vn::launch(vn::vn_rp_count_kernel, "vn_rp_count_kernel", dim3(blocks), dim3(vn::kRpBlock), 0, st, true,
+                            reward, n, t, stride_n, stride_t, labels, scratch);
+    if (rc) return rc;
+    if (blocks <= 256)  // few blocks (an A2C rollout: 80 blocks at 4,096 envs x 20 steps): no separate scan launch
+        return vn::launch(vn::vn_rp_scatter_kernel, "vn_rp_scatter_kernel", dim3(blocks), dim3(vn::kRpBlock), 0, st, true,
+                          reward, n, t, stride_n, stride_t, scratch, 0, counts, zero_idx, nonzero_idx);
+    rc = vn::launch(vn::vn_rp_scan_kernel, "vn_rp_scan_kernel", dim3(1), dim3(1024), 0, st, true, scratch, blocks, n,
+                    counts);
+    if (rc || !(zero_idx || nonzero_idx)) return rc;
+    return vn::launch(vn::vn_rp_scatter_kernel, "vn_rp_scatter_kernel", dim3(blocks), dim3(vn::kRpBlock), 0, st, true,
+                      reward, n, t, stride_n, stride_t, scratch, 1, (int32_t *)nullptr, zero_idx, nonzero_idx);
 }
 
 }  // extern "C"

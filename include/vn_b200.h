@@ -15,8 +15,11 @@
  *     marked [host]; the descriptor structs themselves are read on the host during the call.
  *   - no allocation, no implicit synchronisation: kernels are enqueued on the caller's
  *     cudaStream_t (passed as void*; NULL = legacy default stream) and the call returns.
- *   - re-entrant: there is no global state apart from the thread-local error string and a launch
- *     counter kept for statistics (vn_launch_count).
+ *   - re-entrant.  The global state is: the thread-local error string, a launch counter kept for
+ *     statistics (vn_launch_count), the development trace buffer of vn_debug_gather_trace, per-device
+ *     caches of the SM count and of the dynamic shared-memory limit set on each kernel, and a
+ *     per-thread cache of host pointers already found pinned and device-mapped.  No environment
+ *     variable is read: how a call runs follows from its arguments and the device alone.
  *
  * State numbering: oriented scenes use state = free_cell_rank * 4 + rotation (the numbering of
  * graph/util.py:208-210,229-237 save_graph_as_h5), un-oriented ones state = free_cell_rank; with
