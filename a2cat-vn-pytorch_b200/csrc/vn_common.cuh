@@ -17,8 +17,11 @@ namespace vn {
 void set_error(const char *fmt, ...);
 // Counts a kernel launch whose enqueue returned `e`; VN_ECUDA with `what` in vn_last_error when it failed.
 int32_t launch_result(const char *what, cudaError_t e);
-// The same for a launch written as kernel<<<...>>>, which reports through cudaGetLastError.
-inline int32_t check_launch(const char *what) { return launch_result(what, cudaGetLastError()); }
+// Whether every pointer is 16-byte aligned (a null pointer is).
+template <typename... P>
+inline bool aligned16(const P *...p) {
+    return ((reinterpret_cast<uintptr_t>(p) | ... | uintptr_t(0)) & 15) == 0;
+}
 int sm_count();  // multiprocessors of the current device (cached per device)
 // Raises the kernel's dynamic shared-memory limit on the current device to `bytes` unless an earlier call did; a size
 // is remembered only once the attribute was set.  VN_ECUDA with a message when it cannot be set.

@@ -832,10 +832,8 @@ int32_t ensure_smem(const void *kernel, int bytes) {
 
 static int32_t check_rows_aligned(const GatherParams &gp) {
     for (int pl = 0; pl < gp.store.n_planes; ++pl) {
-        VN_REQUIRE(!gp.obs[pl] || (reinterpret_cast<uintptr_t>(gp.obs[pl]) & 15) == 0,
-                   "gather: obs[%d] must be 16-byte aligned", pl);
-        VN_REQUIRE(!gp.goal_obs[pl] || (reinterpret_cast<uintptr_t>(gp.goal_obs[pl]) & 15) == 0,
-                   "gather: goal_obs[%d] must be 16-byte aligned", pl);
+        VN_REQUIRE(aligned16(gp.obs[pl]), "gather: obs[%d] must be 16-byte aligned", pl);
+        VN_REQUIRE(aligned16(gp.goal_obs[pl]), "gather: goal_obs[%d] must be 16-byte aligned", pl);
     }
     return VN_OK;
 }

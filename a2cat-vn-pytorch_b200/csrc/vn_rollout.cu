@@ -127,53 +127,68 @@ struct PoolGeom {
     int h, w, c, cell, out_h, out_w, top, left;
 };
 
-// out[cell] = mean_c avg_pool_cell(|nxt/255 - cur/255|) for one transition; frames and LUT in shared memory
+// F.avg_pool2d's window sum for output cell (oi, oj) of channel ch: value(byte offset of the pixel in the HWC frame)
+// summed in row-major order
+template <typename Value>
+__device__ __forceinline__ float window_sum(const PoolGeom &g, int oi, int oj, int ch, Value value) {
+    const int row_bytes = g.w * g.c;
+    float acc = 0.f;
+    for (int dy = 0; dy < g.cell; ++dy) {
+        const int rowoff = (g.top + oi * g.cell + dy) * row_bytes + (g.left + oj * g.cell) * g.c + ch;
+        for (int dx = 0; dx < g.cell; ++dx) acc = __fadd_rn(acc, value(rowoff + dx * g.c));
+    }
+    return acc;
+}
+
+// out[cell] = mean_c avg_pool_cell(|nxt/255 - cur/255|) for one transition; frames in shared memory
 __device__ __forceinline__ void pc_cells(const uint8_t *cur, const uint8_t *nxt, const PoolGeom &g,
                                          float *__restrict__ out_row) {
     const int cells = g.out_h * g.out_w;
-    const int row_bytes = g.w * g.c;
     for (int cidx = threadIdx.x; cidx < cells; cidx += blockDim.x) {
         const int oi = cidx / g.out_w, oj = cidx - oi * g.out_w;
         float chan_sum = 0.f;
         for (int ch = 0; ch < g.c; ++ch) {
-            float acc = 0.f;  // F.avg_pool2d: window sum in row-major order, then / cell^2
-            for (int dy = 0; dy < g.cell; ++dy) {
-                const int rowoff = (g.top + oi * g.cell + dy) * row_bytes + (g.left + oj * g.cell) * g.c + ch;
-                for (int dx = 0; dx < g.cell; ++dx) {
-                    const float a = u8_over_255(nxt[rowoff + dx * g.c]);
-                    const float b = u8_over_255(cur[rowoff + dx * g.c]);
-                    acc = __fadd_rn(acc, fabsf(__fsub_rn(a, b)));
-                }
-            }
+            const float acc = window_sum(g, oi, oj, ch, [&](int at) {
+                return fabsf(__fsub_rn(u8_over_255(nxt[at]), u8_over_255(cur[at])));
+            });
             chan_sum = __fadd_rn(chan_sum, __fdiv_rn(acc, (float)(g.cell * g.cell)));
         }
         out_row[cidx] = __fdiv_rn(chan_sum, (float)g.c);  // mean over channels
     }
 }
 
+// The two frames a pixel-control CTA stages in shared memory: frame 1 starts at the 16-byte boundary after frame 0
+struct TwoFrames {
+    uint8_t *f0, *f1;
+    int bytes;
+};
+__device__ __forceinline__ TwoFrames two_frames(uint8_t *smem, const PoolGeom &g) {
+    const int bytes = g.h * g.w * g.c;
+    return {smem, smem + ((bytes + 15) & ~15), bytes};
+}
+
 // CTA per (env n, chunk of time steps).  Frames of consecutive steps are kept in a 2-slot shared ring so
-// each frame is read from HBM/L2 once per chunk: (chunk + 1) / chunk reads per output.
+// each frame is read from HBM/L2 once per chunk: (chunk + 1) / chunk reads per output.  8 CTAs per SM caps ptxas at
+// 32 registers, which it reaches without spills; left free it takes 40 and runs slower (B200, 1,000 W: 131.8 vs
+// 122.5 us for tools/bench_targets.py's pixel_control_direct).
 template <int kChunk>
-__global__ void __launch_bounds__(256) vn_pixel_control_kernel(const vn_store_t store, int plane,
-                                                               const int32_t *__restrict__ states, int n, int t,
-                                                               int64_t sn, int64_t st, PoolGeom g,
-                                                               float *__restrict__ out) {
+__global__ void __launch_bounds__(256, 8) vn_pixel_control_kernel(const uint8_t *__restrict__ pbase,
+                                                                  int64_t pitch, const int32_t *__restrict__ states,
+                                                                  int n, int t, int64_t sn, int64_t st, PoolGeom g,
+                                                                  float *__restrict__ out) {
     extern __shared__ __align__(16) uint8_t smem_raw[];
-    const int fbytes = g.h * g.w * g.c;
-    uint8_t *frame0 = smem_raw;
-    uint8_t *frame1 = frame0 + ((fbytes + 15) & ~15);
+    const TwoFrames fr = two_frames(smem_raw, g);
     const int chunks = (t + kChunk - 1) / kChunk;
     const int env = blockIdx.x / chunks;
     const int k0 = (blockIdx.x - env * chunks) * kChunk;
     const int k1 = min(t, k0 + kChunk);
     const int32_t *srow = states + (int64_t)env * sn;   // observation k of this env lives at srow[k * st]
-    const uint8_t *pbase = store.base + store.plane_off[plane];
 
-    load_frame(frame0, pbase + (size_t)srow[(int64_t)k0 * st] * store.state_pitch, fbytes);
-    uint8_t *cur = frame0, *nxt = frame1;
+    load_frame(fr.f0, pbase + (size_t)srow[(int64_t)k0 * st] * pitch, fr.bytes);
+    uint8_t *cur = fr.f0, *nxt = fr.f1;
     const int cells = g.out_h * g.out_w;
     for (int k = k0; k < k1; ++k) {
-        load_frame(nxt, pbase + (size_t)srow[(int64_t)(k + 1) * st] * store.state_pitch, fbytes);
+        load_frame(nxt, pbase + (size_t)srow[(int64_t)(k + 1) * st] * pitch, fr.bytes);
         __syncthreads();
         pc_cells(cur, nxt, g, out + ((int64_t)env * t + k) * cells);
         __syncthreads();
@@ -186,31 +201,28 @@ __global__ void __launch_bounds__(256) vn_pixel_control_kernel(const vn_store_t 
 // Direct pixel-control reward for a device-resident LIST of transitions (the reset transitions that the
 // per-scene transition table cannot serve).  Persistent CTAs loop over the list; its length is read from
 // device memory, so no host synchronisation is needed between the lookup pass and this one.
-__global__ void __launch_bounds__(512) vn_pixel_control_list_kernel(const vn_store_t store, int plane,
-                                                                    const int32_t *__restrict__ states, int t,
-                                                                    int64_t sn, int64_t st, PoolGeom g,
+__global__ void __launch_bounds__(512) vn_pixel_control_list_kernel(const uint8_t *__restrict__ pbase,
+                                                                    int64_t pitch, const int32_t *__restrict__ states,
+                                                                    int t, int64_t sn, int64_t st, PoolGeom g,
                                                                     const int32_t *__restrict__ pos,
                                                                     const int32_t *__restrict__ count, int max_count,
                                                                     int compact, float *__restrict__ out, int chained) {
     extern __shared__ __align__(16) uint8_t smem_raw[];
     chain_wait(chained);
-    const int fbytes = g.h * g.w * g.c;
-    uint8_t *frame0 = smem_raw;
-    uint8_t *frame1 = frame0 + ((fbytes + 15) & ~15);
+    const TwoFrames fr = two_frames(smem_raw, g);
     const int m_total = min(*count, max_count);
     if ((int)blockIdx.x >= m_total) return;
-    const uint8_t *pbase = store.base + store.plane_off[plane];
     const int cells = g.out_h * g.out_w;
     for (int m = blockIdx.x; m < m_total; m += gridDim.x) {
         const int p = pos[m];
         const int env = p / t, k = p - env * t;
         const int32_t *srow = states + (int64_t)env * sn;
         __syncthreads();
-        load_frame(frame0, pbase + (size_t)srow[(int64_t)k * st] * store.state_pitch, fbytes);
-        load_frame(frame1, pbase + (size_t)srow[(int64_t)(k + 1) * st] * store.state_pitch, fbytes);
+        load_frame(fr.f0, pbase + (size_t)srow[(int64_t)k * st] * pitch, fr.bytes);
+        load_frame(fr.f1, pbase + (size_t)srow[(int64_t)(k + 1) * st] * pitch, fr.bytes);
         __syncthreads();
         // compact: row m of a side buffer (consumed by vn_pixel_control_returns); else row p of the [n][t] output
-        pc_cells(frame0, frame1, g, out + (int64_t)(compact ? m : p) * cells);
+        pc_cells(fr.f0, fr.f1, g, out + (int64_t)(compact ? m : p) * cells);
     }
 }
 
@@ -307,35 +319,31 @@ __global__ void __launch_bounds__(256) vn_gather_rows_kernel(const int4 *__restr
 }
 
 // CTA per gathered frame: out[m][c][out_h][out_w] = avg_pool(crop(frame / 255))
-__global__ void __launch_bounds__(256) vn_aux_target_kernel(const vn_store_t store, int plane,
+__global__ void __launch_bounds__(256) vn_aux_target_kernel(const uint8_t *__restrict__ pbase, int64_t pitch,
                                                             const int32_t *__restrict__ idx, int m, PoolGeom g,
                                                             float *__restrict__ out) {
     extern __shared__ __align__(16) uint8_t smem_raw[];
     const int fbytes = g.h * g.w * g.c;
-    uint8_t *frame = smem_raw;
+    const uint8_t *frame = smem_raw;
     const int cells = g.out_h * g.out_w;
-    const int row_bytes = g.w * g.c;
     for (int f = blockIdx.x; f < m; f += gridDim.x) {
         __syncthreads();
-        load_frame(frame, store.base + store.plane_off[plane] + (size_t)idx[f] * store.state_pitch, fbytes);
+        load_frame(smem_raw, pbase + (size_t)idx[f] * pitch, fbytes);
         __syncthreads();
         for (int o = threadIdx.x; o < cells * g.c; o += blockDim.x) {
             const int ch = o / cells, cidx = o - ch * cells;
             const int oi = cidx / g.out_w, oj = cidx - oi * g.out_w;
-            float acc = 0.f;
-            for (int dy = 0; dy < g.cell; ++dy) {
-                const int rowoff = (g.top + oi * g.cell + dy) * row_bytes + (g.left + oj * g.cell) * g.c + ch;
-                for (int dx = 0; dx < g.cell; ++dx) acc = __fadd_rn(acc, u8_over_255(frame[rowoff + dx * g.c]));
-            }
+            const float acc = window_sum(g, oi, oj, ch, [&](int at) { return u8_over_255(frame[at]); });
             out[(int64_t)f * cells * g.c + o] = __fdiv_rn(acc, (float)(g.cell * g.cell));
         }
     }
 }
 
 // gather + TransposeImage + ScaledFloatFrame: out[i][c][h][w] = float(frame[h][w][c]) / 255
-__global__ void __launch_bounds__(256) vn_gather_f32_chw_kernel(const vn_store_t store, int plane,
-                                                                const int32_t *__restrict__ idx, int idx_stride, int n,
-                                                                int h, int w, int c, float *__restrict__ out) {
+__global__ void __launch_bounds__(256) vn_gather_f32_chw_kernel(const uint8_t *__restrict__ pbase,
+                                                                int64_t pitch, const int32_t *__restrict__ idx,
+                                                                int idx_stride, int n, int h, int w, int c,
+                                                                float *__restrict__ out) {
     extern __shared__ __align__(16) uint8_t smem_raw[];
     const int fbytes = h * w * c;
     const int hw = h * w;
@@ -343,13 +351,31 @@ __global__ void __launch_bounds__(256) vn_gather_f32_chw_kernel(const vn_store_t
         const int rec = idx[(int64_t)f * idx_stride];
         if (rec < 0) continue;  // uniform over the block: row f keeps its content
         __syncthreads();
-        load_frame(smem_raw, store.base + store.plane_off[plane] + (size_t)rec * store.state_pitch, fbytes);
+        load_frame(smem_raw, pbase + (size_t)rec * pitch, fbytes);
         __syncthreads();
         float *o = out + (int64_t)f * fbytes;
         for (int k = threadIdx.x; k < fbytes; k += blockDim.x) {  // k indexes the CHW output: coalesced stores
             const int ch = k / hw, px = k - ch * hw;
             o[k] = __fdiv_rn((float)smem_raw[px * c + ch], 255.0f);
         }
+    }
+}
+
+// One group of 4 pixels as float32 CHW / 255: w holds the group's 4 * C bytes (pixel-major, channel-minor, as in the
+// HWC frame); one streaming 16-byte store per channel plane of the output, o pointing at the group in plane 0.
+template <int C>
+__device__ __forceinline__ void store_group(float *o, const uint32_t *w, int hw) {
+#pragma unroll
+    for (int ch = 0; ch < C; ++ch) {
+        float v[4];
+#pragma unroll
+        for (int px = 0; px < 4; ++px) {
+            const int b = px * C + ch;
+            v[px] = u8_over_255_f(byte_as_float(w[b >> 2], b & 3));
+        }
+        asm volatile("st.global.cs.v4.f32 [%0], {%1,%2,%3,%4};" ::"l"(o + (int64_t)ch * hw), "f"(v[0]), "f"(v[1]),
+                     "f"(v[2]), "f"(v[3])
+                     : "memory");
     }
 }
 
@@ -385,21 +411,8 @@ __global__ void __launch_bounds__(256) vn_gather_f32_chw_vec_kernel(const uint8_
             }
         }
 #pragma unroll
-        for (int u = 0; u < kUnroll; ++u) {
-            if (!o[u]) continue;
-#pragma unroll
-            for (int ch = 0; ch < C; ++ch) {
-                float v[4];
-#pragma unroll
-                for (int px = 0; px < 4; ++px) {
-                    const int b = px * C + ch;  // byte of the group: pixel-major, channel-minor (HWC)
-                    v[px] = u8_over_255_f(byte_as_float(w[u][b >> 2], b & 3));
-                }
-                asm volatile("st.global.cs.v4.f32 [%0], {%1,%2,%3,%4};" ::"l"(o[u] + (int64_t)ch * hw), "f"(v[0]),
-                             "f"(v[1]), "f"(v[2]), "f"(v[3])
-                             : "memory");
-            }
-        }
+        for (int u = 0; u < kUnroll; ++u)
+            if (o[u]) store_group<C>(o[u], w[u], hw);
     }
 }
 
@@ -415,21 +428,6 @@ struct FloatLeaves {
     int32_t n_leaves;
 };
 
-__device__ __forceinline__ void store_group(float *o, const uint32_t *w, int c, int hw) {
-    for (int ch = 0; ch < c; ++ch) {
-        float v[4];
-#pragma unroll
-        for (int px = 0; px < 4; ++px) {
-            const int b = px * c + ch;
-            // w[] is indexed with compile-time constants once c is known (c == 1 or c == 3 below)
-            v[px] = u8_over_255_f(byte_as_float(w[b >> 2], b & 3));
-        }
-        asm volatile("st.global.cs.v4.f32 [%0], {%1,%2,%3,%4};" ::"l"(o + (int64_t)ch * hw), "f"(v[0]), "f"(v[1]),
-                     "f"(v[2]), "f"(v[3])
-                     : "memory");
-    }
-}
-
 // kLeaves = number of leaves (sizes the register arrays), kUnroll = groups per thread and iteration: chosen on the
 // host so that a thread has about a dozen independent loads in flight without running out of registers.
 template <int kLeaves, int kUnroll>
@@ -438,8 +436,7 @@ __global__ void __launch_bounds__(256) vn_gather_leaves_f32_kernel(const FloatLe
                                                                    int early_release) {
     // as part of a step (programmatic launch) the scalar half's descriptors are needed from here on, and the next
     // step's scalar kernel - which touches nothing this kernel reads - may be scheduled while this one runs
-    asm volatile("griddepcontrol.wait;" ::: "memory");
-    if (early_release) asm volatile("griddepcontrol.launch_dependents;" ::: "memory");
+    chain_wait(early_release);
     const int groups = hw >> 2;
     const int64_t total = (int64_t)n * groups;
     const int64_t stride = (int64_t)gridDim.x * blockDim.x;
@@ -478,9 +475,9 @@ __global__ void __launch_bounds__(256) vn_gather_leaves_f32_kernel(const FloatLe
                 if (!live[u][l]) continue;
                 float *o = L.out[l] + ((int64_t)fq[u][0] * L.c[l]) * hw + 4 * fq[u][1];
                 if (L.c[l] == 3)
-                    store_group(o, w[u][l], 3, hw);
+                    store_group<3>(o, w[u][l], hw);
                 else
-                    store_group(o, w[u][l], 1, hw);
+                    store_group<1>(o, w[u][l], hw);
             }
         }
     }
@@ -663,10 +660,7 @@ __global__ void __launch_bounds__(kRpBlock) vn_rp_scatter_kernel(const float *__
 // device-side UNREAL replay ring: uniform sampling of valid windows, one thread per env
 // =====================================================================================================
 struct ReplayParams {
-    const int32_t *before, *after, *goal, *goal_before, *action;  // [cap][n] time-major ring
-    const float *reward;
-    const uint8_t *done;
-    int32_t n, cap, head, count;                     // head = next slot to write, count = filled slots (<= cap)
+    vn_replay_t ring;                                // [cap][n] time-major ring, as the caller described it
     int32_t length;                                  // transitions per sampled window
     int32_t mode;                                    // 0 sequence, 1 reward-prediction (length is 3 history steps)
     int32_t env_id_base;
@@ -694,9 +688,9 @@ struct ReplayParams {
 __global__ void __launch_bounds__(128) vn_replay_sample_kernel(const ReplayParams p) {
     const int lane = threadIdx.x & 31;
     const int e = (blockIdx.x * blockDim.x + threadIdx.x) >> 5;
-    if (e >= p.n) return;   // whole warps leave together
+    if (e >= p.ring.n) return;   // whole warps leave together
     const int L = p.mode == 1 ? 4 : p.length;
-    const int oldest = (p.head - p.count + p.cap) % p.cap;
+    const int oldest = (p.ring.head - p.ring.count + p.ring.cap) % p.ring.cap;
     const Philox4 d = philox4x32_10((uint32_t)(p.env_id_base + e), p.call, 0x5EB1A7u, (uint32_t)p.mode,
                                     (uint32_t)p.seed, (uint32_t)(p.seed >> 32));
     int n_valid[2] = {0, 0};  // [0] all (mode 0) or zero-reward (mode 1); [1] non-zero reward (mode 1)
@@ -715,16 +709,16 @@ __global__ void __launch_bounds__(128) vn_replay_sample_kernel(const ReplayParam
         }
         int carry = -1;   // chronological index of the last episode end seen in earlier chunks
         int seen = 0;     // valid windows of class `cls` in earlier chunks (pass 1)
-        for (int base = 0; base < p.count; base += 32) {
+        for (int base = 0; base < p.ring.count; base += 32) {
             const int i = base + lane;
-            const bool in = i < p.count;
-            const size_t at = (size_t)((oldest + (in ? i : 0)) % p.cap) * p.n + e;
-            const bool dn = in && p.done[at] != 0;
+            const bool in = i < p.ring.count;
+            const size_t at = (size_t)((oldest + (in ? i : 0)) % p.ring.cap) * p.ring.n + e;
+            const bool dn = in && p.ring.done[at] != 0;
             const unsigned m = __ballot_sync(0xffffffffu, dn);
             const unsigned below = m & ((1u << lane) - 1u);
             const int last = below ? base + 31 - __clz((int)below) : carry;
             const bool valid = in && i >= L - 1 && last < i - L + 1;
-            const int c = (p.mode == 1 && valid) ? (p.reward[at] != 0.0f) : 0;
+            const int c = (p.mode == 1 && valid) ? (p.ring.reward[at] != 0.0f) : 0;
             if (pass == 0) {
                 n_valid[0] += __popc(__ballot_sync(0xffffffffu, valid && c == 0));
                 n_valid[1] += __popc(__ballot_sync(0xffffffffu, valid && c == 1));
@@ -744,52 +738,153 @@ __global__ void __launch_bounds__(128) vn_replay_sample_kernel(const ReplayParam
     if (start < 0) return;
     // lanes write the L transitions (and the closing observation) of the window
     for (int k = lane; k < L; k += 32) {
-        const size_t at = (size_t)((oldest + start + k) % p.cap) * p.n + e;
-        p.o_states[(size_t)e * (L + 1) + k] = p.before[at];
+        const size_t at = (size_t)((oldest + start + k) % p.ring.cap) * p.ring.n + e;
+        p.o_states[(size_t)e * (L + 1) + k] = p.ring.before[at];
         // goal of the episode the BEFORE observation belongs to (ring.goal is the goal after the step, i.e. the next
         // episode's goal when the step ended one and the env auto-reset)
-        p.o_goals[(size_t)e * (L + 1) + k] = p.goal_before[at];
-        p.o_actions[(size_t)e * L + k] = p.action[at];
-        p.o_rewards[(size_t)e * L + k] = p.reward[at];
-        p.o_dones[(size_t)e * L + k] = p.done[at];
+        p.o_goals[(size_t)e * (L + 1) + k] = p.ring.goal_before[at];
+        p.o_actions[(size_t)e * L + k] = p.ring.action[at];
+        p.o_rewards[(size_t)e * L + k] = p.ring.reward[at];
+        p.o_dones[(size_t)e * L + k] = p.ring.done[at];
         if (k == L - 1) {
-            p.o_states[(size_t)e * (L + 1) + L] = p.after[at];
-            p.o_goals[(size_t)e * (L + 1) + L] = p.goal[at];
+            p.o_states[(size_t)e * (L + 1) + L] = p.ring.after[at];
+            p.o_goals[(size_t)e * (L + 1) + L] = p.ring.goal[at];
             if (p.o_label) {
-                const float r = p.reward[at];
+                const float r = p.ring.reward[at];
                 p.o_label[e] = r > 0.f ? 1 : (r < 0.f ? 2 : 0);
             }
         }
     }
 }
 
-static int32_t pool_geom(int h, int w, int c, int cell, int out_h, int out_w, PoolGeom *g) {
-    VN_REQUIRE(h > 0 && w > 0 && c > 0 && cell > 0 && out_h > 0 && out_w > 0, "pool: bad geometry");
-    VN_REQUIRE(out_h * cell <= h && out_w * cell <= w, "pool: output %dx%d * cell %d exceeds frame %dx%d", out_h,
+
+// =====================================================================================================
+// host side
+// =====================================================================================================
+constexpr int kMaxSmem = 220 * 1024;   // dynamic shared memory one CTA can have
+
+// A store plane as the frame kernels read it.
+struct FrameArgs {
+    const uint8_t *pbase;   // store base + plane offset
+    int64_t pitch;          // bytes from one record to the next
+    PoolGeom g;             // h, w, c; the pool fields as well when a pool applies
+    int smem;               // bytes of the frames a CTA stages, each padded to 16 bytes
+};
+
+// Validates plane `plane` of the store against the frame geometry (h, w, c) and, when `pool` = {cell, out_h, out_w} is
+// given, the centred pool; `frames` frames are staged in shared memory.  Their size is checked by frame_smem() when a
+// call has work to launch.
+static int32_t frame_args(const vn_store_t *store, int32_t plane, int h, int w, int c, const int *pool, int frames,
+                          const char *who, FrameArgs *f) {
+    VN_REQUIRE(store && store->base, "%s: store is null", who);
+    VN_REQUIRE(plane >= 0 && plane < store->n_planes, "%s: plane=%d", who, plane);
+    const int fb = (h * w * c + 15) & ~15;
+    VN_REQUIRE(store->plane_bytes[plane] == fb, "%s: plane holds %d bytes, geometry says %d (rounded up to 16)", who,
+               store->plane_bytes[plane], h * w * c);
+    VN_REQUIRE((store->plane_bytes[plane] & 15) == 0 && (store->state_pitch & 15) == 0 &&
+                   (store->plane_off[plane] & 15) == 0,
+               "%s: store is not 16-byte aligned", who);
+    f->pbase = store->base + store->plane_off[plane];
+    f->pitch = store->state_pitch;
+    f->smem = frames * fb;
+    f->g = PoolGeom{h, w, c, 1, h, w, 0, 0};
+    if (!pool) return VN_OK;
+    const int cell = pool[0], out_h = pool[1], out_w = pool[2];
+    VN_REQUIRE(h > 0 && w > 0 && c > 0 && cell > 0 && out_h > 0 && out_w > 0, "%s: bad pool geometry", who);
+    VN_REQUIRE(out_h * cell <= h && out_w * cell <= w, "%s: pool output %dx%d * cell %d exceeds frame %dx%d", who, out_h,
                out_w, cell, h, w);
-    g->h = h;
-    g->w = w;
-    g->c = c;
-    g->cell = cell;
-    g->out_h = out_h;
-    g->out_w = out_w;
-    g->top = (h - out_h * cell) / 2;   // autocrop_observations: centred, top margin (H - H') // 2
-    g->left = (w - out_w * cell) / 2;
+    // autocrop_observations: centred, top margin (H - H') // 2
+    f->g = PoolGeom{h, w, c, cell, out_h, out_w, (h - out_h * cell) / 2, (w - out_w * cell) / 2};
     return VN_OK;
+}
+
+// The frames `kernel` stages must fit one CTA's shared memory; raises the kernel's limit to their size.
+template <typename... KArgs>
+static int32_t frame_smem(void (*kernel)(KArgs...), const FrameArgs &f, const char *who) {
+    VN_REQUIRE(f.smem <= kMaxSmem, "%s: frame too large for shared memory", who);
+    return ensure_smem(kernel, f.smem);
+}
+
+// chained: the first kernel of vn_pixel_control_returns_from_states (programmatic launch, releases the list kernel
+// early); otherwise an ordinary launch.
+static int32_t launch_transition_rows(const int32_t *adj, const int32_t *states, int n, int t, int64_t sn, int64_t st,
+                                      int64_t rsn, int64_t rst, int32_t *rows, int32_t *miss_pos, int32_t *miss_count,
+                                      cudaStream_t stream, bool chained) {
+    const int64_t total = (int64_t)n * t;
+    return launch(vn_transition_rows_kernel, "vn_transition_rows_kernel", dim3((unsigned)((total + 255) / 256)),
+                  dim3(256), 0, stream, chained, adj, states, n, t, sn, st, rsn, rst, rows, miss_pos, miss_count,
+                  chained ? 1 : 0);
 }
 
 // The list kernel loops over a device-resident list (episode resets: ~0.1 % of an A2C rollout's transitions, ~2 % at
 // C5's short episodes).  512 threads: one per output cell (20 x 20) in a single round - the kernel sits on the critical
-// path between the row lookup and the back-up.
-static int32_t launch_pc_list(const vn_store_t *store, int plane, const int32_t *states, int t, int64_t sn, int64_t st,
-                              const PoolGeom &g, const int32_t *pos, const int32_t *count, int max_count, int compact,
-                              float *out, int smem, int per_sm, cudaStream_t stream, bool chained) {
-    int32_t rc = ensure_smem(vn_pixel_control_list_kernel, smem);
+// path between the row lookup and the back-up.  chained: the second kernel of vn_pixel_control_returns_from_states.
+static int32_t launch_pc_list(const FrameArgs &f, const int32_t *states, int t, int64_t sn, int64_t st,
+                              const int32_t *pos, const int32_t *count, int max_count, int compact, float *out,
+                              cudaStream_t stream, bool chained, const char *who) {
+    int32_t rc = frame_smem(vn_pixel_control_list_kernel, f, who);
     if (rc) return rc;
-    const int want = sm_count() * (per_sm < 4 ? per_sm : 4);
+    const int want = sm_count() * ctas_per_sm(f.smem, 4);
     const int grid = max_count < want ? max_count : want;
-    return launch(vn_pixel_control_list_kernel, "vn_pixel_control_list_kernel", dim3(grid), dim3(512), (size_t)smem,
-                  stream, true, *store, plane, states, t, sn, st, g, pos, count, max_count, compact, out, chained ? 1 : 0);
+    return launch(vn_pixel_control_list_kernel, "vn_pixel_control_list_kernel", dim3(grid), dim3(512), (size_t)f.smem,
+                  stream, true, f.pbase, f.pitch, states, t, sn, st, f.g, pos, count, max_count, compact, out,
+                  chained ? 1 : 0);
+}
+
+// chained: the last kernel of vn_pixel_control_returns_from_states (programmatic launch), which re-arms the chain's
+// miss counter reset_counter; otherwise an ordinary launch and reset_counter is null.
+static int32_t launch_pc_returns(const float *pc_table, int cells, const int32_t *rows, int64_t rsn, int64_t rst,
+                                 const float *miss_rows, const uint8_t *done, int64_t dsn, int64_t dst,
+                                 const float *bootstrap, float gamma, int n, int t, float *out_returns,
+                                 float *out_reward, int32_t *reset_counter, cudaStream_t stream, bool chained) {
+    const int d4 = cells >> 2;
+    const int64_t threads = (int64_t)n * d4;
+    return launch(vn_pc_returns_kernel, "vn_pc_returns_kernel", dim3((unsigned)((threads + 255) / 256)), dim3(256), 0,
+                  stream, chained, reinterpret_cast<const float4 *>(pc_table), rows, rsn, rst,
+                  reinterpret_cast<const float4 *>(miss_rows), done, dsn, dst,
+                  reinterpret_cast<const float4 *>(bootstrap), gamma, n, t, d4, reinterpret_cast<float4 *>(out_returns),
+                  reinterpret_cast<float4 *>(out_reward), reset_counter);
+}
+
+int32_t launch_float_leaves(const vn_store_t *store, const vn_float_leaf_t *leaves, int32_t n_leaves, const int32_t *desc,
+                            int32_t n, int32_t h, int32_t w, void *stream, bool in_step) {
+    VN_REQUIRE(store && store->base && leaves && desc && n >= 0, "gather_leaves_f32_chw: null pointer");
+    VN_REQUIRE(n_leaves >= 1 && n_leaves <= kMaxFloatLeaves, "gather_leaves_f32_chw: n_leaves=%d (max %d)", n_leaves,
+               kMaxFloatLeaves);
+    if ((h * w) % 4 != 0) {
+        set_error("gather_leaves_f32_chw: %d x %d pixels are not whole groups of 4 (use the per-leaf call)", h, w);
+        return VN_EUNSUPPORTED;
+    }
+    FloatLeaves L = {};
+    L.n_leaves = n_leaves;
+    for (int l = 0; l < n_leaves; ++l) {
+        FrameArgs f;
+        int32_t rc = frame_args(store, leaves[l].plane, h, w, leaves[l].channels, nullptr, 0, "gather_leaves_f32_chw", &f);
+        if (rc) return rc;
+        if (leaves[l].channels != 1 && leaves[l].channels != 3) {
+            set_error("gather_leaves_f32_chw: %d channels (use the per-leaf call)", leaves[l].channels);
+            return VN_EUNSUPPORTED;
+        }
+        VN_REQUIRE(leaves[l].out && aligned16(leaves[l].out), "gather_leaves_f32_chw: out[%d] must be 16-byte aligned",
+                   l);
+        VN_REQUIRE(leaves[l].source == 0 || leaves[l].source == 1, "gather_leaves_f32_chw: source=%d", leaves[l].source);
+        L.pbase[l] = f.pbase;
+        L.out[l] = leaves[l].out;
+        L.c[l] = leaves[l].channels;
+        L.goal[l] = leaves[l].source;
+    }
+    if (n == 0) return VN_OK;
+    const int64_t total = (int64_t)n * (h * w / 4);
+    const int unroll = n_leaves == 1 ? 4 : (n_leaves <= 3 ? 2 : 1);
+    const int64_t want = (total + unroll * 256 - 1) / (unroll * 256), cap = (int64_t)sm_count() * 16;
+    const int grid = (int)(want < cap ? want : cap);
+    void (*const kernels[])(FloatLeaves, int64_t, const int2 *, int, int, int) = {
+        vn_gather_leaves_f32_kernel<1, 4>, vn_gather_leaves_f32_kernel<2, 2>, vn_gather_leaves_f32_kernel<3, 2>,
+        vn_gather_leaves_f32_kernel<4, 1>, vn_gather_leaves_f32_kernel<5, 1>, vn_gather_leaves_f32_kernel<6, 1>};
+    // programmatic launch only as part of a step: there the predecessor is the step's own scalar / gather kernel
+    return launch(kernels[n_leaves - 1], "vn_gather_leaves_f32_kernel", dim3(grid), dim3(256), 0,
+                  static_cast<cudaStream_t>(stream), in_step, L, store->state_pitch, reinterpret_cast<const int2 *>(desc),
+                  n, h * w, in_step ? 1 : 0);
 }
 
 }  // namespace vn
@@ -803,9 +898,9 @@ int32_t vn_nstep_returns(const float *reward, const uint8_t *done, const float *
     VN_REQUIRE(n >= 0 && t >= 1, "nstep_returns: n=%d t=%d", n, t);
     if (n == 0) return VN_OK;
     // 64-thread blocks: 4,096 envs spread over 64 SMs instead of 16 (the loop over T is a chain of dependent FMAs)
-    vn::vn_nstep_returns_kernel<<<(n + 63) / 64, 64, 0, static_cast<cudaStream_t>(stream)>>>(
-        reward, done, last_value, gamma, n, t, stride_n, stride_t, out, out_stride_n, out_stride_t);
-    return vn::check_launch("vn_nstep_returns_kernel");
+    return vn::launch(vn::vn_nstep_returns_kernel, "vn_nstep_returns_kernel", dim3((n + 63) / 64), dim3(64), 0,
+                      static_cast<cudaStream_t>(stream), false, reward, done, last_value, gamma, n, t, stride_n,
+                      stride_t, out, out_stride_n, out_stride_t);
 }
 
 int32_t vn_nstep_returns_scan(const float *reward, const uint8_t *done, const float *last_value, float gamma,
@@ -815,9 +910,9 @@ int32_t vn_nstep_returns_scan(const float *reward, const uint8_t *done, const fl
     VN_REQUIRE(n >= 0 && t >= 1, "nstep_returns_scan: n=%d t=%d", n, t);
     if (n == 0) return VN_OK;
     const int64_t want = ((int64_t)n * 32 + 127) / 128, cap = (int64_t)vn::sm_count() * 16;
-    vn::vn_nstep_returns_scan_kernel<<<(int)(want < cap ? want : cap), 128, 0, static_cast<cudaStream_t>(stream)>>>(
-        reward, done, last_value, gamma, n, t, stride_n, stride_t, out, out_stride_n, out_stride_t);
-    return vn::check_launch("vn_nstep_returns_scan_kernel");
+    return vn::launch(vn::vn_nstep_returns_scan_kernel, "vn_nstep_returns_scan_kernel",
+                      dim3((unsigned)(want < cap ? want : cap)), dim3(128), 0, static_cast<cudaStream_t>(stream), false,
+                      reward, done, last_value, gamma, n, t, stride_n, stride_t, out, out_stride_n, out_stride_t);
 }
 
 int32_t vn_discounted_backup(const float *reward, const uint8_t *done, int64_t done_stride_n, int64_t done_stride_t,
@@ -827,9 +922,9 @@ int32_t vn_discounted_backup(const float *reward, const uint8_t *done, int64_t d
     VN_REQUIRE(n >= 0 && t >= 1 && d >= 1, "discounted_backup: n=%d t=%d d=%d", n, t, d);
     if (n == 0) return VN_OK;
     const int64_t total = (int64_t)n * d;
-    vn::vn_backup_kernel<<<(unsigned)((total + 255) / 256), 256, 0, static_cast<cudaStream_t>(stream)>>>(
-        reward, done, bootstrap, gamma, n, t, d, done_stride_n, done_stride_t, out);
-    return vn::check_launch("vn_backup_kernel");
+    return vn::launch(vn::vn_backup_kernel, "vn_backup_kernel", dim3((unsigned)((total + 255) / 256)), dim3(256), 0,
+                      static_cast<cudaStream_t>(stream), false, reward, done, bootstrap, gamma, n, t, d, done_stride_n,
+                      done_stride_t, out);
 }
 
 int32_t vn_pixel_control_returns(const float *pc_table, int32_t cells, const int32_t *rows, int64_t row_stride_n,
@@ -840,34 +935,13 @@ int32_t vn_pixel_control_returns(const float *pc_table, int32_t cells, const int
     VN_REQUIRE(pc_table && rows && miss_rows && done && bootstrap && out_returns, "pixel_control_returns: null pointer");
     VN_REQUIRE(n >= 0 && t >= 1 && cells >= 4 && (cells & 3) == 0, "pixel_control_returns: n=%d t=%d cells=%d", n, t,
                cells);
-    VN_REQUIRE(((reinterpret_cast<uintptr_t>(pc_table) | reinterpret_cast<uintptr_t>(miss_rows) |
-                 reinterpret_cast<uintptr_t>(bootstrap) | reinterpret_cast<uintptr_t>(out_returns) |
-                 reinterpret_cast<uintptr_t>(out_reward)) & 15) == 0,
+    VN_REQUIRE(vn::aligned16(pc_table, miss_rows, bootstrap, out_returns, out_reward),
                "pixel_control_returns: arrays must be 16-byte aligned");
     if (n == 0) return VN_OK;
-    const int d4 = cells >> 2;
-    const int64_t total = (int64_t)n * d4;
-    vn::vn_pc_returns_kernel<<<(unsigned)((total + 255) / 256), 256, 0, static_cast<cudaStream_t>(stream)>>>(
-        reinterpret_cast<const float4 *>(pc_table), rows, row_stride_n, row_stride_t,
-        reinterpret_cast<const float4 *>(miss_rows), done, done_stride_n, done_stride_t,
-        reinterpret_cast<const float4 *>(bootstrap), gamma, n, t, d4, reinterpret_cast<float4 *>(out_returns),
-        reinterpret_cast<float4 *>(out_reward), nullptr);
-    return vn::check_launch("vn_pc_returns_kernel");
+    return vn::launch_pc_returns(pc_table, cells, rows, row_stride_n, row_stride_t, miss_rows, done, done_stride_n,
+                                 done_stride_t, bootstrap, gamma, n, t, out_returns, out_reward, nullptr,
+                                 static_cast<cudaStream_t>(stream), false);
 }
-
-static int32_t check_plane(const vn_store_t *store, int32_t plane, int h, int w, int c, const char *who) {
-    VN_REQUIRE(store && store->base, "%s: store is null", who);
-    VN_REQUIRE(plane >= 0 && plane < store->n_planes, "%s: plane=%d", who, plane);
-    VN_REQUIRE(store->plane_bytes[plane] == ((h * w * c + 15) & ~15),
-               "%s: plane holds %d bytes, geometry says %d (rounded up to 16)", who, store->plane_bytes[plane],
-               h * w * c);
-    VN_REQUIRE((store->plane_bytes[plane] & 15) == 0 && (store->state_pitch & 15) == 0 &&
-                   (store->plane_off[plane] & 15) == 0,
-               "%s: store is not 16-byte aligned", who);
-    return VN_OK;
-}
-
-static int32_t check_plane(const vn_store_t *store, int32_t plane, int h, int w, int c, const char *who);
 
 int32_t vn_pixel_control_returns_from_states(const vn_store_t *store, int32_t plane, const int32_t *adj,
                                              const float *pc_table, const int32_t *states, int64_t state_stride_n,
@@ -877,73 +951,57 @@ int32_t vn_pixel_control_returns_from_states(const vn_store_t *store, int32_t pl
                                              int32_t out_w, int32_t *rows, int32_t *miss_pos, int32_t *miss_count,
                                              float *miss_rows, int32_t max_miss, float *out_returns, float *out_reward,
                                              void *stream) {
-    int32_t rc = check_plane(store, plane, h, w, c, "pixel_control_returns");
+    const char *who = "pixel_control_returns";
+    const int pool[] = {cell, out_h, out_w};
+    vn::FrameArgs f;
+    int32_t rc = vn::frame_args(store, plane, h, w, c, pool, 2, who, &f);
     if (rc) return rc;
     const int32_t cells = out_h * out_w;
     VN_REQUIRE(adj && pc_table && states && done && bootstrap && rows && miss_pos && miss_count && miss_rows && out_returns,
                "pixel_control_returns: null pointer");
     VN_REQUIRE(n >= 0 && t >= 1 && cells >= 4 && (cells & 3) == 0 && max_miss >= 1,
                "pixel_control_returns: n=%d t=%d cells=%d max_miss=%d", n, t, cells, max_miss);
-    VN_REQUIRE((reinterpret_cast<uintptr_t>(adj) & 15) == 0, "pixel_control_returns: adj must be 16-byte aligned");
-    VN_REQUIRE(((reinterpret_cast<uintptr_t>(pc_table) | reinterpret_cast<uintptr_t>(miss_rows) |
-                 reinterpret_cast<uintptr_t>(bootstrap) | reinterpret_cast<uintptr_t>(out_returns) |
-                 reinterpret_cast<uintptr_t>(out_reward)) & 15) == 0,
+    VN_REQUIRE(vn::aligned16(adj), "pixel_control_returns: adj must be 16-byte aligned");
+    VN_REQUIRE(vn::aligned16(pc_table, miss_rows, bootstrap, out_returns, out_reward),
                "pixel_control_returns: arrays must be 16-byte aligned");
-    vn::PoolGeom g;
-    rc = vn::pool_geom(h, w, c, cell, out_h, out_w, &g);
-    if (rc) return rc;
     if (n == 0) return VN_OK;
     cudaStream_t st = static_cast<cudaStream_t>(stream);
     // (1) table row of every transition; the misses (episode resets) go to a list.  *miss_count must be 0 on entry:
     //     zero it once when the scratch is allocated - kernel (3) re-arms it for the next call
-    const int64_t total = (int64_t)n * t;
     // `rows` is written batch-major whatever the layout of `states` (the lookup kernel orders its threads for coalesced
     // state READS; its 4-byte row writes are then scattered for time-major input, which costs nothing next to what a
     // time-major `rows` costs the back-up kernel: there every step's row index is a dependent load in front of the table
     // load, and batch-major keeps an env's T indices in one or two cache lines - 42 vs 58 us at 4,096 x 20)
     const int64_t rsn = t, rst = 1;
-    rc = vn::launch(vn::vn_transition_rows_kernel, "vn_transition_rows_kernel", dim3((unsigned)((total + 255) / 256)),
-                    dim3(256), 0, st, true, adj, states, n, t, state_stride_n, state_stride_t, rsn, rst, rows, miss_pos,
-                    miss_count, 1);
+    rc = vn::launch_transition_rows(adj, states, n, t, state_stride_n, state_stride_t, rsn, rst, rows, miss_pos,
+                                    miss_count, st, true);
     if (rc) return rc;
     // (2) the misses computed directly from their two frames into the compact side buffer
-    const int fb = (h * w * c + 15) & ~15;
-    const int smem = 2 * fb;
-    VN_REQUIRE(smem <= 220 * 1024, "pixel_control_returns: frame too large for shared memory");
-    rc = vn::launch_pc_list(store, plane, states, t, state_stride_n, state_stride_t, g, miss_pos, miss_count, max_miss, 1,
-                            miss_rows, smem, vn::ctas_per_sm(smem), st, true);
+    rc = vn::launch_pc_list(f, states, t, state_stride_n, state_stride_t, miss_pos, miss_count, max_miss, 1, miss_rows, st,
+                            true, who);
     if (rc) return rc;
     // (3) rewards gathered on the fly + discounted back-up
-    const int d4 = cells >> 2;
-    const int64_t threads = (int64_t)n * d4;
-    return vn::launch(vn::vn_pc_returns_kernel, "vn_pc_returns_kernel", dim3((unsigned)((threads + 255) / 256)), dim3(256),
-                      0, st, true, reinterpret_cast<const float4 *>(pc_table), rows, rsn, rst,
-                      reinterpret_cast<const float4 *>(miss_rows), done, done_stride_n, done_stride_t,
-                      reinterpret_cast<const float4 *>(bootstrap), gamma, n, t, d4,
-                      reinterpret_cast<float4 *>(out_returns), reinterpret_cast<float4 *>(out_reward), miss_count);
+    return vn::launch_pc_returns(pc_table, cells, rows, rsn, rst, miss_rows, done, done_stride_n, done_stride_t,
+                                 bootstrap, gamma, n, t, out_returns, out_reward, miss_count, st, true);
 }
 
 int32_t vn_pixel_control(const vn_store_t *store, int32_t plane, const int32_t *states, int32_t n, int32_t t,
                          int64_t state_stride_n, int64_t state_stride_t, int32_t h, int32_t w, int32_t c, int32_t cell,
                          int32_t out_h, int32_t out_w, float *out, void *stream) {
-    int32_t rc = check_plane(store, plane, h, w, c, "pixel_control");
+    const int pool[] = {cell, out_h, out_w};
+    vn::FrameArgs f;
+    int32_t rc = vn::frame_args(store, plane, h, w, c, pool, 2, "pixel_control", &f);
     if (rc) return rc;
     VN_REQUIRE(states && out && n >= 0 && t >= 1, "pixel_control: bad arguments");
-    vn::PoolGeom g;
-    rc = vn::pool_geom(h, w, c, cell, out_h, out_w, &g);
-    if (rc) return rc;
     if (n == 0) return VN_OK;
     constexpr int kChunk = 16;
-    const int fb = (h * w * c + 15) & ~15;
-    const int smem = 2 * fb;
-    VN_REQUIRE(smem <= 220 * 1024, "pixel_control: frame too large for shared memory");
-    rc = vn::ensure_smem(vn::vn_pixel_control_kernel<kChunk>, smem);
+    rc = vn::frame_smem(vn::vn_pixel_control_kernel<kChunk>, f, "pixel_control");
     if (rc) return rc;
     const int64_t blocks = (int64_t)n * ((t + kChunk - 1) / kChunk);
     VN_REQUIRE(blocks < (1ll << 31), "pixel_control: too many blocks");
-    vn::vn_pixel_control_kernel<kChunk><<<(unsigned)blocks, 256, smem, static_cast<cudaStream_t>(stream)>>>(
-        *store, plane, states, n, t, state_stride_n, state_stride_t, g, out);
-    return vn::check_launch("vn_pixel_control_kernel");
+    return vn::launch(vn::vn_pixel_control_kernel<kChunk>, "vn_pixel_control_kernel", dim3((unsigned)blocks), dim3(256),
+                      (size_t)f.smem, static_cast<cudaStream_t>(stream), false, f.pbase, f.pitch, states, n, t,
+                      state_stride_n, state_stride_t, f.g, out);
 }
 
 int32_t vn_transition_rows(const int32_t *adj, const int32_t *states, int32_t n, int32_t t, int64_t state_stride_n,
@@ -951,14 +1009,17 @@ int32_t vn_transition_rows(const int32_t *adj, const int32_t *states, int32_t n,
                            int32_t *miss_pos, int32_t *miss_count, void *stream) {
     VN_REQUIRE(adj && states && rows && miss_pos && miss_count, "transition_rows: null pointer");
     VN_REQUIRE(n >= 0 && t >= 1, "transition_rows: n=%d t=%d", n, t);
-    VN_REQUIRE((reinterpret_cast<uintptr_t>(adj) & 15) == 0, "transition_rows: adj must be 16-byte aligned");
+    VN_REQUIRE(vn::aligned16(adj), "transition_rows: adj must be 16-byte aligned");
     if (n == 0) return VN_OK;
     cudaStream_t st = static_cast<cudaStream_t>(stream);
-    cudaMemsetAsync(miss_count, 0, sizeof(int32_t), st);
-    const int64_t total = (int64_t)n * t;
-    vn::vn_transition_rows_kernel<<<(unsigned)((total + 255) / 256), 256, 0, st>>>(
-        adj, states, n, t, state_stride_n, state_stride_t, row_stride_n, row_stride_t, rows, miss_pos, miss_count, 0);
-    return vn::check_launch("vn_transition_rows_kernel");
+    const cudaError_t e = cudaMemsetAsync(miss_count, 0, sizeof(int32_t), st);
+    if (e != cudaSuccess) {
+        cudaGetLastError();
+        vn::set_error("transition_rows: zeroing miss_count: %s", cudaGetErrorString(e));
+        return VN_ECUDA;
+    }
+    return vn::launch_transition_rows(adj, states, n, t, state_stride_n, state_stride_t, row_stride_n, row_stride_t, rows,
+                                      miss_pos, miss_count, st, false);
 }
 
 int32_t vn_gather_rows(const void *table, int64_t row_bytes, const int32_t *idx, int64_t n, int32_t idx_t,
@@ -967,32 +1028,26 @@ int32_t vn_gather_rows(const void *table, int64_t row_bytes, const int32_t *idx,
     VN_REQUIRE(idx_t >= 1 && n % idx_t == 0, "gather_rows: n=%lld is not a multiple of idx_t=%d", (long long)n, idx_t);
     VN_REQUIRE(row_bytes > 0 && (row_bytes & 15) == 0, "gather_rows: row_bytes=%lld must be a multiple of 16",
                (long long)row_bytes);
-    VN_REQUIRE(((reinterpret_cast<uintptr_t>(table) | reinterpret_cast<uintptr_t>(out)) & 15) == 0,
-               "gather_rows: table and out must be 16-byte aligned");
+    VN_REQUIRE(vn::aligned16(table, out), "gather_rows: table and out must be 16-byte aligned");
     if (n <= 0) return VN_OK;
     const int64_t cap = (int64_t)vn::sm_count() * 64, warps = n < cap ? n : cap;
-    vn::vn_gather_rows_kernel<<<(unsigned)((warps * 32 + 255) / 256), 256, 0, static_cast<cudaStream_t>(stream)>>>(
-        static_cast<const int4 *>(table), (int)(row_bytes >> 4), idx, n, idx_t, idx_stride_n, idx_stride_t,
-        static_cast<int4 *>(out));
-    return vn::check_launch("vn_gather_rows_kernel");
+    return vn::launch(vn::vn_gather_rows_kernel, "vn_gather_rows_kernel", dim3((unsigned)((warps * 32 + 255) / 256)),
+                      dim3(256), 0, static_cast<cudaStream_t>(stream), false, static_cast<const int4 *>(table),
+                      (int)(row_bytes >> 4), idx, n, idx_t, idx_stride_n, idx_stride_t, static_cast<int4 *>(out));
 }
 
 int32_t vn_pixel_control_list(const vn_store_t *store, int32_t plane, const int32_t *states, int32_t n, int32_t t,
                               int64_t state_stride_n, int64_t state_stride_t, int32_t h, int32_t w, int32_t c,
                               int32_t cell, int32_t out_h, int32_t out_w, const int32_t *pos, const int32_t *count,
                               int32_t max_count, int32_t compact, float *out, void *stream) {
-    int32_t rc = check_plane(store, plane, h, w, c, "pixel_control_list");
+    const int pool[] = {cell, out_h, out_w};
+    vn::FrameArgs f;
+    int32_t rc = vn::frame_args(store, plane, h, w, c, pool, 2, "pixel_control_list", &f);
     if (rc) return rc;
     VN_REQUIRE(states && pos && count && out && n >= 0 && t >= 1 && max_count >= 0, "pixel_control_list: bad arguments");
-    vn::PoolGeom g;
-    rc = vn::pool_geom(h, w, c, cell, out_h, out_w, &g);
-    if (rc) return rc;
     if (n == 0 || max_count == 0) return VN_OK;
-    const int fb = (h * w * c + 15) & ~15;
-    const int smem = 2 * fb;
-    VN_REQUIRE(smem <= 220 * 1024, "pixel_control_list: frame too large for shared memory");
-    return vn::launch_pc_list(store, plane, states, t, state_stride_n, state_stride_t, g, pos, count, max_count, compact, out,
-                              smem, vn::ctas_per_sm(smem, 8), static_cast<cudaStream_t>(stream), false);
+    return vn::launch_pc_list(f, states, t, state_stride_n, state_stride_t, pos, count, max_count, compact, out,
+                              static_cast<cudaStream_t>(stream), false, "pixel_control_list");
 }
 
 int32_t vn_replay_sample(const vn_replay_t *ring, int32_t length, int32_t mode, uint64_t seed, uint32_t call,
@@ -1008,50 +1063,25 @@ int32_t vn_replay_sample(const vn_replay_t *ring, int32_t length, int32_t mode, 
     VN_REQUIRE(mode == 1 || length >= 1, "replay_sample: length=%d", length);
     VN_REQUIRE(o_states && o_goals && o_actions && o_rewards && o_dones && o_start, "replay_sample: null output");
     if (ring->n == 0) return VN_OK;
-    vn::ReplayParams p;
-    p.before = ring->before;
-    p.after = ring->after;
-    p.goal = ring->goal;
-    p.goal_before = ring->goal_before;
-    p.action = ring->action;
-    p.reward = ring->reward;
-    p.done = ring->done;
-    p.n = ring->n;
-    p.cap = ring->cap;
-    p.head = ring->head;
-    p.count = ring->count;
-    p.length = length;
-    p.mode = mode;
-    p.env_id_base = env_id_base;
-    p.call = call;
-    p.seed = seed;
-    p.o_states = o_states;
-    p.o_goals = o_goals;
-    p.o_actions = o_actions;
-    p.o_rewards = o_rewards;
-    p.o_dones = o_dones;
-    p.o_start = o_start;
-    p.o_label = o_label;
-    vn::vn_replay_sample_kernel<<<(ring->n + 3) / 4, 128, 0, static_cast<cudaStream_t>(stream)>>>(p);   // warp per env
-    return vn::check_launch("vn_replay_sample_kernel");
+    const vn::ReplayParams p = {*ring,    length,    mode,      env_id_base, call,    seed,   o_states,
+                                o_goals, o_actions, o_rewards, o_dones,     o_start, o_label};
+    return vn::launch(vn::vn_replay_sample_kernel, "vn_replay_sample_kernel", dim3((ring->n + 3) / 4), dim3(128), 0,
+                      static_cast<cudaStream_t>(stream), false, p);   // warp per env
 }
 
 int32_t vn_aux_target(const vn_store_t *store, int32_t plane, const int32_t *idx, int32_t m, int32_t h, int32_t w,
                       int32_t c, int32_t cell, int32_t out_h, int32_t out_w, float *out, void *stream) {
-    int32_t rc = check_plane(store, plane, h, w, c, "aux_target");
+    const int pool[] = {cell, out_h, out_w};
+    vn::FrameArgs f;
+    int32_t rc = vn::frame_args(store, plane, h, w, c, pool, 1, "aux_target", &f);
     if (rc) return rc;
     VN_REQUIRE(idx && out && m >= 0, "aux_target: bad arguments");
-    vn::PoolGeom g;
-    rc = vn::pool_geom(h, w, c, cell, out_h, out_w, &g);
-    if (rc) return rc;
     if (m == 0) return VN_OK;
-    const int smem = (h * w * c + 15) & ~15;
-    VN_REQUIRE(smem <= 220 * 1024, "aux_target: frame too large for shared memory");
-    rc = vn::ensure_smem(vn::vn_aux_target_kernel, smem);
+    rc = vn::frame_smem(vn::vn_aux_target_kernel, f, "aux_target");
     if (rc) return rc;
     const int grid = m < vn::sm_count() * 8 ? m : vn::sm_count() * 8;
-    vn::vn_aux_target_kernel<<<grid, 256, smem, static_cast<cudaStream_t>(stream)>>>(*store, plane, idx, m, g, out);
-    return vn::check_launch("vn_aux_target_kernel");
+    return vn::launch(vn::vn_aux_target_kernel, "vn_aux_target_kernel", dim3(grid), dim3(256), (size_t)f.smem,
+                      static_cast<cudaStream_t>(stream), false, f.pbase, f.pitch, idx, m, f.g, out);
 }
 
 int32_t vn_gather_plane_f32_chw(const vn_store_t *store, int32_t plane, const int32_t *idx, int32_t n, int32_t h,
@@ -1061,90 +1091,26 @@ int32_t vn_gather_plane_f32_chw(const vn_store_t *store, int32_t plane, const in
 
 int32_t vn_gather_plane_f32_chw_rows(const vn_store_t *store, int32_t plane, const int32_t *idx, int32_t idx_stride,
                                      int32_t n, int32_t h, int32_t w, int32_t c, float *out, void *stream) {
-    int32_t rc = check_plane(store, plane, h, w, c, "gather_plane_f32_chw");
+    vn::FrameArgs f;
+    int32_t rc = vn::frame_args(store, plane, h, w, c, nullptr, 1, "gather_plane_f32_chw", &f);
     if (rc) return rc;
     VN_REQUIRE(idx && out && n >= 0 && idx_stride >= 1, "gather_plane_f32_chw: bad arguments");
     if (n == 0) return VN_OK;
-    if ((h * w) % 4 == 0 && (c == 1 || c == 3) && (reinterpret_cast<uintptr_t>(out) & 15) == 0) {
+    cudaStream_t st = static_cast<cudaStream_t>(stream);
+    if ((h * w) % 4 == 0 && (c == 1 || c == 3) && vn::aligned16(out)) {
         // whole 4-pixel groups: the vectorised kernel (0.36 -> see DESIGN.md of the copy peak for the staged one)
         const int64_t total = (int64_t)n * (h * w / 4);
         const int64_t want = (total + 4 * 256 - 1) / (4 * 256), cap = (int64_t)vn::sm_count() * 16;
-        const int grid = (int)(want < cap ? want : cap);
-        cudaStream_t st = static_cast<cudaStream_t>(stream);
-        const uint8_t *pbase = store->base + store->plane_off[plane];
-        if (c == 1)
-            vn::vn_gather_f32_chw_vec_kernel<1><<<grid, 256, 0, st>>>(pbase, store->state_pitch, idx, idx_stride, n, h * w,
-                                                                      out);
-        else
-            vn::vn_gather_f32_chw_vec_kernel<3><<<grid, 256, 0, st>>>(pbase, store->state_pitch, idx, idx_stride, n, h * w,
-                                                                      out);
-        return vn::check_launch("vn_gather_f32_chw_vec_kernel");
+        return vn::launch(c == 1 ? vn::vn_gather_f32_chw_vec_kernel<1> : vn::vn_gather_f32_chw_vec_kernel<3>,
+                          "vn_gather_f32_chw_vec_kernel", dim3((unsigned)(want < cap ? want : cap)), dim3(256), 0, st,
+                          false, f.pbase, f.pitch, idx, idx_stride, n, h * w, out);
     }
-    const int smem = (h * w * c + 15) & ~15;
-    VN_REQUIRE(smem <= 220 * 1024, "gather_plane_f32_chw: frame too large for shared memory");
-    rc = vn::ensure_smem(vn::vn_gather_f32_chw_kernel, smem);
+    rc = vn::frame_smem(vn::vn_gather_f32_chw_kernel, f, "gather_plane_f32_chw");
     if (rc) return rc;
     const int grid = n < vn::sm_count() * 8 ? n : vn::sm_count() * 8;
-    vn::vn_gather_f32_chw_kernel<<<grid, 256, smem, static_cast<cudaStream_t>(stream)>>>(*store, plane, idx, idx_stride,
-                                                                                        n, h, w, c, out);
-    return vn::check_launch("vn_gather_f32_chw_kernel");
+    return vn::launch(vn::vn_gather_f32_chw_kernel, "vn_gather_f32_chw_kernel", dim3(grid), dim3(256), (size_t)f.smem, st,
+                      false, f.pbase, f.pitch, idx, idx_stride, n, h, w, c, out);
 }
-
-}  // extern "C"
-
-namespace vn {
-
-int32_t launch_float_leaves(const vn_store_t *store, const vn_float_leaf_t *leaves, int32_t n_leaves, const int32_t *desc,
-                            int32_t n, int32_t h, int32_t w, void *stream, bool in_step) {
-    VN_REQUIRE(store && store->base && leaves && desc && n >= 0, "gather_leaves_f32_chw: null pointer");
-    VN_REQUIRE(n_leaves >= 1 && n_leaves <= kMaxFloatLeaves, "gather_leaves_f32_chw: n_leaves=%d (max %d)", n_leaves,
-               kMaxFloatLeaves);
-    if ((h * w) % 4 != 0) {
-        set_error("gather_leaves_f32_chw: %d x %d pixels are not whole groups of 4 (use the per-leaf call)", h, w);
-        return VN_EUNSUPPORTED;
-    }
-    FloatLeaves L;
-    L.n_leaves = n_leaves;
-    for (int l = 0; l < kMaxFloatLeaves; ++l) {
-        L.pbase[l] = nullptr;
-        L.out[l] = nullptr;
-        L.c[l] = 1;
-        L.goal[l] = 0;
-    }
-    for (int l = 0; l < n_leaves; ++l) {
-        int32_t rc = check_plane(store, leaves[l].plane, h, w, leaves[l].channels, "gather_leaves_f32_chw");
-        if (rc) return rc;
-        if (leaves[l].channels != 1 && leaves[l].channels != 3) {
-            set_error("gather_leaves_f32_chw: %d channels (use the per-leaf call)", leaves[l].channels);
-            return VN_EUNSUPPORTED;
-        }
-        VN_REQUIRE(leaves[l].out && (reinterpret_cast<uintptr_t>(leaves[l].out) & 15) == 0,
-                   "gather_leaves_f32_chw: out[%d] must be 16-byte aligned", l);
-        VN_REQUIRE(leaves[l].source == 0 || leaves[l].source == 1, "gather_leaves_f32_chw: source=%d", leaves[l].source);
-        L.pbase[l] = store->base + store->plane_off[leaves[l].plane];
-        L.out[l] = leaves[l].out;
-        L.c[l] = leaves[l].channels;
-        L.goal[l] = leaves[l].source;
-    }
-    if (n == 0) return VN_OK;
-    const int64_t total = (int64_t)n * (h * w / 4);
-    const int unroll = n_leaves == 1 ? 4 : (n_leaves <= 3 ? 2 : 1);
-    const int64_t want = (total + unroll * 256 - 1) / (unroll * 256), cap = (int64_t)sm_count() * 16;
-    const int grid = (int)(want < cap ? want : cap);
-    const int2 *d2 = reinterpret_cast<const int2 *>(desc);
-    const int64_t pitch = store->state_pitch;
-    const int hw = h * w, early = in_step ? 1 : 0;
-    void (*const kernels[])(FloatLeaves, int64_t, const int2 *, int, int, int) = {
-        vn_gather_leaves_f32_kernel<1, 4>, vn_gather_leaves_f32_kernel<2, 2>, vn_gather_leaves_f32_kernel<3, 2>,
-        vn_gather_leaves_f32_kernel<4, 1>, vn_gather_leaves_f32_kernel<5, 1>, vn_gather_leaves_f32_kernel<6, 1>};
-    // programmatic launch only as part of a step: there the predecessor is the step's own scalar / gather kernel
-    return launch(kernels[n_leaves - 1], "vn_gather_leaves_f32_kernel", dim3(grid), dim3(256), 0,
-                  static_cast<cudaStream_t>(stream), in_step, L, pitch, d2, n, hw, early);
-}
-
-}  // namespace vn
-
-extern "C" {
 
 int32_t vn_gather_leaves_f32_chw(const vn_store_t *store, const vn_float_leaf_t *leaves, int32_t n_leaves,
                                  const int32_t *desc, int32_t n, int32_t h, int32_t w, void *stream) {
@@ -1162,14 +1128,17 @@ int32_t vn_rp_labels(const float *reward, int32_t n, int32_t t, int64_t stride_n
     int32_t rc = vn::launch(vn::vn_rp_count_kernel, "vn_rp_count_kernel", dim3(blocks), dim3(vn::kRpBlock), 0, st, true,
                             reward, n, t, stride_n, stride_t, labels, scratch);
     if (rc) return rc;
-    if (blocks <= 256)  // few blocks (an A2C rollout: 80 blocks at 4,096 envs x 20 steps): no separate scan launch
-        return vn::launch(vn::vn_rp_scatter_kernel, "vn_rp_scatter_kernel", dim3(blocks), dim3(vn::kRpBlock), 0, st, true,
-                          reward, n, t, stride_n, stride_t, scratch, 0, counts, zero_idx, nonzero_idx);
-    rc = vn::launch(vn::vn_rp_scan_kernel, "vn_rp_scan_kernel", dim3(1), dim3(1024), 0, st, true, scratch, blocks, n,
-                    counts);
-    if (rc || !(zero_idx || nonzero_idx)) return rc;
+    // few blocks (an A2C rollout: 80 blocks at 4,096 envs x 20 steps): no separate scan launch, the scatter kernel
+    // sums the block counts itself and writes the totals
+    const bool scan = blocks > 256;
+    if (scan) {
+        rc = vn::launch(vn::vn_rp_scan_kernel, "vn_rp_scan_kernel", dim3(1), dim3(1024), 0, st, true, scratch, blocks, n,
+                        counts);
+        if (rc || !(zero_idx || nonzero_idx)) return rc;
+    }
     return vn::launch(vn::vn_rp_scatter_kernel, "vn_rp_scatter_kernel", dim3(blocks), dim3(vn::kRpBlock), 0, st, true,
-                      reward, n, t, stride_n, stride_t, scratch, 1, (int32_t *)nullptr, zero_idx, nonzero_idx);
+                      reward, n, t, stride_n, stride_t, scratch, scan ? 1 : 0, scan ? nullptr : counts, zero_idx,
+                      nonzero_idx);
 }
 
 }  // extern "C"

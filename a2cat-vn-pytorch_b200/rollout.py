@@ -16,8 +16,12 @@ from . import lib as L
 from .store import DeviceWorld
 
 
-def _stream(t):
-    return torch.cuda.current_stream(t.device).cuda_stream
+def _call(device, fn, *args, stream_of=None):
+    """Calls library entry point ``fn`` with ``device`` current and, as its stream argument, the current stream of the
+    device ``stream_of`` lives on (default: ``device``); raises VnError when the call fails."""
+    with torch.cuda.device(device):
+        stream = torch.cuda.current_stream(device if stream_of is None else stream_of.device).cuda_stream
+        L.check(getattr(L.load(), fn)(*args, stream))
 
 
 def _strided2d(x, dtype):
@@ -39,8 +43,7 @@ def nstep_returns(rewards, dones, last_values, gamma, time_major=False, method="
     method="serial" (default): thread per env, the reference's loop order, bit-identical to it.
     method="scan": warp per env, 32 steps per pass composed with shuffles - for few envs and long rollouts; equal
     within ~1e-6 relative (float re-association), not bit for bit."""
-    lib = L.load()
-    fn = {"serial": lib.vn_nstep_returns, "scan": lib.vn_nstep_returns_scan}[method]
+    fn = {"serial": "vn_nstep_returns", "scan": "vn_nstep_returns_scan"}[method]
     rewards, dones = _strided2d(rewards, torch.float32), _strided2d(dones, torch.uint8)
     if time_major:
         rewards, dones = rewards.t(), dones.t()
@@ -51,24 +54,21 @@ def nstep_returns(rewards, dones, last_values, gamma, time_major=False, method="
     if out is None:
         out = torch.empty((t, n) if time_major else (n, t), dtype=torch.float32, device=rewards.device)
     ob = out.t() if time_major else out
-    with torch.cuda.device(rewards.device):
-        L.check(fn(rewards.data_ptr(), dones.data_ptr(), last_values.data_ptr(), float(gamma), n, t, rewards.stride(0),
-                   rewards.stride(1), out.data_ptr(), ob.stride(0), ob.stride(1), _stream(rewards)))
+    _call(rewards.device, fn, rewards.data_ptr(), dones.data_ptr(), last_values.data_ptr(), float(gamma), n, t,
+          rewards.stride(0), rewards.stride(1), out.data_ptr(), ob.stride(0), ob.stride(1), stream_of=rewards)
     return out
 
 
 def discounted_backup(rewards, dones, bootstrap, gamma):
     """rewards [B, T, ...]; dones [B, T] (any strides); bootstrap [B, ...] -> R_t = r_t + gamma (1 - done_t) R_{t+1}."""
-    lib = L.load()
     b, t = rewards.shape[:2]
     d = rewards[0, 0].numel()
     rewards = rewards.contiguous().float()
     dones = _strided2d(dones, torch.uint8)
     bootstrap = bootstrap.contiguous().float()
     out = torch.empty_like(rewards)
-    with torch.cuda.device(rewards.device):
-        L.check(lib.vn_discounted_backup(rewards.data_ptr(), dones.data_ptr(), dones.stride(0), dones.stride(1),
-                                         bootstrap.data_ptr(), float(gamma), b, t, d, out.data_ptr(), _stream(rewards)))
+    _call(rewards.device, "vn_discounted_backup", rewards.data_ptr(), dones.data_ptr(), dones.stride(0), dones.stride(1),
+          bootstrap.data_ptr(), float(gamma), b, t, d, out.data_ptr(), stream_of=rewards)
     return out
 
 
@@ -82,33 +82,34 @@ def _geom(dw, plane, cell, output_size):
     return pi, h, w, c, int(output_size[0]), int(output_size[1])
 
 
-def _states2d(dw, states):
+def _on_device(dw, states):
     if states.device != dw.device or states.dtype != torch.int32:
         states = states.to(device=dw.device, dtype=torch.int32)
+    return states
+
+
+def _states2d(dw, states):
+    states = _on_device(dw, states)
     if states.dim() != 2:
         raise ValueError("states must be [B, T+1]")
     return states
 
 
 def _pixel_control_direct(dw, states, cell_size, output_size, plane):
-    lib = L.load()
     pi, h, w, c, oh, ow = _geom(dw, plane, cell_size, output_size)
     b, t1 = states.shape
     out = torch.empty((b, t1 - 1, 1, oh, ow), dtype=torch.float32, device=dw.device)
-    with torch.cuda.device(dw.device):
-        L.check(lib.vn_pixel_control(C.byref(dw.store), pi, states.data_ptr(), b, t1 - 1, states.stride(0),
-                                     states.stride(1), h, w, c, cell_size, oh, ow, out.data_ptr(), _stream(states)))
+    _call(dw.device, "vn_pixel_control", C.byref(dw.store), pi, states.data_ptr(), b, t1 - 1, states.stride(0),
+          states.stride(1), h, w, c, cell_size, oh, ow, out.data_ptr(), stream_of=states)
     return out
 
 
 def _aux_direct(dw, states, plane, cell_size, output_size):
-    lib = L.load()
     pi, h, w, c, oh, ow = _geom(dw, plane, cell_size, output_size)
     states = states.contiguous()
     out = torch.empty(tuple(states.shape) + (c, oh, ow), dtype=torch.float32, device=dw.device)
-    with torch.cuda.device(dw.device):
-        L.check(lib.vn_aux_target(C.byref(dw.store), pi, states.data_ptr(), states.numel(), h, w, c, cell_size, oh, ow,
-                                  out.data_ptr(), _stream(states)))
+    _call(dw.device, "vn_aux_target", C.byref(dw.store), pi, states.data_ptr(), states.numel(), h, w, c, cell_size, oh,
+          ow, out.data_ptr(), stream_of=states)
     return out
 
 
@@ -158,6 +159,14 @@ class TargetTables:
                                   torch.zeros(1, dtype=torch.int32, device=dev))
         return self._scratch[key]
 
+    def miss_rows(self, max_miss):
+        """float32 [max_miss, oh * ow] side buffer of the chained call (the rewards of the transitions the table cannot
+        serve), reused between calls."""
+        key = ("miss", max_miss)
+        if key not in self._scratch:
+            self._scratch[key] = torch.empty((max_miss, self.pc.shape[1]), dtype=torch.float32, device=self.dw.device)
+        return self._scratch[key]
+
     def nbytes(self):
         return self.pc.numel() * 4 + sum(t.numel() * 4 for t in self._aux.values())
 
@@ -179,7 +188,6 @@ def pixel_control_reward(dw: DeviceWorld, states, cell_size=4, output_size=None,
     method="table" (default): rows of the per-world transition table (TargetTables) are gathered; the few
     transitions the table cannot serve (resets) are computed directly by a list kernel in the same pass.
     method="direct": every transition is computed from the two frames.  Both give identical bits."""
-    lib = L.load()
     pi, h, w, c, oh, ow = _geom(dw, plane, cell_size, output_size)
     states = _states2d(dw, states)
     if method == "direct" or (oh * ow) % 4:
@@ -189,15 +197,14 @@ def pixel_control_reward(dw: DeviceWorld, states, cell_size=4, output_size=None,
     t = t1 - 1
     out = torch.empty((b, t, 1, oh, ow), dtype=torch.float32, device=dw.device)
     rows, miss_pos, miss_count = tab.scratch(b * t)
-    sn, st_ = states.stride()
-    with torch.cuda.device(dw.device):
-        st = _stream(states)
-        rsn, rst = t, 1          # batch-major row scratch (the lookup kernel orders its threads for coalesced state reads)
-        L.check(lib.vn_transition_rows(dw.adj.data_ptr(), states.data_ptr(), b, t, sn, st_, rows.data_ptr(), rsn, rst,
-                                       miss_pos.data_ptr(), miss_count.data_ptr(), st))
-        L.check(lib.vn_gather_rows(tab.pc.data_ptr(), oh * ow * 4, rows.data_ptr(), b * t, t, rsn, rst, out.data_ptr(), st))
-        L.check(lib.vn_pixel_control_list(C.byref(dw.store), pi, states.data_ptr(), b, t, sn, st_, h, w, c, cell_size, oh,
-                                          ow, miss_pos.data_ptr(), miss_count.data_ptr(), b * t, 0, out.data_ptr(), st))
+    sn, st = states.stride()
+    rsn, rst = t, 1          # batch-major row scratch (the lookup kernel orders its threads for coalesced state reads)
+    _call(dw.device, "vn_transition_rows", dw.adj.data_ptr(), states.data_ptr(), b, t, sn, st, rows.data_ptr(), rsn, rst,
+          miss_pos.data_ptr(), miss_count.data_ptr(), stream_of=states)
+    _call(dw.device, "vn_gather_rows", tab.pc.data_ptr(), oh * ow * 4, rows.data_ptr(), b * t, t, rsn, rst, out.data_ptr(),
+          stream_of=states)
+    _call(dw.device, "vn_pixel_control_list", C.byref(dw.store), pi, states.data_ptr(), b, t, sn, st, h, w, c, cell_size,
+          oh, ow, miss_pos.data_ptr(), miss_count.data_ptr(), b * t, 0, out.data_ptr(), stream_of=states)
     return out
 
 
@@ -210,7 +217,6 @@ def pixel_control_returns(dw: DeviceWorld, states, dones, bootstrap, gamma, cell
     states int32 [B, T+1], dones uint8/bool [B, T] (any strides: ``storage.t()`` views are read in place), bootstrap
     float32 [B, h*w] (or [B, h, w]).  Returns float32 [B, T, h*w] (and the rewards [B, T, h*w] with with_reward).
     max_miss bounds the side buffer for the transitions the table cannot serve (episode resets; default: all B*T)."""
-    lib = L.load()
     pi, h, w, c, oh, ow = _geom(dw, plane, cell_size, output_size)
     cells = oh * ow
     if cells % 4:
@@ -226,19 +232,14 @@ def pixel_control_returns(dw: DeviceWorld, states, dones, bootstrap, gamma, cell
     out = torch.empty((b, t, cells), dtype=torch.float32, device=dw.device)
     rew = torch.empty((b, t, cells), dtype=torch.float32, device=dw.device) if with_reward else None
     rows, miss_pos, miss_count = tab.scratch(b * t, chained=True)
-    max_miss = b * t if max_miss is None else int(max_miss)
-    key = ("miss", max_miss, cells)
-    side = tab._aux.get(key)
-    if side is None:
-        side = tab._aux[key] = torch.empty((max(max_miss, 1), cells), dtype=torch.float32, device=dw.device)
-    sn, st_ = states.stride()
-    with torch.cuda.device(dw.device):
-        # one C call, three chained kernels: transition rows -> misses computed directly -> gather + back-up
-        L.check(lib.vn_pixel_control_returns_from_states(
-            C.byref(dw.store), pi, dw.adj.data_ptr(), tab.pc.data_ptr(), states.data_ptr(), sn, st_, dones.data_ptr(),
-            dones.stride(0), dones.stride(1), bootstrap.data_ptr(), float(gamma), b, t, h, w, c, cell_size, oh, ow,
-            rows.data_ptr(), miss_pos.data_ptr(), miss_count.data_ptr(), side.data_ptr(), max(max_miss, 1),
-            out.data_ptr(), L.ptr(rew), _stream(states)))
+    max_miss = max(b * t if max_miss is None else int(max_miss), 1)
+    side = tab.miss_rows(max_miss)
+    sn, st = states.stride()
+    # one C call, three chained kernels: transition rows -> misses computed directly -> gather + back-up
+    _call(dw.device, "vn_pixel_control_returns_from_states", C.byref(dw.store), pi, dw.adj.data_ptr(), tab.pc.data_ptr(),
+          states.data_ptr(), sn, st, dones.data_ptr(), dones.stride(0), dones.stride(1), bootstrap.data_ptr(),
+          float(gamma), b, t, h, w, c, cell_size, oh, ow, rows.data_ptr(), miss_pos.data_ptr(), miss_count.data_ptr(),
+          side.data_ptr(), max_miss, out.data_ptr(), L.ptr(rew), stream_of=states)
     return (out, rew) if with_reward else out
 
 
@@ -246,10 +247,8 @@ def auxiliary_target(dw: DeviceWorld, states, plane, cell_size=4, output_size=No
     """compute_auxiliary_target (experiments/ai2_auxiliary/trainer.py:9-15) from state indices.
     states int32 [B, T] (any strides) -> float32 [B, T, C, h, w].  method="table": one row gather from the per-world
     pooled-plane table; method="direct": pooled from the frame."""
-    lib = L.load()
     pi, h, w, c, oh, ow = _geom(dw, plane, cell_size, output_size)
-    if states.device != dw.device or states.dtype != torch.int32:
-        states = states.to(device=dw.device, dtype=torch.int32)
+    states = _on_device(dw, states)
     if method == "direct" or (c * oh * ow) % 4:
         return _aux_direct(dw, states, plane, cell_size, (oh, ow))
     shape = tuple(states.shape)
@@ -257,9 +256,8 @@ def auxiliary_target(dw: DeviceWorld, states, plane, cell_size=4, output_size=No
         states = states.contiguous().view(-1, 1)
     tab = target_tables(dw, cell_size, (oh, ow)).aux(plane)
     out = torch.empty(shape + (c, oh, ow), dtype=torch.float32, device=dw.device)
-    with torch.cuda.device(dw.device):
-        L.check(lib.vn_gather_rows(tab.data_ptr(), c * oh * ow * 4, states.data_ptr(), states.numel(), states.shape[1],
-                                   states.stride(0), states.stride(1), out.data_ptr(), _stream(states)))
+    _call(dw.device, "vn_gather_rows", tab.data_ptr(), c * oh * ow * 4, states.data_ptr(), states.numel(),
+          states.shape[1], states.stride(0), states.stride(1), out.data_ptr(), stream_of=states)
     return out
 
 
@@ -273,13 +271,11 @@ def auxiliary_targets(dw, states, goal_states, cell_size=4, output_size=None, me
 
 def policy_input(dw: DeviceWorld, states, plane="rgb"):
     """TransposeImage + ScaledFloatFrame fused with the gather: float32 [..., C, H, W] in [0, 1]."""
-    lib = L.load()
     pi, h, w, c, _, _ = _geom(dw, plane, 1, None)
     states = states.to(device=dw.device, dtype=torch.int32).contiguous()
     out = torch.empty(tuple(states.shape) + (c, h, w), dtype=torch.float32, device=dw.device)
-    with torch.cuda.device(dw.device):
-        L.check(lib.vn_gather_plane_f32_chw(C.byref(dw.store), pi, states.data_ptr(), states.numel(), h, w, c,
-                                            out.data_ptr(), _stream(states)))
+    _call(dw.device, "vn_gather_plane_f32_chw", C.byref(dw.store), pi, states.data_ptr(), states.numel(), h, w, c,
+          out.data_ptr(), stream_of=states)
     return out
 
 
@@ -290,7 +286,6 @@ def reward_prediction_labels(rewards, with_lists=True, sync=True, buffers=None):
     Returns (labels int8 [B, T] contiguous, zero_idx int32, nonzero_idx int32).  sync=True: the lists are trimmed
     to their lengths (one 8-byte D2H read for the two counts).  sync=False: nothing waits for the device - the
     lists come back at full length together with a device tensor ``counts`` = (#zero, #non-zero) as a 4th value."""
-    lib = L.load()
     r = rewards if rewards.dtype == torch.float32 else rewards.float()
     flat = r.dim() != 2
     if flat:
@@ -298,21 +293,19 @@ def reward_prediction_labels(rewards, with_lists=True, sync=True, buffers=None):
     n = r.numel()
     if buffers is not None:          # (labels, zero, nonzero, counts, scratch) owned by the caller, reused call after call
         labels, zero, nonzero, counts, scratch = buffers
-        with torch.cuda.device(r.device):
-            L.check(lib.vn_rp_labels(r.data_ptr(), n, r.shape[1], r.stride(0), r.stride(1), labels.data_ptr(), L.ptr(zero),
-                                     L.ptr(nonzero), counts.data_ptr(), scratch.data_ptr(), _stream(r)))
+    else:
+        labels = torch.empty(tuple(rewards.shape), dtype=torch.int8, device=r.device)
+        if n == 0:
+            e = torch.empty(0, dtype=torch.int32, device=r.device)
+            return labels, (e if with_lists else None), (e.clone() if with_lists else None)
+        scratch = torch.empty((n + 1023) // 1024 + 1, dtype=torch.int32, device=r.device)
+        counts = torch.empty(2, dtype=torch.int32, device=r.device)     # always written by the scan kernel
+        zero = torch.empty(n, dtype=torch.int32, device=r.device) if with_lists else None
+        nonzero = torch.empty(n, dtype=torch.int32, device=r.device) if with_lists else None
+    _call(r.device, "vn_rp_labels", r.data_ptr(), n, r.shape[1], r.stride(0), r.stride(1), labels.data_ptr(), L.ptr(zero),
+          L.ptr(nonzero), counts.data_ptr(), scratch.data_ptr(), stream_of=r)
+    if buffers is not None:
         return labels, zero, nonzero, counts
-    labels = torch.empty(tuple(rewards.shape), dtype=torch.int8, device=r.device)
-    if n == 0:
-        e = torch.empty(0, dtype=torch.int32, device=r.device)
-        return labels, (e if with_lists else None), (e.clone() if with_lists else None)
-    scratch = torch.empty((n + 1023) // 1024 + 1, dtype=torch.int32, device=r.device)
-    counts = torch.empty(2, dtype=torch.int32, device=r.device)     # always written by the scan kernel
-    zero = torch.empty(n, dtype=torch.int32, device=r.device) if with_lists else None
-    nonzero = torch.empty(n, dtype=torch.int32, device=r.device) if with_lists else None
-    with torch.cuda.device(r.device):
-        L.check(lib.vn_rp_labels(r.data_ptr(), n, r.shape[1], r.stride(0), r.stride(1), labels.data_ptr(), L.ptr(zero),
-                                 L.ptr(nonzero), counts.data_ptr(), scratch.data_ptr(), _stream(r)))
     if not with_lists:
         return labels, None, None
     if not sync:
@@ -484,7 +477,6 @@ class ReplayRing:
         self.count = min(self.count + T, self.cap)
 
     def _sample(self, length, mode):
-        lib = L.load()
         Lw = 4 if mode == 1 else length
         dev, n = self.dw.device, self.N
         out = dict(states=torch.zeros((n, Lw + 1), dtype=torch.int32, device=dev),
@@ -498,11 +490,9 @@ class ReplayRing:
         ring = L.Replay(self.before.data_ptr(), self.after.data_ptr(), self.goal.data_ptr(), self.goal_before.data_ptr(),
                         self.action.data_ptr(),
                         self.reward.data_ptr(), self.done.data_ptr(), n, self.cap, self.head, self.count)
-        with torch.cuda.device(dev):
-            L.check(lib.vn_replay_sample(C.byref(ring), Lw, mode, C.c_uint64(self.seed), self.calls, self.env_id_base,
-                                         out["states"].data_ptr(), out["goals"].data_ptr(), out["actions"].data_ptr(),
-                                         out["rewards"].data_ptr(), out["dones"].data_ptr(), out["start"].data_ptr(),
-                                         L.ptr(out.get("label")), torch.cuda.current_stream(dev).cuda_stream))
+        _call(dev, "vn_replay_sample", C.byref(ring), Lw, mode, C.c_uint64(self.seed), self.calls, self.env_id_base,
+              out["states"].data_ptr(), out["goals"].data_ptr(), out["actions"].data_ptr(), out["rewards"].data_ptr(),
+              out["dones"].data_ptr(), out["start"].data_ptr(), L.ptr(out.get("label")))
         self.calls += 1
         return out
 
