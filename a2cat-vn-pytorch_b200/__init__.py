@@ -13,7 +13,8 @@ def __getattr__(name):
     # torch / CUDA dependent modules are imported lazily so that the host-side compiler and the
     # synthetic scenes stay usable (and testable) without torch being imported.
     import importlib
-    if name in ("lib", "store", "vec_env", "rollout", "build", "loaders", "single_env", "evaluation"):
+    if name in ("lib", "store", "vec_env", "rollout", "build", "loaders", "single_env", "evaluation",
+                "nn"):
         return importlib.import_module("." + name, __name__)
     if name in ("GraphVecEnv", "shard_range", "gather_plane", "reduce_stats"):
         return getattr(importlib.import_module(".vec_env", __name__), name)

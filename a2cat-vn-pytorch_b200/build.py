@@ -11,7 +11,7 @@ PKG = os.path.dirname(os.path.abspath(__file__))
 ROOT = os.path.dirname(PKG)
 CSRC = os.path.join(PKG, "csrc")
 LIB = os.path.join(PKG, "libvn_b200.so")
-SOURCES = ["vn_env.cu", "vn_rollout.cu"]
+SOURCES = ["vn_env.cu", "vn_rollout.cu", "vn_conv.cu"]
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17", "--use_fast_math=false",
               "-Xcompiler", "-fPIC,-O3,-Wall", "-shared", "-cudart", "shared"]
 

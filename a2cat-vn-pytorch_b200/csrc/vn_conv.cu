@@ -1,0 +1,550 @@
+// libvn_b200 - the policy's first convolution read straight from uint8 frames (sm_100a).
+//
+// Replaces TransposeImage + ScaledFloatFrame (deep_rl.common.env, thor_cached_auxiliary.py:61-62) + the model's first
+// Conv2d (models/goal.py:36-41): y = conv2d(x / 255, weight, bias, stride) with x the uint8 HWC frame of an observation
+// batch row or of a store record, and the weight / bias gradient of that layer.  No float copy of a frame is written.
+//
+// Numerics.  A pixel is an integer 0..255, exact in bf16.  The fp32 operand (the weight in the forward, grad_out in the
+// weight gradient) is split into three bf16 terms hi + mid + lo (24 significant bits in all), so every product on the
+// tensor cores is exact.  Per 16-deep k-step the three terms are chained through one mma.sync accumulator started at
+// zero, and that k-step's sum is added to an fp32 register accumulator with a round-to-nearest FADD; the 1/255 scale is
+// one division at the end.  The weight gradient's partial sums per fixed chunk of frames are reduced in a fixed order
+// by a second kernel: no float atomics, the same bits on any number of SMs.
+#include <cuda_bf16.h>
+
+#include "vn_common.cuh"
+
+namespace vn {
+
+constexpr int kMaxSmemConv = 220 * 1024;  // dynamic shared memory one CTA can have
+constexpr int kMaxFrameSide = 174;        // the reference's native frame (INTEGRATION.md section 1)
+constexpr int kFwdWarps = 4;
+constexpr int kWgradWarps = 8;
+constexpr int kWgradTiles = 13;    // (cout, tap) tiles of 16 x 8 per warp: 4 x 25 at most over 8 warps
+constexpr int kWgradChunk = 32;    // frames per partial gradient
+constexpr int kReduceLanes = 32;   // chunks summed in parallel per output of the reduce kernel
+
+// ---------------------------------------------------------------- device helpers
+__device__ __forceinline__ const uint8_t *frame_src(const vn_u8_frames_t &f, int i) {
+    int64_t rec = i;
+    if (f.idx) {
+        const int a = i / f.idx_t, k = i - a * f.idx_t;
+        rec = f.idx[a * f.idx_stride_n + k * f.idx_stride_t];
+    }
+    return f.base + rec * f.pitch;
+}
+// byte -> float, exact, without the integer-conversion pipe
+__device__ __forceinline__ float u8f(uint32_t v) { return __int_as_float(0x4B000000u | v) - 8388608.f; }
+// two floats of at most 8 significant bits as bf16x2 (exact truncation), lo in the low half
+__device__ __forceinline__ uint32_t pack_exact(float lo, float hi) {
+    return __byte_perm(__float_as_uint(lo), __float_as_uint(hi), 0x7632);
+}
+__device__ __forceinline__ uint32_t bf2_bits(__nv_bfloat162 v) { return *reinterpret_cast<uint32_t *>(&v); }
+// (a, b) = hi + mid + lo, each a bf16x2 with a in the low half; every residual is exact in fp32
+__device__ __forceinline__ void split3(float a, float b, uint32_t &hi, uint32_t &mid, uint32_t &lo) {
+    const __nv_bfloat162 h = __floats2bfloat162_rn(a, b);
+    const float2 hf = __bfloat1622float2(h);
+    const float ra = __fsub_rn(a, hf.x), rb = __fsub_rn(b, hf.y);
+    const __nv_bfloat162 m = __floats2bfloat162_rn(ra, rb);
+    const float2 mf = __bfloat1622float2(m);
+    hi = bf2_bits(h);
+    mid = bf2_bits(m);
+    lo = bf2_bits(__floats2bfloat162_rn(__fsub_rn(ra, mf.x), __fsub_rn(rb, mf.y)));
+}
+// d = a * b + c, m16n8k16, bf16 in, fp32 accumulate
+__device__ __forceinline__ void mma16816(float (&d)[4], const uint32_t (&a)[4], uint32_t b0, uint32_t b1,
+                                         const float (&c)[4]) {
+    asm volatile(
+        "mma.sync.aligned.m16n8k16.row.col.f32.bf16.bf16.f32 {%0,%1,%2,%3}, {%4,%5,%6,%7}, {%8,%9}, "
+        "{%10,%11,%12,%13};"
+        : "=f"(d[0]), "=f"(d[1]), "=f"(d[2]), "=f"(d[3])
+        : "r"(a[0]), "r"(a[1]), "r"(a[2]), "r"(a[3]), "r"(b0), "r"(b1), "f"(c[0]), "f"(c[1]), "f"(c[2]), "f"(c[3]));
+}
+// acc += (a_hi + a_mid + a_lo) * b over one k-step (operand split on A)
+__device__ __forceinline__ void mma_split_a(float (&acc)[4], const uint32_t (&ah)[4], const uint32_t (&am)[4],
+                                            const uint32_t (&al)[4], uint32_t b0, uint32_t b1) {
+    const float z[4] = {0.f, 0.f, 0.f, 0.f};
+    float d[4];
+    mma16816(d, al, b0, b1, z);
+    mma16816(d, am, b0, b1, d);
+    mma16816(d, ah, b0, b1, d);
+#pragma unroll
+    for (int q = 0; q < 4; ++q) acc[q] = __fadd_rn(acc[q], d[q]);
+}
+// acc += a * (b_hi + b_mid + b_lo) over one k-step (operand split on B)
+__device__ __forceinline__ void mma_split_b(float (&acc)[4], const uint32_t (&a)[4], uint2 bh, uint2 bm, uint2 bl) {
+    const float z[4] = {0.f, 0.f, 0.f, 0.f};
+    float d[4];
+    mma16816(d, a, bl.x, bl.y, z);
+    mma16816(d, a, bm.x, bm.y, d);
+    mma16816(d, a, bh.x, bh.y, d);
+#pragma unroll
+    for (int q = 0; q < 4; ++q) acc[q] = __fadd_rn(acc[q], d[q]);
+}
+// byte offset of output pixel p's window corner inside an HWC frame
+__device__ __forceinline__ int pix_base(int p, int ow, int stride, int w, int c) {
+    const int oy = p / ow, ox = p - oy * ow;
+    return (oy * stride * w + ox * stride) * c;
+}
+
+// The frames of a CTA, double-buffered in shared memory (one buffer when two do not fit): frame number `it` of the
+// CTA's sequence sits in buffer it % nbuf and completes phase it / nbuf of that buffer's mbarrier.
+struct FramePipe {
+    uint8_t *buf;
+    uint64_t *bar;
+    int fb, nbuf;
+    __device__ void load(int slot, const uint8_t *src) const {
+        mbar_expect_tx(&bar[slot], (uint32_t)fb);
+        bulk_g2s(buf + (size_t)slot * fb, src, (uint32_t)fb, &bar[slot]);
+    }
+    __device__ const uint8_t *wait(int it) const {
+        const int slot = nbuf == 2 ? (it & 1) : 0;
+        mbar_wait(&bar[slot], (uint32_t)((nbuf == 2 ? it >> 1 : it) & 1));
+        return buf + (size_t)slot * fb;
+    }
+    __device__ int slot(int it) const { return nbuf == 2 ? (it & 1) : 0; }
+};
+
+struct FwdArgs {
+    vn_u8_frames_t src;
+    const float *weight;   // [cout][K], K = c * k * k
+    const float *bias;     // [cout] or null
+    float *out;            // [n][cout][oh][ow]
+    int k, stride, oh, ow, K, ksteps, nbuf, fb;
+};
+
+// Persistent grid; a CTA owns whole frames.  Its prologue splits the weights into shared memory in mma B-fragment order
+// ([k-step][n-tile][hi, mid, lo][lane] uint2).  A warp owns two 16-pixel m-tiles of a frame and every output channel;
+// the A fragments are the frame's bytes picked through a tap-offset table (implicit im2col).  Each C fragment row is 8
+// consecutive pixels of one channel, so every store instruction writes whole 32-byte sectors of the NCHW output.
+template <int NT>   // cout / 8
+__global__ void __launch_bounds__(kFwdWarps * 32) vn_conv_u8_fwd_kernel(const FwdArgs a) {
+    extern __shared__ __align__(128) uint8_t smem[];
+    const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31, g = lane >> 2, tig = lane & 3;
+    const int w = a.src.w, c = a.src.c, K = a.K, ksteps = a.ksteps;
+    uint2 *wfrag = reinterpret_cast<uint2 *>(smem + (size_t)a.nbuf * a.fb);
+    int *tap = reinterpret_cast<int *>(wfrag + ksteps * NT * 3 * 32);
+    float *sbias = reinterpret_cast<float *>(tap + ksteps * 16);
+    uint64_t *bar = reinterpret_cast<uint64_t *>(sbias + NT * 8);
+    const FramePipe pipe{smem, bar, a.fb, a.nbuf};
+
+    const int kk2 = a.k * a.k;
+    for (int t = tid; t < ksteps * 16; t += blockDim.x) {
+        int off = 0;   // padding taps read byte 0: their weight is zero
+        if (t < K) {
+            const int ci = t / kk2, r = t - ci * kk2, ky = r / a.k, kx = r - ky * a.k;
+            off = (ky * w + kx) * c + ci;
+        }
+        tap[t] = off;
+    }
+    if (tid == 0) {
+        mbar_init(&bar[0], 1);
+        mbar_init(&bar[1], 1);
+        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+    }
+    // the weights, indices and frames may be written by the kernels before this one; nothing is released early, so a
+    // following env step cannot rewrite the batch rows or obs_state while they are read here
+    asm volatile("griddepcontrol.wait;" ::: "memory");
+    for (int e = tid; e < ksteps * NT * 32; e += blockDim.x) {
+        const int ln = e & 31, j = (e >> 5) % NT, ks = (e >> 5) / NT;
+        const int n = j * 8 + (ln >> 2), k0 = ks * 16 + (ln & 3) * 2;
+        const float *wr = a.weight + (size_t)n * K;
+        const float v0 = k0 < K ? wr[k0] : 0.f, v1 = k0 + 1 < K ? wr[k0 + 1] : 0.f;
+        const float v8 = k0 + 8 < K ? wr[k0 + 8] : 0.f, v9 = k0 + 9 < K ? wr[k0 + 9] : 0.f;
+        uint32_t h0, m0, l0, h1, m1, l1;
+        split3(v0, v1, h0, m0, l0);
+        split3(v8, v9, h1, m1, l1);
+        uint2 *dst = wfrag + (size_t)(ks * NT + j) * 96 + ln;
+        dst[0] = make_uint2(h0, h1);
+        dst[32] = make_uint2(m0, m1);
+        dst[64] = make_uint2(l0, l1);
+    }
+    for (int co = tid; co < NT * 8; co += blockDim.x) sbias[co] = a.bias ? a.bias[co] : 0.f;
+    const int n = a.src.n;
+    if (tid == 0)
+        for (int s = 0; s < a.nbuf; ++s) {
+            const int f = blockIdx.x + s * gridDim.x;
+            if (f < n) pipe.load(s, frame_src(a.src, f));
+        }
+    __syncthreads();
+
+    const int P = a.oh * a.ow, tasks = ((P + 15) / 16 + 1) / 2;
+    int it = 0;
+    for (int f = blockIdx.x; f < n; f += gridDim.x, ++it) {
+        const uint8_t *x = pipe.wait(it);
+        float *out = a.out + (int64_t)f * (NT * 8) * P;
+        for (int task = warp; task < tasks; task += kFwdWarps) {
+            int pb[2][2];
+#pragma unroll
+            for (int mt = 0; mt < 2; ++mt)
+#pragma unroll
+                for (int r = 0; r < 2; ++r) {
+                    const int p = (task * 2 + mt) * 16 + g + r * 8;
+                    pb[mt][r] = p < P ? pix_base(p, a.ow, a.stride, w, c) : 0;
+                }
+            float acc[2][NT][4];
+#pragma unroll
+            for (int mt = 0; mt < 2; ++mt)
+#pragma unroll
+                for (int j = 0; j < NT; ++j)
+#pragma unroll
+                    for (int q = 0; q < 4; ++q) acc[mt][j][q] = 0.f;
+#pragma unroll 1
+            for (int ks = 0; ks < ksteps; ++ks) {
+                const int2 t01 = *reinterpret_cast<const int2 *>(tap + ks * 16 + tig * 2);
+                const int2 t89 = *reinterpret_cast<const int2 *>(tap + ks * 16 + tig * 2 + 8);
+                uint32_t af[2][4];
+#pragma unroll
+                for (int mt = 0; mt < 2; ++mt)
+#pragma unroll
+                    for (int r = 0; r < 2; ++r) {
+                        const uint8_t *row = x + pb[mt][r];
+                        af[mt][r] = pack_exact(u8f(row[t01.x]), u8f(row[t01.y]));
+                        af[mt][2 + r] = pack_exact(u8f(row[t89.x]), u8f(row[t89.y]));
+                    }
+                const uint2 *wf = wfrag + (size_t)ks * NT * 96 + lane;
+#pragma unroll
+                for (int j = 0; j < NT; ++j) {
+                    const uint2 bh = wf[j * 96], bm = wf[j * 96 + 32], bl = wf[j * 96 + 64];
+                    mma_split_b(acc[0][j], af[0], bh, bm, bl);
+                    mma_split_b(acc[1][j], af[1], bh, bm, bl);
+                }
+            }
+#pragma unroll
+            for (int mt = 0; mt < 2; ++mt)
+#pragma unroll
+                for (int r = 0; r < 2; ++r) {
+                    const int p = (task * 2 + mt) * 16 + g + r * 8;
+                    if (p >= P) continue;
+#pragma unroll
+                    for (int j = 0; j < NT; ++j) {
+                        const int co = j * 8 + tig * 2;
+                        out[(int64_t)co * P + p] = __fadd_rn(__fdiv_rn(acc[mt][j][2 * r], 255.f), sbias[co]);
+                        out[(int64_t)(co + 1) * P + p] =
+                            __fadd_rn(__fdiv_rn(acc[mt][j][2 * r + 1], 255.f), sbias[co + 1]);
+                    }
+                }
+        }
+        __syncthreads();   // every warp is done with this buffer
+        const int next = f + a.nbuf * gridDim.x;
+        if (tid == 0 && next < n) {
+            fence_proxy_async();
+            pipe.load(pipe.slot(it), frame_src(a.src, next));
+        }
+    }
+}
+
+struct WgradArgs {
+    vn_u8_frames_t src;
+    const float *grad_out;   // [n][cout][oh][ow]
+    float *partial;          // [chunks][cout][K + 1]
+    int cout, k, stride, oh, ow, K, mtiles, ntiles, nbuf, fb;
+};
+
+// The frames of chunk q are [q * kWgradChunk, ...): the CTA's next frame after f.
+__device__ __forceinline__ int next_frame(int f, int n) {
+    const int chunk_end = min(n, (f / kWgradChunk + 1) * kWgradChunk);
+    return f + 1 < chunk_end ? f + 1 : (f / kWgradChunk + (int)gridDim.x) * kWgradChunk;
+}
+
+// dW[co][t] = sum over the chunk's frames and output pixels p of g[co][p] * x[tap t of p]: an implicit GEMM with
+// M = cout, N = taps + 1 (the last tap reads 1: the bias gradient), K = pixels.  grad_out is the split operand (A, read
+// from global: each fragment row is 8 consecutive floats of one channel), the frame's bytes are B.  A warp owns up to
+// kWgradTiles (16 x 8) output tiles for the whole chunk.  Its registers sum one frame; the frame sums are added into
+// the thread's own shared-memory column, and the chunk's raw sums go to partial[chunk].
+__global__ void __launch_bounds__(kWgradWarps * 32) vn_conv_u8_wgrad_kernel(const WgradArgs a) {
+    extern __shared__ __align__(128) uint8_t smem[];
+    const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31, g = lane >> 2, tig = lane & 3;
+    const int w = a.src.w, c = a.src.c, K = a.K, K1 = a.K + 1, cout = a.cout;
+    int *tap = reinterpret_cast<int *>(smem + (size_t)a.nbuf * a.fb);
+    uint64_t *bar = reinterpret_cast<uint64_t *>(tap + a.ntiles * 8);
+    float *chunk_acc = reinterpret_cast<float *>(bar + 2) + tid;   // this thread's [kWgradTiles * 4] column
+    const FramePipe pipe{smem, bar, a.fb, a.nbuf};
+
+    const int kk2 = a.k * a.k;
+    for (int t = tid; t < a.ntiles * 8; t += blockDim.x) {
+        int off = t == K ? -1 : -2;   // -1: the bias tap (reads 1), -2: padding (reads 0)
+        if (t < K) {
+            const int ci = t / kk2, r = t - ci * kk2, ky = r / a.k, kx = r - ky * a.k;
+            off = (ky * w + kx) * c + ci;
+        }
+        tap[t] = off;
+    }
+    if (tid == 0) {
+        mbar_init(&bar[0], 1);
+        mbar_init(&bar[1], 1);
+        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+    }
+    asm volatile("griddepcontrol.wait;" ::: "memory");
+    __syncthreads();
+
+    const int tiles = a.mtiles * a.ntiles, per = (tiles + kWgradWarps - 1) / kWgradWarps;
+    const int t0 = warp * per, cnt = max(0, min(per, tiles - t0));
+    int tmi[kWgradTiles], toff[kWgradTiles];
+#pragma unroll
+    for (int i = 0; i < kWgradTiles; ++i) {
+        const int tl = i < cnt ? t0 + i : 0, mi = tl / a.ntiles;
+        tmi[i] = mi;
+        toff[i] = tap[(tl - mi * a.ntiles) * 8 + g];
+    }
+
+    const int n = a.src.n, P = a.oh * a.ow, ksteps = (P + 15) / 16;
+    int f = blockIdx.x * kWgradChunk;
+    if (tid == 0 && f < n) {
+        pipe.load(0, frame_src(a.src, f));
+        const int f1 = next_frame(f, n);
+        if (a.nbuf == 2 && f1 < n) pipe.load(1, frame_src(a.src, f1));
+    }
+    int it = 0;
+    for (int chunk = blockIdx.x; chunk * kWgradChunk < n; chunk += gridDim.x) {
+        float acc[kWgradTiles][4];
+#pragma unroll
+        for (int i = 0; i < kWgradTiles; ++i)
+#pragma unroll
+            for (int q = 0; q < 4; ++q) {
+                acc[i][q] = 0.f;
+                chunk_acc[(i * 4 + q) * kWgradWarps * 32] = 0.f;
+            }
+        const int end = min(n, (chunk + 1) * kWgradChunk);
+        for (; f < end; f = next_frame(f, n), ++it) {
+            const uint8_t *x = pipe.wait(it);
+            const float *gf = a.grad_out + (int64_t)f * cout * P;
+#pragma unroll 1
+            for (int ks = 0; ks < ksteps; ++ks) {
+                const int p0 = ks * 16 + tig * 2;
+                const int pb0 = p0 < P ? pix_base(p0, a.ow, a.stride, w, c) : 0;
+                const int pb1 = p0 + 1 < P ? pix_base(p0 + 1, a.ow, a.stride, w, c) : 0;
+                const int pb8 = p0 + 8 < P ? pix_base(p0 + 8, a.ow, a.stride, w, c) : 0;
+                const int pb9 = p0 + 9 < P ? pix_base(p0 + 9, a.ow, a.stride, w, c) : 0;
+                int cur = -1;
+                uint32_t ah[4], am[4], al[4];
+#pragma unroll
+                for (int i = 0; i < kWgradTiles; ++i) {
+                    if (i >= cnt) break;
+                    if (tmi[i] != cur) {   // warp-uniform: the warp's tiles are sorted by m-tile
+                        cur = tmi[i];
+#pragma unroll
+                        for (int r = 0; r < 2; ++r) {
+                            const int co = cur * 16 + g + r * 8;
+                            const float *gr = gf + (int64_t)co * P;
+                            const bool ok = co < cout;
+                            const float v0 = ok && p0 < P ? gr[p0] : 0.f, v1 = ok && p0 + 1 < P ? gr[p0 + 1] : 0.f;
+                            const float v8 = ok && p0 + 8 < P ? gr[p0 + 8] : 0.f;
+                            const float v9 = ok && p0 + 9 < P ? gr[p0 + 9] : 0.f;
+                            split3(v0, v1, ah[r], am[r], al[r]);
+                            split3(v8, v9, ah[2 + r], am[2 + r], al[2 + r]);
+                        }
+                    }
+                    const int o = toff[i];
+                    float b0, b1, b8, b9;
+                    if (o >= 0) {
+                        b0 = u8f(x[pb0 + o]);
+                        b1 = u8f(x[pb1 + o]);
+                        b8 = u8f(x[pb8 + o]);
+                        b9 = u8f(x[pb9 + o]);
+                    } else {
+                        b0 = b1 = b8 = b9 = o == -1 ? 1.f : 0.f;
+                    }
+                    mma_split_a(acc[i], ah, am, al, pack_exact(b0, b1), pack_exact(b8, b9));
+                }
+            }
+            // the frame's sums join the chunk's in shared memory: no register sum runs over more than one frame
+#pragma unroll
+            for (int i = 0; i < kWgradTiles; ++i)
+#pragma unroll
+                for (int q = 0; q < 4; ++q) {
+                    float &s = chunk_acc[(i * 4 + q) * kWgradWarps * 32];
+                    s = __fadd_rn(s, acc[i][q]);
+                    acc[i][q] = 0.f;
+                }
+            __syncthreads();   // every warp is done with this buffer
+            if (tid == 0) {
+                int nx = next_frame(f, n);
+                if (a.nbuf == 2 && nx < n) nx = next_frame(nx, n);
+                if (nx < n) {
+                    fence_proxy_async();
+                    pipe.load(pipe.slot(it), frame_src(a.src, nx));
+                }
+            }
+        }
+        float *part = a.partial + (int64_t)chunk * cout * K1;
+#pragma unroll
+        for (int i = 0; i < kWgradTiles; ++i) {
+            if (i >= cnt) break;
+            const int tl = t0 + i, mi = tmi[i], nj = tl - mi * a.ntiles;
+#pragma unroll
+            for (int r = 0; r < 2; ++r) {
+                const int co = mi * 16 + g + r * 8, t = nj * 8 + tig * 2;
+                if (co >= cout) continue;
+                if (t < K1) part[(int64_t)co * K1 + t] = chunk_acc[(i * 4 + 2 * r) * kWgradWarps * 32];
+                if (t + 1 < K1) part[(int64_t)co * K1 + t + 1] = chunk_acc[(i * 4 + 2 * r + 1) * kWgradWarps * 32];
+            }
+        }
+    }
+}
+
+// out[o] = sum over chunks of partial[chunk][o], o = co * (K + 1) + t: lane ty of a column sums chunks ty, ty + 32, ...
+// in order, then the 32 lane sums are added in a fixed tree.  Weight columns are scaled by 1/255, the bias column
+// (t == K) is the bias gradient.
+__global__ void __launch_bounds__(kReduceLanes * 32) vn_conv_u8_wgrad_reduce_kernel(const float *__restrict__ partial,
+                                                                                   int chunks, int cout, int K,
+                                                                                   float *__restrict__ grad_weight,
+                                                                                   float *__restrict__ grad_bias) {
+    __shared__ float red[kReduceLanes][33];
+    asm volatile("griddepcontrol.wait;" ::: "memory");
+    const int K1 = K + 1, total = cout * K1;
+    const int tx = threadIdx.x, ty = threadIdx.y, o = blockIdx.x * 32 + tx;
+    float s = 0.f;
+    if (o < total)
+        for (int q = ty; q < chunks; q += kReduceLanes) s = __fadd_rn(s, partial[(int64_t)q * total + o]);
+    red[ty][tx] = s;
+    __syncthreads();
+#pragma unroll
+    for (int st = kReduceLanes / 2; st > 0; st >>= 1) {
+        if (ty < st) red[ty][tx] = __fadd_rn(red[ty][tx], red[ty + st][tx]);
+        __syncthreads();
+    }
+    if (ty != 0 || o >= total) return;
+    const int co = o / K1, t = o - co * K1;
+    if (t < K)
+        grad_weight[(int64_t)co * K + t] = __fdiv_rn(red[0][tx], 255.f);
+    else if (grad_bias)
+        grad_bias[co] = red[0][tx];
+}
+
+// ---------------------------------------------------------------- host side
+struct ConvGeom {
+    int oh, ow, K, fb;
+};
+
+static bool aligned4(const void *p) { return (reinterpret_cast<uintptr_t>(p) & 3) == 0; }
+
+// Checks the frame source and the layer shape shared by the forward and the backward.
+static int32_t conv_args(const vn_u8_frames_t *src, int32_t cout, int32_t k, int32_t stride, const char *who, ConvGeom *g) {
+    VN_REQUIRE(src, "%s: src is null", who);
+    VN_REQUIRE(src->n >= 0, "%s: n=%d", who, src->n);
+    VN_REQUIRE(src->base, "%s: frame base is null", who);
+    VN_REQUIRE(aligned16(src->base) && (src->pitch & 15) == 0, "%s: frame base and pitch (%lld) must be 16-byte aligned",
+               who, (long long)src->pitch);
+    VN_REQUIRE(src->h > 0 && src->w > 0 && src->c > 0, "%s: frame %d x %d x %d", who, src->h, src->w, src->c);
+    VN_REQUIRE(src->pitch >= (int64_t)src->h * src->w * src->c, "%s: pitch %lld is less than a %d x %d x %d frame", who,
+               (long long)src->pitch, src->h, src->w, src->c);
+    VN_REQUIRE(!src->idx || (src->idx_t >= 1 && src->n % src->idx_t == 0), "%s: idx_t=%d does not divide n=%d", who,
+               src->idx_t, src->n);
+    if (src->c != 1 && src->c != 3) {
+        set_error("%s: %d channels (1 or 3 are supported)", who, src->c);
+        return VN_EUNSUPPORTED;
+    }
+    if (k < 1 || k > 8 || stride < 1 || stride > k) {
+        set_error("%s: kernel %d, stride %d (1 <= stride <= kernel <= 8 are supported)", who, k, stride);
+        return VN_EUNSUPPORTED;
+    }
+    if (cout < 8 || cout > 64 || cout % 8) {
+        set_error("%s: %d output channels (multiples of 8 up to 64 are supported)", who, cout);
+        return VN_EUNSUPPORTED;
+    }
+    if (src->h < k || src->w < k || src->h > kMaxFrameSide || src->w > kMaxFrameSide) {
+        set_error("%s: %d x %d frame with kernel %d (frames of kernel .. %d pixels a side are supported)", who, src->h,
+                  src->w, k, kMaxFrameSide);
+        return VN_EUNSUPPORTED;
+    }
+    g->oh = (src->h - k) / stride + 1;
+    g->ow = (src->w - k) / stride + 1;
+    g->K = src->c * k * k;
+    g->fb = (src->h * src->w * src->c + 15) & ~15;
+    return VN_OK;
+}
+
+static int64_t chunks_of(int64_t n) { return (n + kWgradChunk - 1) / kWgradChunk; }
+
+using FwdKernel = void (*)(const FwdArgs);
+static const FwdKernel kFwdKernels[8] = {vn_conv_u8_fwd_kernel<1>, vn_conv_u8_fwd_kernel<2>, vn_conv_u8_fwd_kernel<3>,
+                                  vn_conv_u8_fwd_kernel<4>, vn_conv_u8_fwd_kernel<5>, vn_conv_u8_fwd_kernel<6>,
+                                  vn_conv_u8_fwd_kernel<7>, vn_conv_u8_fwd_kernel<8>};
+
+// Shared memory of `frames_bytes` frame buffers plus `rest`: two buffers when they fit, else one.
+static int frame_buffers(int fb, int rest) { return 2 * fb + rest <= kMaxSmemConv ? 2 : 1; }
+
+// A persistent grid: as many CTAs of `kernel` as are resident at once (registers and shared memory), at most `work`.
+template <typename... KArgs>
+static int32_t persistent_grid(void (*kernel)(KArgs...), int threads, int smem, int64_t work, const char *who,
+                               int *grid) {
+    int per_sm = 0;
+    const cudaError_t e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kernel, threads, smem);
+    if (e != cudaSuccess || per_sm < 1) {
+        cudaGetLastError();
+        set_error("%s: occupancy query: %s", who, cudaGetErrorString(e));
+        return VN_ECUDA;
+    }
+    const int64_t cap = (int64_t)sm_count() * per_sm;
+    *grid = (int)(work < cap ? work : cap);
+    return VN_OK;
+}
+
+}  // namespace vn
+
+extern "C" {
+
+int32_t vn_conv_u8_forward(const vn_u8_frames_t *src, const float *weight, const float *bias, int32_t cout, int32_t k,
+                           int32_t stride, float *out, void *stream) {
+    vn::ConvGeom g;
+    int32_t rc = vn::conv_args(src, cout, k, stride, "conv_u8_forward", &g);
+    if (rc) return rc;
+    VN_REQUIRE(weight && out, "conv_u8_forward: weight and out must not be null");
+    VN_REQUIRE(vn::aligned4(weight) && vn::aligned4(bias) && vn::aligned4(out),
+               "conv_u8_forward: weight, bias and out must be 4-byte aligned");
+    if (src->n == 0) return VN_OK;
+    const int NT = cout / 8, ksteps = (g.K + 15) / 16;
+    const int rest = ksteps * NT * 3 * 32 * 8 + ksteps * 16 * 4 + NT * 8 * 4 + 16;
+    const int nbuf = vn::frame_buffers(g.fb, rest), smem = nbuf * g.fb + rest;
+    const vn::FwdKernel kernel = vn::kFwdKernels[NT - 1];
+    rc = vn::ensure_smem(kernel, smem);
+    if (rc) return rc;
+    int grid;
+    rc = vn::persistent_grid(kernel, vn::kFwdWarps * 32, smem, src->n, "conv_u8_forward", &grid);
+    if (rc) return rc;
+    const vn::FwdArgs a{*src, weight, bias, out, k, stride, g.oh, g.ow, g.K, ksteps, nbuf, g.fb};
+    return vn::launch(kernel, "vn_conv_u8_fwd_kernel", dim3(grid), dim3(vn::kFwdWarps * 32), (size_t)smem,
+                      (cudaStream_t)stream, true, a);
+}
+
+int64_t vn_conv_u8_wgrad_scratch_bytes(int32_t n, int32_t c, int32_t cout, int32_t k) {
+    if (n < 0 || c < 1 || cout < 1 || k < 1) return -1;
+    return vn::chunks_of(n) * cout * ((int64_t)c * k * k + 1) * (int64_t)sizeof(float);
+}
+
+int32_t vn_conv_u8_backward(const vn_u8_frames_t *src, const float *grad_out, int32_t cout, int32_t k, int32_t stride,
+                            float *grad_weight, float *grad_bias, void *scratch, int64_t scratch_bytes, void *stream) {
+    vn::ConvGeom g;
+    int32_t rc = vn::conv_args(src, cout, k, stride, "conv_u8_backward", &g);
+    if (rc) return rc;
+    VN_REQUIRE(grad_out && grad_weight, "conv_u8_backward: grad_out and grad_weight must not be null");
+    VN_REQUIRE(vn::aligned4(grad_out) && vn::aligned4(grad_weight) && vn::aligned4(grad_bias),
+               "conv_u8_backward: grad_out, grad_weight and grad_bias must be 4-byte aligned");
+    const int64_t need = vn_conv_u8_wgrad_scratch_bytes(src->n, src->c, cout, k);
+    VN_REQUIRE(scratch_bytes >= need, "conv_u8_backward: %lld scratch bytes, %lld needed", (long long)scratch_bytes,
+               (long long)need);
+    VN_REQUIRE(need == 0 || (scratch && vn::aligned16(scratch)),
+               "conv_u8_backward: scratch must be a 16-byte aligned device buffer");
+    if (src->n == 0) return VN_OK;
+    const int mtiles = (cout + 15) / 16, ntiles = (g.K + 1 + 7) / 8;
+    const int rest = ntiles * 8 * 4 + 16 + vn::kWgradTiles * 4 * vn::kWgradWarps * 32 * 4;
+    const int nbuf = vn::frame_buffers(g.fb, rest), smem = nbuf * g.fb + rest;
+    rc = vn::ensure_smem(vn::vn_conv_u8_wgrad_kernel, smem);
+    if (rc) return rc;
+    const int64_t chunks = vn::chunks_of(src->n);
+    int grid;
+    rc = vn::persistent_grid(vn::vn_conv_u8_wgrad_kernel, vn::kWgradWarps * 32, smem, chunks, "conv_u8_backward", &grid);
+    if (rc) return rc;
+    const vn::WgradArgs a{*src, grad_out, (float *)scratch, cout, k, stride, g.oh, g.ow, g.K, mtiles, ntiles, nbuf,
+                          g.fb};
+    rc = vn::launch(vn::vn_conv_u8_wgrad_kernel, "vn_conv_u8_wgrad_kernel", dim3(grid), dim3(vn::kWgradWarps * 32),
+                    (size_t)smem, (cudaStream_t)stream, true, a);
+    if (rc) return rc;
+    const int outputs = cout * (g.K + 1);
+    return vn::launch(vn::vn_conv_u8_wgrad_reduce_kernel, "vn_conv_u8_wgrad_reduce_kernel", dim3((outputs + 31) / 32),
+                      dim3(32, vn::kReduceLanes), 0, (cudaStream_t)stream, true, (const float *)scratch, (int)chunks,
+                      (int)cout, g.K, grad_weight, grad_bias);
+}
+
+}  // extern "C"

@@ -1200,6 +1200,7 @@ int32_t vn_abi_struct_size(int32_t which) {
         case 6: return (int32_t)sizeof(vn_replay_t);
         case 7: return (int32_t)sizeof(vn_float_leaf_t);
         case 8: return (int32_t)sizeof(vn_host_call_t);
+        case 9: return (int32_t)sizeof(vn_u8_frames_t);
         default: return -1;
     }
 }

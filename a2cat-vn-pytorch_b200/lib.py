@@ -24,7 +24,7 @@ STEP_ACTIONS_READY = 0x01
 STEP_SKIP_UNCHANGED = 0x02
 STEP_NO_OVERLAP = 0x04
 MODE_SPLIT, MODE_FUSED, MODE_PERSISTENT = 0, 1, 2
-ABI_VERSION = 3
+ABI_VERSION = 4
 STAT_NAMES = ("episodes", "return_sum", "length_sum", "successes", "collisions", "steps", "truncations", "resets",
               "rows_skipped")
 
@@ -85,6 +85,12 @@ class HostCall(C.Structure):
                 ("timeout_us", C.c_int64)]
 
 
+class U8Frames(C.Structure):
+    _fields_ = [("base", _P), ("pitch", C.c_int64), ("idx", _P), ("idx_stride_n", C.c_int64),
+                ("idx_stride_t", C.c_int64), ("n", C.c_int32), ("idx_t", C.c_int32), ("h", C.c_int32),
+                ("w", C.c_int32), ("c", C.c_int32), ("reserved", C.c_int32)]
+
+
 class VnError(RuntimeError):
     pass
 
@@ -96,7 +102,7 @@ EXPORTS = ("vn_abi_version", "vn_abi_struct_size", "vn_last_error", "vn_launch_c
            "vn_env_gather", "vn_env_step_host", "vn_env_step_host_sync", "vn_env_step_host_call", "vn_env_step_mode", "vn_debug_gather_trace", "vn_env_host_seq_words", "vn_host_wait_seq", "vn_event_create", "vn_event_destroy", "vn_event_wait", "vn_gather_plane",
            "vn_gather_plane_f32_chw", "vn_gather_plane_f32_chw_rows", "vn_gather_leaves_f32_chw", "vn_nstep_returns", "vn_nstep_returns_scan", "vn_discounted_backup", "vn_pixel_control",
            "vn_transition_rows", "vn_gather_rows", "vn_pixel_control_list", "vn_pixel_control_returns", "vn_pixel_control_returns_from_states", "vn_replay_sample",
-           "vn_aux_target", "vn_rp_labels")
+           "vn_aux_target", "vn_rp_labels", "vn_conv_u8_forward", "vn_conv_u8_wgrad_scratch_bytes", "vn_conv_u8_backward")
 
 
 def library_path():
@@ -161,6 +167,9 @@ def load(build_if_missing=True):
         "vn_replay_sample": (i32, [C.POINTER(Replay), i32, i32, u64, C.c_uint32, i32, _P, _P, _P, _P, _P, _P, _P, _P]),
         "vn_aux_target": (i32, [S, i32, _P, i32, i32, i32, i32, i32, i32, i32, _P, _P]),
         "vn_rp_labels": (i32, [_P, i32, i32, i64, i64, _P, _P, _P, _P, _P, _P]),
+        "vn_conv_u8_forward": (i32, [C.POINTER(U8Frames), _P, _P, i32, i32, i32, _P, _P]),
+        "vn_conv_u8_wgrad_scratch_bytes": (i64, [i32, i32, i32, i32]),
+        "vn_conv_u8_backward": (i32, [C.POINTER(U8Frames), _P, i32, i32, i32, _P, _P, _P, i64, _P]),
     }
     for name, (res, args) in sig.items():
         fn = getattr(lib, name)
@@ -168,7 +177,8 @@ def load(build_if_missing=True):
     if lib.vn_abi_version() != ABI_VERSION:
         raise VnError("libvn_b200.so ABI version %d, expected %d - rebuild with `python __graft_entry__.py`"
                       % (lib.vn_abi_version(), ABI_VERSION))
-    for which, mirror in enumerate((Store, Tables, Envs, Rules, Inject, StepOut, Replay, FloatLeaf, HostCall)):
+    for which, mirror in enumerate((Store, Tables, Envs, Rules, Inject, StepOut, Replay, FloatLeaf, HostCall,
+                                     U8Frames)):
         if lib.vn_abi_struct_size(which) != C.sizeof(mirror):
             raise VnError("libvn_b200.so is stale: sizeof(%s) is %d in the library, %d in lib.py - rebuild with "
                           "`python __graft_entry__.py`" % (mirror.__name__, lib.vn_abi_struct_size(which), C.sizeof(mirror)))

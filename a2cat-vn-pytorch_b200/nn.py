@@ -1,0 +1,165 @@
+"""The policy's first convolution read straight from uint8 frames (``vn.nn``).
+
+``U8Conv2d`` replaces TransposeImage + ScaledFloatFrame (deep_rl.common.env, thor_cached_auxiliary.py:61-62) + the
+model's first ``Conv2d`` (models/goal.py:36-41): ``layer(frames) == F.conv2d(frames.permute(0, 3, 1, 2).float() / 255,
+weight, bias, stride)`` to fp32 accuracy, with the frames taken as uint8 ``[N, H, W, C]`` - the observation leaves of
+``GraphVecEnv(scaled_float=False)`` - or as state indices read from the HBM store (``forward_states``).  No float copy of
+a frame is ever written: the forward is one library kernel, the weight / bias gradient two, and what autograd keeps for
+the backward is the uint8 batch or the int32 index tensor.
+
+Aliasing rule: the frames must not change between the forward and the backward.  The library rewrites an env's
+observation batch on the next ``step`` without bumping torch's version counter, so autograd cannot notice.  An update
+pass therefore runs ``forward_states`` over the rollout's state indices (``buf.states[:-1].t()``), which is also the
+path that keeps nothing but those indices alive until the backward.
+"""
+import ctypes as C
+
+import torch
+
+from . import lib as L
+from .rollout import _call
+
+
+def _frames_of_batch(x):
+    """vn_u8_frames_t of a uint8 [N, H, W, C] batch whose rows are a multiple of 16 bytes apart (StoreLayout.batch)."""
+    n, h, w, c = x.shape
+    if x.stride()[1:] != (w * c, c, 1):
+        raise ValueError("U8Conv2d: each frame must be HWC-contiguous, got strides %s" % (x.stride(),))
+    pitch = x.stride(0) if n > 1 else (h * w * c + 15) // 16 * 16
+    if pitch % 16 or x.data_ptr() % 16:
+        raise ValueError("U8Conv2d: frames must start on 16-byte boundaries, rows a multiple of 16 bytes apart (got a "
+                         "pitch of %d bytes); StoreLayout.batch / GraphVecEnv observation leaves are" % pitch)
+    return L.U8Frames(x.data_ptr(), pitch, None, 0, 0, n, 1, h, w, c, 0)
+
+
+def _frames_of_states(dw, states, plane):
+    """vn_u8_frames_t of store plane `plane` at the records named by int32 `states` ([N] or [B, T], any strides)."""
+    lay = dw.world.layout
+    pi = dw.plane_index(plane)
+    h, w = lay.frame_hw
+    if states.dim() == 1:
+        idx_t, sn, st = 1, states.stride(0), 0
+    elif states.dim() == 2:
+        idx_t, sn, st = states.shape[1], states.stride(0), states.stride(1)
+    else:
+        raise ValueError("U8Conv2d.forward_states: states must be [N] or [B, T], got %s" % (tuple(states.shape),))
+    n = states.numel()
+    return L.U8Frames(dw.frames.data_ptr() + lay.plane_off[pi], lay.state_pitch, states.data_ptr(), sn, st, n,
+                      max(idx_t, 1), h, w, lay.channels[pi], 0)
+
+
+class _U8Conv(torch.autograd.Function):
+    """y = conv2d(x / 255, weight, bias, stride) for uint8 frames described by ``frames_of(source)``.  Saves only
+    ``source`` (the uint8 batch or the index tensor) for the backward."""
+
+    @staticmethod
+    def forward(ctx, source, weight, bias, frames_of, stride, out_shape):
+        cout, _, k, _ = weight.shape
+        if not weight.is_contiguous() or (bias is not None and not bias.is_contiguous()):
+            raise ValueError("U8Conv2d: weight and bias must be contiguous")
+        src = frames_of(source)
+        out = torch.empty(out_shape, dtype=torch.float32, device=weight.device)
+        _call(weight.device, "vn_conv_u8_forward", C.byref(src), weight.data_ptr(), L.ptr(bias), cout, k, stride,
+              out.data_ptr(), stream_of=weight)
+        ctx.save_for_backward(source)
+        ctx.frames_of, ctx.stride, ctx.has_bias = frames_of, stride, bias is not None
+        ctx.wshape = tuple(weight.shape)
+        return out
+
+    @staticmethod
+    def backward(ctx, grad_out):
+        need_w, need_b = ctx.needs_input_grad[1], ctx.has_bias and ctx.needs_input_grad[2]
+        if not (need_w or need_b):
+            return None, None, None, None, None, None
+        (source,) = ctx.saved_tensors
+        src = ctx.frames_of(source)
+        cout, c, k, _ = ctx.wshape
+        dev = grad_out.device
+        grad_out = grad_out.contiguous()      # a copy kernel only when autograd hands over a non-contiguous gradient
+        gw = torch.empty(ctx.wshape, dtype=torch.float32, device=dev)
+        gb = torch.empty(cout, dtype=torch.float32, device=dev) if ctx.has_bias else None
+        if src.n == 0:
+            gw.zero_()
+            if gb is not None:
+                gb.zero_()
+        else:
+            nbytes = L.load().vn_conv_u8_wgrad_scratch_bytes(src.n, c, cout, k)
+            scratch = torch.empty(nbytes, dtype=torch.uint8, device=dev)
+            _call(dev, "vn_conv_u8_backward", C.byref(src), grad_out.data_ptr(), cout, k, ctx.stride, gw.data_ptr(),
+                  L.ptr(gb), scratch.data_ptr(), nbytes, stream_of=grad_out)
+        return None, (gw if need_w else None), (gb if need_b else None), None, None, None
+
+
+class U8Conv2d(torch.nn.Conv2d):
+    """Drop-in for the model's first ``nn.Conv2d`` whose input is uint8 HWC frames (see the module docstring).
+
+    Same constructor, parameter initialisation and ``state_dict`` keys as ``nn.Conv2d``.  Supported: 1 or 3 input
+    channels, a square kernel of 1..8, stride 1..kernel (square), 8..64 output channels in steps of 8, no padding,
+    dilation or groups, frames of kernel..174 pixels a side; anything else raises ``ValueError`` here."""
+
+    def __init__(self, in_channels, out_channels, kernel_size, stride=1, padding=0, dilation=1, groups=1, bias=True,
+                 padding_mode="zeros", device=None, dtype=None):
+        super().__init__(in_channels, out_channels, kernel_size, stride, padding, dilation, groups, bias, padding_mode,
+                         device, dtype)
+        k, s = self.kernel_size, self.stride
+        why = None
+        if self.padding not in ((0, 0), "valid") or self.dilation != (1, 1) or self.groups != 1:
+            why = "padding, dilation and groups are not supported"
+        elif k[0] != k[1] or s[0] != s[1]:
+            why = "kernel and stride must be square"
+        elif in_channels not in (1, 3):
+            why = "in_channels must be 1 or 3"
+        elif not 1 <= k[0] <= 8 or not 1 <= s[0] <= k[0]:
+            why = "1 <= stride <= kernel_size <= 8"
+        elif out_channels % 8 or not 8 <= out_channels <= 64:
+            why = "out_channels must be a multiple of 8 up to 64"
+        elif self.weight.dtype != torch.float32:
+            why = "the parameters must be float32"
+        if why:
+            raise ValueError("U8Conv2d: " + why)
+
+    @classmethod
+    def from_conv2d(cls, conv):
+        """A U8Conv2d with the parameters of a trained ``nn.Conv2d`` (copied, on the same device)."""
+        layer = cls(conv.in_channels, conv.out_channels, conv.kernel_size, conv.stride, conv.padding, conv.dilation,
+                    conv.groups, conv.bias is not None, conv.padding_mode, device=conv.weight.device,
+                    dtype=conv.weight.dtype)
+        layer.load_state_dict(conv.state_dict())
+        return layer
+
+    def _out_hw(self, h, w):
+        k, s = self.kernel_size[0], self.stride[0]
+        return (h - k) // s + 1, (w - k) // s + 1
+
+    def _check_device(self, t):
+        if not self.weight.is_cuda or t.device != self.weight.device:
+            raise ValueError("U8Conv2d: the layer and its input must be on the same CUDA device")
+
+    def forward(self, frames):
+        """frames: uint8 CUDA ``[N, H, W, C]`` (rows a multiple of 16 bytes apart, e.g. a GraphVecEnv observation leaf)
+        -> float32 ``[N, out_channels, oh, ow]``."""
+        if not torch.is_tensor(frames) or frames.dtype != torch.uint8:
+            raise TypeError("U8Conv2d takes uint8 [N, H, W, C] frames, got %s" %
+                            (frames.dtype if torch.is_tensor(frames) else type(frames).__name__))
+        if frames.dim() != 4 or frames.shape[3] != self.in_channels:
+            raise ValueError("U8Conv2d: expected [N, H, W, %d] frames, got %s" % (self.in_channels, tuple(frames.shape)))
+        self._check_device(frames)
+        n, h, w, _ = frames.shape
+        return _U8Conv.apply(frames, self.weight, self.bias, _frames_of_batch, self.stride[0],
+                             (n, self.out_channels) + self._out_hw(h, w))
+
+    def forward_states(self, dw, states, plane="rgb"):
+        """The frames of store plane `plane` at the records ``states`` (int32 ``[N]`` or ``[B, T]`` with any strides,
+        e.g. ``env.obs_state`` or ``buf.states[:-1].t()``, read in place) -> float32 ``[*states.shape, out_channels,
+        oh, ow]``.  As with ``vn_gather_plane``, ``states`` must hold valid record indices."""
+        lay = dw.world.layout
+        if lay.channels[dw.plane_index(plane)] != self.in_channels:
+            raise ValueError("U8Conv2d: plane %r has %d channels, the layer takes %d"
+                             % (plane, lay.channels[dw.plane_index(plane)], self.in_channels))
+        if states.dtype != torch.int32 or states.device != dw.device:
+            states = states.to(device=dw.device, dtype=torch.int32)
+        self._check_device(states)
+        shape = tuple(states.shape)
+        out = _U8Conv.apply(states, self.weight, self.bias, lambda s: _frames_of_states(dw, s, plane), self.stride[0],
+                            (states.numel(), self.out_channels) + self._out_hw(*lay.frame_hw))
+        return out.view(shape + tuple(out.shape[1:]))

@@ -34,7 +34,7 @@
 extern "C" {
 #endif
 
-#define VN_ABI_VERSION 3
+#define VN_ABI_VERSION 4
 #define VN_MAX_PLANES 6 /* rgb, depth, segmentation (+ the 3 third-person planes of graph/thor_graph.py:25-31) */
 
 /* error codes */
@@ -231,7 +231,7 @@ typedef struct vn_step_out {
 
 int32_t vn_abi_version(void);
 /* sizeof of the descriptor structs as compiled into the library (0 store, 1 tables, 2 envs, 3 rules, 4 inject,
- * 5 step_out, 6 replay, 7 float_leaf, 8 host_call; -1 otherwise): a binding checks its mirrors against these at load
+ * 5 step_out, 6 replay, 7 float_leaf, 8 host_call, 9 u8_frames; -1 otherwise): a binding checks its mirrors against these at load
  * time. */
 int32_t vn_abi_struct_size(int32_t which);
 const char *vn_last_error(void);
@@ -486,6 +486,44 @@ int32_t vn_aux_target(const vn_store_t *store, int32_t plane, const int32_t *idx
  * caller-owned device memory. */
 int32_t vn_rp_labels(const float *reward, int32_t n, int32_t t, int64_t stride_n, int64_t stride_t, int8_t *labels,
                      int32_t *zero_idx, int32_t *nonzero_idx, int32_t *counts, int32_t *scratch, void *stream);
+
+/* The policy's first convolution read straight from uint8 frames.  Replaces TransposeImage + ScaledFloatFrame
+ * (deep_rl.common.env, thor_cached_auxiliary.py:61-62) + the model's first Conv2d (models/goal.py:36-41):
+ *   y = conv2d(x / 255, weight, bias, stride), x = frame i as [c][h][w] (the frame is stored HWC), padding 0.
+ * The frames are never written as float32: the forward reads each uint8 frame once, and the weight gradient reads it
+ * again, so an update pass keeps only the state indices alive between its forward and its backward.
+ *
+ * Frame source.  Frame i of a batch (idx == NULL) is row i: base + i * pitch.  With idx it is record
+ * idx[a * idx_stride_n + k * idx_stride_t], a = i / idx_t, k = i % idx_t (vn_gather_rows' convention: a [B, T] view of
+ * time-major rollout states is read in place), at base + record * pitch.  base is a store plane
+ * (store->base + plane_off[p], pitch state_pitch) or a uint8 observation batch (pitch plane_bytes); base and pitch are
+ * multiples of 16, pitch >= h * w * c, and idx holds valid record indices. */
+typedef struct vn_u8_frames {
+    const uint8_t *base;
+    int64_t pitch;
+    const int32_t *idx;
+    int64_t idx_stride_n, idx_stride_t;
+    int32_t n, idx_t, h, w, c, reserved;
+} vn_u8_frames_t;
+
+/* Supported: c 1 or 3, 1 <= k <= 8, 1 <= stride <= k, cout a multiple of 8 up to 64, k <= h, w <= 174; anything else
+ * is VN_EUNSUPPORTED.  n == 0 launches nothing (and writes nothing).  The kernels run on the tensor cores with the fp32
+ * operand split into three exact bf16 terms: fp32-class results (see vn_conv.cu).  A programmatic launch that waits for
+ * its predecessor before it reads anything and does not release its successor early: like vn_gather_plane, idx may be
+ * live env state (out->obs_state), and a batch row may be one a following vn_env_step* call rewrites. */
+/* out [n][cout][oh][ow] float32, oh = (h - k) / stride + 1; weight [cout][c][k][k]; bias [cout] or NULL. */
+int32_t vn_conv_u8_forward(const vn_u8_frames_t *src, const float *weight, const float *bias, int32_t cout, int32_t k,
+                           int32_t stride, float *out, void *stream);
+/* Bytes of device scratch vn_conv_u8_backward needs: ceil(n / 32) * cout * (c * k * k + 1) * 4 (one partial gradient
+ * per chunk of 32 frames); -1 for negative or zero sizes.  Host only. */
+int64_t vn_conv_u8_wgrad_scratch_bytes(int32_t n, int32_t c, int32_t cout, int32_t k);
+/* The weight and bias gradient of vn_conv_u8_forward for grad_out [n][cout][oh][ow]:
+ *   grad_weight[co][ci][ky][kx] = sum_{i, oy, ox} grad_out[i][co][oy][ox] * x_i[ci][oy * stride + ky][ox * stride + kx] / 255,
+ *   grad_bias[co] (optional) = sum_{i, oy, ox} grad_out[i][co][oy][ox].
+ * Both are written, not accumulated.  Two kernels: partial sums per chunk of 32 frames into scratch, then a reduction
+ * over the chunks in a fixed order - no atomics, the same bits on every run and every device size. */
+int32_t vn_conv_u8_backward(const vn_u8_frames_t *src, const float *grad_out, int32_t cout, int32_t k, int32_t stride,
+                            float *grad_weight, float *grad_bias, void *scratch, int64_t scratch_bytes, void *stream);
 
 #ifdef __cplusplus
 }
