@@ -10,7 +10,15 @@
 // zero, and that k-step's sum is added to an fp32 register accumulator with a round-to-nearest FADD; the 1/255 scale is
 // one division at the end.  The weight gradient's partial sums per fixed chunk of frames are reduced in a fixed order
 // by a second kernel: no float atomics, the same bits on any number of SMs.
+//
+// The 16-bit variants (the *_lp entry points, torch.autocast) have fp16 or bf16 as the element type T.  The weight is
+// rounded to T once (round-to-nearest-even, as autocast's cast), grad_out arrives in T, and a pixel is exact in either
+// type, so every product is exact with ONE term: one mma.sync per k-step instead of three.  Accumulation, the 1/255
+// scale and the reduction are those of the fp32 kernels; the forward rounds its fp32 result to T once.
 #include <cuda_bf16.h>
+#include <cuda_fp16.h>
+
+#include <type_traits>
 
 #include "vn_common.cuh"
 
@@ -51,14 +59,72 @@ __device__ __forceinline__ void split3(float a, float b, uint32_t &hi, uint32_t 
     mid = bf2_bits(m);
     lo = bf2_bits(__floats2bfloat162_rn(__fsub_rn(ra, mf.x), __fsub_rn(rb, mf.y)));
 }
-// d = a * b + c, m16n8k16, bf16 in, fp32 accumulate
+// Element type T of a kernel: float = the fp32 operand split into three bf16 terms, __half / __nv_bfloat16 = one term.
+template <typename T>
+constexpr int kTerms = std::is_same_v<T, float> ? 3 : 1;
+// two floats rounded to T x2 (round-to-nearest-even), lo in the low half
+template <typename T>
+__device__ __forceinline__ uint32_t pack_rn(float lo, float hi) {
+    if constexpr (std::is_same_v<T, __half>) {
+        const __half2 v = __floats2half2_rn(lo, hi);
+        return *reinterpret_cast<const uint32_t *>(&v);
+    } else {
+        return bf2_bits(__floats2bfloat162_rn(lo, hi));
+    }
+}
+// two pixels 0..255 as the mma operand type of T, exactly
+template <typename T>
+__device__ __forceinline__ uint32_t pack_px(float lo, float hi) {
+    if constexpr (std::is_same_v<T, __half>)
+        return pack_rn<__half>(lo, hi);
+    else
+        return pack_exact(lo, hi);
+}
+// x rounded to T and back (the value autocast's cast gives)
+template <typename T>
+__device__ __forceinline__ float round_to(float x) {
+    if constexpr (std::is_same_v<T, __half>)
+        return __half2float(__float2half_rn(x));
+    else if constexpr (std::is_same_v<T, __nv_bfloat16>)
+        return __bfloat162float(__float2bfloat16_rn(x));
+    else
+        return x;
+}
+// the output element of x: x itself, or x rounded once to T (fp16 overflows to +-inf)
+template <typename T>
+__device__ __forceinline__ T to_out(float x) {
+    if constexpr (std::is_same_v<T, __half>)
+        return __float2half_rn(x);
+    else if constexpr (std::is_same_v<T, __nv_bfloat16>)
+        return __float2bfloat16_rn(x);
+    else
+        return x;
+}
+// d = a * b + c, m16n8k16, fp32 accumulate; f16 operands for T = __half, bf16 otherwise
+template <typename T = float>
 __device__ __forceinline__ void mma16816(float (&d)[4], const uint32_t (&a)[4], uint32_t b0, uint32_t b1,
                                          const float (&c)[4]) {
-    asm volatile(
-        "mma.sync.aligned.m16n8k16.row.col.f32.bf16.bf16.f32 {%0,%1,%2,%3}, {%4,%5,%6,%7}, {%8,%9}, "
-        "{%10,%11,%12,%13};"
-        : "=f"(d[0]), "=f"(d[1]), "=f"(d[2]), "=f"(d[3])
-        : "r"(a[0]), "r"(a[1]), "r"(a[2]), "r"(a[3]), "r"(b0), "r"(b1), "f"(c[0]), "f"(c[1]), "f"(c[2]), "f"(c[3]));
+    if constexpr (std::is_same_v<T, __half>)
+        asm volatile(
+            "mma.sync.aligned.m16n8k16.row.col.f32.f16.f16.f32 {%0,%1,%2,%3}, {%4,%5,%6,%7}, {%8,%9}, "
+            "{%10,%11,%12,%13};"
+            : "=f"(d[0]), "=f"(d[1]), "=f"(d[2]), "=f"(d[3])
+            : "r"(a[0]), "r"(a[1]), "r"(a[2]), "r"(a[3]), "r"(b0), "r"(b1), "f"(c[0]), "f"(c[1]), "f"(c[2]), "f"(c[3]));
+    else
+        asm volatile(
+            "mma.sync.aligned.m16n8k16.row.col.f32.bf16.bf16.f32 {%0,%1,%2,%3}, {%4,%5,%6,%7}, {%8,%9}, "
+            "{%10,%11,%12,%13};"
+            : "=f"(d[0]), "=f"(d[1]), "=f"(d[2]), "=f"(d[3])
+            : "r"(a[0]), "r"(a[1]), "r"(a[2]), "r"(a[3]), "r"(b0), "r"(b1), "f"(c[0]), "f"(c[1]), "f"(c[2]), "f"(c[3]));
+}
+// acc += a * b over one k-step, one term of type T
+template <typename T>
+__device__ __forceinline__ void mma_one(float (&acc)[4], const uint32_t (&a)[4], uint32_t b0, uint32_t b1) {
+    const float z[4] = {0.f, 0.f, 0.f, 0.f};
+    float d[4];
+    mma16816<T>(d, a, b0, b1, z);
+#pragma unroll
+    for (int q = 0; q < 4; ++q) acc[q] = __fadd_rn(acc[q], d[q]);
 }
 // acc += (a_hi + a_mid + a_lo) * b over one k-step (operand split on A)
 __device__ __forceinline__ void mma_split_a(float (&acc)[4], const uint32_t (&ah)[4], const uint32_t (&am)[4],
@@ -109,21 +175,24 @@ struct FwdArgs {
     vn_u8_frames_t src;
     const float *weight;   // [cout][K], K = c * k * k
     const float *bias;     // [cout] or null
-    float *out;            // [n][cout][oh][ow]
+    void *out;             // [n][cout][oh][ow] of the kernel's element type
     int k, stride, oh, ow, K, ksteps, nbuf, fb;
 };
 
-// Persistent grid; a CTA owns whole frames.  Its prologue splits the weights into shared memory in mma B-fragment order
-// ([k-step][n-tile][hi, mid, lo][lane] uint2).  A warp owns two 16-pixel m-tiles of a frame and every output channel;
-// the A fragments are the frame's bytes picked through a tap-offset table (implicit im2col).  Each C fragment row is 8
-// consecutive pixels of one channel, so every store instruction writes whole 32-byte sectors of the NCHW output.
-template <int NT>   // cout / 8
+// Persistent grid; a CTA owns whole frames.  Its prologue splits (fp32) or rounds (16-bit T) the weights into shared
+// memory in mma B-fragment order ([k-step][n-tile][hi, mid, lo or the one term][lane] uint2).  A warp owns two 16-pixel
+// m-tiles of a frame and every output channel; the A fragments are the frame's bytes picked through a tap-offset table
+// (implicit im2col).  Each C fragment row is 8 consecutive pixels of one channel, so every fp32 store instruction
+// writes whole 32-byte sectors of the NCHW output (16-bit ones write half sectors, which L2 joins: the other half is
+// the same thread's row g + 8).
+template <int NT, typename T>   // cout / 8, element type
 __global__ void __launch_bounds__(kFwdWarps * 32) vn_conv_u8_fwd_kernel(const FwdArgs a) {
+    constexpr int TERMS = kTerms<T>;
     extern __shared__ __align__(128) uint8_t smem[];
     const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31, g = lane >> 2, tig = lane & 3;
     const int w = a.src.w, c = a.src.c, K = a.K, ksteps = a.ksteps;
     uint2 *wfrag = reinterpret_cast<uint2 *>(smem + (size_t)a.nbuf * a.fb);
-    int *tap = reinterpret_cast<int *>(wfrag + ksteps * NT * 3 * 32);
+    int *tap = reinterpret_cast<int *>(wfrag + ksteps * NT * TERMS * 32);
     float *sbias = reinterpret_cast<float *>(tap + ksteps * 16);
     uint64_t *bar = reinterpret_cast<uint64_t *>(sbias + NT * 8);
     const FramePipe pipe{smem, bar, a.fb, a.nbuf};
@@ -151,15 +220,19 @@ __global__ void __launch_bounds__(kFwdWarps * 32) vn_conv_u8_fwd_kernel(const Fw
         const float *wr = a.weight + (size_t)n * K;
         const float v0 = k0 < K ? wr[k0] : 0.f, v1 = k0 + 1 < K ? wr[k0 + 1] : 0.f;
         const float v8 = k0 + 8 < K ? wr[k0 + 8] : 0.f, v9 = k0 + 9 < K ? wr[k0 + 9] : 0.f;
-        uint32_t h0, m0, l0, h1, m1, l1;
-        split3(v0, v1, h0, m0, l0);
-        split3(v8, v9, h1, m1, l1);
-        uint2 *dst = wfrag + (size_t)(ks * NT + j) * 96 + ln;
-        dst[0] = make_uint2(h0, h1);
-        dst[32] = make_uint2(m0, m1);
-        dst[64] = make_uint2(l0, l1);
+        if constexpr (TERMS == 3) {
+            uint32_t h0, m0, l0, h1, m1, l1;
+            split3(v0, v1, h0, m0, l0);
+            split3(v8, v9, h1, m1, l1);
+            uint2 *dst = wfrag + (size_t)(ks * NT + j) * 96 + ln;
+            dst[0] = make_uint2(h0, h1);
+            dst[32] = make_uint2(m0, m1);
+            dst[64] = make_uint2(l0, l1);
+        } else {
+            wfrag[(size_t)(ks * NT + j) * 32 + ln] = make_uint2(pack_rn<T>(v0, v1), pack_rn<T>(v8, v9));
+        }
     }
-    for (int co = tid; co < NT * 8; co += blockDim.x) sbias[co] = a.bias ? a.bias[co] : 0.f;
+    for (int co = tid; co < NT * 8; co += blockDim.x) sbias[co] = a.bias ? round_to<T>(a.bias[co]) : 0.f;
     const int n = a.src.n;
     if (tid == 0)
         for (int s = 0; s < a.nbuf; ++s) {
@@ -172,7 +245,7 @@ __global__ void __launch_bounds__(kFwdWarps * 32) vn_conv_u8_fwd_kernel(const Fw
     int it = 0;
     for (int f = blockIdx.x; f < n; f += gridDim.x, ++it) {
         const uint8_t *x = pipe.wait(it);
-        float *out = a.out + (int64_t)f * (NT * 8) * P;
+        T *out = static_cast<T *>(a.out) + (int64_t)f * (NT * 8) * P;
         for (int task = warp; task < tasks; task += kFwdWarps) {
             int pb[2][2];
 #pragma unroll
@@ -199,15 +272,21 @@ __global__ void __launch_bounds__(kFwdWarps * 32) vn_conv_u8_fwd_kernel(const Fw
 #pragma unroll
                     for (int r = 0; r < 2; ++r) {
                         const uint8_t *row = x + pb[mt][r];
-                        af[mt][r] = pack_exact(u8f(row[t01.x]), u8f(row[t01.y]));
-                        af[mt][2 + r] = pack_exact(u8f(row[t89.x]), u8f(row[t89.y]));
+                        af[mt][r] = pack_px<T>(u8f(row[t01.x]), u8f(row[t01.y]));
+                        af[mt][2 + r] = pack_px<T>(u8f(row[t89.x]), u8f(row[t89.y]));
                     }
-                const uint2 *wf = wfrag + (size_t)ks * NT * 96 + lane;
+                const uint2 *wf = wfrag + (size_t)ks * NT * TERMS * 32 + lane;
 #pragma unroll
                 for (int j = 0; j < NT; ++j) {
-                    const uint2 bh = wf[j * 96], bm = wf[j * 96 + 32], bl = wf[j * 96 + 64];
-                    mma_split_b(acc[0][j], af[0], bh, bm, bl);
-                    mma_split_b(acc[1][j], af[1], bh, bm, bl);
+                    if constexpr (TERMS == 3) {
+                        const uint2 bh = wf[j * 96], bm = wf[j * 96 + 32], bl = wf[j * 96 + 64];
+                        mma_split_b(acc[0][j], af[0], bh, bm, bl);
+                        mma_split_b(acc[1][j], af[1], bh, bm, bl);
+                    } else {
+                        const uint2 b = wf[j * 32];
+                        mma_one<T>(acc[0][j], af[0], b.x, b.y);
+                        mma_one<T>(acc[1][j], af[1], b.x, b.y);
+                    }
                 }
             }
 #pragma unroll
@@ -219,9 +298,9 @@ __global__ void __launch_bounds__(kFwdWarps * 32) vn_conv_u8_fwd_kernel(const Fw
 #pragma unroll
                     for (int j = 0; j < NT; ++j) {
                         const int co = j * 8 + tig * 2;
-                        out[(int64_t)co * P + p] = __fadd_rn(__fdiv_rn(acc[mt][j][2 * r], 255.f), sbias[co]);
+                        out[(int64_t)co * P + p] = to_out<T>(__fadd_rn(__fdiv_rn(acc[mt][j][2 * r], 255.f), sbias[co]));
                         out[(int64_t)(co + 1) * P + p] =
-                            __fadd_rn(__fdiv_rn(acc[mt][j][2 * r + 1], 255.f), sbias[co + 1]);
+                            to_out<T>(__fadd_rn(__fdiv_rn(acc[mt][j][2 * r + 1], 255.f), sbias[co + 1]));
                     }
                 }
         }
@@ -236,7 +315,7 @@ __global__ void __launch_bounds__(kFwdWarps * 32) vn_conv_u8_fwd_kernel(const Fw
 
 struct WgradArgs {
     vn_u8_frames_t src;
-    const float *grad_out;   // [n][cout][oh][ow]
+    const void *grad_out;    // [n][cout][oh][ow] of the kernel's element type
     float *partial;          // [chunks][cout][K + 1]
     int cout, k, stride, oh, ow, K, mtiles, ntiles, nbuf, fb;
 };
@@ -248,11 +327,14 @@ __device__ __forceinline__ int next_frame(int f, int n) {
 }
 
 // dW[co][t] = sum over the chunk's frames and output pixels p of g[co][p] * x[tap t of p]: an implicit GEMM with
-// M = cout, N = taps + 1 (the last tap reads 1: the bias gradient), K = pixels.  grad_out is the split operand (A, read
-// from global: each fragment row is 8 consecutive floats of one channel), the frame's bytes are B.  A warp owns up to
-// kWgradTiles (16 x 8) output tiles for the whole chunk.  Its registers sum one frame; the frame sums are added into
-// the thread's own shared-memory column, and the chunk's raw sums go to partial[chunk].
+// M = cout, N = taps + 1 (the last tap reads 1: the bias gradient), K = pixels.  grad_out is A (read from global: each
+// fragment row is 8 consecutive elements of one channel), split into three terms when it is fp32, and the frame's bytes
+// are B.  A warp owns up to kWgradTiles (16 x 8) output tiles for the whole chunk.  Its registers sum one frame; the
+// frame sums are added into the thread's own shared-memory column, and the chunk's raw sums go to partial[chunk].
+// 16-bit grad_out is read one element at a time: a channel row is only 2-byte aligned when oh * ow is odd.
+template <typename T>
 __global__ void __launch_bounds__(kWgradWarps * 32) vn_conv_u8_wgrad_kernel(const WgradArgs a) {
+    constexpr int TERMS = kTerms<T>;
     extern __shared__ __align__(128) uint8_t smem[];
     const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31, g = lane >> 2, tig = lane & 3;
     const int w = a.src.w, c = a.src.c, K = a.K, K1 = a.K + 1, cout = a.cout;
@@ -308,7 +390,7 @@ __global__ void __launch_bounds__(kWgradWarps * 32) vn_conv_u8_wgrad_kernel(cons
         const int end = min(n, (chunk + 1) * kWgradChunk);
         for (; f < end; f = next_frame(f, n), ++it) {
             const uint8_t *x = pipe.wait(it);
-            const float *gf = a.grad_out + (int64_t)f * cout * P;
+            const T *gf = static_cast<const T *>(a.grad_out) + (int64_t)f * cout * P;
 #pragma unroll 1
             for (int ks = 0; ks < ksteps; ++ks) {
                 const int p0 = ks * 16 + tig * 2;
@@ -326,13 +408,22 @@ __global__ void __launch_bounds__(kWgradWarps * 32) vn_conv_u8_wgrad_kernel(cons
 #pragma unroll
                         for (int r = 0; r < 2; ++r) {
                             const int co = cur * 16 + g + r * 8;
-                            const float *gr = gf + (int64_t)co * P;
                             const bool ok = co < cout;
-                            const float v0 = ok && p0 < P ? gr[p0] : 0.f, v1 = ok && p0 + 1 < P ? gr[p0 + 1] : 0.f;
-                            const float v8 = ok && p0 + 8 < P ? gr[p0 + 8] : 0.f;
-                            const float v9 = ok && p0 + 9 < P ? gr[p0 + 9] : 0.f;
-                            split3(v0, v1, ah[r], am[r], al[r]);
-                            split3(v8, v9, ah[2 + r], am[2 + r], al[2 + r]);
+                            if constexpr (TERMS == 3) {
+                                const float *gr = gf + (int64_t)co * P;
+                                const float v0 = ok && p0 < P ? gr[p0] : 0.f, v1 = ok && p0 + 1 < P ? gr[p0 + 1] : 0.f;
+                                const float v8 = ok && p0 + 8 < P ? gr[p0 + 8] : 0.f;
+                                const float v9 = ok && p0 + 9 < P ? gr[p0 + 9] : 0.f;
+                                split3(v0, v1, ah[r], am[r], al[r]);
+                                split3(v8, v9, ah[2 + r], am[2 + r], al[2 + r]);
+                            } else {   // the raw 16-bit patterns; 0 is +0 in both types
+                                const uint16_t *gr = reinterpret_cast<const uint16_t *>(gf) + (int64_t)co * P;
+                                const uint32_t v0 = ok && p0 < P ? gr[p0] : 0u, v1 = ok && p0 + 1 < P ? gr[p0 + 1] : 0u;
+                                const uint32_t v8 = ok && p0 + 8 < P ? gr[p0 + 8] : 0u;
+                                const uint32_t v9 = ok && p0 + 9 < P ? gr[p0 + 9] : 0u;
+                                ah[r] = v0 | v1 << 16;
+                                ah[2 + r] = v8 | v9 << 16;
+                            }
                         }
                     }
                     const int o = toff[i];
@@ -345,7 +436,10 @@ __global__ void __launch_bounds__(kWgradWarps * 32) vn_conv_u8_wgrad_kernel(cons
                     } else {
                         b0 = b1 = b8 = b9 = o == -1 ? 1.f : 0.f;
                     }
-                    mma_split_a(acc[i], ah, am, al, pack_exact(b0, b1), pack_exact(b8, b9));
+                    if constexpr (TERMS == 3)
+                        mma_split_a(acc[i], ah, am, al, pack_exact(b0, b1), pack_exact(b8, b9));
+                    else
+                        mma_one<T>(acc[i], ah, pack_px<T>(b0, b1), pack_px<T>(b8, b9));
                 }
             }
             // the frame's sums join the chunk's in shared memory: no register sum runs over more than one frame
@@ -418,6 +512,7 @@ struct ConvGeom {
 };
 
 static bool aligned4(const void *p) { return (reinterpret_cast<uintptr_t>(p) & 3) == 0; }
+static bool aligned2(const void *p) { return (reinterpret_cast<uintptr_t>(p) & 1) == 0; }
 
 // Checks the frame source and the layer shape shared by the forward and the backward.
 static int32_t conv_args(const vn_u8_frames_t *src, int32_t cout, int32_t k, int32_t stride, const char *who, ConvGeom *g) {
@@ -458,9 +553,11 @@ static int32_t conv_args(const vn_u8_frames_t *src, int32_t cout, int32_t k, int
 static int64_t chunks_of(int64_t n) { return (n + kWgradChunk - 1) / kWgradChunk; }
 
 using FwdKernel = void (*)(const FwdArgs);
-static const FwdKernel kFwdKernels[8] = {vn_conv_u8_fwd_kernel<1>, vn_conv_u8_fwd_kernel<2>, vn_conv_u8_fwd_kernel<3>,
-                                  vn_conv_u8_fwd_kernel<4>, vn_conv_u8_fwd_kernel<5>, vn_conv_u8_fwd_kernel<6>,
-                                  vn_conv_u8_fwd_kernel<7>, vn_conv_u8_fwd_kernel<8>};
+template <typename T>
+static const FwdKernel kFwdKernels[8] = {vn_conv_u8_fwd_kernel<1, T>, vn_conv_u8_fwd_kernel<2, T>,
+                                         vn_conv_u8_fwd_kernel<3, T>, vn_conv_u8_fwd_kernel<4, T>,
+                                         vn_conv_u8_fwd_kernel<5, T>, vn_conv_u8_fwd_kernel<6, T>,
+                                         vn_conv_u8_fwd_kernel<7, T>, vn_conv_u8_fwd_kernel<8, T>};
 
 // Shared memory of `frames_bytes` frame buffers plus `rest`: two buffers when they fit, else one.
 static int frame_buffers(int fb, int rest) { return 2 * fb + rest <= kMaxSmemConv ? 2 : 1; }
@@ -481,6 +578,59 @@ static int32_t persistent_grid(void (*kernel)(KArgs...), int threads, int smem, 
     return VN_OK;
 }
 
+// The forward launch of element type T for checked arguments and n > 0.
+template <typename T>
+static int32_t conv_forward(const vn_u8_frames_t *src, const ConvGeom &g, const float *weight, const float *bias,
+                            int32_t cout, int32_t k, int32_t stride, void *out, void *stream, const char *who) {
+    const int NT = cout / 8, ksteps = (g.K + 15) / 16;
+    const int rest = ksteps * NT * kTerms<T> * 32 * 8 + ksteps * 16 * 4 + NT * 8 * 4 + 16;
+    const int nbuf = frame_buffers(g.fb, rest), smem = nbuf * g.fb + rest;
+    const FwdKernel kernel = kFwdKernels<T>[NT - 1];
+    int32_t rc = ensure_smem(kernel, smem);
+    if (rc) return rc;
+    int grid;
+    rc = persistent_grid(kernel, kFwdWarps * 32, smem, src->n, who, &grid);
+    if (rc) return rc;
+    const FwdArgs a{*src, weight, bias, out, k, stride, g.oh, g.ow, g.K, ksteps, nbuf, g.fb};
+    return launch(kernel, "vn_conv_u8_fwd_kernel", dim3(grid), dim3(kFwdWarps * 32), (size_t)smem,
+                  (cudaStream_t)stream, true, a);
+}
+
+// Checks the weight-gradient scratch shared by both backward entry points.
+static int32_t scratch_args(const vn_u8_frames_t *src, int32_t cout, int32_t k, const void *scratch,
+                            int64_t scratch_bytes, const char *who) {
+    const int64_t need = vn_conv_u8_wgrad_scratch_bytes(src->n, src->c, cout, k);
+    VN_REQUIRE(scratch_bytes >= need, "%s: %lld scratch bytes, %lld needed", who, (long long)scratch_bytes,
+               (long long)need);
+    VN_REQUIRE(need == 0 || (scratch && aligned16(scratch)), "%s: scratch must be a 16-byte aligned device buffer",
+               who);
+    return VN_OK;
+}
+
+// The two backward launches of element type T for checked arguments and n > 0.
+template <typename T>
+static int32_t conv_backward(const vn_u8_frames_t *src, const ConvGeom &g, const void *grad_out, int32_t cout,
+                             int32_t k, int32_t stride, float *grad_weight, float *grad_bias, void *scratch,
+                             void *stream, const char *who) {
+    const int mtiles = (cout + 15) / 16, ntiles = (g.K + 1 + 7) / 8;
+    const int rest = ntiles * 8 * 4 + 16 + kWgradTiles * 4 * kWgradWarps * 32 * 4;
+    const int nbuf = frame_buffers(g.fb, rest), smem = nbuf * g.fb + rest;
+    int32_t rc = ensure_smem(vn_conv_u8_wgrad_kernel<T>, smem);
+    if (rc) return rc;
+    const int64_t chunks = chunks_of(src->n);
+    int grid;
+    rc = persistent_grid(vn_conv_u8_wgrad_kernel<T>, kWgradWarps * 32, smem, chunks, who, &grid);
+    if (rc) return rc;
+    const WgradArgs a{*src, grad_out, (float *)scratch, cout, k, stride, g.oh, g.ow, g.K, mtiles, ntiles, nbuf, g.fb};
+    rc = launch(vn_conv_u8_wgrad_kernel<T>, "vn_conv_u8_wgrad_kernel", dim3(grid), dim3(kWgradWarps * 32),
+                (size_t)smem, (cudaStream_t)stream, true, a);
+    if (rc) return rc;
+    const int outputs = cout * (g.K + 1);
+    return launch(vn_conv_u8_wgrad_reduce_kernel, "vn_conv_u8_wgrad_reduce_kernel", dim3((outputs + 31) / 32),
+                  dim3(32, kReduceLanes), 0, (cudaStream_t)stream, true, (const float *)scratch, (int)chunks,
+                  (int)cout, g.K, grad_weight, grad_bias);
+}
+
 }  // namespace vn
 
 extern "C" {
@@ -494,18 +644,26 @@ int32_t vn_conv_u8_forward(const vn_u8_frames_t *src, const float *weight, const
     VN_REQUIRE(vn::aligned4(weight) && vn::aligned4(bias) && vn::aligned4(out),
                "conv_u8_forward: weight, bias and out must be 4-byte aligned");
     if (src->n == 0) return VN_OK;
-    const int NT = cout / 8, ksteps = (g.K + 15) / 16;
-    const int rest = ksteps * NT * 3 * 32 * 8 + ksteps * 16 * 4 + NT * 8 * 4 + 16;
-    const int nbuf = vn::frame_buffers(g.fb, rest), smem = nbuf * g.fb + rest;
-    const vn::FwdKernel kernel = vn::kFwdKernels[NT - 1];
-    rc = vn::ensure_smem(kernel, smem);
+    return vn::conv_forward<float>(src, g, weight, bias, cout, k, stride, out, stream, "conv_u8_forward");
+}
+
+int32_t vn_conv_u8_forward_lp(const vn_u8_frames_t *src, const float *weight, const float *bias, int32_t cout,
+                              int32_t k, int32_t stride, int32_t dtype, void *out, void *stream) {
+    vn::ConvGeom g;
+    int32_t rc = vn::conv_args(src, cout, k, stride, "conv_u8_forward_lp", &g);
     if (rc) return rc;
-    int grid;
-    rc = vn::persistent_grid(kernel, vn::kFwdWarps * 32, smem, src->n, "conv_u8_forward", &grid);
-    if (rc) return rc;
-    const vn::FwdArgs a{*src, weight, bias, out, k, stride, g.oh, g.ow, g.K, ksteps, nbuf, g.fb};
-    return vn::launch(kernel, "vn_conv_u8_fwd_kernel", dim3(grid), dim3(vn::kFwdWarps * 32), (size_t)smem,
-                      (cudaStream_t)stream, true, a);
+    if (dtype != VN_DTYPE_F16 && dtype != VN_DTYPE_BF16) {
+        vn::set_error("conv_u8_forward_lp: dtype %d (VN_DTYPE_F16 or VN_DTYPE_BF16 are supported)", dtype);
+        return VN_EUNSUPPORTED;
+    }
+    VN_REQUIRE(weight && out, "conv_u8_forward_lp: weight and out must not be null");
+    VN_REQUIRE(vn::aligned4(weight) && vn::aligned4(bias), "conv_u8_forward_lp: weight and bias must be 4-byte aligned");
+    VN_REQUIRE(vn::aligned2(out), "conv_u8_forward_lp: out must be 2-byte aligned");
+    if (src->n == 0) return VN_OK;
+    return dtype == VN_DTYPE_F16
+               ? vn::conv_forward<__half>(src, g, weight, bias, cout, k, stride, out, stream, "conv_u8_forward_lp")
+               : vn::conv_forward<__nv_bfloat16>(src, g, weight, bias, cout, k, stride, out, stream,
+                                                 "conv_u8_forward_lp");
 }
 
 int64_t vn_conv_u8_wgrad_scratch_bytes(int32_t n, int32_t c, int32_t cout, int32_t k) {
@@ -521,30 +679,34 @@ int32_t vn_conv_u8_backward(const vn_u8_frames_t *src, const float *grad_out, in
     VN_REQUIRE(grad_out && grad_weight, "conv_u8_backward: grad_out and grad_weight must not be null");
     VN_REQUIRE(vn::aligned4(grad_out) && vn::aligned4(grad_weight) && vn::aligned4(grad_bias),
                "conv_u8_backward: grad_out, grad_weight and grad_bias must be 4-byte aligned");
-    const int64_t need = vn_conv_u8_wgrad_scratch_bytes(src->n, src->c, cout, k);
-    VN_REQUIRE(scratch_bytes >= need, "conv_u8_backward: %lld scratch bytes, %lld needed", (long long)scratch_bytes,
-               (long long)need);
-    VN_REQUIRE(need == 0 || (scratch && vn::aligned16(scratch)),
-               "conv_u8_backward: scratch must be a 16-byte aligned device buffer");
+    rc = vn::scratch_args(src, cout, k, scratch, scratch_bytes, "conv_u8_backward");
+    if (rc) return rc;
     if (src->n == 0) return VN_OK;
-    const int mtiles = (cout + 15) / 16, ntiles = (g.K + 1 + 7) / 8;
-    const int rest = ntiles * 8 * 4 + 16 + vn::kWgradTiles * 4 * vn::kWgradWarps * 32 * 4;
-    const int nbuf = vn::frame_buffers(g.fb, rest), smem = nbuf * g.fb + rest;
-    rc = vn::ensure_smem(vn::vn_conv_u8_wgrad_kernel, smem);
+    return vn::conv_backward<float>(src, g, grad_out, cout, k, stride, grad_weight, grad_bias, scratch, stream,
+                                    "conv_u8_backward");
+}
+
+int32_t vn_conv_u8_backward_lp(const vn_u8_frames_t *src, const void *grad_out, int32_t dtype, int32_t cout,
+                               int32_t k, int32_t stride, float *grad_weight, float *grad_bias, void *scratch,
+                               int64_t scratch_bytes, void *stream) {
+    vn::ConvGeom g;
+    int32_t rc = vn::conv_args(src, cout, k, stride, "conv_u8_backward_lp", &g);
     if (rc) return rc;
-    const int64_t chunks = vn::chunks_of(src->n);
-    int grid;
-    rc = vn::persistent_grid(vn::vn_conv_u8_wgrad_kernel, vn::kWgradWarps * 32, smem, chunks, "conv_u8_backward", &grid);
+    if (dtype != VN_DTYPE_F16 && dtype != VN_DTYPE_BF16) {
+        vn::set_error("conv_u8_backward_lp: dtype %d (VN_DTYPE_F16 or VN_DTYPE_BF16 are supported)", dtype);
+        return VN_EUNSUPPORTED;
+    }
+    VN_REQUIRE(grad_out && grad_weight, "conv_u8_backward_lp: grad_out and grad_weight must not be null");
+    VN_REQUIRE(vn::aligned2(grad_out), "conv_u8_backward_lp: grad_out must be 2-byte aligned");
+    VN_REQUIRE(vn::aligned4(grad_weight) && vn::aligned4(grad_bias),
+               "conv_u8_backward_lp: grad_weight and grad_bias must be 4-byte aligned");
+    rc = vn::scratch_args(src, cout, k, scratch, scratch_bytes, "conv_u8_backward_lp");
     if (rc) return rc;
-    const vn::WgradArgs a{*src, grad_out, (float *)scratch, cout, k, stride, g.oh, g.ow, g.K, mtiles, ntiles, nbuf,
-                          g.fb};
-    rc = vn::launch(vn::vn_conv_u8_wgrad_kernel, "vn_conv_u8_wgrad_kernel", dim3(grid), dim3(vn::kWgradWarps * 32),
-                    (size_t)smem, (cudaStream_t)stream, true, a);
-    if (rc) return rc;
-    const int outputs = cout * (g.K + 1);
-    return vn::launch(vn::vn_conv_u8_wgrad_reduce_kernel, "vn_conv_u8_wgrad_reduce_kernel", dim3((outputs + 31) / 32),
-                      dim3(32, vn::kReduceLanes), 0, (cudaStream_t)stream, true, (const float *)scratch, (int)chunks,
-                      (int)cout, g.K, grad_weight, grad_bias);
+    if (src->n == 0) return VN_OK;
+    return dtype == VN_DTYPE_F16 ? vn::conv_backward<__half>(src, g, grad_out, cout, k, stride, grad_weight, grad_bias,
+                                                             scratch, stream, "conv_u8_backward_lp")
+                                 : vn::conv_backward<__nv_bfloat16>(src, g, grad_out, cout, k, stride, grad_weight,
+                                                                    grad_bias, scratch, stream, "conv_u8_backward_lp");
 }
 
 }  // extern "C"

@@ -7,6 +7,15 @@ weight, bias, stride)`` to fp32 accuracy, with the frames taken as uint8 ``[N, H
 a frame is ever written: the forward is one library kernel, the weight / bias gradient two, and what autograd keeps for
 the backward is the uint8 batch or the int32 index tensor.
 
+Mixed precision: inside ``torch.autocast("cuda", dtype=torch.float16)`` or ``bfloat16`` the layer returns that dtype and
+runs one-term 16-bit tensor-core kernels, as ``nn.Conv2d`` does there: ``round_to_dtype(fp32(conv2d(x / 255,
+weight.to(dtype), bias.to(dtype), stride)))``.  Pixels are exact, the weight and bias are rounded like autocast's cast, the
+products are exact and accumulate in fp32, and the result is rounded once.  torch's own autocast conv also rounds
+``x / 255`` to ``dtype``; this layer does not, so its results are more accurate than that and not bit-equal to it.  The
+backward takes ``grad_out`` in ``dtype`` and returns fp32 gradients for the fp32 parameters; a non-finite ``grad_out``
+element makes its output channel's gradients non-finite, which is what ``GradScaler`` looks for.  Outside autocast, with
+any other autocast dtype, or under a nested ``autocast(enabled=False)``, the fp32 kernels run.
+
 Aliasing rule: the frames must not change between the forward and the backward.  The library rewrites an env's
 observation batch on the next ``step`` without bumping torch's version counter, so autograd cannot notice.  An update
 pass therefore runs ``forward_states`` over the rollout's state indices (``buf.states[:-1].t()``), which is also the
@@ -18,6 +27,17 @@ import torch
 
 from . import lib as L
 from .rollout import _call
+
+_LP_DTYPES = {torch.float16: L.DTYPE_F16, torch.bfloat16: L.DTYPE_BF16}
+
+
+def _autocast_dtype():
+    """The 16-bit dtype of an enabled CUDA autocast region, or None (fp32 kernels)."""
+    if torch.is_autocast_enabled("cuda"):
+        dt = torch.get_autocast_dtype("cuda")
+        if dt in _LP_DTYPES:
+            return dt
+    return None
 
 
 def _frames_of_batch(x):
@@ -49,8 +69,9 @@ def _frames_of_states(dw, states, plane):
 
 
 class _U8Conv(torch.autograd.Function):
-    """y = conv2d(x / 255, weight, bias, stride) for uint8 frames described by ``frames_of(source)``.  Saves only
-    ``source`` (the uint8 batch or the index tensor) for the backward."""
+    """y = conv2d(x / 255, weight, bias, stride) for uint8 frames described by ``frames_of(source)``, in float32 or in the
+    autocast dtype the forward ran under (recorded for the backward).  Saves only ``source`` (the uint8 batch or the
+    index tensor) for the backward."""
 
     @staticmethod
     def forward(ctx, source, weight, bias, frames_of, stride, out_shape):
@@ -58,11 +79,16 @@ class _U8Conv(torch.autograd.Function):
         if not weight.is_contiguous() or (bias is not None and not bias.is_contiguous()):
             raise ValueError("U8Conv2d: weight and bias must be contiguous")
         src = frames_of(source)
-        out = torch.empty(out_shape, dtype=torch.float32, device=weight.device)
-        _call(weight.device, "vn_conv_u8_forward", C.byref(src), weight.data_ptr(), L.ptr(bias), cout, k, stride,
-              out.data_ptr(), stream_of=weight)
+        dtype = _autocast_dtype()
+        out = torch.empty(out_shape, dtype=dtype or torch.float32, device=weight.device)
+        if dtype is None:
+            _call(weight.device, "vn_conv_u8_forward", C.byref(src), weight.data_ptr(), L.ptr(bias), cout, k, stride,
+                  out.data_ptr(), stream_of=weight)
+        else:
+            _call(weight.device, "vn_conv_u8_forward_lp", C.byref(src), weight.data_ptr(), L.ptr(bias), cout, k,
+                  stride, _LP_DTYPES[dtype], out.data_ptr(), stream_of=weight)
         ctx.save_for_backward(source)
-        ctx.frames_of, ctx.stride, ctx.has_bias = frames_of, stride, bias is not None
+        ctx.frames_of, ctx.stride, ctx.has_bias, ctx.dtype = frames_of, stride, bias is not None, dtype
         ctx.wshape = tuple(weight.shape)
         return out
 
@@ -75,6 +101,8 @@ class _U8Conv(torch.autograd.Function):
         src = ctx.frames_of(source)
         cout, c, k, _ = ctx.wshape
         dev = grad_out.device
+        if ctx.dtype is not None:
+            grad_out = grad_out.to(ctx.dtype)  # a copy kernel only when the gradient arrives in another dtype
         grad_out = grad_out.contiguous()      # a copy kernel only when autograd hands over a non-contiguous gradient
         gw = torch.empty(ctx.wshape, dtype=torch.float32, device=dev)
         gb = torch.empty(cout, dtype=torch.float32, device=dev) if ctx.has_bias else None
@@ -85,8 +113,12 @@ class _U8Conv(torch.autograd.Function):
         else:
             nbytes = L.load().vn_conv_u8_wgrad_scratch_bytes(src.n, c, cout, k)
             scratch = torch.empty(nbytes, dtype=torch.uint8, device=dev)
-            _call(dev, "vn_conv_u8_backward", C.byref(src), grad_out.data_ptr(), cout, k, ctx.stride, gw.data_ptr(),
-                  L.ptr(gb), scratch.data_ptr(), nbytes, stream_of=grad_out)
+            if ctx.dtype is None:
+                _call(dev, "vn_conv_u8_backward", C.byref(src), grad_out.data_ptr(), cout, k, ctx.stride,
+                      gw.data_ptr(), L.ptr(gb), scratch.data_ptr(), nbytes, stream_of=grad_out)
+            else:
+                _call(dev, "vn_conv_u8_backward_lp", C.byref(src), grad_out.data_ptr(), _LP_DTYPES[ctx.dtype], cout, k,
+                      ctx.stride, gw.data_ptr(), L.ptr(gb), scratch.data_ptr(), nbytes, stream_of=grad_out)
         return None, (gw if need_w else None), (gb if need_b else None), None, None, None
 
 
@@ -95,7 +127,9 @@ class U8Conv2d(torch.nn.Conv2d):
 
     Same constructor, parameter initialisation and ``state_dict`` keys as ``nn.Conv2d``.  Supported: 1 or 3 input
     channels, a square kernel of 1..8, stride 1..kernel (square), 8..64 output channels in steps of 8, no padding,
-    dilation or groups, frames of kernel..174 pixels a side; anything else raises ``ValueError`` here."""
+    dilation or groups, frames of kernel..174 pixels a side; anything else raises ``ValueError`` here.  Under
+    ``torch.autocast`` with fp16 or bf16 the output has that dtype (see the module docstring for the numerics); the
+    autocast state is the only switch, as for ``nn.Conv2d``."""
 
     def __init__(self, in_channels, out_channels, kernel_size, stride=1, padding=0, dilation=1, groups=1, bias=True,
                  padding_mode="zeros", device=None, dtype=None):
@@ -137,7 +171,7 @@ class U8Conv2d(torch.nn.Conv2d):
 
     def forward(self, frames):
         """frames: uint8 CUDA ``[N, H, W, C]`` (rows a multiple of 16 bytes apart, e.g. a GraphVecEnv observation leaf)
-        -> float32 ``[N, out_channels, oh, ow]``."""
+        -> float32 ``[N, out_channels, oh, ow]`` (fp16 / bf16 under autocast with that dtype)."""
         if not torch.is_tensor(frames) or frames.dtype != torch.uint8:
             raise TypeError("U8Conv2d takes uint8 [N, H, W, C] frames, got %s" %
                             (frames.dtype if torch.is_tensor(frames) else type(frames).__name__))
@@ -151,7 +185,7 @@ class U8Conv2d(torch.nn.Conv2d):
     def forward_states(self, dw, states, plane="rgb"):
         """The frames of store plane `plane` at the records ``states`` (int32 ``[N]`` or ``[B, T]`` with any strides,
         e.g. ``env.obs_state`` or ``buf.states[:-1].t()``, read in place) -> float32 ``[*states.shape, out_channels,
-        oh, ow]``.  As with ``vn_gather_plane``, ``states`` must hold valid record indices."""
+        oh, ow]`` (fp16 / bf16 under autocast with that dtype).  As with ``vn_gather_plane``, ``states`` must hold valid record indices."""
         lay = dw.world.layout
         if lay.channels[dw.plane_index(plane)] != self.in_channels:
             raise ValueError("U8Conv2d: plane %r has %d channels, the layer takes %d"

@@ -34,7 +34,7 @@
 extern "C" {
 #endif
 
-#define VN_ABI_VERSION 4
+#define VN_ABI_VERSION 5
 #define VN_MAX_PLANES 6 /* rgb, depth, segmentation (+ the 3 third-person planes of graph/thor_graph.py:25-31) */
 
 /* error codes */
@@ -524,6 +524,25 @@ int64_t vn_conv_u8_wgrad_scratch_bytes(int32_t n, int32_t c, int32_t cout, int32
  * over the chunks in a fixed order - no atomics, the same bits on every run and every device size. */
 int32_t vn_conv_u8_backward(const vn_u8_frames_t *src, const float *grad_out, int32_t cout, int32_t k, int32_t stride,
                             float *grad_weight, float *grad_bias, void *scratch, int64_t scratch_bytes, void *stream);
+
+/* The same layer under torch.autocast with a 16-bit dtype (mixed precision).  out and grad_out are of `dtype`, weight,
+ * bias, grad_weight and grad_bias stay float32.  The forward computes
+ *   out = round_to_dtype(fp32(conv2d(x / 255, round_to_dtype(weight), round_to_dtype(bias), stride)))
+ * with the weight and bias rounded to nearest-even in its prologue (autocast's cast), the pixel NOT rounded (0..255 is
+ * exact in both types; 1/255 is applied in fp32 as in vn_conv_u8_forward), every product exact on the tensor cores
+ * with one term per operand, fp32 accumulation, and one rounding of the result (fp16 overflows to +-inf).  The backward
+ * takes grad_out in `dtype`, forms every product exactly, and writes the fp32 weight / bias gradient with the two
+ * kernels and the scratch (vn_conv_u8_wgrad_scratch_bytes) of vn_conv_u8_backward; a non-finite grad_out element makes
+ * its output channel's gradients non-finite.  Arguments, limits and launch behaviour are those of the fp32 entry
+ * points; in addition out and grad_out must be 2-byte aligned (any oh * ow, odd ones included), and a dtype other
+ * than VN_DTYPE_F16 / VN_DTYPE_BF16 is VN_EUNSUPPORTED. */
+#define VN_DTYPE_F16 1
+#define VN_DTYPE_BF16 2
+int32_t vn_conv_u8_forward_lp(const vn_u8_frames_t *src, const float *weight, const float *bias, int32_t cout,
+                              int32_t k, int32_t stride, int32_t dtype, void *out, void *stream);
+int32_t vn_conv_u8_backward_lp(const vn_u8_frames_t *src, const void *grad_out, int32_t dtype, int32_t cout,
+                               int32_t k, int32_t stride, float *grad_weight, float *grad_bias,
+                               void *scratch, int64_t scratch_bytes, void *stream);
 
 #ifdef __cplusplus
 }

@@ -8,6 +8,11 @@ torch.cuda.max_memory_allocated over forward + backward (above what was allocate
 its HBM share against bench.measured_peak(), and the tensor-core rate of the fused kernels.  Then one "step + first
 layer" loop: the aux5 uint8 env + U8Conv2d on the rgb and goal leaves against scaled_float=True + nn.Conv2d.
 
+Every row also runs under torch.autocast with bf16 and fp16 (keys "ac_bf16_*" / "ac_f16_*"): U8Conv2d's one-term 16-bit
+kernels against torch's own float path under the same autocast, with grad_out in the autocast dtype.  Their issued
+tensor-core work is a third of the fp32 kernels' (one mma per k-step instead of three); "useful" counts the
+convolution's multiply-adds alone (forward, plus as many again for the weight gradient).
+
     python tools/bench_u8conv.py [--reps 20] [--out record.json]
 """
 import argparse
@@ -28,6 +33,7 @@ import bench  # noqa: E402
 
 GEOMS = {"ref_3x32_k7s4": (3, 32, 7, 4), "example_3x16_k8s4": (3, 16, 8, 4)}
 ENVS, STEPS = 4096, 20
+AUTOCAST = {"bf16": torch.bfloat16, "f16": torch.float16}
 
 
 def gpu_info():
@@ -136,6 +142,37 @@ def main():
             res["update_float_tf32_%s_peak_bytes" % tf32] = peak_bytes(float_update)
         torch.backends.cudnn.allow_tf32 = True
         res["update_float_bytes_min"] = n * (frame_u8 + 4 * frame_u8 + 2 * 4 * frame_u8 + 2 * out_b)
+        for tag, dtype in AUTOCAST.items():
+            ac = "ac_%s_" % tag
+            go_lp = go.to(dtype)
+
+            def lp_update():
+                layer.zero_grad(set_to_none=True)
+                with torch.autocast("cuda", dtype=dtype):
+                    y = layer.forward_states(dw, states)
+                y.backward(go_lp)
+
+            def lp_float_update():
+                conv.zero_grad(set_to_none=True)
+                with torch.autocast("cuda", dtype=dtype):
+                    y = conv(vn.rollout.policy_input(dw, states).flatten(0, 1))
+                y.backward(go_lp.flatten(0, 1))
+
+            with torch.no_grad(), torch.autocast("cuda", dtype=dtype):
+                t = timed(lambda: layer(obs), args.reps)
+                res[ac + "act_fused_ms"] = t
+                res[ac + "act_fused_tensor_tflops_issued"] = ENVS * mma_flop / 3 / (t * 1e-3) / 1e12
+                res[ac + "act_useful_tflops"] = ENVS * useful / (t * 1e-3) / 1e12
+                res[ac + "act_float_ms"] = timed(lambda: conv(vn.rollout.policy_input(dw, env.obs_state)), args.reps)
+                res[ac + "update_fused_fwd_ms"] = timed(lambda: layer.forward_states(dw, states), args.reps)
+            t = timed(lp_update, args.reps)
+            res[ac + "update_fused_fwd_bwd_ms"] = t
+            res[ac + "update_fused_peak_bytes"] = peak_bytes(lp_update)
+            res[ac + "update_fused_tensor_tflops_issued"] = n * (mma_flop + wg_flop) / 3 / (t * 1e-3) / 1e12
+            res[ac + "update_useful_tflops"] = n * 2 * useful / (t * 1e-3) / 1e12
+            res[ac + "update_float_fwd_bwd_ms"] = timed(lp_float_update, args.reps)
+            res[ac + "update_float_peak_bytes"] = peak_bytes(lp_float_update)
+            del go_lp
         rec["results"][name] = res
         del go
 
@@ -169,6 +206,12 @@ def main():
         torch.backends.cudnn.allow_tf32 = True
         ms = timed(u8_loop, 3, warmup=1)
         loop["u8_env_steps_per_s"] = ENVS * args.loop_steps / (ms * 1e-3)
+        for tag, dtype in AUTOCAST.items():
+            with torch.autocast("cuda", dtype=dtype):
+                ms = timed(float_loop, 3, warmup=1)
+                loop["ac_%s_float_env_steps_per_s" % tag] = ENVS * args.loop_steps / (ms * 1e-3)
+                ms = timed(u8_loop, 3, warmup=1)
+                loop["ac_%s_u8_env_steps_per_s" % tag] = ENVS * args.loop_steps / (ms * 1e-3)
     rec["step_plus_first_layer"] = loop
     line = json.dumps(rec)
     print(line)
