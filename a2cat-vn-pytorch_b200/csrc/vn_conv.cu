@@ -15,6 +15,17 @@
 // rounded to T once (round-to-nearest-even, as autocast's cast), grad_out arrives in T, and a pixel is exact in either
 // type, so every product is exact with ONE term: one mma.sync per k-step instead of three.  Accumulation, the 1/255
 // scale and the reduction are those of the fp32 kernels; the forward rounds its fp32 result to T once.
+//
+// Plane sets (the vn_conv_u8_planes_* entry points, S = kMaxSrcs) read the frames of up to four sources (RGB-D,
+// observation + goal) as one input of C = sum c_s channels in source order.  Each source's frame has its own region of
+// the frame buffer, filled by its own bulk copy on the buffer's one mbarrier; a tap of the table is packed as
+// (region byte offset of its channel at pixel (ky, kx)) << 2 | c_s, so the byte of output pixel p is at
+// off + pixel(p) * c_s.  K = C * k * k grows to 512, so the forward splits the output channels into groups of NT * 8
+// whose weight fragments fit in shared memory (a CTA keeps one group for its whole life and reads every frame it owns
+// once per group), and the weight gradient splits the (cout, tap) tiles into groups of at most kWgradWarps * kWgradTiles
+// (a CTA keeps one group and sums its chunks' frames for that group).  Both kernels keep the k-step and frame order of
+// the single-frame kernels, so every output element is computed with the same operations in the same order.  The S = 1
+// instantiations behind vn_conv_u8_forward / vn_conv_u8_backward compile none of this.
 #include <cuda_bf16.h>
 #include <cuda_fp16.h>
 
@@ -31,6 +42,8 @@ constexpr int kWgradWarps = 8;
 constexpr int kWgradTiles = 13;    // (cout, tap) tiles of 16 x 8 per warp: 4 x 25 at most over 8 warps
 constexpr int kWgradChunk = 32;    // frames per partial gradient
 constexpr int kReduceLanes = 32;   // chunks summed in parallel per output of the reduce kernel
+constexpr int kMaxSrcs = 4;        // frame sources of a plane set
+constexpr int kMaxSetChannels = 8; // channels of a plane set
 
 // ---------------------------------------------------------------- device helpers
 __device__ __forceinline__ const uint8_t *frame_src(const vn_u8_frames_t &f, int i) {
@@ -152,6 +165,22 @@ __device__ __forceinline__ int pix_base(int p, int ow, int stride, int w, int c)
     const int oy = p / ow, ox = p - oy * ow;
     return (oy * stride * w + ox * stride) * c;
 }
+// the packed plane-set tap of input channel ci (of the set) at window pixel pix = ky * w + kx; 0 (byte 0) past the set
+template <int S>
+__device__ __forceinline__ int set_tap(const vn_u8_frames_t (&src)[S], const int (&region)[S + 1], int n_srcs, int ci,
+                                       int pix) {
+    int t = 0;
+#pragma unroll
+    for (int s = 0; s < S; ++s)
+        if (s < n_srcs) {
+            const int cs = src[s].c;
+            if (ci >= 0 && ci < cs) t = (region[s] + pix * cs + ci) << 2 | cs;
+            ci -= cs;
+        }
+    return t;
+}
+// the plane-set byte of tap t for the output pixel whose window corner is pixel pp of the frame
+__device__ __forceinline__ uint32_t set_px(const uint8_t *x, int pp, int t) { return x[(t >> 2) + pp * (t & 3)]; }
 
 // The frames of a CTA, double-buffered in shared memory (one buffer when two do not fit): frame number `it` of the
 // CTA's sequence sits in buffer it % nbuf and completes phase it / nbuf of that buffer's mbarrier.
@@ -169,28 +198,57 @@ struct FramePipe {
         return buf + (size_t)slot * fb;
     }
     __device__ int slot(int it) const { return nbuf == 2 ? (it & 1) : 0; }
+    // a plane set's frame f: one bulk copy per source into its region, all on the slot's one transaction
+    template <int S>
+    __device__ void load_set(int slot, const vn_u8_frames_t (&src)[S], const int (&region)[S + 1], int n_srcs,
+                             int f) const {
+        mbar_expect_tx(&bar[slot], (uint32_t)fb);
+        uint8_t *dst = buf + (size_t)slot * fb;
+#pragma unroll
+        for (int s = 0; s < S; ++s)
+            if (s < n_srcs)
+                bulk_g2s(dst + region[s], frame_src(src[s], f), (uint32_t)(region[s + 1] - region[s]), &bar[slot]);
+    }
 };
 
+// The frame sources of a kernel: one (S = 1), or a plane set of n_srcs <= S sources whose frames sit at region[s] of a
+// frame buffer (region[n_srcs] = fb), their output channels or tiles split into `groups` groups.
+template <int S>
 struct FwdArgs {
-    vn_u8_frames_t src;
+    vn_u8_frames_t src[S];
     const float *weight;   // [cout][K], K = c * k * k
     const float *bias;     // [cout] or null
     void *out;             // [n][cout][oh][ow] of the kernel's element type
     int k, stride, oh, ow, K, ksteps, nbuf, fb;
+    int n_srcs, groups, cout;
+    int region[S + 1];
 };
+
+template <int S>
+__device__ __forceinline__ void load_frame(const FramePipe &pipe, int slot, const FwdArgs<S> &a, int f) {
+    if constexpr (S == 1)
+        pipe.load(slot, frame_src(a.src[0], f));
+    else
+        pipe.load_set(slot, a.src, a.region, a.n_srcs, f);
+}
 
 // Persistent grid; a CTA owns whole frames.  Its prologue splits (fp32) or rounds (16-bit T) the weights into shared
 // memory in mma B-fragment order ([k-step][n-tile][hi, mid, lo or the one term][lane] uint2).  A warp owns two 16-pixel
 // m-tiles of a frame and every output channel; the A fragments are the frame's bytes picked through a tap-offset table
 // (implicit im2col).  Each C fragment row is 8 consecutive pixels of one channel, so every fp32 store instruction
 // writes whole 32-byte sectors of the NCHW output (16-bit ones write half sectors, which L2 joins: the other half is
-// the same thread's row g + 8).
-template <int NT, typename T>   // cout / 8, element type
-__global__ void __launch_bounds__(kFwdWarps * 32) vn_conv_u8_fwd_kernel(const FwdArgs a) {
+// the same thread's row g + 8).  A plane-set CTA owns output channels [grp * NT * 8, ...) of its frames.
+template <int NT, typename T, int S>   // output channels of a CTA / 8, element type, frame sources
+__global__ void __launch_bounds__(kFwdWarps * 32, 1) vn_conv_u8_fwd_kernel(const FwdArgs<S> a) {
     constexpr int TERMS = kTerms<T>;
+    constexpr bool SET = S > 1;
     extern __shared__ __align__(128) uint8_t smem[];
     const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31, g = lane >> 2, tig = lane & 3;
-    const int w = a.src.w, c = a.src.c, K = a.K, ksteps = a.ksteps;
+    const int w = a.src[0].w, c = a.src[0].c, K = a.K, ksteps = a.ksteps;
+    // a plane-set CTA's first frame, frame step and first output channel (blockIdx.x, gridDim.x and 0 otherwise)
+    const auto f0 = [&] { if constexpr (SET) return (int)blockIdx.x / a.groups; else return blockIdx.x; };
+    const auto fstep = [&] { if constexpr (SET) return (int)gridDim.x / a.groups; else return gridDim.x; };
+    const auto co0 = [&] { if constexpr (SET) return (int)blockIdx.x % a.groups * NT * 8; else return 0; };
     uint2 *wfrag = reinterpret_cast<uint2 *>(smem + (size_t)a.nbuf * a.fb);
     int *tap = reinterpret_cast<int *>(wfrag + ksteps * NT * TERMS * 32);
     float *sbias = reinterpret_cast<float *>(tap + ksteps * 16);
@@ -202,7 +260,10 @@ __global__ void __launch_bounds__(kFwdWarps * 32) vn_conv_u8_fwd_kernel(const Fw
         int off = 0;   // padding taps read byte 0: their weight is zero
         if (t < K) {
             const int ci = t / kk2, r = t - ci * kk2, ky = r / a.k, kx = r - ky * a.k;
-            off = (ky * w + kx) * c + ci;
+            if constexpr (SET)
+                off = set_tap(a.src, a.region, a.n_srcs, ci, ky * w + kx);
+            else
+                off = (ky * w + kx) * c + ci;
         }
         tap[t] = off;
     }
@@ -217,7 +278,7 @@ __global__ void __launch_bounds__(kFwdWarps * 32) vn_conv_u8_fwd_kernel(const Fw
     for (int e = tid; e < ksteps * NT * 32; e += blockDim.x) {
         const int ln = e & 31, j = (e >> 5) % NT, ks = (e >> 5) / NT;
         const int n = j * 8 + (ln >> 2), k0 = ks * 16 + (ln & 3) * 2;
-        const float *wr = a.weight + (size_t)n * K;
+        const float *wr = a.weight + (size_t)(co0() + n) * K;
         const float v0 = k0 < K ? wr[k0] : 0.f, v1 = k0 + 1 < K ? wr[k0 + 1] : 0.f;
         const float v8 = k0 + 8 < K ? wr[k0 + 8] : 0.f, v9 = k0 + 9 < K ? wr[k0 + 9] : 0.f;
         if constexpr (TERMS == 3) {
@@ -232,20 +293,21 @@ __global__ void __launch_bounds__(kFwdWarps * 32) vn_conv_u8_fwd_kernel(const Fw
             wfrag[(size_t)(ks * NT + j) * 32 + ln] = make_uint2(pack_rn<T>(v0, v1), pack_rn<T>(v8, v9));
         }
     }
-    for (int co = tid; co < NT * 8; co += blockDim.x) sbias[co] = a.bias ? round_to<T>(a.bias[co]) : 0.f;
-    const int n = a.src.n;
+    for (int co = tid; co < NT * 8; co += blockDim.x) sbias[co] = a.bias ? round_to<T>(a.bias[co0() + co]) : 0.f;
+    const int n = a.src[0].n;
     if (tid == 0)
         for (int s = 0; s < a.nbuf; ++s) {
-            const int f = blockIdx.x + s * gridDim.x;
-            if (f < n) pipe.load(s, frame_src(a.src, f));
+            const int f = f0() + s * fstep();
+            if (f < n) load_frame(pipe, s, a, f);
         }
     __syncthreads();
 
     const int P = a.oh * a.ow, tasks = ((P + 15) / 16 + 1) / 2;
     int it = 0;
-    for (int f = blockIdx.x; f < n; f += gridDim.x, ++it) {
+    for (int f = f0(); f < n; f += fstep(), ++it) {
         const uint8_t *x = pipe.wait(it);
-        T *out = static_cast<T *>(a.out) + (int64_t)f * (NT * 8) * P;
+        T *out = static_cast<T *>(a.out) + (int64_t)f * (SET ? a.cout : NT * 8) * P;
+        if constexpr (SET) out += (int64_t)co0() * P;
         for (int task = warp; task < tasks; task += kFwdWarps) {
             int pb[2][2];
 #pragma unroll
@@ -253,7 +315,7 @@ __global__ void __launch_bounds__(kFwdWarps * 32) vn_conv_u8_fwd_kernel(const Fw
 #pragma unroll
                 for (int r = 0; r < 2; ++r) {
                     const int p = (task * 2 + mt) * 16 + g + r * 8;
-                    pb[mt][r] = p < P ? pix_base(p, a.ow, a.stride, w, c) : 0;
+                    pb[mt][r] = p < P ? pix_base(p, a.ow, a.stride, w, SET ? 1 : c) : 0;
                 }
             float acc[2][NT][4];
 #pragma unroll
@@ -271,9 +333,15 @@ __global__ void __launch_bounds__(kFwdWarps * 32) vn_conv_u8_fwd_kernel(const Fw
                 for (int mt = 0; mt < 2; ++mt)
 #pragma unroll
                     for (int r = 0; r < 2; ++r) {
-                        const uint8_t *row = x + pb[mt][r];
-                        af[mt][r] = pack_px<T>(u8f(row[t01.x]), u8f(row[t01.y]));
-                        af[mt][2 + r] = pack_px<T>(u8f(row[t89.x]), u8f(row[t89.y]));
+                        if constexpr (SET) {
+                            const int pp = pb[mt][r];
+                            af[mt][r] = pack_px<T>(u8f(set_px(x, pp, t01.x)), u8f(set_px(x, pp, t01.y)));
+                            af[mt][2 + r] = pack_px<T>(u8f(set_px(x, pp, t89.x)), u8f(set_px(x, pp, t89.y)));
+                        } else {
+                            const uint8_t *row = x + pb[mt][r];
+                            af[mt][r] = pack_px<T>(u8f(row[t01.x]), u8f(row[t01.y]));
+                            af[mt][2 + r] = pack_px<T>(u8f(row[t89.x]), u8f(row[t89.y]));
+                        }
                     }
                 const uint2 *wf = wfrag + (size_t)ks * NT * TERMS * 32 + lane;
 #pragma unroll
@@ -305,25 +373,36 @@ __global__ void __launch_bounds__(kFwdWarps * 32) vn_conv_u8_fwd_kernel(const Fw
                 }
         }
         __syncthreads();   // every warp is done with this buffer
-        const int next = f + a.nbuf * gridDim.x;
+        const int next = f + a.nbuf * fstep();
         if (tid == 0 && next < n) {
             fence_proxy_async();
-            pipe.load(pipe.slot(it), frame_src(a.src, next));
+            load_frame(pipe, pipe.slot(it), a, next);
         }
     }
 }
 
+template <int S>
 struct WgradArgs {
-    vn_u8_frames_t src;
+    vn_u8_frames_t src[S];
     const void *grad_out;    // [n][cout][oh][ow] of the kernel's element type
     float *partial;          // [chunks][cout][K + 1]
     int cout, k, stride, oh, ow, K, mtiles, ntiles, nbuf, fb;
+    int n_srcs, groups, group_tiles;
+    int region[S + 1];
 };
 
-// The frames of chunk q are [q * kWgradChunk, ...): the CTA's next frame after f.
-__device__ __forceinline__ int next_frame(int f, int n) {
+template <int S>
+__device__ __forceinline__ void load_frame(const FramePipe &pipe, int slot, const WgradArgs<S> &a, int f) {
+    if constexpr (S == 1)
+        pipe.load(slot, frame_src(a.src[0], f));
+    else
+        pipe.load_set(slot, a.src, a.region, a.n_srcs, f);
+}
+
+// The frames of chunk q are [q * kWgradChunk, ...): the CTA's next frame after f, its chunks `cstep` apart.
+__device__ __forceinline__ int next_frame(int f, int n, int cstep) {
     const int chunk_end = min(n, (f / kWgradChunk + 1) * kWgradChunk);
-    return f + 1 < chunk_end ? f + 1 : (f / kWgradChunk + (int)gridDim.x) * kWgradChunk;
+    return f + 1 < chunk_end ? f + 1 : (f / kWgradChunk + cstep) * kWgradChunk;
 }
 
 // dW[co][t] = sum over the chunk's frames and output pixels p of g[co][p] * x[tap t of p]: an implicit GEMM with
@@ -332,12 +411,17 @@ __device__ __forceinline__ int next_frame(int f, int n) {
 // are B.  A warp owns up to kWgradTiles (16 x 8) output tiles for the whole chunk.  Its registers sum one frame; the
 // frame sums are added into the thread's own shared-memory column, and the chunk's raw sums go to partial[chunk].
 // 16-bit grad_out is read one element at a time: a channel row is only 2-byte aligned when oh * ow is odd.
-template <typename T>
-__global__ void __launch_bounds__(kWgradWarps * 32) vn_conv_u8_wgrad_kernel(const WgradArgs a) {
+// A plane-set CTA owns tiles [grp * group_tiles, ...) of its chunks.
+template <typename T, int S>
+__global__ void __launch_bounds__(kWgradWarps * 32) vn_conv_u8_wgrad_kernel(const WgradArgs<S> a) {
     constexpr int TERMS = kTerms<T>;
+    constexpr bool SET = S > 1;
     extern __shared__ __align__(128) uint8_t smem[];
     const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31, g = lane >> 2, tig = lane & 3;
-    const int w = a.src.w, c = a.src.c, K = a.K, K1 = a.K + 1, cout = a.cout;
+    const int w = a.src[0].w, c = a.src[0].c, K = a.K, K1 = a.K + 1, cout = a.cout;
+    // a plane-set CTA's first chunk and chunk step (blockIdx.x and gridDim.x otherwise)
+    const auto chunk0 = [&] { if constexpr (SET) return (int)blockIdx.x / a.groups; else return blockIdx.x; };
+    const auto cstep = [&] { if constexpr (SET) return (int)gridDim.x / a.groups; else return (int)gridDim.x; };
     int *tap = reinterpret_cast<int *>(smem + (size_t)a.nbuf * a.fb);
     uint64_t *bar = reinterpret_cast<uint64_t *>(tap + a.ntiles * 8);
     float *chunk_acc = reinterpret_cast<float *>(bar + 2) + tid;   // this thread's [kWgradTiles * 4] column
@@ -348,7 +432,10 @@ __global__ void __launch_bounds__(kWgradWarps * 32) vn_conv_u8_wgrad_kernel(cons
         int off = t == K ? -1 : -2;   // -1: the bias tap (reads 1), -2: padding (reads 0)
         if (t < K) {
             const int ci = t / kk2, r = t - ci * kk2, ky = r / a.k, kx = r - ky * a.k;
-            off = (ky * w + kx) * c + ci;
+            if constexpr (SET)
+                off = set_tap(a.src, a.region, a.n_srcs, ci, ky * w + kx);
+            else
+                off = (ky * w + kx) * c + ci;
         }
         tap[t] = off;
     }
@@ -360,8 +447,13 @@ __global__ void __launch_bounds__(kWgradWarps * 32) vn_conv_u8_wgrad_kernel(cons
     asm volatile("griddepcontrol.wait;" ::: "memory");
     __syncthreads();
 
-    const int tiles = a.mtiles * a.ntiles, per = (tiles + kWgradWarps - 1) / kWgradWarps;
-    const int t0 = warp * per, cnt = max(0, min(per, tiles - t0));
+    int tiles = a.mtiles * a.ntiles, g0 = 0;   // this CTA's tiles: [g0, tiles)
+    if constexpr (SET) {
+        g0 = (int)blockIdx.x % a.groups * a.group_tiles;
+        tiles = min(tiles, g0 + a.group_tiles);
+    }
+    const int per = (tiles - g0 + kWgradWarps - 1) / kWgradWarps;
+    const int t0 = g0 + warp * per, cnt = max(0, min(per, tiles - t0));
     int tmi[kWgradTiles], toff[kWgradTiles];
 #pragma unroll
     for (int i = 0; i < kWgradTiles; ++i) {
@@ -370,15 +462,15 @@ __global__ void __launch_bounds__(kWgradWarps * 32) vn_conv_u8_wgrad_kernel(cons
         toff[i] = tap[(tl - mi * a.ntiles) * 8 + g];
     }
 
-    const int n = a.src.n, P = a.oh * a.ow, ksteps = (P + 15) / 16;
-    int f = blockIdx.x * kWgradChunk;
+    const int n = a.src[0].n, P = a.oh * a.ow, ksteps = (P + 15) / 16;
+    int f = chunk0() * kWgradChunk;
     if (tid == 0 && f < n) {
-        pipe.load(0, frame_src(a.src, f));
-        const int f1 = next_frame(f, n);
-        if (a.nbuf == 2 && f1 < n) pipe.load(1, frame_src(a.src, f1));
+        load_frame(pipe, 0, a, f);
+        const int f1 = next_frame(f, n, cstep());
+        if (a.nbuf == 2 && f1 < n) load_frame(pipe, 1, a, f1);
     }
     int it = 0;
-    for (int chunk = blockIdx.x; chunk * kWgradChunk < n; chunk += gridDim.x) {
+    for (int chunk = chunk0(); chunk * kWgradChunk < n; chunk += cstep()) {
         float acc[kWgradTiles][4];
 #pragma unroll
         for (int i = 0; i < kWgradTiles; ++i)
@@ -388,16 +480,16 @@ __global__ void __launch_bounds__(kWgradWarps * 32) vn_conv_u8_wgrad_kernel(cons
                 chunk_acc[(i * 4 + q) * kWgradWarps * 32] = 0.f;
             }
         const int end = min(n, (chunk + 1) * kWgradChunk);
-        for (; f < end; f = next_frame(f, n), ++it) {
+        for (; f < end; f = next_frame(f, n, cstep()), ++it) {
             const uint8_t *x = pipe.wait(it);
             const T *gf = static_cast<const T *>(a.grad_out) + (int64_t)f * cout * P;
 #pragma unroll 1
             for (int ks = 0; ks < ksteps; ++ks) {
-                const int p0 = ks * 16 + tig * 2;
-                const int pb0 = p0 < P ? pix_base(p0, a.ow, a.stride, w, c) : 0;
-                const int pb1 = p0 + 1 < P ? pix_base(p0 + 1, a.ow, a.stride, w, c) : 0;
-                const int pb8 = p0 + 8 < P ? pix_base(p0 + 8, a.ow, a.stride, w, c) : 0;
-                const int pb9 = p0 + 9 < P ? pix_base(p0 + 9, a.ow, a.stride, w, c) : 0;
+                const int p0 = ks * 16 + tig * 2, cp = SET ? 1 : c;
+                const int pb0 = p0 < P ? pix_base(p0, a.ow, a.stride, w, cp) : 0;
+                const int pb1 = p0 + 1 < P ? pix_base(p0 + 1, a.ow, a.stride, w, cp) : 0;
+                const int pb8 = p0 + 8 < P ? pix_base(p0 + 8, a.ow, a.stride, w, cp) : 0;
+                const int pb9 = p0 + 9 < P ? pix_base(p0 + 9, a.ow, a.stride, w, cp) : 0;
                 int cur = -1;
                 uint32_t ah[4], am[4], al[4];
 #pragma unroll
@@ -429,10 +521,17 @@ __global__ void __launch_bounds__(kWgradWarps * 32) vn_conv_u8_wgrad_kernel(cons
                     const int o = toff[i];
                     float b0, b1, b8, b9;
                     if (o >= 0) {
-                        b0 = u8f(x[pb0 + o]);
-                        b1 = u8f(x[pb1 + o]);
-                        b8 = u8f(x[pb8 + o]);
-                        b9 = u8f(x[pb9 + o]);
+                        if constexpr (SET) {
+                            b0 = u8f(set_px(x, pb0, o));
+                            b1 = u8f(set_px(x, pb1, o));
+                            b8 = u8f(set_px(x, pb8, o));
+                            b9 = u8f(set_px(x, pb9, o));
+                        } else {
+                            b0 = u8f(x[pb0 + o]);
+                            b1 = u8f(x[pb1 + o]);
+                            b8 = u8f(x[pb8 + o]);
+                            b9 = u8f(x[pb9 + o]);
+                        }
                     } else {
                         b0 = b1 = b8 = b9 = o == -1 ? 1.f : 0.f;
                     }
@@ -453,11 +552,11 @@ __global__ void __launch_bounds__(kWgradWarps * 32) vn_conv_u8_wgrad_kernel(cons
                 }
             __syncthreads();   // every warp is done with this buffer
             if (tid == 0) {
-                int nx = next_frame(f, n);
-                if (a.nbuf == 2 && nx < n) nx = next_frame(nx, n);
+                int nx = next_frame(f, n, cstep());
+                if (a.nbuf == 2 && nx < n) nx = next_frame(nx, n, cstep());
                 if (nx < n) {
                     fence_proxy_async();
-                    pipe.load(pipe.slot(it), frame_src(a.src, nx));
+                    load_frame(pipe, pipe.slot(it), a, nx);
                 }
             }
         }
@@ -509,14 +608,15 @@ __global__ void __launch_bounds__(kReduceLanes * 32) vn_conv_u8_wgrad_reduce_ker
 // ---------------------------------------------------------------- host side
 struct ConvGeom {
     int oh, ow, K, fb;
+    int c;                      // input channels (of the whole set)
+    int region[kMaxSrcs + 1];   // plane sets: byte offset of each source's frame in a frame buffer
 };
 
 static bool aligned4(const void *p) { return (reinterpret_cast<uintptr_t>(p) & 3) == 0; }
 static bool aligned2(const void *p) { return (reinterpret_cast<uintptr_t>(p) & 1) == 0; }
 
-// Checks the frame source and the layer shape shared by the forward and the backward.
-static int32_t conv_args(const vn_u8_frames_t *src, int32_t cout, int32_t k, int32_t stride, const char *who, ConvGeom *g) {
-    VN_REQUIRE(src, "%s: src is null", who);
+// Checks one frame source up to its channel count.
+static int32_t source_args(const vn_u8_frames_t *src, const char *who) {
     VN_REQUIRE(src->n >= 0, "%s: n=%d", who, src->n);
     VN_REQUIRE(src->base, "%s: frame base is null", who);
     VN_REQUIRE(aligned16(src->base) && (src->pitch & 15) == 0, "%s: frame base and pitch (%lld) must be 16-byte aligned",
@@ -530,6 +630,12 @@ static int32_t conv_args(const vn_u8_frames_t *src, int32_t cout, int32_t k, int
         set_error("%s: %d channels (1 or 3 are supported)", who, src->c);
         return VN_EUNSUPPORTED;
     }
+    return VN_OK;
+}
+
+// Checks the layer shape for frames of `src`'s size with c input channels in all.
+static int32_t layer_args(const vn_u8_frames_t *src, int c, int32_t cout, int32_t k, int32_t stride, const char *who,
+                          ConvGeom *g) {
     if (k < 1 || k > 8 || stride < 1 || stride > k) {
         set_error("%s: kernel %d, stride %d (1 <= stride <= kernel <= 8 are supported)", who, k, stride);
         return VN_EUNSUPPORTED;
@@ -545,27 +651,88 @@ static int32_t conv_args(const vn_u8_frames_t *src, int32_t cout, int32_t k, int
     }
     g->oh = (src->h - k) / stride + 1;
     g->ow = (src->w - k) / stride + 1;
-    g->K = src->c * k * k;
+    g->K = c * k * k;
+    g->c = c;
+    return VN_OK;
+}
+
+// Checks the frame source and the layer shape shared by the forward and the backward.
+static int32_t conv_args(const vn_u8_frames_t *src, int32_t cout, int32_t k, int32_t stride, const char *who, ConvGeom *g) {
+    VN_REQUIRE(src, "%s: src is null", who);
+    int32_t rc = source_args(src, who);
+    if (rc) return rc;
+    rc = layer_args(src, src->c, cout, k, stride, who, g);
+    if (rc) return rc;
     g->fb = (src->h * src->w * src->c + 15) & ~15;
+    g->region[0] = 0;
+    g->region[1] = g->fb;
+    return VN_OK;
+}
+
+// Shared memory past the frame buffers: the forward's weight fragments of nt n-tiles, tap table and bias, and the
+// weight gradient's tap table and per-thread chunk sums.
+template <typename T>
+static int fwd_rest(int ksteps, int nt) { return ksteps * nt * kTerms<T> * 32 * 8 + ksteps * 16 * 4 + nt * 8 * 4 + 16; }
+static int wgrad_rest(int ntiles) { return ntiles * 8 * 4 + 16 + kWgradTiles * 4 * kWgradWarps * 32 * 4; }
+
+// Checks a plane set (1 .. kMaxSrcs sources of one size and index shape, 1 or 3 channels each, kMaxSetChannels in all)
+// and the layer shape, and that one frame buffer of the set fits beside the tables of both kernels.
+static int32_t set_args(const vn_u8_frames_t *srcs, int32_t n_srcs, int32_t cout, int32_t k, int32_t stride,
+                        const char *who, ConvGeom *g) {
+    VN_REQUIRE(srcs, "%s: srcs is null", who);
+    VN_REQUIRE(n_srcs >= 1, "%s: %d sources", who, n_srcs);
+    if (n_srcs > kMaxSrcs) {
+        set_error("%s: %d sources (1 to %d are supported)", who, n_srcs, kMaxSrcs);
+        return VN_EUNSUPPORTED;
+    }
+    int c = 0;
+    g->region[0] = 0;
+    for (int s = 0; s < n_srcs; ++s) {
+        const vn_u8_frames_t *f = &srcs[s];
+        char whos[96];
+        snprintf(whos, sizeof whos, "%s: source %d", who, s);
+        const int32_t rc = source_args(f, whos);
+        if (rc) return rc;
+        VN_REQUIRE(f->n == srcs[0].n && f->idx_t == srcs[0].idx_t && f->h == srcs[0].h && f->w == srcs[0].w,
+                   "%s: n, idx_t, h, w (%d, %d, %d, %d) differ from source 0's (%d, %d, %d, %d)", whos, f->n, f->idx_t,
+                   f->h, f->w, srcs[0].n, srcs[0].idx_t, srcs[0].h, srcs[0].w);
+        c += f->c;
+        g->region[s + 1] = g->region[s] + ((f->h * f->w * f->c + 15) & ~15);
+    }
+    if (c > kMaxSetChannels) {
+        set_error("%s: %d channels in all (at most %d are supported)", who, c, kMaxSetChannels);
+        return VN_EUNSUPPORTED;
+    }
+    const int32_t rc = layer_args(srcs, c, cout, k, stride, who, g);
+    if (rc) return rc;
+    g->fb = g->region[n_srcs];
+    const int ksteps = (g->K + 15) / 16, ntiles = (g->K + 1 + 7) / 8;
+    if (g->fb + fwd_rest<float>(ksteps, 1) > kMaxSmemConv || g->fb + wgrad_rest(ntiles) > kMaxSmemConv) {
+        set_error("%s: a %d x %d frame set of %d channels (%d bytes) does not fit in shared memory", who, srcs->h,
+                  srcs->w, c, g->fb);
+        return VN_EUNSUPPORTED;
+    }
     return VN_OK;
 }
 
 static int64_t chunks_of(int64_t n) { return (n + kWgradChunk - 1) / kWgradChunk; }
 
-using FwdKernel = void (*)(const FwdArgs);
-template <typename T>
-static const FwdKernel kFwdKernels[8] = {vn_conv_u8_fwd_kernel<1, T>, vn_conv_u8_fwd_kernel<2, T>,
-                                         vn_conv_u8_fwd_kernel<3, T>, vn_conv_u8_fwd_kernel<4, T>,
-                                         vn_conv_u8_fwd_kernel<5, T>, vn_conv_u8_fwd_kernel<6, T>,
-                                         vn_conv_u8_fwd_kernel<7, T>, vn_conv_u8_fwd_kernel<8, T>};
+template <typename T, int S>
+using FwdKernel = void (*)(const FwdArgs<S>);
+template <typename T, int S>
+static const FwdKernel<T, S> kFwdKernels[8] = {
+    vn_conv_u8_fwd_kernel<1, T, S>, vn_conv_u8_fwd_kernel<2, T, S>, vn_conv_u8_fwd_kernel<3, T, S>,
+    vn_conv_u8_fwd_kernel<4, T, S>, vn_conv_u8_fwd_kernel<5, T, S>, vn_conv_u8_fwd_kernel<6, T, S>,
+    vn_conv_u8_fwd_kernel<7, T, S>, vn_conv_u8_fwd_kernel<8, T, S>};
 
 // Shared memory of `frames_bytes` frame buffers plus `rest`: two buffers when they fit, else one.
 static int frame_buffers(int fb, int rest) { return 2 * fb + rest <= kMaxSmemConv ? 2 : 1; }
 
-// A persistent grid: as many CTAs of `kernel` as are resident at once (registers and shared memory), at most `work`.
+// A persistent grid: as many CTAs of `kernel` as are resident at once (registers and shared memory), at most `work`,
+// a multiple of `groups` (work is).
 template <typename... KArgs>
 static int32_t persistent_grid(void (*kernel)(KArgs...), int threads, int smem, int64_t work, const char *who,
-                               int *grid) {
+                               int *grid, int groups = 1) {
     int per_sm = 0;
     const cudaError_t e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kernel, threads, smem);
     if (e != cudaSuccess || per_sm < 1) {
@@ -573,33 +740,65 @@ static int32_t persistent_grid(void (*kernel)(KArgs...), int threads, int smem, 
         set_error("%s: occupancy query: %s", who, cudaGetErrorString(e));
         return VN_ECUDA;
     }
-    const int64_t cap = (int64_t)sm_count() * per_sm;
+    const int64_t cap = (int64_t)sm_count() * per_sm / groups * groups;
     *grid = (int)(work < cap ? work : cap);
     return VN_OK;
 }
 
-// The forward launch of element type T for checked arguments and n > 0.
-template <typename T>
-static int32_t conv_forward(const vn_u8_frames_t *src, const ConvGeom &g, const float *weight, const float *bias,
-                            int32_t cout, int32_t k, int32_t stride, void *out, void *stream, const char *who) {
-    const int NT = cout / 8, ksteps = (g.K + 15) / 16;
-    const int rest = ksteps * NT * kTerms<T> * 32 * 8 + ksteps * 16 * 4 + NT * 8 * 4 + 16;
+template <typename A>
+static void set_sources(A &a, const vn_u8_frames_t *src, int n_srcs, const ConvGeom &g) {
+    for (int s = 0; s < n_srcs; ++s) a.src[s] = src[s];
+    a.n_srcs = n_srcs;
+    for (int s = 0; s <= n_srcs; ++s) a.region[s] = g.region[s];
+}
+
+// The forward launch of element type T and S frame sources for checked arguments and n > 0.  A plane set splits its
+// output channels into the fewest groups whose weight fragments fit beside two frame buffers, else beside one.
+template <typename T, int S>
+static int32_t conv_forward(const vn_u8_frames_t *src, int n_srcs, const ConvGeom &g, const float *weight,
+                            const float *bias, int32_t cout, int32_t k, int32_t stride, void *out, void *stream,
+                            const char *who) {
+    const int ksteps = (g.K + 15) / 16;
+    int NT = cout / 8, groups = 1;
+    if (S > 1) {
+        int pick = 0;
+        for (int nbuf = 2; nbuf >= 1 && !pick; --nbuf)
+            for (int gr = 1; gr <= NT && !pick; ++gr)
+                if (NT % gr == 0 && nbuf * g.fb + fwd_rest<T>(ksteps, NT / gr) <= kMaxSmemConv) pick = gr;
+        groups = pick;   // set_args checked that one n-tile fits beside one buffer
+        NT /= groups;
+    }
+    const int rest = fwd_rest<T>(ksteps, NT);
     const int nbuf = frame_buffers(g.fb, rest), smem = nbuf * g.fb + rest;
-    const FwdKernel kernel = kFwdKernels<T>[NT - 1];
+    const FwdKernel<T, S> kernel = kFwdKernels<T, S>[NT - 1];
     int32_t rc = ensure_smem(kernel, smem);
     if (rc) return rc;
     int grid;
-    rc = persistent_grid(kernel, kFwdWarps * 32, smem, src->n, who, &grid);
+    rc = persistent_grid(kernel, kFwdWarps * 32, smem, (int64_t)src->n * groups, who, &grid, groups);
     if (rc) return rc;
-    const FwdArgs a{*src, weight, bias, out, k, stride, g.oh, g.ow, g.K, ksteps, nbuf, g.fb};
+    FwdArgs<S> a{};
+    set_sources(a, src, n_srcs, g);
+    a.weight = weight;
+    a.bias = bias;
+    a.out = out;
+    a.k = k;
+    a.stride = stride;
+    a.oh = g.oh;
+    a.ow = g.ow;
+    a.K = g.K;
+    a.ksteps = ksteps;
+    a.nbuf = nbuf;
+    a.fb = g.fb;
+    a.groups = groups;
+    a.cout = cout;
     return launch(kernel, "vn_conv_u8_fwd_kernel", dim3(grid), dim3(kFwdWarps * 32), (size_t)smem,
                   (cudaStream_t)stream, true, a);
 }
 
-// Checks the weight-gradient scratch shared by both backward entry points.
-static int32_t scratch_args(const vn_u8_frames_t *src, int32_t cout, int32_t k, const void *scratch,
-                            int64_t scratch_bytes, const char *who) {
-    const int64_t need = vn_conv_u8_wgrad_scratch_bytes(src->n, src->c, cout, k);
+// Checks the weight-gradient scratch shared by the backward entry points.
+static int32_t scratch_args(const vn_u8_frames_t *src, const ConvGeom &g, int32_t cout, int32_t k,
+                            const void *scratch, int64_t scratch_bytes, const char *who) {
+    const int64_t need = vn_conv_u8_wgrad_scratch_bytes(src->n, g.c, cout, k);
     VN_REQUIRE(scratch_bytes >= need, "%s: %lld scratch bytes, %lld needed", who, (long long)scratch_bytes,
                (long long)need);
     VN_REQUIRE(need == 0 || (scratch && aligned16(scratch)), "%s: scratch must be a 16-byte aligned device buffer",
@@ -607,22 +806,39 @@ static int32_t scratch_args(const vn_u8_frames_t *src, int32_t cout, int32_t k, 
     return VN_OK;
 }
 
-// The two backward launches of element type T for checked arguments and n > 0.
-template <typename T>
-static int32_t conv_backward(const vn_u8_frames_t *src, const ConvGeom &g, const void *grad_out, int32_t cout,
-                             int32_t k, int32_t stride, float *grad_weight, float *grad_bias, void *scratch,
-                             void *stream, const char *who) {
-    const int mtiles = (cout + 15) / 16, ntiles = (g.K + 1 + 7) / 8;
-    const int rest = ntiles * 8 * 4 + 16 + kWgradTiles * 4 * kWgradWarps * 32 * 4;
+// The two backward launches of element type T and S frame sources for checked arguments and n > 0.  A plane set
+// splits its (cout, tap) tiles into the fewest groups of at most kWgradWarps * kWgradTiles.
+template <typename T, int S>
+static int32_t conv_backward(const vn_u8_frames_t *src, int n_srcs, const ConvGeom &g, const void *grad_out,
+                             int32_t cout, int32_t k, int32_t stride, float *grad_weight, float *grad_bias,
+                             void *scratch, void *stream, const char *who) {
+    const int mtiles = (cout + 15) / 16, ntiles = (g.K + 1 + 7) / 8, tiles = mtiles * ntiles;
+    const int groups = S > 1 ? (tiles + kWgradWarps * kWgradTiles - 1) / (kWgradWarps * kWgradTiles) : 1;
+    const int rest = wgrad_rest(ntiles);
     const int nbuf = frame_buffers(g.fb, rest), smem = nbuf * g.fb + rest;
-    int32_t rc = ensure_smem(vn_conv_u8_wgrad_kernel<T>, smem);
+    int32_t rc = ensure_smem(vn_conv_u8_wgrad_kernel<T, S>, smem);
     if (rc) return rc;
     const int64_t chunks = chunks_of(src->n);
     int grid;
-    rc = persistent_grid(vn_conv_u8_wgrad_kernel<T>, kWgradWarps * 32, smem, chunks, who, &grid);
+    rc = persistent_grid(vn_conv_u8_wgrad_kernel<T, S>, kWgradWarps * 32, smem, chunks * groups, who, &grid, groups);
     if (rc) return rc;
-    const WgradArgs a{*src, grad_out, (float *)scratch, cout, k, stride, g.oh, g.ow, g.K, mtiles, ntiles, nbuf, g.fb};
-    rc = launch(vn_conv_u8_wgrad_kernel<T>, "vn_conv_u8_wgrad_kernel", dim3(grid), dim3(kWgradWarps * 32),
+    WgradArgs<S> a{};
+    set_sources(a, src, n_srcs, g);
+    a.grad_out = grad_out;
+    a.partial = (float *)scratch;
+    a.cout = cout;
+    a.k = k;
+    a.stride = stride;
+    a.oh = g.oh;
+    a.ow = g.ow;
+    a.K = g.K;
+    a.mtiles = mtiles;
+    a.ntiles = ntiles;
+    a.nbuf = nbuf;
+    a.fb = g.fb;
+    a.groups = groups;
+    a.group_tiles = (tiles + groups - 1) / groups;
+    rc = launch(vn_conv_u8_wgrad_kernel<T, S>, "vn_conv_u8_wgrad_kernel", dim3(grid), dim3(kWgradWarps * 32),
                 (size_t)smem, (cudaStream_t)stream, true, a);
     if (rc) return rc;
     const int outputs = cout * (g.K + 1);
@@ -631,39 +847,102 @@ static int32_t conv_backward(const vn_u8_frames_t *src, const ConvGeom &g, const
                   (int)cout, g.K, grad_weight, grad_bias);
 }
 
+// The launch of S frame sources in fp32 (lp false) or in the checked 16-bit `dtype`.
+template <int S>
+static int32_t forward_of(const vn_u8_frames_t *src, int n_srcs, const ConvGeom &g, const float *weight,
+                          const float *bias, int32_t cout, int32_t k, int32_t stride, bool lp, int32_t dtype, void *out,
+                          void *stream, const char *who) {
+    if (!lp) return conv_forward<float, S>(src, n_srcs, g, weight, bias, cout, k, stride, out, stream, who);
+    if (dtype == VN_DTYPE_F16) return conv_forward<__half, S>(src, n_srcs, g, weight, bias, cout, k, stride, out, stream, who);
+    return conv_forward<__nv_bfloat16, S>(src, n_srcs, g, weight, bias, cout, k, stride, out, stream, who);
+}
+
+template <int S>
+static int32_t backward_of(const vn_u8_frames_t *src, int n_srcs, const ConvGeom &g, const void *grad_out,
+                           int32_t cout, int32_t k, int32_t stride, float *grad_weight, float *grad_bias,
+                           void *scratch, bool lp, int32_t dtype, void *stream, const char *who) {
+    if (!lp)
+        return conv_backward<float, S>(src, n_srcs, g, grad_out, cout, k, stride, grad_weight, grad_bias, scratch,
+                                       stream, who);
+    if (dtype == VN_DTYPE_F16)
+        return conv_backward<__half, S>(src, n_srcs, g, grad_out, cout, k, stride, grad_weight, grad_bias, scratch,
+                                        stream, who);
+    return conv_backward<__nv_bfloat16, S>(src, n_srcs, g, grad_out, cout, k, stride, grad_weight, grad_bias, scratch,
+                                           stream, who);
+}
+
+static int32_t dtype_arg(int32_t dtype, const char *who) {
+    if (dtype != VN_DTYPE_F16 && dtype != VN_DTYPE_BF16) {
+        set_error("%s: dtype %d (VN_DTYPE_F16 or VN_DTYPE_BF16 are supported)", who, dtype);
+        return VN_EUNSUPPORTED;
+    }
+    return VN_OK;
+}
+
+// The argument checks and launch of every forward entry point: one source (set false) or a plane set of n_srcs, in
+// fp32 (lp false) or in a 16-bit dtype (the _lp entry points).
+static int32_t forward_entry(const vn_u8_frames_t *src, int32_t n_srcs, bool set, const float *weight,
+                             const float *bias, int32_t cout, int32_t k, int32_t stride, bool lp, int32_t dtype,
+                             void *out, void *stream, const char *who) {
+    ConvGeom g;
+    int32_t rc = set ? set_args(src, n_srcs, cout, k, stride, who, &g) : conv_args(src, cout, k, stride, who, &g);
+    if (rc) return rc;
+    if (!lp) {
+        VN_REQUIRE(weight && out, "%s: weight and out must not be null", who);
+        VN_REQUIRE(aligned4(weight) && aligned4(bias) && aligned4(out), "%s: weight, bias and out must be 4-byte aligned",
+                   who);
+    } else {
+        rc = dtype_arg(dtype, who);
+        if (rc) return rc;
+        VN_REQUIRE(weight && out, "%s: weight and out must not be null", who);
+        VN_REQUIRE(aligned4(weight) && aligned4(bias), "%s: weight and bias must be 4-byte aligned", who);
+        VN_REQUIRE(aligned2(out), "%s: out must be 2-byte aligned", who);
+    }
+    if (src->n == 0) return VN_OK;
+    return set ? forward_of<kMaxSrcs>(src, n_srcs, g, weight, bias, cout, k, stride, lp, dtype, out, stream, who)
+               : forward_of<1>(src, 1, g, weight, bias, cout, k, stride, lp, dtype, out, stream, who);
+}
+
+// The argument checks and launches of every backward entry point (see forward_entry).
+static int32_t backward_entry(const vn_u8_frames_t *src, int32_t n_srcs, bool set, const void *grad_out, bool lp,
+                              int32_t dtype, int32_t cout, int32_t k, int32_t stride, float *grad_weight,
+                              float *grad_bias, void *scratch, int64_t scratch_bytes, void *stream, const char *who) {
+    ConvGeom g;
+    int32_t rc = set ? set_args(src, n_srcs, cout, k, stride, who, &g) : conv_args(src, cout, k, stride, who, &g);
+    if (rc) return rc;
+    if (!lp) {
+        VN_REQUIRE(grad_out && grad_weight, "%s: grad_out and grad_weight must not be null", who);
+        VN_REQUIRE(aligned4(grad_out) && aligned4(grad_weight) && aligned4(grad_bias),
+                   "%s: grad_out, grad_weight and grad_bias must be 4-byte aligned", who);
+    } else {
+        rc = dtype_arg(dtype, who);
+        if (rc) return rc;
+        VN_REQUIRE(grad_out && grad_weight, "%s: grad_out and grad_weight must not be null", who);
+        VN_REQUIRE(aligned2(grad_out), "%s: grad_out must be 2-byte aligned", who);
+        VN_REQUIRE(aligned4(grad_weight) && aligned4(grad_bias), "%s: grad_weight and grad_bias must be 4-byte aligned",
+                   who);
+    }
+    rc = scratch_args(src, g, cout, k, scratch, scratch_bytes, who);
+    if (rc) return rc;
+    if (src->n == 0) return VN_OK;
+    return set ? backward_of<kMaxSrcs>(src, n_srcs, g, grad_out, cout, k, stride, grad_weight, grad_bias, scratch, lp,
+                                       dtype, stream, who)
+               : backward_of<1>(src, 1, g, grad_out, cout, k, stride, grad_weight, grad_bias, scratch, lp, dtype,
+                                stream, who);
+}
+
 }  // namespace vn
 
 extern "C" {
 
 int32_t vn_conv_u8_forward(const vn_u8_frames_t *src, const float *weight, const float *bias, int32_t cout, int32_t k,
                            int32_t stride, float *out, void *stream) {
-    vn::ConvGeom g;
-    int32_t rc = vn::conv_args(src, cout, k, stride, "conv_u8_forward", &g);
-    if (rc) return rc;
-    VN_REQUIRE(weight && out, "conv_u8_forward: weight and out must not be null");
-    VN_REQUIRE(vn::aligned4(weight) && vn::aligned4(bias) && vn::aligned4(out),
-               "conv_u8_forward: weight, bias and out must be 4-byte aligned");
-    if (src->n == 0) return VN_OK;
-    return vn::conv_forward<float>(src, g, weight, bias, cout, k, stride, out, stream, "conv_u8_forward");
+    return vn::forward_entry(src, 1, false, weight, bias, cout, k, stride, false, 0, out, stream, "conv_u8_forward");
 }
 
 int32_t vn_conv_u8_forward_lp(const vn_u8_frames_t *src, const float *weight, const float *bias, int32_t cout,
                               int32_t k, int32_t stride, int32_t dtype, void *out, void *stream) {
-    vn::ConvGeom g;
-    int32_t rc = vn::conv_args(src, cout, k, stride, "conv_u8_forward_lp", &g);
-    if (rc) return rc;
-    if (dtype != VN_DTYPE_F16 && dtype != VN_DTYPE_BF16) {
-        vn::set_error("conv_u8_forward_lp: dtype %d (VN_DTYPE_F16 or VN_DTYPE_BF16 are supported)", dtype);
-        return VN_EUNSUPPORTED;
-    }
-    VN_REQUIRE(weight && out, "conv_u8_forward_lp: weight and out must not be null");
-    VN_REQUIRE(vn::aligned4(weight) && vn::aligned4(bias), "conv_u8_forward_lp: weight and bias must be 4-byte aligned");
-    VN_REQUIRE(vn::aligned2(out), "conv_u8_forward_lp: out must be 2-byte aligned");
-    if (src->n == 0) return VN_OK;
-    return dtype == VN_DTYPE_F16
-               ? vn::conv_forward<__half>(src, g, weight, bias, cout, k, stride, out, stream, "conv_u8_forward_lp")
-               : vn::conv_forward<__nv_bfloat16>(src, g, weight, bias, cout, k, stride, out, stream,
-                                                 "conv_u8_forward_lp");
+    return vn::forward_entry(src, 1, false, weight, bias, cout, k, stride, true, dtype, out, stream, "conv_u8_forward_lp");
 }
 
 int64_t vn_conv_u8_wgrad_scratch_bytes(int32_t n, int32_t c, int32_t cout, int32_t k) {
@@ -673,40 +952,42 @@ int64_t vn_conv_u8_wgrad_scratch_bytes(int32_t n, int32_t c, int32_t cout, int32
 
 int32_t vn_conv_u8_backward(const vn_u8_frames_t *src, const float *grad_out, int32_t cout, int32_t k, int32_t stride,
                             float *grad_weight, float *grad_bias, void *scratch, int64_t scratch_bytes, void *stream) {
-    vn::ConvGeom g;
-    int32_t rc = vn::conv_args(src, cout, k, stride, "conv_u8_backward", &g);
-    if (rc) return rc;
-    VN_REQUIRE(grad_out && grad_weight, "conv_u8_backward: grad_out and grad_weight must not be null");
-    VN_REQUIRE(vn::aligned4(grad_out) && vn::aligned4(grad_weight) && vn::aligned4(grad_bias),
-               "conv_u8_backward: grad_out, grad_weight and grad_bias must be 4-byte aligned");
-    rc = vn::scratch_args(src, cout, k, scratch, scratch_bytes, "conv_u8_backward");
-    if (rc) return rc;
-    if (src->n == 0) return VN_OK;
-    return vn::conv_backward<float>(src, g, grad_out, cout, k, stride, grad_weight, grad_bias, scratch, stream,
-                                    "conv_u8_backward");
+    return vn::backward_entry(src, 1, false, grad_out, false, 0, cout, k, stride, grad_weight, grad_bias, scratch,
+                              scratch_bytes, stream, "conv_u8_backward");
 }
 
 int32_t vn_conv_u8_backward_lp(const vn_u8_frames_t *src, const void *grad_out, int32_t dtype, int32_t cout,
                                int32_t k, int32_t stride, float *grad_weight, float *grad_bias, void *scratch,
                                int64_t scratch_bytes, void *stream) {
-    vn::ConvGeom g;
-    int32_t rc = vn::conv_args(src, cout, k, stride, "conv_u8_backward_lp", &g);
-    if (rc) return rc;
-    if (dtype != VN_DTYPE_F16 && dtype != VN_DTYPE_BF16) {
-        vn::set_error("conv_u8_backward_lp: dtype %d (VN_DTYPE_F16 or VN_DTYPE_BF16 are supported)", dtype);
-        return VN_EUNSUPPORTED;
-    }
-    VN_REQUIRE(grad_out && grad_weight, "conv_u8_backward_lp: grad_out and grad_weight must not be null");
-    VN_REQUIRE(vn::aligned2(grad_out), "conv_u8_backward_lp: grad_out must be 2-byte aligned");
-    VN_REQUIRE(vn::aligned4(grad_weight) && vn::aligned4(grad_bias),
-               "conv_u8_backward_lp: grad_weight and grad_bias must be 4-byte aligned");
-    rc = vn::scratch_args(src, cout, k, scratch, scratch_bytes, "conv_u8_backward_lp");
-    if (rc) return rc;
-    if (src->n == 0) return VN_OK;
-    return dtype == VN_DTYPE_F16 ? vn::conv_backward<__half>(src, g, grad_out, cout, k, stride, grad_weight, grad_bias,
-                                                             scratch, stream, "conv_u8_backward_lp")
-                                 : vn::conv_backward<__nv_bfloat16>(src, g, grad_out, cout, k, stride, grad_weight,
-                                                                    grad_bias, scratch, stream, "conv_u8_backward_lp");
+    return vn::backward_entry(src, 1, false, grad_out, true, dtype, cout, k, stride, grad_weight, grad_bias, scratch,
+                              scratch_bytes, stream, "conv_u8_backward_lp");
+}
+
+int32_t vn_conv_u8_planes_forward(const vn_u8_frames_t *srcs, int32_t n_srcs, const float *weight, const float *bias,
+                                  int32_t cout, int32_t k, int32_t stride, float *out, void *stream) {
+    return vn::forward_entry(srcs, n_srcs, true, weight, bias, cout, k, stride, false, 0, out, stream,
+                             "conv_u8_planes_forward");
+}
+
+int32_t vn_conv_u8_planes_forward_lp(const vn_u8_frames_t *srcs, int32_t n_srcs, const float *weight,
+                                     const float *bias, int32_t cout, int32_t k, int32_t stride, int32_t dtype,
+                                     void *out, void *stream) {
+    return vn::forward_entry(srcs, n_srcs, true, weight, bias, cout, k, stride, true, dtype, out, stream,
+                             "conv_u8_planes_forward_lp");
+}
+
+int32_t vn_conv_u8_planes_backward(const vn_u8_frames_t *srcs, int32_t n_srcs, const float *grad_out, int32_t cout,
+                                   int32_t k, int32_t stride, float *grad_weight, float *grad_bias, void *scratch,
+                                   int64_t scratch_bytes, void *stream) {
+    return vn::backward_entry(srcs, n_srcs, true, grad_out, false, 0, cout, k, stride, grad_weight, grad_bias, scratch,
+                              scratch_bytes, stream, "conv_u8_planes_backward");
+}
+
+int32_t vn_conv_u8_planes_backward_lp(const vn_u8_frames_t *srcs, int32_t n_srcs, const void *grad_out, int32_t dtype,
+                                      int32_t cout, int32_t k, int32_t stride, float *grad_weight, float *grad_bias,
+                                      void *scratch, int64_t scratch_bytes, void *stream) {
+    return vn::backward_entry(srcs, n_srcs, true, grad_out, true, dtype, cout, k, stride, grad_weight, grad_bias, scratch,
+                              scratch_bytes, stream, "conv_u8_planes_backward_lp");
 }
 
 }  // extern "C"

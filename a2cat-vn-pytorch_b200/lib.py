@@ -24,7 +24,7 @@ STEP_ACTIONS_READY = 0x01
 STEP_SKIP_UNCHANGED = 0x02
 STEP_NO_OVERLAP = 0x04
 MODE_SPLIT, MODE_FUSED, MODE_PERSISTENT = 0, 1, 2
-ABI_VERSION = 5
+ABI_VERSION = 6
 DTYPE_F16, DTYPE_BF16 = 1, 2
 STAT_NAMES = ("episodes", "return_sum", "length_sum", "successes", "collisions", "steps", "truncations", "resets",
               "rows_skipped")
@@ -104,7 +104,8 @@ EXPORTS = ("vn_abi_version", "vn_abi_struct_size", "vn_last_error", "vn_launch_c
            "vn_gather_plane_f32_chw", "vn_gather_plane_f32_chw_rows", "vn_gather_leaves_f32_chw", "vn_nstep_returns", "vn_nstep_returns_scan", "vn_discounted_backup", "vn_pixel_control",
            "vn_transition_rows", "vn_gather_rows", "vn_pixel_control_list", "vn_pixel_control_returns", "vn_pixel_control_returns_from_states", "vn_replay_sample",
            "vn_aux_target", "vn_rp_labels", "vn_conv_u8_forward", "vn_conv_u8_wgrad_scratch_bytes", "vn_conv_u8_backward",
-           "vn_conv_u8_forward_lp", "vn_conv_u8_backward_lp")
+           "vn_conv_u8_forward_lp", "vn_conv_u8_backward_lp", "vn_conv_u8_planes_forward", "vn_conv_u8_planes_forward_lp",
+           "vn_conv_u8_planes_backward", "vn_conv_u8_planes_backward_lp")
 
 
 def library_path():
@@ -174,6 +175,10 @@ def load(build_if_missing=True):
         "vn_conv_u8_backward": (i32, [C.POINTER(U8Frames), _P, i32, i32, i32, _P, _P, _P, i64, _P]),
         "vn_conv_u8_forward_lp": (i32, [C.POINTER(U8Frames), _P, _P, i32, i32, i32, i32, _P, _P]),
         "vn_conv_u8_backward_lp": (i32, [C.POINTER(U8Frames), _P, i32, i32, i32, i32, _P, _P, _P, i64, _P]),
+        "vn_conv_u8_planes_forward": (i32, [C.POINTER(U8Frames), i32, _P, _P, i32, i32, i32, _P, _P]),
+        "vn_conv_u8_planes_forward_lp": (i32, [C.POINTER(U8Frames), i32, _P, _P, i32, i32, i32, i32, _P, _P]),
+        "vn_conv_u8_planes_backward": (i32, [C.POINTER(U8Frames), i32, _P, i32, i32, i32, _P, _P, _P, i64, _P]),
+        "vn_conv_u8_planes_backward_lp": (i32, [C.POINTER(U8Frames), i32, _P, i32, i32, i32, i32, _P, _P, _P, i64, _P]),
     }
     for name, (res, args) in sig.items():
         fn = getattr(lib, name)

@@ -34,7 +34,7 @@
 extern "C" {
 #endif
 
-#define VN_ABI_VERSION 5
+#define VN_ABI_VERSION 6
 #define VN_MAX_PLANES 6 /* rgb, depth, segmentation (+ the 3 third-person planes of graph/thor_graph.py:25-31) */
 
 /* error codes */
@@ -515,7 +515,8 @@ typedef struct vn_u8_frames {
 int32_t vn_conv_u8_forward(const vn_u8_frames_t *src, const float *weight, const float *bias, int32_t cout, int32_t k,
                            int32_t stride, float *out, void *stream);
 /* Bytes of device scratch vn_conv_u8_backward needs: ceil(n / 32) * cout * (c * k * k + 1) * 4 (one partial gradient
- * per chunk of 32 frames); -1 for negative or zero sizes.  Host only. */
+ * per chunk of 32 frames); -1 for negative or zero sizes.  Host only.  With c the set's channel count, also the
+ * scratch of vn_conv_u8_planes_backward[_lp]. */
 int64_t vn_conv_u8_wgrad_scratch_bytes(int32_t n, int32_t c, int32_t cout, int32_t k);
 /* The weight and bias gradient of vn_conv_u8_forward for grad_out [n][cout][oh][ow]:
  *   grad_weight[co][ci][ky][kx] = sum_{i, oy, ox} grad_out[i][co][oy][ox] * x_i[ci][oy * stride + ky][ox * stride + kx] / 255,
@@ -543,6 +544,29 @@ int32_t vn_conv_u8_forward_lp(const vn_u8_frames_t *src, const float *weight, co
 int32_t vn_conv_u8_backward_lp(const vn_u8_frames_t *src, const void *grad_out, int32_t dtype, int32_t cout,
                                int32_t k, int32_t stride, float *grad_weight, float *grad_bias,
                                void *scratch, int64_t scratch_bytes, void *stream);
+
+/* The same layer over a plane set: the frames of n_srcs sources stacked along channels in source order (RGB-D:
+ * {rgb, depth}; early-fused goal: {obs rgb, goal rgb}):
+ *   y = conv2d(cat_c(x_0, ..., x_{n_srcs-1}) / 255, weight, bias, stride), weight [cout][C][k][k], C = sum of srcs[s].c.
+ * Every source has its own base, pitch, idx and index strides (the observation and the goal may come from two index
+ * tensors, or a store plane and an observation batch); all share n, idx_t, h and w (a mismatch is VN_EINVAL).
+ * Supported: 1 to 4 sources of 1 or 3 channels, 8 channels in all, the kernel, stride and cout of vn_conv_u8_forward,
+ * and frames whose set (sum of h * w * c rounded up to 16 bytes per source) fits in shared memory beside the kernels'
+ * tables: every such set on frames up to 84 x 84, and up to 5 channels (e.g. RGB-D) on the reference's 174 x 174;
+ * anything else is VN_EUNSUPPORTED.  Numerics, results (one source gives the bits of vn_conv_u8_forward / _backward),
+ * scratch (vn_conv_u8_wgrad_scratch_bytes with c = C), alignment and launch behaviour are those of the one-source entry
+ * points above, in fp32 and in fp16 / bf16 (_lp). */
+int32_t vn_conv_u8_planes_forward(const vn_u8_frames_t *srcs, int32_t n_srcs, const float *weight, const float *bias,
+                                  int32_t cout, int32_t k, int32_t stride, float *out, void *stream);
+int32_t vn_conv_u8_planes_forward_lp(const vn_u8_frames_t *srcs, int32_t n_srcs, const float *weight,
+                                     const float *bias, int32_t cout, int32_t k, int32_t stride, int32_t dtype,
+                                     void *out, void *stream);
+int32_t vn_conv_u8_planes_backward(const vn_u8_frames_t *srcs, int32_t n_srcs, const float *grad_out, int32_t cout,
+                                   int32_t k, int32_t stride, float *grad_weight, float *grad_bias, void *scratch,
+                                   int64_t scratch_bytes, void *stream);
+int32_t vn_conv_u8_planes_backward_lp(const vn_u8_frames_t *srcs, int32_t n_srcs, const void *grad_out, int32_t dtype,
+                                      int32_t cout, int32_t k, int32_t stride, float *grad_weight, float *grad_bias,
+                                      void *scratch, int64_t scratch_bytes, void *stream);
 
 #ifdef __cplusplus
 }

@@ -13,7 +13,12 @@ kernels against torch's own float path under the same autocast, with grad_out in
 tensor-core work is a third of the fp32 kernels' (one mma per k-step instead of three); "useful" counts the
 convolution's multiply-adds alone (forward, plus as many again for the weight gradient).
 
-    python tools/bench_u8conv.py [--reps 20] [--out record.json]
+With --planes it runs the plane-set cases instead: vn.nn.U8PlanesConv2d for RGB-D ((3, 1): obs rgb + depth) and
+observation + goal ((3, 3): obs rgb + goal rgb, the goals from a second [4096, 20] index view) at (k 7, stride 4,
+cout 32), against the float path it replaces (policy_input per plane + torch.cat + nn.Conv2d), in fp32 (TF32 on and off
+for the float path) and under autocast with bf16 and fp16, with the update pass's peak memory.
+
+    python tools/bench_u8conv.py [--reps 20] [--planes] [--out record.json]
 """
 import argparse
 import importlib
@@ -37,7 +42,7 @@ AUTOCAST = {"bf16": torch.bfloat16, "f16": torch.float16}
 
 
 def gpu_info():
-    q = subprocess.run(["nvidia-smi", "--query-gpu=name,power.limit,clocks.max.sm", "--format=csv,noheader"],
+    q = subprocess.run(["nvidia-smi", "--query-gpu=name,power.limit,clocks.max.sm,clocks.sm", "--format=csv,noheader"],
                        capture_output=True, text=True)
     return q.stdout.strip().splitlines()[0] if q.returncode == 0 and q.stdout.strip() else "unknown"
 
@@ -66,10 +71,71 @@ def peak_bytes(fn):
     return torch.cuda.max_memory_allocated() - base
 
 
+PLANE_CASES = {"rgbd_3+1_32_k7s4": ((3, 1), ("rgb", "depth")), "obs_goal_3+3_32_k7s4": ((3, 3), ("rgb", "goal_rgb"))}
+
+
+def planes(vn, env, dw, states, goals, reps, gen):
+    """The plane-set rows: {case: {key: value}}.  "goal_rgb" is the goal leaf for the act size and the rgb plane at
+    the goal indices for the update size."""
+    dev = states.device
+    h, w = dw.world.layout.frame_hw
+    out = {}
+    for name, (pcs, leaves) in PLANE_CASES.items():
+        torch.manual_seed(0)
+        layer = vn.nn.U8PlanesConv2d(pcs, 32, 7, stride=4).to(dev)
+        conv = torch.nn.Conv2d(sum(pcs), 32, 7, stride=4).to(dev)
+        conv.load_state_dict(layer.state_dict())
+        oh = (h - 7) // 4 + 1
+        batch = [env.goal_buf["rgb"] if lf == "goal_rgb" else env.obs_buf[lf] for lf in leaves]
+        act_idx = [(env.goal if lf == "goal_rgb" else env.obs_state, "rgb" if lf == "goal_rgb" else lf)
+                   for lf in leaves]
+        upd = [(goals if lf == "goal_rgb" else states, "rgb" if lf == "goal_rgb" else lf) for lf in leaves]
+        go = torch.randn((ENVS, STEPS, 32, oh, oh), device=dev, generator=gen)
+        res = {"plane_channels": list(pcs), "act_frames": ENVS, "update_frames": ENVS * STEPS,
+               "float_frame_bytes": 4 * sum(pcs) * h * w}
+
+        def float_x(src):
+            return torch.cat([vn.rollout.policy_input(dw, s, p) for s, p in src], -3)
+
+        for tag, dtype in [("", None)] + [("ac_%s_" % t, d) for t, d in AUTOCAST.items()]:
+            ac = dict(device_type="cuda", dtype=dtype or torch.float16, enabled=dtype is not None)
+            g = go if dtype is None else go.to(dtype)
+
+            def fused_update():
+                layer.zero_grad(set_to_none=True)
+                with torch.autocast(**ac):
+                    y = layer.forward_states(dw, *upd)
+                y.backward(g)
+
+            def float_update():
+                conv.zero_grad(set_to_none=True)
+                with torch.autocast(**ac):
+                    y = conv(float_x(upd).flatten(0, 1))
+                y.backward(g.flatten(0, 1))
+
+            with torch.no_grad(), torch.autocast(**ac):
+                res[tag + "act_fused_ms"] = timed(lambda: layer(*batch), reps)
+            res[tag + "update_fused_fwd_bwd_ms"] = timed(fused_update, reps)
+            res[tag + "update_fused_peak_bytes"] = peak_bytes(fused_update)
+            for tf32 in ((True, False) if dtype is None else (True,)):
+                torch.backends.cudnn.allow_tf32 = tf32
+                key = tag + ("float_tf32_%s_" % tf32 if dtype is None else "float_")
+                with torch.no_grad(), torch.autocast(**ac):
+                    res[key + "act_ms"] = timed(lambda: conv(float_x(act_idx)), reps)
+                res[key + "update_fwd_bwd_ms"] = timed(float_update, reps)
+                res[key + "update_peak_bytes"] = peak_bytes(float_update)
+            torch.backends.cudnn.allow_tf32 = True
+            del g
+        out[name] = res
+        del go
+    return out
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--reps", type=int, default=20)
     ap.add_argument("--loop-steps", type=int, default=200)
+    ap.add_argument("--planes", action="store_true", help="run the plane-set cases (U8PlanesConv2d) only")
     ap.add_argument("--out", default=None)
     args = ap.parse_args()
     vn = importlib.import_module("a2cat-vn-pytorch_b200")
@@ -87,6 +153,17 @@ def main():
     states = storage[:-1].t()                                  # [4096, 20] strided view, read in place
     h, w = world.layout.frame_hw
     rec = dict(gpu=gpu_info(), hbm_peak_gbs=peak_gbs, hbm_peak_source=peak_src, results={})
+    if args.planes:
+        goals = torch.randint(0, world.n_states, (STEPS + 1, ENVS), dtype=torch.int32, device=dev, generator=gen)
+        rec["gpu_fields"] = "name, power.limit, clocks.max.sm, clocks.sm"
+        rec["results"] = planes(vn, env, dw, states, goals[:-1].t(), args.reps, gen)
+        line = json.dumps(rec)
+        print(line)
+        if args.out:
+            with open(args.out, "w") as f:
+                f.write(json.dumps(rec, indent=1) + "\n")
+        env.close()
+        return
     frame_u8 = h * w * 3
     for name, (cin, cout, k, s) in GEOMS.items():
         torch.manual_seed(0)
