@@ -99,14 +99,11 @@ class _U8Conv(torch.autograd.Function):
         src = frames_of(*sources)
         dtype = _autocast_dtype()
         out = torch.empty(out_shape, dtype=dtype or torch.float32, device=weight.device)
-        if dtype is None:
-            fn, head, _ = _entry(src, "forward")
-            _call(weight.device, fn, *head, weight.data_ptr(), L.ptr(bias), cout, k, stride, out.data_ptr(),
+        fn, head, n = _entry(src, "forward" if dtype is None else "forward_lp")
+        if n:   # an empty batch launches nothing: a freshly allocated one has a null data pointer
+            dt = () if dtype is None else (_LP_DTYPES[dtype],)
+            _call(weight.device, fn, *head, weight.data_ptr(), L.ptr(bias), cout, k, stride, *dt, out.data_ptr(),
                   stream_of=weight)
-        else:
-            fn, head, _ = _entry(src, "forward_lp")
-            _call(weight.device, fn, *head, weight.data_ptr(), L.ptr(bias), cout, k, stride, _LP_DTYPES[dtype],
-                  out.data_ptr(), stream_of=weight)
         ctx.save_for_backward(*sources)
         ctx.frames_of, ctx.stride, ctx.has_bias, ctx.dtype = frames_of, stride, bias is not None, dtype
         ctx.wshape = tuple(weight.shape)
