@@ -153,6 +153,15 @@ __device__ __forceinline__ void step_env(const StepParams &p, const int i, EnvSt
             if (terminal) r = p.rules.reward_goal;
             if (collided) r = p.rules.reward_collision;
         }
+        if (p.rules.reward_progress != 0.0f) {
+            // geodesic progress (vn_b200.h, vn_rules_t.reward_progress): distance of the current task's goal from the
+            // state the action was taken in minus that from the state it led to, before any auto-reset
+            const int32_t *dist = p.tab.task_dist + (size_t)p.env.task[i] * p.tab.n_states;
+            const int d_prev = __ldg(dist + s_old);
+            const int d_next = s == s_old ? d_prev : __ldg(dist + s);
+            const int delta = (d_prev < 0 || d_next < 0) ? 0 : d_prev - d_next;
+            r = __fadd_rn(r, __fmul_rn(p.rules.reward_progress, (float)delta));
+        }
         bool done = terminal, trunc = false, at_limit = false;
         elapsed += 1;
         ep_ret += r;
@@ -918,6 +927,10 @@ static int32_t make_step_params(StepParams &sp, const vn_tables_t *tab, const vn
                "envs: null pointer");
     VN_REQUIRE(rules && rules->n_actions >= 1 && rules->n_actions <= 16, "rules: n_actions");
     VN_REQUIRE(rules->goal_compare >= 0 && rules->goal_compare <= 2, "rules: goal_compare=%d", rules->goal_compare);
+    VN_REQUIRE(isfinite(rules->reward_progress), "rules: reward_progress=%g is not finite", (double)rules->reward_progress);
+    VN_REQUIRE(rules->reward_progress == 0.0f || tab->task_dist,
+               "rules: reward_progress=%g needs tables->task_dist (the [n_tasks][n_states] distance table)",
+               (double)rules->reward_progress);
     VN_REQUIRE(out && out->obs_state, "out: obs_state scratch is required");
     VN_REQUIRE(reset || actions, "step: actions is null");
     VN_REQUIRE(!inj || !inj->start || inj->stride > 0, "inject: stride=%d", inj ? inj->stride : 0);

@@ -24,7 +24,7 @@ STEP_ACTIONS_READY = 0x01
 STEP_SKIP_UNCHANGED = 0x02
 STEP_NO_OVERLAP = 0x04
 MODE_SPLIT, MODE_FUSED, MODE_PERSISTENT = 0, 1, 2
-ABI_VERSION = 6
+ABI_VERSION = 7
 DTYPE_F16, DTYPE_BF16 = 1, 2
 STAT_NAMES = ("episodes", "return_sum", "length_sum", "successes", "collisions", "steps", "truncations", "resets",
               "rows_skipped")
@@ -39,7 +39,7 @@ class Store(C.Structure):
 
 class Tables(C.Structure):
     _fields_ = [("adj", _P), ("task_goal", _P), ("task_cand_off", _P), ("task_prefix", _P), ("cand_state", _P),
-                ("n_states", C.c_int32), ("n_tasks", C.c_int32)]
+                ("n_states", C.c_int32), ("n_tasks", C.c_int32), ("task_dist", _P)]
 
 
 class Envs(C.Structure):
@@ -51,7 +51,7 @@ class Envs(C.Structure):
 class Rules(C.Structure):
     _fields_ = [("reward_goal", C.c_float), ("reward_step", C.c_float), ("reward_collision", C.c_float),
                 ("max_episode_steps", C.c_int32), ("goal_compare", C.c_int32), ("flags", C.c_int32),
-                ("n_actions", C.c_int32), ("reserved", C.c_int32), ("seed", C.c_uint64)]
+                ("n_actions", C.c_int32), ("reward_progress", C.c_float), ("seed", C.c_uint64)]
 
 
 class Inject(C.Structure):

@@ -194,7 +194,8 @@ def make_vec(id, tasks, num_envs=None, screen_size=None, graph_files=None, **env
     environments/gym_graph/__init__.py ('AuxiliaryGraph-v0', 'OrientedGraph-v0', 'Graph<Scene>-v0'), ``tasks`` the
     experiment's ``[(scene_name, [goal, ...]), ...]`` list (``None`` goals = the table of download.py:21-29).  One env
     per (scene, goal) unless ``num_envs`` says otherwise; scene pickles come from ``graph_files[scene_name]`` or the
-    reference's cache directory.  Returns a GraphVecEnv (extra keyword arguments are passed on)."""
+    reference's cache directory.  Returns a GraphVecEnv (extra keyword arguments, e.g. ``reward_progress``, are passed
+    on)."""
     from .tables import GYM_GRAPH, compile_world
     from .vec_env import GraphVecEnv
     if id in GYM_IDS:

@@ -46,6 +46,10 @@ class GraphEnv:
     def set_complexity(self, complexity=None):
         self._vec.set_complexity(complexity)
 
+    def set_reward_progress(self, coef):
+        """GraphVecEnv.set_reward_progress (also the ``reward_progress`` keyword of the constructor)."""
+        self._vec.set_reward_progress(coef)
+
     def reset(self):
         return self._one(self._vec.reset())
 

@@ -53,6 +53,7 @@ class DeviceWorld:
         self.tables.n_states = n
         self.tables.n_tasks = len(world.tasks)
         self.complexity = None
+        self._shortest = None
         if fill:
             self.fill()
 
@@ -90,6 +91,28 @@ class DeviceWorld:
         self.complexity = complexity
         pre = torch.from_numpy(self.world.prefixes(complexity))
         self.task_prefix.copy_(pre.to(self.device), non_blocking=False)
+
+    def shortest_paths(self):
+        """(action, dist) int32 CUDA tensors ``[n_tasks, n_states]``: for every task and GLOBAL state the first action of
+        a shortest action sequence to the task's goal and its length, -1 where the goal cannot be reached (and for the
+        states of other scenes) - tables.optimal_policy_table on the state graph, orientation included.  Built on the host
+        the first time it is asked for, then kept: ``n_tasks * n_states * 4`` bytes of device memory each (C2: 96 KB,
+        C4's 30 scenes: 86.4 MB).  ``dist`` is also the table the step kernel reads for the geodesic-progress reward
+        (vn_tables_t.task_dist), so GraphVecEnv.optimal_actions() and the reward share one copy."""
+        if self._shortest is None:
+            from .tables import optimal_policy_table
+            w = self.world
+            act = np.full((len(w.tasks), w.n_states), -1, np.int32)
+            dst = np.full((len(w.tasks), w.n_states), -1, np.int32)
+            for ti, t in enumerate(w.tasks):
+                b = int(w.scene_base[t.scene])
+                d, a = optimal_policy_table(w, ti)
+                act[ti, b:b + len(a)] = a
+                dst[ti, b:b + len(d)] = d
+            with torch.cuda.device(self.device):
+                self._shortest = (torch.from_numpy(act).to(self.device), torch.from_numpy(dst).to(self.device))
+            self.tables.task_dist = self._shortest[1].data_ptr()
+        return self._shortest
 
     def plane_index(self, name):
         return self.world.layout.planes.index(name)

@@ -161,7 +161,7 @@ class GraphVecEnv:
     def __init__(self, world, num_envs, *, device="cuda", seed=0, max_episode_steps=900, rewards=(1.0, 0.0, 0.0),
                  obs_layout="aux5", unreal_wrapper=True, env_tasks=None, auto_reset=True, rank=0, world_size=1,
                  gather="auto", inject=None, host_outputs=True, device_world=None, scaled_float=False,
-                 episode_info=True, skip_unchanged=True, numpy_obs=False):
+                 episode_info=True, skip_unchanged=True, numpy_obs=False, reward_progress=0.0):
         """
         world            tables.World (compiled scenes) - or pass a ready ``device_world``
         num_envs         TOTAL number of envs of the job; this process owns shard_range(num_envs, rank, world_size)
@@ -185,6 +185,7 @@ class GraphVecEnv:
                          row of an env whose state did not change (collision, no-op) is not copied again
                          (VN_STEP_SKIP_UNCHANGED).  Pass False if the returned observation tensors are modified in
                          place between steps.
+        reward_progress  dense geodesic-progress reward, NOT part of the reference (see set_reward_progress); 0 = off
         """
         self.dw = device_world if device_world is not None else DeviceWorld(world, device)
         self.world: World = self.dw.world
@@ -284,7 +285,9 @@ class GraphVecEnv:
         flags |= L.RULE_NOOP_ACTION if fam.noop_action else 0
         flags |= L.RULE_AUTO_RESET if auto_reset else 0
         self._c_rules = L.Rules(float(rewards[0]), float(rewards[1]), float(rewards[2]), self.max_episode_steps,
-                                fam.goal_compare, flags, self.n_actions, 0, C.c_uint64(seed & (2 ** 64 - 1)))
+                                fam.goal_compare, flags, self.n_actions, 0.0, C.c_uint64(seed & (2 ** 64 - 1)))
+        self.reward_progress = 0.0
+        self.set_reward_progress(reward_progress)
         out = L.StepOut()
         for i, p in enumerate(lay.planes):
             out.obs[i] = self.obs_buf[p].data_ptr() if p in self.obs_buf else None
@@ -751,6 +754,23 @@ class GraphVecEnv:
     def set_complexity(self, complexity=None):
         self.dw.set_complexity(complexity)
 
+    def set_reward_progress(self, coef):
+        """Dense geodesic-progress reward from the next step on (call between steps, like set_hardness): every step adds
+        ``coef * (d(s_t, g) - d(s_t+1, g))`` to the reward, ``d`` the number of actions on the shortest path to the env's
+        current goal (the distances optimal_actions() returns), ``s_t+1`` the state the action led to before any auto-reset,
+        and 0 where either distance is -1 (unreachable).  The step kernel adds it in float32, ``coef`` rounded to float32,
+        so rewards, episode returns, statistics, last_action_reward and rollout rows all carry the shaped reward.  The
+        reference has no such term; 0 (the default) gives the reference's rewards bit for bit.  A non-zero coefficient
+        builds the distance table (DeviceWorld.shortest_paths) on first use.  A CUDA graph captured earlier
+        (capture_steps) keeps the coefficient it was captured with."""
+        coef = float(coef)
+        if not np.isfinite(coef):
+            raise ValueError("reward_progress must be finite, got %r" % coef)
+        if coef != 0.0:
+            self.dw.shortest_paths()
+        self._c_rules.reward_progress = coef
+        self.reward_progress = float(np.float32(coef))
+
     # ------------------------------------------------------------------ extras
     def states(self):
         """Current states as reference tuples (x, y[, r]) - host copy."""
@@ -773,20 +793,9 @@ class GraphVecEnv:
     def optimal_actions(self):
         """Evaluation service (SURVEY.md section 8(f) rank 4): for every env the first action of a shortest
         action sequence to its current goal, and the remaining distance, from per-task tables computed once
-        on the host (tables.optimal_policy_table) and kept on the device.  Returns (actions, dist) int32 [N]."""
-        if not hasattr(self, "_opt"):
-            from .tables import optimal_policy_table
-            S = self.world.n_states
-            T_ = len(self.world.tasks)
-            act = np.full((T_, S), -1, np.int32)
-            dst = np.full((T_, S), -1, np.int32)
-            for ti, t in enumerate(self.world.tasks):
-                b = int(self.world.scene_base[t.scene])
-                d, a = optimal_policy_table(self.world, ti)
-                act[ti, b:b + len(a)] = a
-                dst[ti, b:b + len(d)] = d
-            self._opt = (torch.from_numpy(act).to(self.device), torch.from_numpy(dst).to(self.device))
-        act, dst = self._opt
+        on the host (tables.optimal_policy_table) and kept on the device (DeviceWorld.shortest_paths, shared with the
+        geodesic-progress reward).  Returns (actions, dist) int32 [N]."""
+        act, dst = self.dw.shortest_paths()
         t, s = self.task.long(), self.state.long()
         return act[t, s], dst[t, s]
 

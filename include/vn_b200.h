@@ -34,7 +34,7 @@
 extern "C" {
 #endif
 
-#define VN_ABI_VERSION 6
+#define VN_ABI_VERSION 7
 #define VN_MAX_PLANES 6 /* rgb, depth, segmentation (+ the 3 third-person planes of graph/thor_graph.py:25-31) */
 
 /* error codes */
@@ -51,6 +51,15 @@ extern "C" {
 #define VN_RULE_TWO_LEVEL 0x10            /* graph/util.py:103-116: 0.9 / 0.1 curriculum buckets */
 #define VN_RULE_NOOP_ACTION 0x20          /* graph/env.py:118-120: action -1 is a no-op with reward 0.0 */
 #define VN_RULE_AUTO_RESET 0x40           /* baselines VecEnv worker: if done: ob = env.reset() */
+/* vn_rules_t.reward_progress (not a flag; the reference has NO such reward): a dense geodesic-progress term for
+ * training without a curriculum, the shaping of PointNav / ObjectNav trainers.  When it is not 0 every step's reward is
+ *   reward = __fadd_rn(base, __fmul_rn(reward_progress, (float)(d_prev - d_next)))
+ * with base the reward of the rules above, d_prev = task_dist of the state before the action and d_next that of the
+ * state the action leads to (before any auto-reset; a collision or a no-op leaves the state, and so the distance,
+ * unchanged), both for the env's current task (vn_tables_t.task_dist).  Where either distance is -1 (unreachable) the
+ * difference is taken as 0.  The shaped reward is the reward everywhere the step writes one: out->reward, rec_reward,
+ * the host pack, ep_return / episode_return, VN_STAT_RETURN_SUM and last_action_reward.  0 leaves every output
+ * bit-identical to a library without the term (no table is read). */
 
 /* vn_step_out_t.flags */
 #define VN_STEP_ACTIONS_READY 0x01 /* the caller guarantees that the action buffer was complete before the PREVIOUS
@@ -112,6 +121,8 @@ typedef struct vn_tables {
     const int32_t *cand_state;    /* candidates of each task sorted by curriculum distance */
     int32_t n_states;
     int32_t n_tasks;
+    const int32_t *task_dist;     /* [n_tasks][n_states] fewest actions to the task's goal, -1 = unreachable; read only
+                                     when vn_rules_t.reward_progress != 0 (may be NULL otherwise) */
 } vn_tables_t;
 
 /* Per-env mutable state (struct of arrays, n_envs each). */
@@ -135,7 +146,7 @@ typedef struct vn_rules {
     int32_t goal_compare;
     int32_t flags;
     int32_t n_actions;                                /* 4 */
-    int32_t reserved;
+    float reward_progress;                            /* geodesic-progress coefficient, 0 = off (see above) */
     uint64_t seed;
 } vn_rules_t;
 
