@@ -1,6 +1,8 @@
 // Rollout / target builders (sm_100a): n-step returns, discounted back-up, pixel-control reward and
 // auxiliary targets computed straight from the HBM frame store, reward-prediction labels + compaction,
 // and the fused gather -> float32 CHW conversion for the policy input.
+#include <climits>
+
 #include "vn_common.cuh"
 
 namespace vn {
@@ -485,13 +487,17 @@ __global__ void __launch_bounds__(256) vn_gather_leaves_f32_kernel(const FloatLe
 
 // Pixel-control returns in ONE pass over the table rows: thread per (env, group of 4 cells), backward over t,
 //   pc(n, k) = table[rows[n][k]] | 0 (rows == -1: identical frames) | miss_rows[m] (rows == -(2 + m): reset transition,
-//              computed directly by vn_pixel_control_list in compact mode)
+//              computed directly by vn_pixel_control_list in compact mode) | NaN (m >= max_miss: no side-buffer row)
 //   R_T = bootstrap;  R_k = pc(n, k) + gamma * (1 - done(n, k)) * R_{k+1}     (same operation order as vn_backup_kernel)
 // The rewards are never written to memory unless out_reward is given: 1,600 B read + 1,600 B written per transition
 // instead of twice that for gather + back-up.
+// The float4 a miss past the side buffer reads (m >= max_miss: the list kernel computed no row for it).  Selecting its
+// address keeps the miss branch one unconditional load: a select of the loaded value cost 1.8 % of the fused chain.
+__device__ __align__(16) const uint32_t kQuietNaN4[4] = {0x7fc00000u, 0x7fc00000u, 0x7fc00000u, 0x7fc00000u};
+
 __global__ void __launch_bounds__(256) vn_pc_returns_kernel(const float4 *__restrict__ table,
                                                             const int32_t *__restrict__ rows, int64_t rsn, int64_t rst,
-                                                            const float4 *__restrict__ miss_rows,
+                                                            const float4 *__restrict__ miss_rows, int max_miss,
                                                             const uint8_t *__restrict__ done, int64_t dsn, int64_t dst,
                                                             const float4 *__restrict__ bootstrap, float gamma, int n,
                                                             int t, int d4, float4 *__restrict__ out,
@@ -517,7 +523,8 @@ __global__ void __launch_bounds__(256) vn_pc_returns_kernel(const float4 *__rest
                 if (r >= 0)
                     v[u] = __ldg(table + (int64_t)r * d4 + f);
                 else if (r <= kRowMiss)
-                    v[u] = __ldg(miss_rows + (int64_t)(kRowMiss - r) * d4 + f);
+                    v[u] = __ldg(kRowMiss - r < max_miss ? miss_rows + (int64_t)(kRowMiss - r) * d4 + f
+                                                         : reinterpret_cast<const float4 *>(kQuietNaN4));
                 nd[u] = 1.0f - (float)done[(int64_t)i * dsn + (int64_t)k * dst];
             }
         }
@@ -834,14 +841,14 @@ static int32_t launch_pc_list(const FrameArgs &f, const int32_t *states, int t, 
 // chained: the last kernel of vn_pixel_control_returns_from_states (programmatic launch), which re-arms the chain's
 // miss counter reset_counter; otherwise an ordinary launch and reset_counter is null.
 static int32_t launch_pc_returns(const float *pc_table, int cells, const int32_t *rows, int64_t rsn, int64_t rst,
-                                 const float *miss_rows, const uint8_t *done, int64_t dsn, int64_t dst,
+                                 const float *miss_rows, int max_miss, const uint8_t *done, int64_t dsn, int64_t dst,
                                  const float *bootstrap, float gamma, int n, int t, float *out_returns,
                                  float *out_reward, int32_t *reset_counter, cudaStream_t stream, bool chained) {
     const int d4 = cells >> 2;
     const int64_t threads = (int64_t)n * d4;
     return launch(vn_pc_returns_kernel, "vn_pc_returns_kernel", dim3((unsigned)((threads + 255) / 256)), dim3(256), 0,
                   stream, chained, reinterpret_cast<const float4 *>(pc_table), rows, rsn, rst,
-                  reinterpret_cast<const float4 *>(miss_rows), done, dsn, dst,
+                  reinterpret_cast<const float4 *>(miss_rows), max_miss, done, dsn, dst,
                   reinterpret_cast<const float4 *>(bootstrap), gamma, n, t, d4, reinterpret_cast<float4 *>(out_returns),
                   reinterpret_cast<float4 *>(out_reward), reset_counter);
 }
@@ -938,8 +945,9 @@ int32_t vn_pixel_control_returns(const float *pc_table, int32_t cells, const int
     VN_REQUIRE(vn::aligned16(pc_table, miss_rows, bootstrap, out_returns, out_reward),
                "pixel_control_returns: arrays must be 16-byte aligned");
     if (n == 0) return VN_OK;
-    return vn::launch_pc_returns(pc_table, cells, rows, row_stride_n, row_stride_t, miss_rows, done, done_stride_n,
-                                 done_stride_t, bootstrap, gamma, n, t, out_returns, out_reward, nullptr,
+    // the caller built rows and miss_rows: every miss index it wrote has its row
+    return vn::launch_pc_returns(pc_table, cells, rows, row_stride_n, row_stride_t, miss_rows, INT_MAX, done,
+                                 done_stride_n, done_stride_t, bootstrap, gamma, n, t, out_returns, out_reward, nullptr,
                                  static_cast<cudaStream_t>(stream), false);
 }
 
@@ -980,8 +988,9 @@ int32_t vn_pixel_control_returns_from_states(const vn_store_t *store, int32_t pl
     rc = vn::launch_pc_list(f, states, t, state_stride_n, state_stride_t, miss_pos, miss_count, max_miss, 1, miss_rows, st,
                             true, who);
     if (rc) return rc;
-    // (3) rewards gathered on the fly + discounted back-up
-    return vn::launch_pc_returns(pc_table, cells, rows, rsn, rst, miss_rows, done, done_stride_n, done_stride_t,
+    // (3) rewards gathered on the fly + discounted back-up; a miss past the side buffer (m >= max_miss: kernel (2)
+    //     computed no row for it) contributes NaN instead of a read past miss_rows
+    return vn::launch_pc_returns(pc_table, cells, rows, rsn, rst, miss_rows, max_miss, done, done_stride_n, done_stride_t,
                                  bootstrap, gamma, n, t, out_returns, out_reward, miss_count, st, true);
 }
 

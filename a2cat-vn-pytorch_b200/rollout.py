@@ -53,6 +53,8 @@ def nstep_returns(rewards, dones, last_values, gamma, time_major=False, method="
     n, t = rewards.shape
     if out is None:
         out = torch.empty((t, n) if time_major else (n, t), dtype=torch.float32, device=rewards.device)
+    if n == 0:
+        return out
     ob = out.t() if time_major else out
     _call(rewards.device, fn, rewards.data_ptr(), dones.data_ptr(), last_values.data_ptr(), float(gamma), n, t,
           rewards.stride(0), rewards.stride(1), out.data_ptr(), ob.stride(0), ob.stride(1), stream_of=rewards)
@@ -62,11 +64,13 @@ def nstep_returns(rewards, dones, last_values, gamma, time_major=False, method="
 def discounted_backup(rewards, dones, bootstrap, gamma):
     """rewards [B, T, ...]; dones [B, T] (any strides); bootstrap [B, ...] -> R_t = r_t + gamma (1 - done_t) R_{t+1}."""
     b, t = rewards.shape[:2]
-    d = rewards[0, 0].numel()
+    d = rewards.shape[2:].numel()
     rewards = rewards.contiguous().float()
     dones = _strided2d(dones, torch.uint8)
     bootstrap = bootstrap.contiguous().float()
     out = torch.empty_like(rewards)
+    if b == 0:
+        return out
     _call(rewards.device, "vn_discounted_backup", rewards.data_ptr(), dones.data_ptr(), dones.stride(0), dones.stride(1),
           bootstrap.data_ptr(), float(gamma), b, t, d, out.data_ptr(), stream_of=rewards)
     return out
@@ -99,6 +103,8 @@ def _pixel_control_direct(dw, states, cell_size, output_size, plane):
     pi, h, w, c, oh, ow = _geom(dw, plane, cell_size, output_size)
     b, t1 = states.shape
     out = torch.empty((b, t1 - 1, 1, oh, ow), dtype=torch.float32, device=dw.device)
+    if b == 0:
+        return out
     _call(dw.device, "vn_pixel_control", C.byref(dw.store), pi, states.data_ptr(), b, t1 - 1, states.stride(0),
           states.stride(1), h, w, c, cell_size, oh, ow, out.data_ptr(), stream_of=states)
     return out
@@ -108,20 +114,21 @@ def _aux_direct(dw, states, plane, cell_size, output_size):
     pi, h, w, c, oh, ow = _geom(dw, plane, cell_size, output_size)
     states = states.contiguous()
     out = torch.empty(tuple(states.shape) + (c, oh, ow), dtype=torch.float32, device=dw.device)
+    if states.numel() == 0:
+        return out
     _call(dw.device, "vn_aux_target", C.byref(dw.store), pi, states.data_ptr(), states.numel(), h, w, c, cell_size, oh,
           ow, out.data_ptr(), stream_of=states)
     return out
 
 
 class TargetTables:
-    """Per-world tables that turn the target builders into row gathers.  On a cached graph both targets
-    are pure functions of state indices, so they are evaluated once (with the direct kernels) and kept
-    resident in HBM - the same move as caching the frames themselves:
+    """Per-world table that turns the pixel-control builders into row gathers.  On a cached graph the target is a
+    pure function of state indices, so it is evaluated once (with the direct kernel) and kept resident in HBM - the
+    same move as caching the frames themselves:
 
       pc[s * 4 + a]  = pixel-control reward of the transition s -> adj[s][a]     [4 S, oh * ow] f32
-      aux[plane][s]  = avg_pool(crop(plane(s) / 255))                             [S, C, oh, ow] f32
 
-    C2 (6,000 states, 20x20): 38 MB + 10 MB (depth) + 29 MB (segmentation).
+    C2 (6,000 states, 20x20): 38 MB.  The auxiliary targets have tables of their own (_aux_table).
     """
 
     def __init__(self, dw: DeviceWorld, cell_size=4, output_size=None, plane="rgb"):
@@ -137,15 +144,7 @@ class TargetTables:
         pairs = torch.stack([me.repeat_interleave(4), nxt.reshape(-1)], 1).contiguous()
         for lo in range(0, 4 * S, step):
             self.pc[lo:lo + step] = _pixel_control_direct(dw, pairs[lo:lo + step], cell_size, (oh, ow), plane).view(-1, oh * ow)
-        self._aux = {}
         self._scratch = {}
-
-    def aux(self, plane):
-        if plane not in self._aux:
-            S = self.dw.world.n_states
-            me = torch.arange(S, dtype=torch.int32, device=self.dw.device)
-            self._aux[plane] = _aux_direct(self.dw, me, plane, self.cell, self.out_hw).contiguous()
-        return self._aux[plane]
 
     def scratch(self, n, chained=False):
         """(rows, miss_pos, miss_count) int32 scratch for n transitions, reused between calls on the same stream.
@@ -168,7 +167,7 @@ class TargetTables:
         return self._scratch[key]
 
     def nbytes(self):
-        return self.pc.numel() * 4 + sum(t.numel() * 4 for t in self._aux.values())
+        return self.pc.numel() * 4
 
 
 def target_tables(dw: DeviceWorld, cell_size=4, output_size=None, plane="rgb") -> TargetTables:
@@ -181,6 +180,17 @@ def target_tables(dw: DeviceWorld, cell_size=4, output_size=None, plane="rgb") -
     return cache[key]
 
 
+def _aux_table(dw: DeviceWorld, plane, cell_size, out_hw):
+    """aux[s] = avg_pool(crop(plane(s) / 255)), float32 [S, C, oh, ow], built with the direct kernel on first use and
+    cached per (world, plane, cell, output size).  C2 (6,000 states, 20x20): 10 MB (depth), 29 MB (segmentation)."""
+    cache = dw.__dict__.setdefault("_aux_tables", {})
+    key = (plane, cell_size) + tuple(out_hw)
+    if key not in cache:
+        me = torch.arange(dw.world.n_states, dtype=torch.int32, device=dw.device)
+        cache[key] = _aux_direct(dw, me, plane, cell_size, out_hw).contiguous()
+    return cache[key]
+
+
 def pixel_control_reward(dw: DeviceWorld, states, cell_size=4, output_size=None, plane="rgb", method="table"):
     """deep_rl.a2c_unreal.util.pixel_control_reward (SURVEY.md D5) computed from state indices.
     states: int32 [B, T+1] (any strides) GLOBAL state of every observation of the sequence -> float32 [B, T, 1, h, w].
@@ -190,7 +200,7 @@ def pixel_control_reward(dw: DeviceWorld, states, cell_size=4, output_size=None,
     method="direct": every transition is computed from the two frames.  Both give identical bits."""
     pi, h, w, c, oh, ow = _geom(dw, plane, cell_size, output_size)
     states = _states2d(dw, states)
-    if method == "direct" or (oh * ow) % 4:
+    if method == "direct" or (oh * ow) % 4 or states.shape[0] == 0:
         return _pixel_control_direct(dw, states, cell_size, (oh, ow), plane)
     tab = target_tables(dw, cell_size, (oh, ow), plane)
     b, t1 = states.shape
@@ -216,7 +226,10 @@ def pixel_control_returns(dw: DeviceWorld, states, dones, bootstrap, gamma, cell
 
     states int32 [B, T+1], dones uint8/bool [B, T] (any strides: ``storage.t()`` views are read in place), bootstrap
     float32 [B, h*w] (or [B, h, w]).  Returns float32 [B, T, h*w] (and the rewards [B, T, h*w] with with_reward).
-    max_miss bounds the side buffer for the transitions the table cannot serve (episode resets; default: all B*T)."""
+    max_miss bounds the side buffer for the transitions the table cannot serve (episode resets; default: all B*T).  When
+    more transitions than that miss the table, the ones past the bound (which ones is up to the device) get no reward:
+    their rows of the rewards are NaN, and so are the returns of their env at their step and every earlier one.  All
+    other elements are what an unbounded call gives."""
     pi, h, w, c, oh, ow = _geom(dw, plane, cell_size, output_size)
     cells = oh * ow
     if cells % 4:
@@ -225,12 +238,14 @@ def pixel_control_returns(dw: DeviceWorld, states, dones, bootstrap, gamma, cell
         return (ret, r) if with_reward else ret
     states = _states2d(dw, states)
     dones = _strided2d(dones, torch.uint8)
-    tab = target_tables(dw, cell_size, (oh, ow), plane)
     b, t1 = states.shape
     t = t1 - 1
-    bootstrap = bootstrap.reshape(b, cells).contiguous().float()
     out = torch.empty((b, t, cells), dtype=torch.float32, device=dw.device)
     rew = torch.empty((b, t, cells), dtype=torch.float32, device=dw.device) if with_reward else None
+    if b == 0:
+        return (out, rew) if with_reward else out
+    tab = target_tables(dw, cell_size, (oh, ow), plane)
+    bootstrap = bootstrap.reshape(b, cells).contiguous().float()
     rows, miss_pos, miss_count = tab.scratch(b * t, chained=True)
     max_miss = max(b * t if max_miss is None else int(max_miss), 1)
     side = tab.miss_rows(max_miss)
@@ -249,12 +264,12 @@ def auxiliary_target(dw: DeviceWorld, states, plane, cell_size=4, output_size=No
     pooled-plane table; method="direct": pooled from the frame."""
     pi, h, w, c, oh, ow = _geom(dw, plane, cell_size, output_size)
     states = _on_device(dw, states)
-    if method == "direct" or (c * oh * ow) % 4:
+    if method == "direct" or (c * oh * ow) % 4 or states.numel() == 0:
         return _aux_direct(dw, states, plane, cell_size, (oh, ow))
     shape = tuple(states.shape)
     if states.dim() != 2:
         states = states.contiguous().view(-1, 1)
-    tab = target_tables(dw, cell_size, (oh, ow)).aux(plane)
+    tab = _aux_table(dw, plane, cell_size, (oh, ow))
     out = torch.empty(shape + (c, oh, ow), dtype=torch.float32, device=dw.device)
     _call(dw.device, "vn_gather_rows", tab.data_ptr(), c * oh * ow * 4, states.data_ptr(), states.numel(),
           states.shape[1], states.stride(0), states.stride(1), out.data_ptr(), stream_of=states)
@@ -274,6 +289,8 @@ def policy_input(dw: DeviceWorld, states, plane="rgb"):
     pi, h, w, c, _, _ = _geom(dw, plane, 1, None)
     states = states.to(device=dw.device, dtype=torch.int32).contiguous()
     out = torch.empty(tuple(states.shape) + (c, h, w), dtype=torch.float32, device=dw.device)
+    if states.numel() == 0:
+        return out
     _call(dw.device, "vn_gather_plane_f32_chw", C.byref(dw.store), pi, states.data_ptr(), states.numel(), h, w, c,
           out.data_ptr(), stream_of=states)
     return out
@@ -295,22 +312,22 @@ def reward_prediction_labels(rewards, with_lists=True, sync=True, buffers=None):
         labels, zero, nonzero, counts, scratch = buffers
     else:
         labels = torch.empty(tuple(rewards.shape), dtype=torch.int8, device=r.device)
-        if n == 0:
-            e = torch.empty(0, dtype=torch.int32, device=r.device)
-            return labels, (e if with_lists else None), (e.clone() if with_lists else None)
         scratch = torch.empty((n + 1023) // 1024 + 1, dtype=torch.int32, device=r.device)
         counts = torch.empty(2, dtype=torch.int32, device=r.device)     # always written by the scan kernel
         zero = torch.empty(n, dtype=torch.int32, device=r.device) if with_lists else None
         nonzero = torch.empty(n, dtype=torch.int32, device=r.device) if with_lists else None
-    _call(r.device, "vn_rp_labels", r.data_ptr(), n, r.shape[1], r.stride(0), r.stride(1), labels.data_ptr(), L.ptr(zero),
-          L.ptr(nonzero), counts.data_ptr(), scratch.data_ptr(), stream_of=r)
+    if n > 0:
+        _call(r.device, "vn_rp_labels", r.data_ptr(), n, r.shape[1], r.stride(0), r.stride(1), labels.data_ptr(),
+              L.ptr(zero), L.ptr(nonzero), counts.data_ptr(), scratch.data_ptr(), stream_of=r)
+    else:
+        counts.zero_()
     if buffers is not None:
         return labels, zero, nonzero, counts
     if not with_lists:
         return labels, None, None
     if not sync:
         return labels, zero, nonzero, counts
-    cz, cn = counts.tolist()
+    cz, cn = counts.tolist() if n > 0 else (0, 0)
     return labels, zero[:cz], nonzero[:cn]
 
 

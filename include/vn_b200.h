@@ -449,7 +449,11 @@ int32_t vn_pixel_control_returns(const float *pc_table, int32_t cells, const int
 /* The three steps above as ONE call for a rollout's states: vn_transition_rows, vn_pixel_control_list (compact, into
  * miss_rows [max_miss][cells]) and vn_pixel_control_returns, chained with programmatic dependent launches (each kernel's
  * launch latency hides behind its predecessor).  rows / miss_pos are int32 scratch of n * t entries; *miss_count must be
- * 0 on entry - zero it once when the scratch is allocated, the last kernel re-arms it for the next call. */
+ * 0 on entry - zero it once when the scratch is allocated, the last kernel re-arms it for the next call.
+ * max_miss bounds the side buffer, not the misses: when more than max_miss transitions miss the table, only the first
+ * max_miss of the list (an order the device picks) get a row.  Each of the others reads nothing and contributes a
+ * quiet NaN: its out_reward row is NaN, and so is out_returns of its env at that step and at every earlier one.  Every
+ * other output is what an unbounded call gives.  max_miss = n * t never overflows. */
 int32_t vn_pixel_control_returns_from_states(const vn_store_t *store, int32_t plane, const int32_t *adj,
                                              const float *pc_table, const int32_t *states, int64_t state_stride_n,
                                              int64_t state_stride_t, const uint8_t *done, int64_t done_stride_n,
