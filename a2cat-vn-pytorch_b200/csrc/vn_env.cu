@@ -2,7 +2,8 @@
 //
 // A vectorised step is, in stream order, programmatically chained:
 //   K1 vn_step_kernel   one thread per env: adjacency lookup, collision + goal test, reward, TimeLimit,
-//                       done, auto-reset (Philox4x32-10 or injected stream), RewardCollector accumulators,
+//                       done, auto-reset (Philox4x32-10, injected stream or a fixed episode list whose results it
+//                       records), RewardCollector accumulators,
 //                       last_action_reward, warp-aggregated episode statistics.  ~40 B per env.
 //   K2 vn_gather_*      copies each env's observation planes (and, only if the env just reset, its goal planes)
 //                       from the HBM store into the contiguous policy batch.  >99.9 % of the bytes; HBM-bound; two
@@ -53,6 +54,7 @@ struct StepParams {
     vn_rules_t rules;
     vn_inject_t inj;
     vn_step_out_t out;
+    vn_episodes_t eps;       // copy of *env.episodes; eps.cursor == NULL: no list
     const int32_t *actions;  // NULL in reset mode
     const uint8_t *mask;     // reset mode only
     int32_t *actions_copy;   // optional device copy of the actions (host-actions path)
@@ -120,6 +122,7 @@ __device__ __forceinline__ void step_env(const StepParams &p, const int i, EnvSt
     const bool may_skip = !kReset && p.skip_rows;
     const int prev_obs = may_skip ? p.out.obs_state[i] : -1;
     int obs_s = s;
+    int listed = -1;  // listed episode (vn_episodes_t) that ended on this step, -1 = none
     bool do_reset;
 
     if (kReset) {
@@ -208,6 +211,18 @@ __device__ __forceinline__ void step_env(const StepParams &p, const int i, EnvSt
             st.ret = ep_ret;
             st.succ = terminal;
             st.trunc = trunc;
+            if (p.eps.cursor) {
+                // the result of a listed episode, written once, by the step that ends it (vn_b200.h, vn_episodes_t)
+                listed = p.eps.cursor[i];
+                if (listed >= 0) {
+                    p.eps.length[listed] = ep_len;
+                    p.eps.ret[listed] = ep_ret;
+                    p.eps.win[listed] = terminal;
+                    p.eps.truncated[listed] = trunc;
+                    p.eps.final_state[listed] = s;
+                    atomicAdd(p.eps.count, 1u);
+                }
+            }
         }
         st.coll = collided;
         st.steps = 1;
@@ -223,7 +238,18 @@ __device__ __forceinline__ void step_env(const StepParams &p, const int i, EnvSt
         const uint32_t e = p.env.epoch[i];
         const int tlo = p.env.task_lo[i];
         int t, start;
-        if (p.inj.start) {
+        int next = -1;  // listed episode this reset starts, -1 = the ordinary source
+        if (p.eps.cursor) {
+            // the env's first listed episode is its global id, each later one `stride` further on (vn_episodes_t)
+            const int64_t j = kReset ? (int64_t)p.env.env_id_base + i
+                                     : (listed >= 0 ? (int64_t)listed + p.eps.stride : (int64_t)-1);
+            next = (j >= 0 && j < p.eps.n_episodes) ? (int)j : -1;
+            p.eps.cursor[i] = next;
+        }
+        if (next >= 0) {
+            t = __ldg(p.eps.task + next);
+            start = __ldg(p.eps.start + next);
+        } else if (p.inj.start) {
             const uint32_t k = e < (uint32_t)p.inj.stride ? e : (uint32_t)p.inj.stride - 1;
             const size_t at = (size_t)i * p.inj.stride + k;
             t = tlo + (p.inj.task ? p.inj.task[at] : 0);
@@ -934,6 +960,23 @@ static int32_t make_step_params(StepParams &sp, const vn_tables_t *tab, const vn
     VN_REQUIRE(out && out->obs_state, "out: obs_state scratch is required");
     VN_REQUIRE(reset || actions, "step: actions is null");
     VN_REQUIRE(!inj || !inj->start || inj->stride > 0, "inject: stride=%d", inj ? inj->stride : 0);
+    const vn_episodes_t *ep = envs->episodes;
+    if (ep) {
+        VN_REQUIRE(!inj || !inj->start, "episodes: a list cannot be combined with an injected reset stream (inject)");
+        VN_REQUIRE(rules->flags & VN_RULE_AUTO_RESET, "episodes: a list needs VN_RULE_AUTO_RESET in rules->flags");
+        VN_REQUIRE(!(reset && mask), "episodes: a masked reset cannot run while a list is installed");
+        VN_REQUIRE(ep->n_episodes >= 0, "episodes: n_episodes=%d", ep->n_episodes);
+        VN_REQUIRE(ep->cursor && ep->count, "episodes: cursor and count are required");
+        VN_REQUIRE(ep->n_episodes == 0 || (ep->task && ep->start && ep->length && ep->ret && ep->win &&
+                                           ep->truncated && ep->final_state),
+                   "episodes: null list or result pointer with n_episodes=%d", ep->n_episodes);
+        VN_REQUIRE(envs->env_id_base >= 0 && ep->stride >= (int64_t)envs->env_id_base + envs->n_envs,
+                   "episodes: stride=%d is less than env_id_base + n_envs = %d + %d", ep->stride, envs->env_id_base,
+                   envs->n_envs);
+        sp.eps = *ep;
+    } else {
+        memset(&sp.eps, 0, sizeof(sp.eps));
+    }
     sp.tab = *tab;
     sp.env = *envs;
     sp.rules = *rules;
@@ -1214,6 +1257,7 @@ int32_t vn_abi_struct_size(int32_t which) {
         case 7: return (int32_t)sizeof(vn_float_leaf_t);
         case 8: return (int32_t)sizeof(vn_host_call_t);
         case 9: return (int32_t)sizeof(vn_u8_frames_t);
+        case 10: return (int32_t)sizeof(vn_episodes_t);
         default: return -1;
     }
 }

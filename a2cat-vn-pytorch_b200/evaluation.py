@@ -6,7 +6,12 @@ experiments/thor_cached_auxiliary.py:45).  Everything stays on the device; only 
 SPL (success weighted by path length): mean over episodes of ``success * l / max(p, l)`` with ``l`` the
 fewest actions from the episode's start state to its goal on the STATE graph (tables.optimal_policy_table) and
 ``p`` the number of actions the agent took.
+
+Two ways to evaluate: ``evaluate`` counts the first episodes to finish on the env's own random resets (quick, but biased
+toward short episodes and dependent on ``num_envs``); ``evaluate_episodes`` runs a fixed list of (task, start) episodes
+exactly once each - the benchmark protocol - and ``episode_set`` draws such a list reproducibly.
 """
+import numpy as np
 import torch
 
 
@@ -68,3 +73,81 @@ def evaluate(env, policy, episodes, max_steps=None):
     vals = acc.cpu().tolist()
     return dict(episodes=int(vals[0]), success_rate=vals[1] / e, episode_length=vals[2] / e, reward=vals[3] / e,
                 spl=vals[4] / e, truncated_rate=vals[5] / e, steps=steps)
+
+
+def episode_set(world, per_task, seed, complexity=None):
+    """A reproducible evaluation list ``(task, start)`` (int32 numpy ``[E]``, GLOBAL indices) for
+    ``evaluate_episodes`` / ``GraphVecEnv.set_episodes``: for every task, ``per_task`` start states drawn without
+    replacement (all of them when ``per_task`` is None or exceeds the pool) from the task's candidate starts within the
+    curriculum prefix at ``complexity`` (tables.curriculum_prefix; None = every candidate), in draw order, tasks in
+    order.  Candidates that cannot reach the goal are dropped first (thor-cached lists unreachable cells at "distance"
+    1, tables.build_task).  Task ``t`` draws from ``numpy.random.default_rng([seed, t])``, so its starts do not depend
+    on the other tasks."""
+    from .tables import optimal_policy_table
+    pre = world.prefixes(complexity)
+    tasks, starts = [], []
+    for ti, t in enumerate(world.tasks):
+        dist, _ = optimal_policy_table(world, ti)
+        cand = np.asarray(t.cand_state[:int(pre[ti])], np.int64)
+        cand = cand[dist[cand] >= 1]
+        k = len(cand) if per_task is None else min(int(per_task), len(cand))
+        pick = np.random.default_rng([int(seed), ti]).choice(len(cand), k, replace=False)
+        tasks.append(np.full(k, ti, np.int32))
+        starts.append((cand[pick] + int(world.scene_base[t.scene])).astype(np.int32))
+    return np.concatenate(tasks), np.concatenate(starts)
+
+
+@torch.no_grad()
+def evaluate_episodes(env, policy, task, start, check_every=64, max_steps=None):
+    """Runs ``policy(obs) -> actions [N]`` (CUDA int32 tensor, or anything ``env.step`` takes) on ``env`` over a fixed
+    list of episodes, each (``task[j]``, ``start[j]``) exactly once (GraphVecEnv.set_episodes: episode ``j`` runs on the
+    env with global id ``j % num_envs_total``), and scores them.  Unlike ``evaluate`` - the first episodes to finish on
+    random resets, a sample biased toward short episodes that changes with ``num_envs`` - every listed episode counts,
+    however long it runs, so the numbers are unbiased and the same for any batch size or shard count.  The step kernel
+    records each result on the device; the host reads one counter every ``check_every`` steps.  Each rank scores the
+    episodes its envs own (``env.episodes_owned``); the list is removed again before returning.
+
+    Stops when all of this shard's episodes have ended or after ``max_steps`` steps; with neither a TimeLimit
+    (``max_episode_steps > 0``) nor ``max_steps`` an episode might never end, so that is refused.  Returns a dict: the
+    summary over the recorded episodes - ``episodes``, ``success_rate``, ``spl`` (mean of ``win * l / max(p, l)``,
+    ``l`` = shortest-path distance of the start, ``p`` = actions taken), ``episode_length``, ``reward``,
+    ``truncated_rate``, ``distance_to_goal`` (mean shortest-path distance of the final state), ``steps``,
+    ``complete`` - and ``per_episode``: numpy arrays over ``env.episodes_owned`` (``index``, ``task``, ``start``,
+    ``length`` (-1 = not finished), ``reward``, ``win``, ``truncated``, ``final_state``, ``distance``,
+    ``final_distance``, ``spl``)."""
+    if env.max_episode_steps <= 0 and max_steps is None:
+        raise ValueError("evaluate_episodes needs a TimeLimit (max_episode_steps > 0) or max_steps: without one an "
+                         "episode might never end")
+    if check_every < 1:
+        raise ValueError("check_every must be >= 1")
+    env.set_episodes(task, start)
+    try:
+        owned = env.episodes_owned
+        obs = env.reset()
+        steps = 0
+        while env.episodes_recorded < len(owned) and (max_steps is None or steps < max_steps):
+            k = check_every if max_steps is None else min(check_every, max_steps - steps)
+            for _ in range(k):
+                obs = env.step(policy(obs))[0]
+            steps += k
+        res = {k: v.cpu().numpy() for k, v in env.episode_results().items()}
+    finally:
+        env.set_episodes(None)
+    _, dist = env.dw.shortest_paths()
+    t = torch.from_numpy(res["task"][owned].astype(np.int64)).to(env.device)
+    l = dist[t, torch.from_numpy(res["start"][owned].astype(np.int64)).to(env.device)].cpu().numpy()
+    fs = res["final_state"][owned].astype(np.int64)
+    fd = dist[t, torch.from_numpy(np.maximum(fs, 0)).to(env.device)].cpu().numpy()
+    length = res["length"][owned]
+    done = length >= 0
+    fd = np.where(done, fd, -1)
+    win = res["win"][owned].astype(np.float64)
+    spl = np.where(done, win * l / np.maximum(np.maximum(length, l), 1), 0.0)
+    per = dict(index=owned, task=res["task"][owned], start=res["start"][owned], length=length,
+               reward=res["ret"][owned], win=res["win"][owned], truncated=res["truncated"][owned],
+               final_state=res["final_state"][owned], distance=l, final_distance=fd, spl=spl)
+    m = int(done.sum())
+    mean = (lambda x: float(np.mean(x[done])) if m else float("nan"))
+    return dict(episodes=m, success_rate=mean(win), spl=mean(spl), episode_length=mean(length.astype(np.float64)),
+                reward=mean(per["reward"].astype(np.float64)), truncated_rate=mean(per["truncated"].astype(np.float64)),
+                distance_to_goal=mean(fd.astype(np.float64)), steps=steps, complete=m == len(owned), per_episode=per)

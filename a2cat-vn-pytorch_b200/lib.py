@@ -45,7 +45,7 @@ class Tables(C.Structure):
 class Envs(C.Structure):
     _fields_ = [("n_envs", C.c_int32), ("env_id_base", C.c_int32), ("state", _P), ("goal", _P), ("task", _P),
                 ("elapsed", _P), ("epoch", _P), ("ep_return", _P), ("ep_length", _P), ("task_lo", _P),
-                ("task_cnt", _P)]
+                ("task_cnt", _P), ("episodes", _P)]
 
 
 class Rules(C.Structure):
@@ -72,6 +72,11 @@ class StepOut(C.Structure):
                 ("rec_action", _P), ("rec_reward", _P), ("rec_done", _P), ("rec_state", _P), ("rec_goal", _P),
                 ("float_leaves", _P), ("n_float_leaves", C.c_int32), ("float_h", C.c_int32), ("float_w", C.c_int32),
                 ("reserved2", C.c_int32)]
+
+
+class Episodes(C.Structure):
+    _fields_ = [("task", _P), ("start", _P), ("n_episodes", C.c_int32), ("stride", C.c_int32), ("cursor", _P),
+                ("length", _P), ("ret", _P), ("win", _P), ("truncated", _P), ("final_state", _P), ("count", _P)]
 
 
 class Replay(C.Structure):
@@ -187,7 +192,7 @@ def load(build_if_missing=True):
         raise VnError("libvn_b200.so ABI version %d, expected %d - rebuild with `python __graft_entry__.py`"
                       % (lib.vn_abi_version(), ABI_VERSION))
     for which, mirror in enumerate((Store, Tables, Envs, Rules, Inject, StepOut, Replay, FloatLeaf, HostCall,
-                                     U8Frames)):
+                                     U8Frames, Episodes)):
         if lib.vn_abi_struct_size(which) != C.sizeof(mirror):
             raise VnError("libvn_b200.so is stale: sizeof(%s) is %d in the library, %d in lib.py - rebuild with "
                           "`python __graft_entry__.py`" % (mirror.__name__, lib.vn_abi_struct_size(which), C.sizeof(mirror)))

@@ -269,6 +269,7 @@ class GraphVecEnv:
             self._actions_host = torch.zeros(n, dtype=torch.int32).pin_memory()
         self._inject_keep = None
         self._c_inject = None
+        self._episodes = None       # installed episode list (set_episodes): tensors + the vn_episodes_t descriptor
         if inject is not None:
             self.set_inject(*inject)
 
@@ -284,6 +285,7 @@ class GraphVecEnv:
         flags |= L.RULE_TWO_LEVEL if fam.two_level_sampling else 0
         flags |= L.RULE_NOOP_ACTION if fam.noop_action else 0
         flags |= L.RULE_AUTO_RESET if auto_reset else 0
+        self.auto_reset = bool(auto_reset)
         self._c_rules = L.Rules(float(rewards[0]), float(rewards[1]), float(rewards[2]), self.max_episode_steps,
                                 fam.goal_compare, flags, self.n_actions, 0.0, C.c_uint64(seed & (2 ** 64 - 1)))
         self.reward_progress = 0.0
@@ -475,7 +477,11 @@ class GraphVecEnv:
         self._check_open()
         m = None
         if mask is not None:
+            if self._episodes is not None:
+                raise ValueError("reset(mask) cannot run while an episode list is installed (set_episodes)")
             m = torch.as_tensor(mask).to(device=self.device, dtype=torch.uint8)
+        if self._episodes is not None:
+            self._rearm_episodes()
         self._tick(self._c_out, 0)
         r = self._ref
         self._call(self.lib.vn_env_reset, r["store"], r["tables"], r["envs"], r["rules"],
@@ -596,6 +602,8 @@ class GraphVecEnv:
         if not (torch.is_tensor(actions) and actions.is_cuda and actions.dtype == torch.int32 and actions.dim() == 2):
             raise ValueError("capture_steps needs a CUDA int32 [T, N] action tensor")
         saved = self.state_dict()
+        if self._episodes is not None:      # the warm-up step may end listed episodes: their state is restored too
+            saved["_episodes"] = {k: v.clone() for k, v in self._episodes.items() if torch.is_tensor(v)}
         side = torch.cuda.Stream(self.device)
         side.wait_stream(torch.cuda.current_stream(self.device))
         with torch.cuda.stream(side):                 # warm-up outside the capture (lazy CUDA / torch initialisation)
@@ -616,11 +624,15 @@ class GraphVecEnv:
                 if after_step is not None:
                     after_step(t)
         self._restore(saved)
-        return CapturedSteps(self, graph)
+        cap = CapturedSteps(self, graph)
+        cap.episodes = self._episodes       # the buffers the captured steps write live as long as the graph
+        return cap
 
     def _restore(self, d):
         for k in ("state", "goal", "task", "elapsed", "epoch", "ep_return", "ep_length", "stats"):
             getattr(self, k).copy_(d[k].to(self.device))
+        for k, v in d.get("_episodes", {}).items():
+            self._episodes[k].copy_(v)
         self.gather_current()
         torch.cuda.synchronize(self.device)
 
@@ -770,6 +782,109 @@ class GraphVecEnv:
             self.dw.shortest_paths()
         self._c_rules.reward_progress = coef
         self.reward_progress = float(np.float32(coef))
+
+    # ------------------------------------------------------------------ fixed episode lists (evaluation)
+    def set_episodes(self, task, start=None):
+        """Installs a fixed list of evaluation episodes that the step runs and scores itself (vn_b200.h vn_episodes_t,
+        vn_envs_t.episodes); ``set_episodes(None)`` removes it.  ``task`` / ``start`` (numpy or tensors, ``[E]``) are the GLOBAL list of the
+        whole job: task indices into ``world.tasks`` (any task, whatever the env's ``env_tasks`` range) and global start
+        states.  Listed episode ``j`` belongs to the env with global id ``j % num_envs_total`` and each env runs its
+        episodes in increasing ``j``, so the results do not depend on ``num_envs`` per shard or on the number of shards.
+
+        Takes effect at the next ``reset()`` (which must be unmasked), and every later ``reset()`` starts the list
+        again from the top with zeroed results.  When a listed episode ends, the step writes its length, return (the
+        bits of ``info['episode']['r']``), win, truncation (``info['TimeLimit.truncated']`` is True) and final state
+        (``info['state']``) at index ``j`` of ``episode_results()`` and counts it in ``episodes_recorded``; the env
+        then starts its next listed episode or, past its list, goes back to its ordinary (Philox) resets and is never
+        scored again.  Needs ``auto_reset`` and no injected reset stream.  Checked here: indices in range, each start
+        in its task's scene and able to reach the goal (``DeviceWorld.shortest_paths()`` distance >= 1).
+        ``state_dict()`` does not carry the list or its results; a CUDA graph captured with ``capture_steps`` keeps the
+        list it was captured with (and its buffers alive)."""
+        if task is None:
+            self._episodes = None
+            self._c_envs.episodes = None
+            return
+        if start is None:
+            raise ValueError("set_episodes(task, start): start is missing")
+        if not self.auto_reset:
+            raise ValueError("an episode list needs auto_reset=True")
+        if self._c_inject is not None:
+            raise ValueError("an episode list cannot be combined with an injected reset stream (inject)")
+        task = np.asarray(task.cpu() if torch.is_tensor(task) else task).reshape(-1)
+        start = np.asarray(start.cpu() if torch.is_tensor(start) else start).reshape(-1)
+        if task.shape != start.shape:
+            raise ValueError("task and start must have the same length (%d != %d)" % (task.size, start.size))
+        if task.size >= 2 ** 31 or not (np.issubdtype(task.dtype, np.integer) or task.size == 0) or \
+                not (np.issubdtype(start.dtype, np.integer) or start.size == 0):
+            raise ValueError("task and start must be integer arrays of fewer than 2**31 episodes")
+        w = self.world
+        E = int(task.size)
+        task, start = task.astype(np.int64), start.astype(np.int64)
+        if E and (task.min() < 0 or task.max() >= len(w.tasks)):
+            raise ValueError("task indices must lie in [0, %d)" % len(w.tasks))
+        if E and (start.min() < 0 or start.max() >= w.n_states):
+            raise ValueError("start states must lie in [0, %d)" % w.n_states)
+        if E:
+            scene = np.array([t.scene for t in w.tasks], np.int64)[task]
+            bad = np.nonzero(w.scene_of_state(start) != scene)[0]
+            if bad.size:
+                raise ValueError("episode %d: start state %d is not in the scene of task %d"
+                                 % (bad[0], start[bad[0]], task[bad[0]]))
+            _, dist = self.dw.shortest_paths()
+            d = dist[torch.from_numpy(task).to(self.device), torch.from_numpy(start).to(self.device)].cpu().numpy()
+            bad = np.nonzero(d < 1)[0]
+            if bad.size:
+                raise ValueError("episode %d: start state %d cannot reach the goal of task %d (distance %d)"
+                                 % (bad[0], start[bad[0]], task[bad[0]], d[bad[0]]))
+        n, dev = self.num_envs, self.device
+        with torch.cuda.device(dev):
+            i32 = lambda fill: torch.full((max(E, 1),), fill, dtype=torch.int32, device=dev)
+            e = dict(task=torch.from_numpy(task.astype(np.int32)).to(dev) if E else i32(0),
+                     start=torch.from_numpy(start.astype(np.int32)).to(dev) if E else i32(0),
+                     cursor=torch.full((max(n, 1),), -1, dtype=torch.int32, device=dev),
+                     length=i32(-1), ret=torch.zeros(max(E, 1), dtype=torch.float32, device=dev),
+                     win=torch.zeros(max(E, 1), dtype=torch.uint8, device=dev),
+                     truncated=torch.zeros(max(E, 1), dtype=torch.uint8, device=dev), final_state=i32(-1),
+                     count=torch.zeros(1, dtype=torch.int32, device=dev))       # uint32 on the device side
+        ids = np.arange(E, dtype=np.int64) % self.num_envs_total
+        e["n"] = E
+        e["owned"] = np.nonzero((ids >= self.env_lo) & (ids < self.env_lo + n))[0]
+        e["c"] = L.Episodes(e["task"].data_ptr(), e["start"].data_ptr(), E, self.num_envs_total,
+                            *(e[k].data_ptr() for k in ("cursor", "length", "ret", "win", "truncated", "final_state",
+                                                        "count")))
+        self._episodes = e
+        self._c_envs.episodes = C.cast(C.pointer(e["c"]), C.c_void_p)
+
+    def _rearm_episodes(self):
+        """A reset starts the list from the top: results and counter back to 'nothing recorded'."""
+        e = self._episodes
+        e["length"].fill_(-1)
+        e["final_state"].fill_(-1)
+        for k in ("ret", "win", "truncated", "count"):
+            e[k].zero_()
+
+    @property
+    def episodes_owned(self):
+        """Ids of the listed episodes this shard runs (``j`` with ``j % num_envs_total`` one of its envs), ascending;
+        None without a list."""
+        return None if self._episodes is None else self._episodes["owned"]
+
+    @property
+    def episodes_recorded(self):
+        """Results the step has written since the last reset() (reads one device word: synchronises the stream)."""
+        if self._episodes is None:
+            return 0
+        return int(self._episodes["count"].item())
+
+    def episode_results(self):
+        """CUDA tensors ``[E]`` of the installed list, indexed by listed episode: ``task``, ``start``, ``length``
+        (int32, -1 = not recorded by this process: still running, or run by another shard), ``ret`` (float32),
+        ``win``, ``truncated`` (uint8), ``final_state`` (int32).  Views of the buffers the step writes."""
+        e = self._episodes
+        if e is None:
+            raise RuntimeError("no episode list is installed (set_episodes)")
+        E = e["n"]
+        return {k: e[k][:E] for k in ("task", "start", "length", "ret", "win", "truncated", "final_state")}
 
     # ------------------------------------------------------------------ extras
     def states(self):

@@ -138,6 +138,9 @@ typedef struct vn_envs {
     int32_t *ep_length;
     const int32_t *task_lo;  /* [n_envs] first task this env may draw (gym_graph/graph.py:47 goals list) */
     const int32_t *task_cnt; /* [n_envs] number of tasks it draws from */
+    /* Optional fixed episode list (evaluation): [host] descriptor read during each reset / step call, see vn_episodes_t
+     * below; NULL = off, and every output is what it is without the field. */
+    const struct vn_episodes *episodes;
 } vn_envs_t;
 
 typedef struct vn_rules {
@@ -223,6 +226,36 @@ typedef struct vn_step_out {
     int32_t reserved2;
 } vn_step_out_t;
 
+/* A fixed list of evaluation episodes that the step runs and scores itself (vn_envs_t.episodes).
+ *
+ * Deal: listed episode j belongs to the env whose GLOBAL id (env_id_base + i) is j mod stride, and each env runs its
+ * episodes in increasing j - g, g + stride, g + 2 * stride, ... with g its global id - so, as with the Philox stream,
+ * the results do not depend on how the envs are sharded.  An unmasked vn_env_reset starts env i on episode g when
+ * g < n_episodes (goal task_goal[task[g]], env.task = task[g], start state start[g]; the env's task_lo / task_cnt are
+ * ignored) and on its ordinary reset source otherwise.  When a listed episode ends (done: goal or TimeLimit), the step
+ * writes its result at index j and adds 1 to *count; the auto-reset of that step starts episode j + stride if it is
+ * listed, else the env returns to its ordinary source (Philox at its current epoch) with cursor -1 and writes no
+ * result again.  Envs past their list keep running ordinary episodes: every other output keeps its meaning.  epoch
+ * counts every reset, listed or not.
+ *
+ * Rejected with VN_EINVAL: a list together with vn_inject_t, without VN_RULE_AUTO_RESET, a masked vn_env_reset, null
+ * list / result pointers while n_episodes > 0, a null cursor or count, stride < env_id_base + n_envs.  task[] and
+ * start[] must hold valid global indices (not checked on the device). */
+typedef struct vn_episodes {
+    const int32_t *task;     /* [n_episodes] GLOBAL task index of each listed episode */
+    const int32_t *start;    /* [n_episodes] GLOBAL start state */
+    int32_t n_episodes;
+    int32_t stride;          /* total envs of the job (all shards) */
+    int32_t *cursor;         /* [n_envs] listed episode the env is running, -1 = none (written by the step) */
+    /* per-episode results [n_episodes], written once, by the step on which the episode ends */
+    int32_t *length;         /* info['episode']['l'] */
+    float *ret;              /* info['episode']['r'], same bits */
+    uint8_t *win;            /* info['win'] */
+    uint8_t *truncated;      /* 1 where info['TimeLimit.truncated'] is True */
+    int32_t *final_state;    /* info['state']: the state the last action led to */
+    uint32_t *count;         /* results written so far (device counter; the caller zeroes it) */
+} vn_episodes_t;
+
 /* gather kernel variants (all bit-identical; see DESIGN.md) */
 #define VN_GATHER_AUTO 0
 #define VN_GATHER_LDG 1      /* 16-byte vector loads/stores through registers */
@@ -242,7 +275,7 @@ typedef struct vn_step_out {
 
 int32_t vn_abi_version(void);
 /* sizeof of the descriptor structs as compiled into the library (0 store, 1 tables, 2 envs, 3 rules, 4 inject,
- * 5 step_out, 6 replay, 7 float_leaf, 8 host_call, 9 u8_frames; -1 otherwise): a binding checks its mirrors against these at load
+ * 5 step_out, 6 replay, 7 float_leaf, 8 host_call, 9 u8_frames, 10 episodes; -1 otherwise): a binding checks its mirrors against these at load
  * time. */
 int32_t vn_abi_struct_size(int32_t which);
 const char *vn_last_error(void);
